@@ -15,7 +15,10 @@
 //     dH_l MMAs, by the elected lanes of warps 1-3 (two or three K-steps each, so nobody issues for long) -- and the
 //     in-place store waits for it (by then the epilogue arithmetic has hidden most of its latency).
 //   * ALL groups accumulate their weight gradients into ONE set of TMEM columns (zeroed once with tcgen05.st; every
-//     MMA accumulates): 7 x 32 result columns + 80 gradient columns = 304 of the SM's 512, one partial per SM.
+//     MMA accumulates): 7 x (32 result + 24 A-operand) columns + 80 gradient columns = 472 of the SM's 512, one partial per SM.
+//   * shared memory is read by the tensor core only where an operand must be MN-major (the weight gradients) and for the
+//     weights: every forward and dH MMA takes its A operand from TMEM, where the epilogue that writes A_l / dZ_l puts a
+//     second copy with tcgen05.st (A_0 included, K0P / 2 columns).
 //   * features mode: the fp32 tile is brought by one bulk-async copy into the slot's A_1.. region, which is dead between
 //     the previous tile's last weight-gradient MMA and this tile's first epilogue -- no staging buffer.
 // Forward-only launches (render) keep fused_v1_kernel: nothing is kept for a gradient there and nine 16 KB tiles
@@ -30,8 +33,7 @@ struct MgLayout {
     using LY = TcLayout<HP>;
     static constexpr int HSL = HP / 8;
     __host__ __device__ static int a0s(int c_in) { return (c_in + 8) >> 3; }   // slabs holding features 0..c_in (ones column included)
-    // slot: A_0 [a0s] | dZ_{L-1} [1] | A_1 [HSL] .. A_{L-1} [HSL].  A K-padding read past A_0 lands in the dZ slab and one past
-    // the dZ slab in A_1: bf16 values a previous stage wrote (finite), never raw fp32 staging bytes.
+    // slot: A_0 [a0s] | dZ_{L-1} [1] | A_1 [HSL] .. A_{L-1} [HSL]
     __host__ __device__ static int dzl_off(int A0S) { return A0S * SLAB; }
     __host__ __device__ static int a_off(int l, int A0S) { return l == 0 ? 0 : (A0S + 1 + (l - 1) * HSL) * SLAB; }
     __host__ __device__ static int slot_bytes(int L, int c_in, int K0P, bool rays)
@@ -45,8 +47,10 @@ struct MgLayout {
         return nat;
     }
     __host__ __device__ static int ndw(int L) { return (L - 1) * HP + 16; }
-    // per group HP result columns + HP/2 columns of bf16 A operand (the forward / dH MMAs of layers >= 1 take A from TMEM)
-    __host__ __device__ static int tmem_need(int L, int ng) { return ng * (HP + HP / 2) + ndw(L); }
+    // per group HP result columns + the bf16 A operand of the forward / dH MMAs, whose widest is A_0 (K0P / 2 columns) or a
+    // hidden layer (HP / 2)
+    __host__ __device__ static int acols(int K0P) { return (K0P > HP ? K0P : HP) / 2; }
+    __host__ __device__ static int tmem_need(int L, int K0P, int ng) { return ng * (HP + acols(K0P)) + ndw(L); }
     __host__ __device__ static size_t total(int L, int c_in, int K0P, bool rays, int ng)
     {
         const int A0S = a0s(c_in);
@@ -73,7 +77,10 @@ __device__ __forceinline__ void bulk_prefetch_l2(const void *src, uint32_t bytes
     asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src), "r"(bytes) : "memory");
 }
 __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-
+__device__ __forceinline__ void tmem_st4(uint32_t taddr, uint4 v)   // one 8-feature slab of a row: 4 columns
+{
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1,%2,%3,%4};" ::"r"(taddr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
+}
 template <int HP> constexpr int mg_max_groups() { return HP <= 32 ? MG_MAX_GROUPS : 4; }   // registers: 64 K / (groups x 128 threads)
 
 template <bool RAYS, int HP>
@@ -132,10 +139,8 @@ __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel
         return reinterpret_cast<const void *>(a16);
     };
 
-    // ---- one-time setup.  Every buffer is fully rewritten each tile before an MMA reads it as data; the one K-padding read
-    // that can come first is the layer-0 MMA's look into the dZ_{L-1} slab behind A_0 (zero weights, but the values must be
-    // finite): zero that slab.  (Zeroing the whole 200 KB cost 0.8 us of every launch.)
-    *reinterpret_cast<uint4 *>(slot + MG::dzl_off(A0S) + tid * 16) = make_uint4(0, 0, 0, 0);
+    // ---- one-time setup.  Every buffer is fully rewritten each tile before an MMA reads it as data (the K padding of A_0
+    // included, in TMEM); what an M = 64 weight-gradient MMA reads past a short A_l only reaches accumulator rows never read.
     if (tid == 0) {
         mbar_init(bar_mma, 1);
         mbar_init(bar_x, 1);
@@ -158,13 +163,12 @@ __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel
     // the MMA program: one record per stage, one THREAD per record (a single thread building all of them cost 3 us)
     if (tid >= 32 && tid < 32 + 3 * L) {
         const int r = tid - 32, kind = r / L, l = r % L;
-        const uint32_t dcol = (uint32_t)(g * HP), acol = (uint32_t)(NG * HP + MG::ndw(L) + g * (HP / 2));
+        const uint32_t dcol = (uint32_t)(g * HP), acol = (uint32_t)(NG * HP + MG::ndw(L) + g * MG::acols(K0P));
         const int Np = LY::np(l, L), Kp = LY::kp(l, K0P);
         const uint32_t wl = smem_u32(Wbase + LY::w_off(l, L, K0P));
-        if (kind == 0) {               // D[128 x Np] = A_l[128 x Kp] * W_l   (A, B K-major)
-            prog[l] = StageRec{smem_desc(smem_u32(a_buf(l)), SLAB, 128), smem_desc(wl, Np * 16, 128), (uint32_t)(2 * SLAB) >> 4, (uint32_t)(2 * Np * 16) >> 4,
-                               instr_desc(128, Np, 0, 0), dcol, (uint32_t)(Kp / 16), 0u, 0u, 0u};
-            if (l > 0) { prog[l].a = (uint64_t)acol; prog[l].inc_a = 8u; prog[l].pad0 = 1u; }    // A from TMEM, 8 columns per K-step
+        if (kind == 0) {               // D[128 x Np] = A_l[128 x Kp] * W_l: A from TMEM (8 columns per K-step), B K-major
+            prog[l] = StageRec{(uint64_t)acol, smem_desc(wl, Np * 16, 128), 8u, (uint32_t)(2 * Np * 16) >> 4,
+                               instr_desc(128, Np, 0, 0), dcol, (uint32_t)(Kp / 16), 0u, 1u, 0u};
         } else if (kind == 1) {        // dH_l[128 x Kp] = dZ_l[128 x Np] * W_l^T (same W bytes, MN-major); unused for l = 0
             prog[L + l] = StageRec{(uint64_t)acol, smem_desc(wl, 128, Np * 16), 8u, 256u >> 4,
                                    instr_desc(128, Kp, 0, 1), dcol, (uint32_t)(Np / 16), 0u, 1u, 0u};       // A = dZ_l from TMEM
@@ -173,7 +177,7 @@ __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel
                                        instr_desc(64, Np, 1, 1), (uint32_t)(NG * HP + l * HP), (uint32_t)(TILE / 16), 1u, 0u, 0u};
         }
     }
-    const int tmem_need = MG::tmem_need(L, NG);
+    const int tmem_need = MG::tmem_need(L, K0P, NG);
     const uint32_t tmem_cols = tmem_need <= 32 ? 32u : (tmem_need <= 64 ? 64u : (tmem_need <= 128 ? 128u : (tmem_need <= 256 ? 256u : 512u)));
     if (g == 0 && warp == 0) tmem_alloc(smem_u32(tmem_slot), tmem_cols);
     fence_async_smem();
@@ -229,7 +233,7 @@ __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel
             alo += r1.x; blo += r1.y; acc = 1u;
         }
     };
-    const uint32_t a_tm = tmem + lane_base + (uint32_t)(NG * HP + MG::ndw(L) + g * (HP / 2));   // this row's bf16 A operand
+    const uint32_t a_tm = tmem + lane_base + (uint32_t)(NG * HP + MG::ndw(L) + g * MG::acols(K0P));   // this row's bf16 A operand
     auto commit_and_wait = [&]() {
         if (tid == 0) umma_commit(bar_mma);
         mbar_wait_mg(bar_mma, phase);
@@ -238,6 +242,14 @@ __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel
     };
     auto publish_smem = [&]() { // generic-proxy smem writes -> visible to the tensor core, all threads of the group
         fence_async_smem();
+        tc_fence_before();
+        bar_group(g);
+        tc_fence_after();
+    };
+    // the same for tcgen05.st -> MMA only.  The forward's shared-memory stores (A_0 .. A_{L-1}) are read by the tensor core
+    // only through the weight-gradient MMAs, which are issued after the backward's first publish_smem: its proxy fence
+    // covers them, so the forward needs none of its own.
+    auto publish_tmem = [&]() {
         tc_fence_before();
         bar_group(g);
         tc_fence_after();
@@ -335,7 +347,7 @@ __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel
             for (int c = 0; c < 3; ++c) pe_sincos(x[c], &sn[c], &cs[c]);
             // feature f = 3 * slot + coord as bf16 pairs (pair j = features 2j, 2j+1); band i fills pairs 1+3i .. 3+3i and leaves
             // its last cosine pending; the ones column (feature 3 + 6E, odd) closes the pending pair.  Four pairs make this row's
-            // 16 bytes of a slab, stored as soon as they are complete.
+            // 16 bytes of a slab, stored to shared memory and TMEM as soon as they are complete.
             {
                 uint8_t *const a0 = a_buf(0);
                 uint32_t q4[4] = {pack_bf16(x[0], x[1]), 0u, 0u, 0u};
@@ -343,7 +355,14 @@ __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel
                 bool closed = false;
                 auto put = [&](int j, uint32_t v) {            // j is a compile-time constant at every call site
                     q4[j & 3] = v;
-                    if ((j & 3) == 3) { if ((j >> 2) < A0S) *row_ptr(a0, j >> 2) = make_uint4(q4[0], q4[1], q4[2], q4[3]); q4[0] = q4[1] = q4[2] = q4[3] = 0u; }
+                    if ((j & 3) == 3) {
+                        if ((j >> 2) < A0S) {
+                            const uint4 q = make_uint4(q4[0], q4[1], q4[2], q4[3]);
+                            *row_ptr(a0, j >> 2) = q;
+                            tmem_st4(a_tm + (uint32_t)(j >> 2) * 4u, q);
+                        }
+                        q4[0] = q4[1] = q4[2] = q4[3] = 0u;
+                    }
                 };
                 // warp-uniform branches: the bands that are off cost nothing
 #pragma unroll
@@ -378,30 +397,40 @@ __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel
             xphase ^= 1;
             uint8_t *a0 = a_buf(0);
             const float *xr = stage + lead + tid * c_in;
-            if (tid < valid) {
-                for (int c8 = 0; c8 < A0S - 1; ++c8) {     // (A0S - 1) * 8 <= c_in: every column of these slabs is a feature
+            const bool row_live = tid < valid;
+            // (tcgen05.st is warp-wide: the rows past `valid` store zeros in the same instruction)
+            auto put = [&](int c8, uint4 q) { *row_ptr(a0, c8) = q; tmem_st4(a_tm + (uint32_t)c8 * 4u, q); };
+            for (int c8 = 0; c8 < A0S - 1; ++c8) {         // (A0S - 1) * 8 <= c_in: every column of these slabs is a feature
+                uint4 q = make_uint4(0, 0, 0, 0);
+                if (row_live) {
                     float f[8];
 #pragma unroll
                     for (int j = 0; j < 8; ++j) f[j] = xr[c8 * 8 + j];
-                    *row_ptr(a0, c8) = make_uint4(pack_bf16(f[0], f[1]), pack_bf16(f[2], f[3]), pack_bf16(f[4], f[5]), pack_bf16(f[6], f[7]));
+                    q = make_uint4(pack_bf16(f[0], f[1]), pack_bf16(f[2], f[3]), pack_bf16(f[4], f[5]), pack_bf16(f[6], f[7]));
                 }
-                {
-                    const int c8 = A0S - 1;
+                put(c8, q);
+            }
+            {
+                const int c8 = A0S - 1;
+                uint4 q = make_uint4(0, 0, 0, 0);
+                if (row_live) {
                     float f[8];
 #pragma unroll
                     for (int j = 0; j < 8; ++j) { const int c = c8 * 8 + j; f[j] = c < c_in ? xr[c] : (c == c_in ? 1.0f : 0.0f); }
-                    *row_ptr(a0, c8) = make_uint4(pack_bf16(f[0], f[1]), pack_bf16(f[2], f[3]), pack_bf16(f[4], f[5]), pack_bf16(f[6], f[7]));
+                    q = make_uint4(pack_bf16(f[0], f[1]), pack_bf16(f[2], f[3]), pack_bf16(f[4], f[5]), pack_bf16(f[6], f[7]));
                 }
-            } else {
-                for (int c8 = 0; c8 < A0S; ++c8) *row_ptr(a0, c8) = make_uint4(0, 0, 0, 0);
+                put(c8, q);
             }
         }
+        // A_0's K padding in TMEM: explicit zeros (they meet zero weight rows, but stale TMEM bits could be NaN)
+        for (int c8 = A0S; c8 < K0P / 8; ++c8) tmem_st4(a_tm + (uint32_t)c8 * 4u, make_uint4(0, 0, 0, 0));
+        tmem_st_wait();
         if (!have_weights) {
             mbar_wait(bar_w, 0);             // weights + biases have landed (and the previous kernel has completed)
             have_weights = true;
             MG_STAMP(2);
         }
-        publish_smem(); // also: every thread is done reading `stage` (the first epilogue overwrites it)
+        publish_tmem(); // also: every thread is done reading `stage` (the first epilogue overwrites it)
         // ---- forward
         float hz[4];
         for (int l = 0; l < L; ++l) {
@@ -426,7 +455,7 @@ __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel
                     tmem_st8(a_tm + (uint32_t)(c16 * 8), o);                          // for the next layer's MMA (A from TMEM)
                 }
                 tmem_st_wait_();
-                publish_smem();
+                publish_tmem();
             } else {
                 uint32_t v[16];
                 tmem_ld16(tmem + lane_base + (uint32_t)(g * HP), v);

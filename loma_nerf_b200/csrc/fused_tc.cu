@@ -1307,7 +1307,7 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
     do {                                                                                                         \
         mg_fn = rays ? (const void *)fused_mg_kernel<true, HPV> : (const void *)fused_mg_kernel<false, HPV>;     \
         ng = mg_max_groups<HPV>();                                                                               \
-        while (ng > 1 && (MgLayout<HPV>::total(L, c_in, K0P, rays, ng) > 232448 || MgLayout<HPV>::tmem_need(L, ng) > 512)) --ng; \
+        while (ng > 1 && (MgLayout<HPV>::total(L, c_in, K0P, rays, ng) > 232448 || MgLayout<HPV>::tmem_need(L, K0P, ng) > 512)) --ng; \
     } while (0)
         if (HP == 16) LNB_MG_PICK(16);
         else if (HP == 32) LNB_MG_PICK(32);
