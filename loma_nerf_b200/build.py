@@ -19,7 +19,7 @@ INCLUDE = os.path.join(os.path.dirname(HERE), "include")
 
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
-CFLAGS = (["-DLNB_TC_CLK"] if os.environ.get("LNB_TC_CLK") else []) + (["-DLNB_WIDE_CLK"] if os.environ.get("LNB_WIDE_CLK") else []) + (["-DLNB_TC_ISSUE_TWICE"] if os.environ.get("LNB_TC_ISSUE_TWICE") else []) + ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC,-fvisibility=hidden",
+CFLAGS = (["-DLNB_TC_CLK"] if os.environ.get("LNB_TC_CLK") else []) + (["-DLNB_WIDE_CLK"] if os.environ.get("LNB_WIDE_CLK") else []) + ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC,-fvisibility=hidden",
           "--expt-relaxed-constexpr", "-I", INCLUDE]
 
 

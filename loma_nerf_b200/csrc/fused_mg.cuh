@@ -1,5 +1,5 @@
 // fused_mg.cuh -- the fused tensor-core TRAIN step, multi-group form.  Included by fused_tc.cu inside its anonymous
-// namespace (PTX wrappers, TcParams, TcLayout, SLAB / TILE / MAXL come from there).
+// namespace (PTX wrappers, TcParams, TcLayout, the per-tile stages, SLAB / TILE / MAXL come from there).
 //
 // Why: a 128-sample tile takes ~10 000 cycles from features to weight gradients even alone on an SM (six dependent
 // tcgen05 stages at ~555 + 145 g cycles each, three scans, five epilogues), a 4096 x 64 batch is only 13.8 tiles per
@@ -63,11 +63,6 @@ struct MgLayout {
     }
 };
 
-// mbarrier wait of the group threads.  With seven groups on an SM a hardware-suspended try_wait is woken by the other groups'
-// barrier traffic and re-polls several times per wait; mbar_wait_tight (fused_tc.cu) keeps an iteration at the try_wait and one
-// branch (an explicit __nanosleep between polls, tried before, does not actually sleep here and costs five instructions).
-__device__ __forceinline__ void mbar_wait_mg(uint32_t bar, uint32_t parity) { mbar_wait_tight(bar, parity); }
-__device__ __forceinline__ void bar_group(int g) { asm volatile("bar.sync %0, %1;" ::"r"(g + 1), "r"(TILE) : "memory"); }
 __device__ __forceinline__ void tmem_st16_zero(uint32_t taddr)
 {
     asm volatile("tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%1,%1,%1,%1,%1,%1,%1,%1,%1,%1,%1,%1,%1,%1,%1};" ::"r"(taddr), "r"(0u) : "memory");
@@ -76,7 +71,6 @@ __device__ __forceinline__ void bulk_prefetch_l2(const void *src, uint32_t bytes
 {
     asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src), "r"(bytes) : "memory");
 }
-__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 __device__ __forceinline__ void tmem_st4(uint32_t taddr, uint4 v)   // one 8-feature slab of a row: 4 columns
 {
     asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1,%2,%3,%4};" ::"r"(taddr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
@@ -119,25 +113,13 @@ __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel
     const uint32_t bar_mma = smem_u32(bar_p), bar_x = smem_u32(bar_p + 1), bar_dw = smem_u32(bar_p + 2);
     const uint32_t bar_w = smem_u32(globals);
     uint32_t *const tmem_slot = reinterpret_cast<uint32_t *>(globals + 8);
-    struct StageRec { uint64_t a, b; uint32_t inc_a, inc_b, idesc, dcol; uint32_t count, first_acc, pad0, pad1; };
+    const CompScratch scratch{color_s, tgt_s, tailp, tail_s, headq, headA, headB};
     StageRec *const prog = reinterpret_cast<StageRec *>(misc + 1728);   // fwd l | dH l (L + l) | dW l (2L + l)
 
     auto a_buf = [&](int l) { return slot + MG::a_off(l, A0S); };
     uint8_t *const dzl_buf = slot + MG::dzl_off(A0S);
     // where the adjoint dZ_l lives: the last layer's in its own slab, the others in place of A_{l+1}
     auto dz_buf = [&](int l) { return l == L - 1 ? dzl_buf : a_buf(l + 1); };
-
-    // TMA source of a tile's features (16 B aligned start, `lead` floats in front of the tile)
-    auto x_src = [&](int tile, int &lead, uint32_t &bytes) -> const void * {
-        const long long row0 = (long long)tile * p.rows_per_tile;
-        long long rem = p.N - row0;
-        const int valid = rem < p.rows_per_tile ? (int)rem : p.rows_per_tile;
-        const uintptr_t a = reinterpret_cast<uintptr_t>(p.X + row0 * c_in);
-        const uintptr_t a16 = a & ~(uintptr_t)15;
-        lead = (int)((a - a16) >> 2);
-        bytes = (uint32_t)(((a - a16) + (uintptr_t)valid * c_in * 4 + 15) & ~(uintptr_t)15);
-        return reinterpret_cast<const void *>(a16);
-    };
 
     // ---- one-time setup.  Every buffer is fully rewritten each tile before an MMA reads it as data (the K padding of A_0
     // included, in TMEM); what an M = 64 weight-gradient MMA reads past a short A_l only reaches accumulator rows never read.
@@ -154,7 +136,7 @@ __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel
             const int t0 = g * (int)gridDim.x + (int)blockIdx.x;
             if (t0 < p.n_tiles) {
                 int lead; uint32_t bytes;
-                const void *src = x_src(t0, lead, bytes);
+                const void *src = x_src(p, t0, c_in, lead, bytes);
                 mbar_expect_tx(bar_x, bytes);
                 bulk_g2s(smem_u32(stage), src, bytes, bar_x);
             }
@@ -168,17 +150,16 @@ __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel
         const uint32_t wl = smem_u32(Wbase + LY::w_off(l, L, K0P));
         if (kind == 0) {               // D[128 x Np] = A_l[128 x Kp] * W_l: A from TMEM (8 columns per K-step), B K-major
             prog[l] = StageRec{(uint64_t)acol, smem_desc(wl, Np * 16, 128), 8u, (uint32_t)(2 * Np * 16) >> 4,
-                               instr_desc(128, Np, 0, 0), dcol, (uint32_t)(Kp / 16), 0u, 1u, 0u};
+                               instr_desc(128, Np, 0, 0), dcol, (uint32_t)(Kp / 16), 1u, 0u, 0u};
         } else if (kind == 1) {        // dH_l[128 x Kp] = dZ_l[128 x Np] * W_l^T (same W bytes, MN-major); unused for l = 0
             prog[L + l] = StageRec{(uint64_t)acol, smem_desc(wl, 128, Np * 16), 8u, 256u >> 4,
-                                   instr_desc(128, Kp, 0, 1), dcol, (uint32_t)(Np / 16), 0u, 1u, 0u};       // A = dZ_l from TMEM
+                                   instr_desc(128, Kp, 0, 1), dcol, (uint32_t)(Np / 16), 1u, 0u, 0u};       // A = dZ_l from TMEM
         } else {                       // dW_l[features x Np] += A_l^T dZ_l, K = the tile's 128 samples, both MN-major
             prog[2 * L + l] = StageRec{smem_desc(smem_u32(a_buf(l)), 128, SLAB), smem_desc(smem_u32(dz_buf(l)), 128, SLAB), 256u >> 4, 256u >> 4,
-                                       instr_desc(64, Np, 1, 1), (uint32_t)(NG * HP + l * HP), (uint32_t)(TILE / 16), 1u, 0u, 0u};
+                                       instr_desc(64, Np, 1, 1), (uint32_t)(NG * HP + l * HP), (uint32_t)(TILE / 16), 0u, 0u, 0u};
         }
     }
-    const int tmem_need = MG::tmem_need(L, K0P, NG);
-    const uint32_t tmem_cols = tmem_need <= 32 ? 32u : (tmem_need <= 64 ? 64u : (tmem_need <= 128 ? 128u : (tmem_need <= 256 ? 256u : 512u)));
+    const uint32_t tmem_cols = tmem_alloc_cols(MG::tmem_need(L, K0P, NG));
     if (g == 0 && warp == 0) tmem_alloc(smem_u32(tmem_slot), tmem_cols);
     fence_async_smem();
     tc_fence_before();
@@ -199,51 +180,29 @@ __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel
     // ONE thread waits for it and issues the bulk copy of the image; the others go straight to their first tile's features
     // and meet the image at its mbarrier (which also orders their later global writes behind that kernel).  No-op without PDL.
     if (threadIdx.x == 64) {
-        asm volatile("griddepcontrol.wait;" ::: "memory");
+        pdl_wait();
         const uint32_t wb = (uint32_t)LY::wimg_bytes(L, K0P);
         mbar_expect_tx(bar_w, wb);
         bulk_g2s(smem_u32(Wbase), p.wimg, wb, bar_w);
     }
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+    pdl_trigger();
     uint32_t phase = 0, xphase = 0, dwphase = 0;
     float loss_acc = 0.0f;
     bool dw_pending = false, have_weights = false;
     MG_STAMP(1);
 
     auto row_ptr = [&](uint8_t *buf, int slab) { return reinterpret_cast<uint4 *>(buf + slab * SLAB + tid * 16); };
-    // issue K-steps [k0, k1) of one stage of the MMA program (one thread)
-    auto issue_steps = [&](int stage_id, uint32_t k0, uint32_t k1) {
-        const uint4 r0 = *reinterpret_cast<const uint4 *>(prog + stage_id);
-        const uint4 r1 = *(reinterpret_cast<const uint4 *>(prog + stage_id) + 1);
-        const uint4 r2 = *(reinterpret_cast<const uint4 *>(prog + stage_id) + 2);
-        if (k1 > r2.x) k1 = r2.x;
-        uint32_t alo = r0.x + k0 * r1.x, blo = r0.z + k0 * r1.y;
-        const uint32_t ahi = r0.y, bhi = r0.w;
-        uint32_t acc = (k0 > 0) ? 1u : r2.y;
-        const uint32_t d = tmem + r1.w;
-        if (r2.z) {                        // A operand in tensor memory
-            for (uint32_t k = k0; k < k1; ++k) {
-                umma_bf16_ts(d, tmem + alo, ((uint64_t)bhi << 32) | blo, r1.z, acc);
-                alo += r1.x; blo += r1.y; acc = 1u;
-            }
-            return;
-        }
-        for (uint32_t k = k0; k < k1; ++k) {
-            umma_bf16(d, ((uint64_t)ahi << 32) | alo, ((uint64_t)bhi << 32) | blo, r1.z, acc);
-            alo += r1.x; blo += r1.y; acc = 1u;
-        }
-    };
     const uint32_t a_tm = tmem + lane_base + (uint32_t)(NG * HP + MG::ndw(L) + g * MG::acols(K0P));   // this row's bf16 A operand
     auto commit_and_wait = [&]() {
         if (tid == 0) umma_commit(bar_mma);
-        mbar_wait_mg(bar_mma, phase);
+        mbar_wait_tight(bar_mma, phase);
         phase ^= 1;
         tc_fence_after();
     };
     auto publish_smem = [&]() { // generic-proxy smem writes -> visible to the tensor core, all threads of the group
         fence_async_smem();
         tc_fence_before();
-        bar_group(g);
+        bar_tile(g + 1);
         tc_fence_after();
     };
     // the same for tcgen05.st -> MMA only.  The forward's shared-memory stores (A_0 .. A_{L-1}) are read by the tensor core
@@ -251,18 +210,19 @@ __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel
     // covers them, so the forward needs none of its own.
     auto publish_tmem = [&]() {
         tc_fence_before();
-        bar_group(g);
+        bar_tile(g + 1);
         tc_fence_after();
     };
-    // the weight-gradient MMAs of layer l: 8 K-steps of 16 samples, dealt 3 / 3 / 2 to the elected lanes of warps 1-3
+    // the weight-gradient MMAs of layer l: 8 K-steps of 16 samples, dealt 3 / 3 / 2 to the elected lanes of warps 1-3; every
+    // one accumulates into the shared accumulator
     auto issue_dw = [&](int l) {
         if (lane == 0 && warp > 0) {
             const uint32_t k0 = warp == 1 ? 0u : (warp == 2 ? 3u : 6u), k1 = warp == 1 ? 3u : (warp == 2 ? 6u : 8u);
-            issue_steps(2 * L + l, k0, k1);
+            issue_steps<true>(prog + 2 * L + l, tmem, k0, k1, 1u);
             umma_commit(bar_dw);
         }
     };
-    auto wait_dw = [&]() { mbar_wait_mg(bar_dw, dwphase); dwphase ^= 1; tc_fence_after(); };
+    auto wait_dw = [&]() { mbar_wait_tight(bar_dw, dwphase); dwphase ^= 1; tc_fence_after(); };
 
     // tiles are dealt statically (tile -> group fixed): with equal tile costs nothing is gained by claiming them, and
     // nothing here then depends on the previous kernel in the stream except the weight image
@@ -278,149 +238,31 @@ __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel
         if (!RAYS && tid == 0) {
             int lead; uint32_t bytes;
             if (have_weights) {                    // (the first tile's copy was issued in the prologue)
-                const void *src = x_src(tile, lead, bytes);
+                const void *src = x_src(p, tile, c_in, lead, bytes);
                 mbar_expect_tx(bar_x, bytes);
                 bulk_g2s(smem_u32(stage), src, bytes, bar_x);
             }
             const int nxt = tile + (int)gridDim.x * NG;
-            if (nxt < p.n_tiles) { const void *src = x_src(nxt, lead, bytes); bulk_prefetch_l2(src, bytes); }
+            if (nxt < p.n_tiles) { const void *src = x_src(p, nxt, c_in, lead, bytes); bulk_prefetch_l2(src, bytes); }
         }
-        // early, latency-tolerant loads for this tile (consumed after the MLP forward)
-        float my_dist = 0.0f, tg0 = 0.0f, tg1 = 0.0f, tg2 = 0.0f;
-        if (p.head == LNB_HEAD_NERF && live) {
-            if (!RAYS) my_dist = __ldg(p.dists + row0 + tid);
-            if (p.target && smp == 0) {
-                const float *tg = p.target + (size_t)(tile * p.G + ray_l) * 3   /* ray = row0 / S + ray_l: a tile holds G whole rays; R is an int */;
-                tg0 = __ldg(tg); tg1 = __ldg(tg + 1); tg2 = __ldg(tg + 2);
-            }
-        }
+        float x[3], my_dist, tg[3];
+        sample_inputs<RAYS>(p, row0, tile * p.G, tid, smp, ray_l, live, x, my_dist, tg);
+        // A_0 goes to shared memory (for the weight gradient, MN-major) and to TMEM (the layer-0 MMA's A operand)
+        auto store_a0 = [&](int c8, uint4 q) { *row_ptr(a_buf(0), c8) = q; tmem_st4(a_tm + (uint32_t)c8 * 4u, q); };
         if (RAYS) {
-            // ---- features from rays: pts = o + d t (train_nerf.py:289-299), PE (pos_encoding.py:38-70),
-            // dist = t[s+1] - t[s], last 1e8 (train_nerf.py:306-311); written straight into A_0
-            float x[3] = {0.f, 0.f, 0.f};
-            if (live && p.cam_mode) {
-                // ray of pixel q and depth of sample smp straight from the pose (get_rays, train_nerf.py:23-62; linspace /
-                // stratified depths, train_nerf.py:289-311): no per-ray or per-sample input at all
-                const CamF32 &c = p.cam;
-                const long long ray = tile * p.G + ray_l;
-                const long long q = c.pixels ? (long long)__ldg(c.pixels + ray) : c.first_pixel + ray;
-                // q / width by the 64-bit reciprocal the launcher computed (exact for every 32-bit q)
-                const unsigned uq = (unsigned)q, row = c.width == 1 ? uq : (unsigned)__umul64hi((unsigned long long)uq, c.w_magic), col = uq - row * (unsigned)c.width;
-                const float fi = col == (unsigned)c.width - 1 ? 1.0f : (float)col * c.step, fj = row == (unsigned)c.width - 1 ? 1.0f : (float)row * c.step;
-                const float dx = (fi - c.cx) * c.inv_fx, dy = (c.cy - fj) * c.inv_fy;
-                float tt, tn;
-                if (c.stratified) {
-                    tt = fmaf((float)smp + (float)lnb_uniform_bits(c.seed, q, smp) * (1.0f / 16777216.0f), c.dt_str, c.near);
-                    tn = fmaf((float)(smp + 1) + (float)lnb_uniform_bits(c.seed, q, smp + 1) * (1.0f / 16777216.0f), c.dt_str, c.near);
-                } else {
-                    tt = smp == S - 1 && S > 1 ? c.far : fmaf((float)smp, c.dt_lin, c.near);
-                    tn = smp + 1 == S - 1 ? c.far : fmaf((float)(smp + 1), c.dt_lin, c.near);
-                }
-                my_dist = smp + 1 < S ? tn - tt : 1e8f;
-#pragma unroll
-                for (int k = 0; k < 3; ++k) {
-                    const float dk = fmaf(dx, c.c2w[4 * k], fmaf(dy, c.c2w[4 * k + 1], 0.0f - c.c2w[4 * k + 2]));
-                    x[k] = fmaf(dk, tt, c.c2w[4 * k + 3]);
-                }
-            } else if (live) {
-                const long long ray = tile * p.G + ray_l, smpl = row0 + tid;
-                if (p.ray_f64) {
-                    const double *o = reinterpret_cast<const double *>(p.rays_o) + ray * 3;
-                    const double *d = reinterpret_cast<const double *>(p.rays_d) + ray * 3;
-                    const double *tv = reinterpret_cast<const double *>(p.tvals) + smpl;
-                    const double tt = __ldg(tv);
-                    my_dist = smp + 1 < S ? (float)(__ldg(tv + 1) - tt) : 1e8f;
-#pragma unroll
-                    for (int c = 0; c < 3; ++c) x[c] = (float)(__ldg(o + c) + __ldg(d + c) * tt);
-                } else {
-                    const float *o = reinterpret_cast<const float *>(p.rays_o) + ray * 3;
-                    const float *d = reinterpret_cast<const float *>(p.rays_d) + ray * 3;
-                    const float *tv = reinterpret_cast<const float *>(p.tvals) + smpl;
-                    const float tt = __ldg(tv);
-                    my_dist = smp + 1 < S ? __ldg(tv + 1) - tt : 1e8f;
-#pragma unroll
-                    for (int c = 0; c < 3; ++c) x[c] = fmaf(__ldg(d + c), tt, __ldg(o + c));
-                }
-            }
+            // ---- features from rays: the positional encoding, written straight into A_0
             float sn[3], cs[3];
 #pragma unroll
             for (int c = 0; c < 3; ++c) pe_sincos(x[c], &sn[c], &cs[c]);
-            // feature f = 3 * slot + coord as bf16 pairs (pair j = features 2j, 2j+1); band i fills pairs 1+3i .. 3+3i and leaves
-            // its last cosine pending; the ones column (feature 3 + 6E, odd) closes the pending pair.  Four pairs make this row's
-            // 16 bytes of a slab, stored to shared memory and TMEM as soon as they are complete.
-            {
-                uint8_t *const a0 = a_buf(0);
-                uint32_t q4[4] = {pack_bf16(x[0], x[1]), 0u, 0u, 0u};
-                float pend = x[2];
-                bool closed = false;
-                auto put = [&](int j, uint32_t v) {            // j is a compile-time constant at every call site
-                    q4[j & 3] = v;
-                    if ((j & 3) == 3) {
-                        if ((j >> 2) < A0S) {
-                            const uint4 q = make_uint4(q4[0], q4[1], q4[2], q4[3]);
-                            *row_ptr(a0, j >> 2) = q;
-                            tmem_st4(a_tm + (uint32_t)(j >> 2) * 4u, q);
-                        }
-                        q4[0] = q4[1] = q4[2] = q4[3] = 0u;
-                    }
-                };
-                // warp-uniform branches: the bands that are off cost nothing
-#pragma unroll
-                for (int i = 0; i < 10; ++i) {
-                    if (i < p.pe_bands) {
-                        put(1 + 3 * i, pack_bf16(pend, sn[0]));
-                        put(2 + 3 * i, pack_bf16(sn[1], sn[2]));
-                        put(3 + 3 * i, pack_bf16(cs[0], cs[1]));
-                        pend = cs[2];
-#pragma unroll
-                        for (int c = 0; c < 3; ++c) {
-                            const float s2 = 2.0f * sn[c] * cs[c], c2 = fmaf(-2.0f * sn[c], sn[c], 1.0f);
-                            sn[c] = s2; cs[c] = c2;
-                        }
-                    } else {
-                        if (closed && ((1 + 3 * i) >> 2) >= A0S) break;   // no live slab left to store (slab 7 then is not live either)
-                        put(1 + 3 * i, closed ? 0u : pack_bf16(pend, 1.0f));
-                        put(2 + 3 * i, 0u);
-                        put(3 + 3 * i, 0u);
-                        closed = true;
-                    }
-                }
-                put(31, closed ? 0u : pack_bf16(pend, 1.0f));
-            }
+            pack_pe(x, sn, cs, p.pe_bands, A0S, store_a0);
         } else {
-            // ---- features: wait for the TMA, convert this thread's row to bf16 slabs.  Columns beyond c_in read the
-            // following floats of `stage` (finite: next row / zeroed or stale bf16 bytes seen as tiny floats... they meet
-            // zero weight rows only if finite) -- so only columns < 8 * A0S are converted, and column c_in is patched to 1.
+            // ---- features: wait for the TMA, convert this thread's row to bf16 slabs (tcgen05.st is warp-wide: the rows
+            // past `valid` store zeros in the same instruction)
             int lead; uint32_t bytes;
-            (void)x_src(tile, lead, bytes);
+            (void)x_src(p, tile, c_in, lead, bytes);
             mbar_wait(bar_x, xphase);
             xphase ^= 1;
-            uint8_t *a0 = a_buf(0);
-            const float *xr = stage + lead + tid * c_in;
-            const bool row_live = tid < valid;
-            // (tcgen05.st is warp-wide: the rows past `valid` store zeros in the same instruction)
-            auto put = [&](int c8, uint4 q) { *row_ptr(a0, c8) = q; tmem_st4(a_tm + (uint32_t)c8 * 4u, q); };
-            for (int c8 = 0; c8 < A0S - 1; ++c8) {         // (A0S - 1) * 8 <= c_in: every column of these slabs is a feature
-                uint4 q = make_uint4(0, 0, 0, 0);
-                if (row_live) {
-                    float f[8];
-#pragma unroll
-                    for (int j = 0; j < 8; ++j) f[j] = xr[c8 * 8 + j];
-                    q = make_uint4(pack_bf16(f[0], f[1]), pack_bf16(f[2], f[3]), pack_bf16(f[4], f[5]), pack_bf16(f[6], f[7]));
-                }
-                put(c8, q);
-            }
-            {
-                const int c8 = A0S - 1;
-                uint4 q = make_uint4(0, 0, 0, 0);
-                if (row_live) {
-                    float f[8];
-#pragma unroll
-                    for (int j = 0; j < 8; ++j) { const int c = c8 * 8 + j; f[j] = c < c_in ? xr[c] : (c == c_in ? 1.0f : 0.0f); }
-                    q = make_uint4(pack_bf16(f[0], f[1]), pack_bf16(f[2], f[3]), pack_bf16(f[4], f[5]), pack_bf16(f[6], f[7]));
-                }
-                put(c8, q);
-            }
+            pack_features(stage + lead + tid * c_in, c_in, tid < valid, store_a0);
         }
         // A_0's K padding in TMEM: explicit zeros (they meet zero weight rows, but stale TMEM bits could be NaN)
         for (int c8 = A0S; c8 < K0P / 8; ++c8) tmem_st4(a_tm + (uint32_t)c8 * 4u, make_uint4(0, 0, 0, 0));
@@ -434,7 +276,7 @@ __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel
         // ---- forward
         float hz[4];
         for (int l = 0; l < L; ++l) {
-            if (tid == 0) issue_steps(l, 0u, 64u);
+            if (tid == 0) issue_steps<true>(prog + l, tmem, 0u, 64u, 0u);
             commit_and_wait();
             const float *bl = bias_s + l * HP;
             if (l < L - 1) {
@@ -454,7 +296,7 @@ __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel
                     *row_ptr(an, c16 * 2 + 1) = make_uint4(o[4], o[5], o[6], o[7]);
                     tmem_st8(a_tm + (uint32_t)(c16 * 8), o);                          // for the next layer's MMA (A from TMEM)
                 }
-                tmem_st_wait_();
+                tmem_st_wait();
                 publish_tmem();
             } else {
                 uint32_t v[16];
@@ -465,112 +307,18 @@ __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel
             }
         }
         // ---- head + loss + adjoint of the head's pre-activation (unit seed)
-        float dz[4] = {0.f, 0.f, 0.f, 0.f};
-        if (p.head == LNB_HEAD_SIGMOID) {
-            // mlp_fit: row r <-> target row (scripts/mlp_fit.py:121-145)
-            if (tid < valid && row0 + tid < p.R) {
-                const float *tg = p.target + (row0 + tid) * p.Wt;
-                for (int c = 0; c < p.Wt && c < 4; ++c) {
-                    float y = sigmoid_f(hz[c]);
-                    float d = y - __ldg(tg + c);
-                    loss_acc = fmaf(d, d, loss_acc);
-                    dz[c] = 2.0f * d * (y * (1.0f - y));
-                }
-            }
-        } else {
-            // Compositing with one thread per sample (thread r <-> sample r of the tile): segmented warp-shuffle scans
-            // inside each warp, carries across the 4 warps through shared memory.  scripts/nerf.py:176-288 and its reverse.
-            const float cr = sigmoid_f(hz[0]), cg = sigmoid_f(hz[1]), cb = sigmoid_f(hz[2]);
-            const float sg = fmaxf(hz[3], 0.0f);
-            const float e = __expf((0.0f - sg) * my_dist);
-            const float a = 1.0f - e;
-            const float qv = live ? (1.0f - a) + 1e-10f : 1.0f;
-            float pr = qv;                                   // segmented inclusive product
-#pragma unroll
-            for (int d = 1; d < 32; d <<= 1) {
-                float o = __shfl_up_sync(0xffffffffu, pr, d);
-                if (lane >= d && smp >= d) pr *= o;
-            }
-            if (lane == 31) { tailp[warp] = pr; tail_s[warp] = smp; }
-            if (lane == 0) headq[warp] = qv;
-            if (live && smp == 0) {
-                color_s[ray_l * 3] = 0.f; color_s[ray_l * 3 + 1] = 0.f; color_s[ray_l * 3 + 2] = 0.f;
-                tgt_s[ray_l * 3] = tg0; tgt_s[ray_l * 3 + 1] = tg1; tgt_s[ray_l * 3 + 2] = tg2;
-            }
-            bar_group(g);
-            float carry = 1.0f;                              // product of this ray's samples in earlier warps
-            if (smp > lane) {
-                for (int w2 = warp - 1; w2 >= 0; --w2) {
-                    carry *= tailp[w2];
-                    if (tail_s[w2] < 32) break;              // that warp's last segment started inside it
-                }
-            }
-            const float Cpre = pr * carry;                   // true inclusive product prod_{k<=s} q_k
-            const float T = (smp == 0) ? 1.0f : Cpre;
-            const float wgt = a * T;
-            {   // colour: segmented inclusive sums, one shared-memory atomic per (warp, ray) segment
-                float s0 = live ? wgt * cr : 0.f, s1 = live ? wgt * cg : 0.f, s2 = live ? wgt * cb : 0.f;
-#pragma unroll
-                for (int d = 1; d < 32; d <<= 1) {
-                    float o0 = __shfl_up_sync(0xffffffffu, s0, d), o1 = __shfl_up_sync(0xffffffffu, s1, d), o2 = __shfl_up_sync(0xffffffffu, s2, d);
-                    if (lane >= d && smp >= d) { s0 += o0; s1 += o1; s2 += o2; }
-                }
-                if (live && (lane == 31 || smp == S - 1)) {
-                    atomicAdd(color_s + ray_l * 3, s0); atomicAdd(color_s + ray_l * 3 + 1, s1); atomicAdd(color_s + ray_l * 3 + 2, s2);
-                }
-            }
-            bar_group(g);
-            float dc0 = 0.f, dc1 = 0.f, dc2 = 0.f;
-            if (live) {
-                const float c0 = color_s[ray_l * 3], c1 = color_s[ray_l * 3 + 1], c2 = color_s[ray_l * 3 + 2];
-                if (smp == 0 && p.color) {
-                    float *co = p.color + (size_t)(tile * p.G + ray_l) * 3;
-                    co[0] = c0; co[1] = c1; co[2] = c2;
-                }
-                const float d0 = c0 - tgt_s[ray_l * 3], d1 = c1 - tgt_s[ray_l * 3 + 1], d2 = c2 - tgt_s[ray_l * 3 + 2];
-                if (smp == 0) loss_acc += d0 * d0 + d1 * d1 + d2 * d2;
-                dc0 = 2.0f * d0; dc1 = 2.0f * d1; dc2 = 2.0f * d2;
-            }
-            {
-                // G_s = dT_s + q_{s+1} G_{s+1}: suffix scan of affine maps; B = 0 at a ray's last sample
-                const float d_w = cr * dc0 + cg * dc1 + cb * dc2;
-                const float dT = (smp == 0 || !live) ? 0.0f : d_w * a;
-                float qn = __shfl_down_sync(0xffffffffu, qv, 1);
-                if (lane == 31) qn = warp < 3 ? headq[warp + 1] : 0.0f;
-                float Aa = dT, Bb = (live && smp + 1 < S) ? qn : 0.0f;
-#pragma unroll
-                for (int d = 1; d < 32; d <<= 1) {
-                    float A2 = __shfl_down_sync(0xffffffffu, Aa, d);
-                    float B2 = __shfl_down_sync(0xffffffffu, Bb, d);
-                    if (lane + d < 32) { Aa = fmaf(Bb, A2, Aa); Bb = Bb * B2; }
-                }
-                if (lane == 0) { headA[warp] = Aa; headB[warp] = Bb; }
-                bar_group(g);
-                float Gn = 0.0f;                             // G at lane 0 of the next warp
-                for (int w2 = 3; w2 > warp; --w2) Gn = fmaf(headB[w2], Gn, headA[w2]);
-                const float Gv = fmaf(Bb, Gn, Aa);
-                float Cm1 = __shfl_up_sync(0xffffffffu, Cpre, 1);
-                if (lane == 0) Cm1 = carry;
-                if (smp == 0) Cm1 = 1.0f;
-                const float d_alpha = d_w * T - Cm1 * Gv;
-                if (live) {
-                    dz[0] = (wgt * dc0) * (cr * (1.0f - cr));
-                    dz[1] = (wgt * dc1) * (cg * (1.0f - cg));
-                    dz[2] = (wgt * dc2) * (cb * (1.0f - cb));
-                    dz[3] = sg > 0.0f ? d_alpha * e * my_dist : 0.0f;
-                }
-            }
-        }
+        float dz[4];
+        head_and_composite<true>(p, scratch, g + 1, hz, my_dist, tg, row0, tile * p.G, valid, tid, smp, ray_l, live, loss_acc, dz);
         // ---- backward.  dZ_{L-1}: 4 live features of its one slab
         {
             const uint32_t o[8] = {pack_bf16(dz[0], dz[1]), pack_bf16(dz[2], dz[3]), 0u, 0u, 0u, 0u, 0u, 0u};
             *row_ptr(dzl_buf, 0) = make_uint4(o[0], o[1], 0u, 0u);
             tmem_st8(a_tm, o);
-            tmem_st_wait_();
+            tmem_st_wait();
         }
         publish_smem();
         for (int l = L - 1; l >= 1; --l) {
-            if (tid == 0) issue_steps(L + l, 0u, 64u);
+            if (tid == 0) issue_steps<true>(prog + L + l, tmem, 0u, 64u, 0u);
             issue_dw(l);                       // dW_l = A_l^T dZ_l while both are still there
             commit_and_wait();
             uint8_t *al = a_buf(l);
@@ -582,25 +330,14 @@ __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel
             for (int c8 = 0; c8 < HP / 8; ++c8) hm[c8] = *row_ptr(al, c8);
             tmem_ld_wait();
             uint4 oz[HP / 8];
-#pragma unroll
-            for (int c8 = 0; c8 < HP / 8; ++c8) {
-                // ReLU mask: bf16 post-ReLU values are >= 0, so positive <=> non-zero halfword
-                const uint32_t hw[4] = {hm[c8].x, hm[c8].y, hm[c8].z, hm[c8].w};
-                uint32_t o[4];
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    const int e = (c8 & 1) * 8 + 2 * j;
-                    o[j] = pack_bf16(__uint_as_float(v[c8 >> 1][e]), __uint_as_float(v[c8 >> 1][e + 1])) & gt0_mask_bf16x2(hw[j]);
-                }
-                oz[c8] = make_uint4(o[0], o[1], o[2], o[3]);
-            }
+            relu_adjoint<HP>(v, hm, oz);
             if (l > 1) {                       // dZ_{l-1} is the A operand of the next dH MMA
 #pragma unroll
                 for (int c16 = 0; c16 < HP / 16; ++c16) {
                     const uint32_t o[8] = {oz[2 * c16].x, oz[2 * c16].y, oz[2 * c16].z, oz[2 * c16].w, oz[2 * c16 + 1].x, oz[2 * c16 + 1].y, oz[2 * c16 + 1].z, oz[2 * c16 + 1].w};
                     tmem_st8(a_tm + (uint32_t)(c16 * 8), o);
                 }
-                tmem_st_wait_();
+                tmem_st_wait();
             }
             wait_dw();                         // ... and only now may A_l become dZ_{l-1}
 #pragma unroll

@@ -35,10 +35,12 @@
 #include <stdio.h>
 #include <stdlib.h>
 
+#include <type_traits>
 #include <vector>
 
 #include "camera.cuh"
 #include "lnb_internal.h"
+#include "tc_ptx.cuh"
 
 namespace {
 
@@ -62,7 +64,7 @@ struct TcParams {
     float *color;      // [R][3] or NULL
     float *part;       // [grid][part_stride]
     float *dbg;        // optional [N][4] head outputs (debug)
-    const void *wimg;  // weight image built by tc_prep_kernel (TcLayout::wimg_bytes)
+    const void *wimg;  // weight image built by tc_prep_kernel (ImgMap)
     // rays mode (X == NULL): features are computed in the kernel from rays and sample depths
     const void *rays_o, *rays_d, *tvals; // [R][3], [R][3], [R][S]; float64 when ray_f64 else float32
     int ray_f64, pe_bands;
@@ -80,14 +82,8 @@ struct TcParams {
 };
 
 // ---------------------------------------------------------------------------------------------
-// PTX wrappers
+// PTX wrappers of these kernels only (the shared ones are in tc_ptx.cuh)
 // ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count)
-{
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity)
 {
     uint32_t done = 0;
@@ -111,7 +107,10 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity)
 // The forward-only kernel's wait for an MMA stage: nine CTAs share an SM and a stage takes ~1 us there, during which the
 // hardware-suspended try_wait comes back ~10 times (any barrier event of the SM wakes it).  The render kernel is bound by
 // instruction issue and these polls were 30 % of its instructions at nine per iteration (counter, time-out test, sleep);
-// here an iteration is the try_wait and one branch, the counter ticks once per four polls.
+// here an iteration is the try_wait and one branch, the counter ticks once per four polls.  The multi-group train kernel's
+// groups wait with it too: with seven groups on an SM a hardware-suspended try_wait is woken by the other groups' barrier
+// traffic and re-polls several times per wait (an explicit __nanosleep between polls, tried before, does not actually sleep
+// there and costs five instructions).
 __device__ __forceinline__ void mbar_wait_tight(uint32_t bar, uint32_t parity)
 {
     asm volatile(
@@ -136,27 +135,7 @@ __device__ __forceinline__ void mbar_wait_tight(uint32_t bar, uint32_t parity)
         "}"
         :: "r"(bar), "r"(parity), "r"(100000u) : "memory");
 }
-__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 
-__device__ __forceinline__ void tmem_alloc(uint32_t smem_dst, uint32_t cols)
-{
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_dst), "r"(cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t cols)
-{
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
-}
-__device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate)
-{
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
-}
 // A operand from tensor memory (M = 128 rows = TMEM lanes; a 16-bit K-step of 16 is 8 columns, element 2c in the low half
 // of column c), B from shared memory
 __device__ __forceinline__ void umma_bf16_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t b_desc, uint32_t idesc, uint32_t accumulate)
@@ -172,20 +151,10 @@ __device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint32_t (&v)[8])
     asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};"
                  ::"r"(taddr), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]) : "memory");
 }
-__device__ __forceinline__ void tmem_st_wait_() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ void umma_commit(uint32_t bar)
-{
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&v)[16])
-{
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
-          "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-        : "r"(taddr) : "memory");
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
+// named barrier of the 128 threads of one tile: id 0 in the one-tile-per-CTA kernel (the whole CTA, = __syncthreads()),
+// g + 1 for group g of the multi-group kernel
+__device__ __forceinline__ void bar_tile(int id) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(TILE) : "memory"); }
 
 // UMMA shared-memory descriptor, SWIZZLE_NONE (cute::UMMA::SmemDescriptor): start>>4 [0,14),
 // LBO>>4 [16,30), SBO>>4 [32,46), version=1 [46,48), layout_type=0 [61,64)
@@ -194,18 +163,7 @@ __device__ __forceinline__ uint64_t smem_desc(uint32_t addr, uint32_t lbo, uint3
     return (uint64_t)((addr >> 4) & 0x3FFF) | ((uint64_t)((lbo >> 4) & 0x3FFF) << 16) |
            ((uint64_t)((sbo >> 4) & 0x3FFF) << 32) | (1ull << 46);
 }
-// instruction descriptor (cute::UMMA::InstrDescriptor): D=f32, A=B=bf16
-__device__ __forceinline__ uint32_t instr_desc(int M, int N, int a_mn_major, int b_mn_major)
-{
-    return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)a_mn_major << 15) | ((uint32_t)b_mn_major << 16) |
-           ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
 
-__device__ __forceinline__ uint32_t pack_bf16(float a, float b)
-{
-    __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
-    return *reinterpret_cast<uint32_t *>(&h);
-}
 __device__ __forceinline__ float sigmoid_f(float z) { return __fdividef(1.0f, 1.0f + __expf(0.0f - z)); }
 // two floats -> packed bf16 pair (lo = first), with ReLU: ONE instruction (F2FP.RELU.BF16)
 __device__ __forceinline__ uint32_t pack_relu_bf16(float lo, float hi)
@@ -233,17 +191,6 @@ __device__ __forceinline__ void pe_sincos(float x, float *s, float *c)
     __sincosf(r, s, c);
 }
 
-
-__device__ __forceinline__ float warp_incl_prod(float p, int lane)
-{
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-        float o = __shfl_up_sync(0xffffffffu, p, d);
-        if (lane >= d) p *= o;
-    }
-    return p;
-}
-
 // ---------------------------------------------------------------------------------------------
 // the kernel.  HP = padded hidden width (16/32/64): every hidden layer has width+1 <= HP.
 // 128 threads: thread r owns row r of the tile (TMEM lane r).  Thread 0 issues the MMAs and the
@@ -264,15 +211,49 @@ __device__ __forceinline__ float warp_incl_prod(float p, int lane)
 // Every MMA's operands are tile-invariant, so the descriptors are computed once per CTA into a
 // shared-memory "MMA program"; issuing a stage is a loop of (load 32 B record, tcgen05.mma).
 // ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes)
-{
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
 __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar)
 {
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
                  ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
 }
+
+// tensor-memory allocation for `need` columns: a power of two, at least 32
+__host__ __device__ inline uint32_t tmem_alloc_cols(int need)
+{
+    return need <= 32 ? 32 : (need <= 64 ? 64 : (need <= 128 ? 128 : (need <= 256 ? 256 : 512)));
+}
+
+// The weight image every CTA of the fused kernels copies: [W_0 .. W_{L-1} bf16 slabs][bias fp32 MAXL x HP], built by
+// tc_prep_kernel in global memory and refreshed in place by the fused Adam update.  W_l holds Kp = kp(l) input rows
+// (K0P for the first layer, HP after) of Np = np(l) columns (HP, 16 for the head) in the slab layout.  The A operands carry
+// an all-ones feature at column in_l (it exists for the bias gradient), so row in_l of a HIDDEN layer's W holds the bias
+// b_l (the MMA adds it) and, at column out_l, a 1.0 that re-creates the ones feature in the layer's output: the hidden-layer
+// epilogue is then just ReLU + pack.  The head keeps its bias in the fp32 tail [MAXL][HP] (zero for hidden layers).  In
+// the adjoint pass these extra entries only feed column in_l of dH_l, which becomes the ones column of dZ_{l-1}: it meets
+// zero weight columns and lands in weight-gradient entries nobody reads.
+struct ImgMap {
+    int L, HP, K0P;
+    int dims[MAXL + 1];
+    __host__ __device__ int np(int l) const { return l < L - 1 ? HP : 16; }
+    __host__ __device__ int kp(int l) const { return l == 0 ? K0P : HP; }
+    __host__ __device__ int w_off(int l) const
+    {
+        int o = 0;
+        for (int i = 0; i < l; ++i) o += np(i) * kp(i) * 2;
+        return o;
+    }
+    __host__ __device__ int bytes() const { return w_off(L) + MAXL * HP * 4; }
+    __device__ float *bias(uint8_t *img) const { return reinterpret_cast<float *>(img + w_off(L)); }
+    __device__ void put_w(uint8_t *img, int l, int k, int j, float v) const
+    {
+        reinterpret_cast<__nv_bfloat16 *>(img + w_off(l))[(k >> 3) * (np(l) * 8) + j * 8 + (k & 7)] = __float2bfloat16_rn(v);
+    }
+    __device__ void put_b(uint8_t *img, int l, int j, float v) const
+    {
+        if (l < L - 1) put_w(img, l, dims[l], j, v);   // hidden layers: bias row of the MMA operand
+        else bias(img)[l * HP + j] = v;                 // head: fp32
+    }
+};
 
 template <int HP>
 struct TcLayout {
@@ -283,8 +264,7 @@ struct TcLayout {
     // forward only (render): no adjoint buffers, no dW accumulator -> more CTAs per SM
     __host__ __device__ static uint32_t tmem_cols(int L, bool grad = true)
     {
-        const int need = grad ? HP + ndw(L) : HP + HP / 2;   // forward only: result columns + the next layer's bf16 A operand
-        return need <= 32 ? 32 : (need <= 64 ? 64 : (need <= 128 ? 128 : (need <= 256 ? 256 : 512)));
+        return tmem_alloc_cols(grad ? HP + ndw(L) : HP + HP / 2);   // forward only: result columns + the next layer's bf16 A operand
     }
     static constexpr int MAX_STAGES = 2 * MAXL + 1; // records of the per-CTA MMA program
     __host__ __device__ static int a_off(int l, int K0P) { return l == 0 ? 0 : (K0P / 8 + (l - 1) * HSL) * SLAB; }
@@ -297,17 +277,11 @@ struct TcLayout {
     {
         return grad ? (K0P / 8 + 2 * (L - 1) * HSL + 2) * SLAB : (fwd_slabs(K0P) + 2) * SLAB;
     }
-    __host__ __device__ static int np(int l, int L) { return l < L - 1 ? HP : 16; }
-    __host__ __device__ static int kp(int l, int K0P) { return l == 0 ? K0P : HP; }
-    __host__ __device__ static int w_off(int l, int L, int K0P)
-    {
-        int o = 0;
-        for (int i = 0; i < l; ++i) o += np(i, L) * kp(i, K0P) * 2;
-        return o;
-    }
-    // weight image = [W_0 .. W_{L-1} bf16 slabs][bias fp32 MAXL x HP], built once per step by
-    // tc_prep_kernel in global memory
-    __host__ __device__ static int wimg_bytes(int L, int K0P) { return w_off(L, L, K0P) + MAXL * HP * 4; }
+    // the weight image of this width (ImgMap)
+    __host__ __device__ static int np(int l, int L) { return ImgMap{L, HP, 0, {}}.np(l); }
+    __host__ __device__ static int kp(int l, int K0P) { return ImgMap{0, HP, K0P, {}}.kp(l); }
+    __host__ __device__ static int w_off(int l, int L, int K0P) { return ImgMap{L, HP, K0P, {}}.w_off(l); }
+    __host__ __device__ static int wimg_bytes(int L, int K0P) { return ImgMap{L, HP, K0P, {}}.bytes(); }
     __host__ __device__ static int stage_bytes(int c_in, int K0P) { return (TILE * c_in * 4 + 32 + K0P * 4 + 15) / 16 * 16; }
     static constexpr int SCRATCH_FLOATS = 48; // colour + target per ray, scan carries, loss
     __host__ __device__ static size_t total(int L, int K0P, int c_in, bool rays = false, bool grad = true)
@@ -319,41 +293,349 @@ struct TcLayout {
     }
 };
 
-// fp32 padded weights -> the bf16 slab image every CTA of the fused kernel copies.  The A operands carry an
-// all-ones feature at column in_l (it exists for the bias gradient), so row in_l of a HIDDEN layer's W holds
-// the bias b_l (the MMA adds it) and, at column out_l, a 1.0 that re-creates the ones feature in the layer's
-// output: the hidden-layer epilogue is then just ReLU + pack.  The head keeps its bias in fp32 (the image's
-// fp32 tail [MAXL][HP]; zero for hidden layers).  In the adjoint pass these extra entries only feed column
-// in_l of dH_l, which becomes the ones column of dZ_{l-1}: it meets zero weight columns and lands in
-// weight-gradient entries nobody reads.
-template <int HP>
-__global__ void tc_prep_kernel(const TcParams p, uint8_t *__restrict__ img)
+// fp32 padded weights and biases -> the weight image (ImgMap)
+__global__ void tc_prep_kernel(const TcParams p, const ImgMap im, uint8_t *__restrict__ img)
 {
-    using LY = TcLayout<HP>;
-    const int L = p.L, K0P = p.K0P;
+    const int L = im.L;
     for (int l = 0; l < L; ++l) {
-        const int in_l = p.dims[l], out_l = p.dims[l + 1], Np = LY::np(l, L), Kp = LY::kp(l, K0P);
+        const int in_l = im.dims[l], out_l = im.dims[l + 1], Np = im.np(l), Kp = im.kp(l);
         const float *wl = p.ws + (size_t)l * p.max_in * p.max_out;
         const float *bl = p.bs + (size_t)l * p.max_out;
-        __nv_bfloat16 *w = reinterpret_cast<__nv_bfloat16 *>(img + LY::w_off(l, L, K0P));
         for (int e = threadIdx.x; e < Np * Kp; e += blockDim.x) {
             const int k = e / Np, j = e % Np; // consecutive threads -> consecutive j (coalesced reads)
-            float v = 0.0f;
-            if (k < in_l && j < out_l) v = __ldg(wl + (size_t)k * p.max_out + j);
-            else if (k == in_l && l < L - 1) v = j < out_l ? __ldg(bl + j) : (j == out_l ? 1.0f : 0.0f);
-            w[(k >> 3) * (Np * 8) + j * 8 + (k & 7)] = __float2bfloat16_rn(v);
+            if (k == in_l && l < L - 1) im.put_b(img, l, j, j < out_l ? __ldg(bl + j) : (j == out_l ? 1.0f : 0.0f));
+            else im.put_w(img, l, k, j, k < in_l && j < out_l ? __ldg(wl + (size_t)k * p.max_out + j) : 0.0f);
         }
     }
-    float *b = reinterpret_cast<float *>(img + LY::w_off(L, L, K0P));
-    for (int e = threadIdx.x; e < MAXL * HP; e += blockDim.x) {
-        const int l = e / HP, j = e % HP;
-        b[e] = (l == L - 1 && j < p.dims[l + 1]) ? __ldg(p.bs + (size_t)l * p.max_out + j) : 0.0f;
+    for (int e = threadIdx.x; e < MAXL * im.HP; e += blockDim.x) {
+        const int l = e / im.HP, j = e % im.HP;
+        im.bias(img)[e] = (l == L - 1 && j < im.dims[l + 1]) ? __ldg(p.bs + (size_t)l * p.max_out + j) : 0.0f;
     }
 }
 
-// fp32 sin/cos of the positional encoding (pos_encoding.py:38-70): one accurate sincosf per
-// coordinate, higher bands by angle doubling (sin 2a = 2 s c, cos 2a = 1 - 2 s^2).  The doubling
-// amplifies the base error by 2^(E-1): ~1e-6 at E = 5, far below the bf16 operand rounding.
+// ---------------------------------------------------------------------------------------------
+// Per-tile stages of the one-tile-per-CTA kernel (below) and the multi-group train kernel (fused_mg.cuh).  Thread tid of a
+// tile's 128 owns row tid: sample smp of the tile's ray ray_l.
+// ---------------------------------------------------------------------------------------------
+
+// TMA source of a tile's features (16 B aligned start, `lead` floats in front of the tile)
+__device__ __forceinline__ const void *x_src(const TcParams &p, int tile, int c_in, int &lead, uint32_t &bytes)
+{
+    const long long row0 = (long long)tile * p.rows_per_tile;
+    long long rem = p.N - row0;
+    const int valid = rem < p.rows_per_tile ? (int)rem : p.rows_per_tile;
+    const uintptr_t a = reinterpret_cast<uintptr_t>(p.X + row0 * c_in);
+    const uintptr_t a16 = a & ~(uintptr_t)15;
+    lead = (int)((a - a16) >> 2);
+    bytes = (uint32_t)(((a - a16) + (uintptr_t)valid * c_in * 4 + 15) & ~(uintptr_t)15);
+    return reinterpret_cast<const void *>(a16);
+}
+
+// This row's inputs other than its features, loaded early (latency-tolerant, consumed after the MLP forward): the sample
+// spacing `dist` and, at a ray's first sample, the ray's target colour.  From rays (RAYS) also the sample point x:
+// pts = o + d t (train_nerf.py:289-299), dist = t[s+1] - t[s], last 1e8 (train_nerf.py:306-311).  x and dist stay 0 in a
+// row past the tile's live samples.
+template <bool RAYS>
+__device__ __forceinline__ void sample_inputs(const TcParams &p, long long row0, int ray0, int tid, int smp, int ray_l, bool live,
+                                              float (&x)[3], float &dist, float (&tg)[3])
+{
+    const int S = p.S;
+    dist = 0.0f;
+    tg[0] = tg[1] = tg[2] = 0.0f;
+    if (p.head == LNB_HEAD_NERF && live) {
+        if (!RAYS) dist = __ldg(p.dists + row0 + tid);
+        if (p.target && smp == 0) {
+            const float *t = p.target + (size_t)(ray0 + ray_l) * 3;   // a tile holds G whole rays: ray0 = row0 / S (R is an int)
+            tg[0] = __ldg(t); tg[1] = __ldg(t + 1); tg[2] = __ldg(t + 2);
+        }
+    }
+    x[0] = x[1] = x[2] = 0.0f;
+    if (!RAYS || !live) return;
+    const long long ray = ray0 + ray_l;
+    if (p.cam_mode) {
+        // ray of pixel q and depth of sample smp straight from the pose (get_rays, train_nerf.py:23-62; linspace /
+        // stratified depths, train_nerf.py:289-311): no per-ray or per-sample input at all
+        const CamF32 &c = p.cam;
+        const long long q = c.pixels ? (long long)__ldg(c.pixels + ray) : c.first_pixel + ray;
+        // q / width by the 64-bit reciprocal the launcher computed (exact for every 32-bit q)
+        const unsigned uq = (unsigned)q, row = c.width == 1 ? uq : (unsigned)__umul64hi((unsigned long long)uq, c.w_magic), col = uq - row * (unsigned)c.width;
+        const float fi = col == (unsigned)c.width - 1 ? 1.0f : (float)col * c.step, fj = row == (unsigned)c.width - 1 ? 1.0f : (float)row * c.step;
+        const float dx = (fi - c.cx) * c.inv_fx, dy = (c.cy - fj) * c.inv_fy;
+        float tt, tn;
+        if (c.stratified) {
+            tt = fmaf((float)smp + (float)lnb_uniform_bits(c.seed, q, smp) * (1.0f / 16777216.0f), c.dt_str, c.near);
+            tn = fmaf((float)(smp + 1) + (float)lnb_uniform_bits(c.seed, q, smp + 1) * (1.0f / 16777216.0f), c.dt_str, c.near);
+        } else {
+            tt = smp == S - 1 && S > 1 ? c.far : fmaf((float)smp, c.dt_lin, c.near);
+            tn = smp + 1 == S - 1 ? c.far : fmaf((float)(smp + 1), c.dt_lin, c.near);
+        }
+        dist = smp + 1 < S ? tn - tt : 1e8f;
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+            const float dk = fmaf(dx, c.c2w[4 * k], fmaf(dy, c.c2w[4 * k + 1], 0.0f - c.c2w[4 * k + 2]));
+            x[k] = fmaf(dk, tt, c.c2w[4 * k + 3]);
+        }
+    } else if (p.ray_f64) {
+        const double *o = reinterpret_cast<const double *>(p.rays_o) + ray * 3;
+        const double *d = reinterpret_cast<const double *>(p.rays_d) + ray * 3;
+        const double *tv = reinterpret_cast<const double *>(p.tvals) + row0 + tid;
+        const double tt = __ldg(tv);
+        dist = smp + 1 < S ? (float)(__ldg(tv + 1) - tt) : 1e8f;
+#pragma unroll
+        for (int c = 0; c < 3; ++c) x[c] = (float)(__ldg(o + c) + __ldg(d + c) * tt);
+    } else {
+        const float *o = reinterpret_cast<const float *>(p.rays_o) + ray * 3;
+        const float *d = reinterpret_cast<const float *>(p.rays_d) + ray * 3;
+        const float *tv = reinterpret_cast<const float *>(p.tvals) + row0 + tid;
+        const float tt = __ldg(tv);
+        dist = smp + 1 < S ? __ldg(tv + 1) - tt : 1e8f;
+#pragma unroll
+        for (int c = 0; c < 3; ++c) x[c] = fmaf(__ldg(d + c), tt, __ldg(o + c));
+    }
+}
+
+// The positional encoding (pos_encoding.py:38-70) of the sample point x into this row's first `live_slabs` slabs of A_0,
+// through store(slab, its 16 bytes of the row).  sn / cs: sin / cos of x (pe_sincos); the higher bands by angle doubling
+// (sin 2a = 2 s c, cos 2a = 1 - 2 s^2), which amplifies the base error by 2^(E-1): ~1e-6 at E = 5, far below the bf16
+// operand rounding.  Feature f = 3 * slot + coord: x0 x1 | x2 s0 | s1 s2 | c0 c1 | c2 s0' | ... as bf16 pairs (pair j =
+// features 2j, 2j+1); band i fills pairs 1+3i .. 3+3i and leaves its last cosine pending; the ones column (feature 3 + 6E,
+// odd) closes the pending pair.  Four pairs make a slab's 16 bytes, stored as soon as they are complete.
+template <class Store>
+__device__ __forceinline__ void pack_pe(const float (&x)[3], float (&sn)[3], float (&cs)[3], int pe_bands, int live_slabs, Store &&store)
+{
+    uint32_t q4[4] = {pack_bf16(x[0], x[1]), 0u, 0u, 0u};
+    float pend = x[2];
+    bool closed = false;
+    auto put = [&](int j, uint32_t v) {            // j is a compile-time constant at every call site
+        q4[j & 3] = v;
+        if ((j & 3) == 3) {
+            if ((j >> 2) < live_slabs) store(j >> 2, make_uint4(q4[0], q4[1], q4[2], q4[3]));
+            q4[0] = q4[1] = q4[2] = q4[3] = 0u;
+        }
+    };
+    // warp-uniform branches: the bands that are off cost nothing
+#pragma unroll
+    for (int i = 0; i < 10; ++i) {
+        if (i < pe_bands) {
+            put(1 + 3 * i, pack_bf16(pend, sn[0]));
+            put(2 + 3 * i, pack_bf16(sn[1], sn[2]));
+            put(3 + 3 * i, pack_bf16(cs[0], cs[1]));
+            pend = cs[2];
+#pragma unroll
+            for (int c = 0; c < 3; ++c) {
+                const float s2 = 2.0f * sn[c] * cs[c], c2 = fmaf(-2.0f * sn[c], sn[c], 1.0f);
+                sn[c] = s2; cs[c] = c2;
+            }
+        } else {
+            if (closed && ((1 + 3 * i) >> 2) >= live_slabs) break;   // no live slab left to store (slab 7 then is not live either)
+            put(1 + 3 * i, closed ? 0u : pack_bf16(pend, 1.0f));
+            put(2 + 3 * i, 0u);
+            put(3 + 3 * i, 0u);
+            closed = true;
+        }
+    }
+    put(31, closed ? 0u : pack_bf16(pend, 1.0f));
+}
+
+// Features mode: this row's c_in fp32 features (xr) -> its first (c_in + 8) / 8 slabs of A_0, through store(slab, its
+// 16 bytes of the row): full slabs, then the last one with the ones column (feature c_in, the bias-gradient feature)
+// written explicitly and zeros after it.  A row past the tile's valid ones stores zeros.
+template <class Store>
+__device__ __forceinline__ void pack_features(const float *xr, int c_in, bool row_live, Store &&store)
+{
+    // the slab count from an opaque copy of c_in: otherwise the compiler hoists the loop's trip-count arithmetic out of the
+    // caller's tile loop, where it holds registers for the whole tile (a dozen more in the one-tile-per-CTA kernel)
+    int n = c_in;
+    asm volatile("" : "+r"(n));
+    const int a0s = (n + 8) >> 3;
+    for (int c8 = 0; c8 < a0s - 1; ++c8) {         // (a0s - 1) * 8 <= c_in: every column of these slabs is a feature
+        uint4 q = make_uint4(0, 0, 0, 0);
+        if (row_live) {
+            float f[8];
+#pragma unroll
+            for (int j = 0; j < 8; ++j) f[j] = xr[c8 * 8 + j];
+            q = make_uint4(pack_bf16(f[0], f[1]), pack_bf16(f[2], f[3]), pack_bf16(f[4], f[5]), pack_bf16(f[6], f[7]));
+        }
+        store(c8, q);
+    }
+    const int c8 = a0s - 1;
+    uint4 q = make_uint4(0, 0, 0, 0);
+    if (row_live) {
+        float f[8];
+#pragma unroll
+        for (int j = 0; j < 8; ++j) { const int c = c8 * 8 + j; f[j] = c < c_in ? xr[c] : (c == c_in ? 1.0f : 0.0f); }
+        q = make_uint4(pack_bf16(f[0], f[1]), pack_bf16(f[2], f[3]), pack_bf16(f[4], f[5]), pack_bf16(f[6], f[7]));
+    }
+    store(c8, q);
+}
+
+// shared-memory scratch of the head and compositing stage of one tile
+struct CompScratch {
+    float *color, *tgt;             // [rays of the tile][3]: colour sums, targets
+    float *tailp;                   // [4] inclusive product at lane 31 of each warp
+    int *tail_s;                    // [4] sample index at lane 31
+    float *headq, *headA, *headB;   // [5] q at lane 0 of each warp; the affine suffix scan's head of each warp
+};
+
+// The head on the last layer's pre-activations hz, the loss (added to loss_acc) and, with GRAD, dz = the adjoint of hz
+// (unit seed).  `bar` is the tile's named barrier (bar_tile).
+template <bool GRAD>
+__device__ __forceinline__ void head_and_composite(const TcParams &p, const CompScratch &s, int bar, const float (&hz)[4], float dist,
+                                                   const float (&tg)[3], long long row0, int ray0, int valid, int tid, int smp,
+                                                   int ray_l, bool live, float &loss_acc, float (&dz)[4])
+{
+    const int warp = tid >> 5, lane = tid & 31, S = p.S;
+    dz[0] = dz[1] = dz[2] = dz[3] = 0.0f;
+    if (p.head == LNB_HEAD_SIGMOID) {
+        // mlp_fit: row r <-> target row (scripts/mlp_fit.py:121-145)
+        if (tid < valid && row0 + tid < p.R) {
+            const float *t = p.target + (row0 + tid) * p.Wt;
+            for (int c = 0; c < p.Wt && c < 4; ++c) {
+                float y = sigmoid_f(hz[c]);
+                float d = y - __ldg(t + c);
+                loss_acc = fmaf(d, d, loss_acc);
+                dz[c] = 2.0f * d * (y * (1.0f - y));
+            }
+        }
+        return;
+    }
+    // Compositing with one thread per sample (thread r <-> sample r of the tile): segmented warp-shuffle scans inside each
+    // warp, carries across the 4 warps through shared memory.  scripts/nerf.py:176-288 and its reverse (SURVEY.md
+    // Appendix B).
+    const float cr = sigmoid_f(hz[0]), cg = sigmoid_f(hz[1]), cb = sigmoid_f(hz[2]);
+    const float sg = fmaxf(hz[3], 0.0f);
+    const float e = __expf((0.0f - sg) * dist);
+    const float a = 1.0f - e;
+    const float qv = live ? (1.0f - a) + 1e-10f : 1.0f;
+    float pr = qv;                                   // segmented inclusive product
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        float o = __shfl_up_sync(0xffffffffu, pr, d);
+        if (lane >= d && smp >= d) pr *= o;
+    }
+    if (lane == 31) { s.tailp[warp] = pr; s.tail_s[warp] = smp; }
+    if (lane == 0) s.headq[warp] = qv;
+    if (live && smp == 0) {
+        s.color[ray_l * 3] = 0.f; s.color[ray_l * 3 + 1] = 0.f; s.color[ray_l * 3 + 2] = 0.f;
+        s.tgt[ray_l * 3] = tg[0]; s.tgt[ray_l * 3 + 1] = tg[1]; s.tgt[ray_l * 3 + 2] = tg[2];
+    }
+    bar_tile(bar);
+    float carry = 1.0f;                              // product of this ray's samples in earlier warps
+    if (smp > lane) {
+        for (int w2 = warp - 1; w2 >= 0; --w2) {
+            carry *= s.tailp[w2];
+            if (s.tail_s[w2] < 32) break;            // that warp's last segment started inside it
+        }
+    }
+    const float Cpre = pr * carry;                   // true inclusive product prod_{k<=s} q_k
+    const float T = (smp == 0) ? 1.0f : Cpre;
+    const float wgt = a * T;
+    {   // colour: segmented inclusive sums, one shared-memory atomic per (warp, ray) segment
+        float s0 = live ? wgt * cr : 0.f, s1 = live ? wgt * cg : 0.f, s2 = live ? wgt * cb : 0.f;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            float o0 = __shfl_up_sync(0xffffffffu, s0, d), o1 = __shfl_up_sync(0xffffffffu, s1, d), o2 = __shfl_up_sync(0xffffffffu, s2, d);
+            if (lane >= d && smp >= d) { s0 += o0; s1 += o1; s2 += o2; }
+        }
+        if (live && (lane == 31 || smp == S - 1)) {
+            atomicAdd(s.color + ray_l * 3, s0); atomicAdd(s.color + ray_l * 3 + 1, s1); atomicAdd(s.color + ray_l * 3 + 2, s2);
+        }
+    }
+    bar_tile(bar);
+    float dc0 = 0.f, dc1 = 0.f, dc2 = 0.f;
+    if (live) {
+        const float c0 = s.color[ray_l * 3], c1 = s.color[ray_l * 3 + 1], c2 = s.color[ray_l * 3 + 2];
+        if (smp == 0 && p.color) {
+            float *co = p.color + (size_t)(ray0 + ray_l) * 3;
+            co[0] = c0; co[1] = c1; co[2] = c2;
+        }
+        // a train step always has a target (the launcher refuses a gradient without one); a forward-only call may pass none
+        if (GRAD || p.target) {
+            const float d0 = c0 - s.tgt[ray_l * 3], d1 = c1 - s.tgt[ray_l * 3 + 1], d2 = c2 - s.tgt[ray_l * 3 + 2];
+            if (smp == 0) loss_acc += d0 * d0 + d1 * d1 + d2 * d2;
+            dc0 = 2.0f * d0; dc1 = 2.0f * d1; dc2 = 2.0f * d2;
+        }
+    }
+    if (!GRAD) return;
+    // G_s = dT_s + q_{s+1} G_{s+1}: suffix scan of affine maps; B = 0 at a ray's last sample
+    const float d_w = cr * dc0 + cg * dc1 + cb * dc2;
+    const float dT = (smp == 0 || !live) ? 0.0f : d_w * a;
+    float qn = __shfl_down_sync(0xffffffffu, qv, 1);
+    if (lane == 31) qn = warp < 3 ? s.headq[warp + 1] : 0.0f;
+    float Aa = dT, Bb = (live && smp + 1 < S) ? qn : 0.0f;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        float A2 = __shfl_down_sync(0xffffffffu, Aa, d);
+        float B2 = __shfl_down_sync(0xffffffffu, Bb, d);
+        if (lane + d < 32) { Aa = fmaf(Bb, A2, Aa); Bb = Bb * B2; }
+    }
+    if (lane == 0) { s.headA[warp] = Aa; s.headB[warp] = Bb; }
+    bar_tile(bar);
+    float Gn = 0.0f;                                 // G at lane 0 of the next warp
+    for (int w2 = 3; w2 > warp; --w2) Gn = fmaf(s.headB[w2], Gn, s.headA[w2]);
+    const float Gv = fmaf(Bb, Gn, Aa);
+    float Cm1 = __shfl_up_sync(0xffffffffu, Cpre, 1);
+    if (lane == 0) Cm1 = carry;
+    if (smp == 0) Cm1 = 1.0f;
+    const float d_alpha = d_w * T - Cm1 * Gv;
+    if (live) {
+        dz[0] = (wgt * dc0) * (cr * (1.0f - cr));
+        dz[1] = (wgt * dc1) * (cg * (1.0f - cg));
+        dz[2] = (wgt * dc2) * (cb * (1.0f - cb));
+        dz[3] = sg > 0.0f ? d_alpha * e * dist : 0.0f;
+    }
+}
+
+// One stage of an MMA program, built once per CTA (group) in shared memory: the MMAs of a stage differ only by constant
+// increments of the descriptors' start-address fields (the K-steps).  With a_tmem set, `a` is the tensor-memory column of
+// the A operand (8 columns per K-step) instead of a shared-memory descriptor.
+struct StageRec { uint64_t a, b; uint32_t inc_a, inc_b, idesc, dcol; uint32_t count, a_tmem, pad0, pad1; };
+
+// issue K-steps [k0, min(k1, count)) of a stage (one thread): the first accumulates into D when `acc` is set, the others
+// always.  TS: the program has stages that take A from tensor memory.
+template <bool TS>
+__device__ __forceinline__ void issue_steps(const StageRec *rec, uint32_t tmem, uint32_t k0, uint32_t k1, uint32_t acc)
+{
+    const uint4 r0 = *reinterpret_cast<const uint4 *>(rec);
+    const uint4 r1 = *(reinterpret_cast<const uint4 *>(rec) + 1);
+    const uint4 r2 = *(reinterpret_cast<const uint4 *>(rec) + 2);
+    if (k1 > r2.x) k1 = r2.x;
+    uint32_t alo = r0.x + k0 * r1.x, blo = r0.z + k0 * r1.y;
+    const uint32_t ahi = r0.y, bhi = r0.w;
+    const uint32_t d = tmem + r1.w;
+    if (TS && r2.y) {
+        for (uint32_t k = k0; k < k1; ++k) {
+            umma_bf16_ts(d, tmem + alo, ((uint64_t)bhi << 32) | blo, r1.z, acc);
+            alo += r1.x; blo += r1.y; acc = 1u;
+        }
+        return;
+    }
+    for (uint32_t k = k0; k < k1; ++k) {
+        umma_bf16(d, ((uint64_t)ahi << 32) | alo, ((uint64_t)bhi << 32) | blo, r1.z, acc);
+        alo += r1.x; blo += r1.y; acc = 1u;
+    }
+}
+
+// The ReLU adjoint of one row: dz = dH_l (the fp32 TMEM values v, rounded to bf16) where the stored bf16 activation a of
+// A_l is positive, 0 elsewhere; 8 features per uint4.  Post-ReLU values are >= 0, so positive <=> non-zero halfword.
+template <int HP>
+__device__ __forceinline__ void relu_adjoint(const uint32_t (&v)[HP / 16][16], const uint4 (&a)[HP / 8], uint4 (&dz)[HP / 8])
+{
+#pragma unroll
+    for (int c8 = 0; c8 < HP / 8; ++c8) {
+        const uint32_t hw[4] = {a[c8].x, a[c8].y, a[c8].z, a[c8].w};
+        uint32_t o[4];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            const int e = (c8 & 1) * 8 + 2 * j;
+            o[j] = pack_bf16(__uint_as_float(v[c8 >> 1][e]), __uint_as_float(v[c8 >> 1][e + 1])) & gt0_mask_bf16x2(hw[j]);
+        }
+        dz[c8] = make_uint4(o[0], o[1], o[2], o[3]);
+    }
+}
+
+// ---------------------------------------------------------------------------------------------
+// the one-tile-per-CTA kernel.
 // FWD: the forward-only (render) form, compiled separately: nothing of the backward pass in its register budget.  Its
 // launch bounds are the CTAs per SM that tensor memory admits (512 columns / 64 per CTA = 8; 4 for the 64-wide form), not
 // more: a ninth CTA could never allocate its columns and the tighter register budget only bought a spill.
@@ -388,31 +670,16 @@ __global__ void __launch_bounds__(TILE, FWD ? (HP == 64 ? 4 : 8) : 1) fused_v1_k
     uint64_t *const bar_p = reinterpret_cast<uint64_t *>(tailp + 48);
     uint32_t *const tmem_slot = reinterpret_cast<uint32_t *>(bar_p + 4);
     const uint32_t bar_mma = smem_u32(bar_p), bar_x = smem_u32(bar_p + 1), bar_w = smem_u32(bar_p + 2), bar_dw = smem_u32(bar_p + 3);
-    // MMA program: one record per stage; the MMAs of a stage differ only by constant increments of
-    // the descriptors' start-address fields (the K-steps)
-    struct StageRec { uint64_t a, b; uint32_t inc_a, inc_b, idesc, dcol; uint32_t count, first_acc, pad0, pad1; };
-    StageRec *const prog = reinterpret_cast<StageRec *>(reinterpret_cast<uint8_t *>(bar_p) + 64);
+    const CompScratch scratch{color_s, tgt_s, tailp, tail_s, headq, headA, headB};
+    StageRec *const prog = reinterpret_cast<StageRec *>(reinterpret_cast<uint8_t *>(bar_p) + 64);   // the MMA program
 
-    // TMA source of a tile's features (16 B aligned start, `lead` floats in front of the tile)
-    auto x_src = [&](int tile, int &lead, uint32_t &bytes) -> const void * {
-        const long long row0 = (long long)tile * p.rows_per_tile;
-        long long rem = p.N - row0;
-        const int valid = rem < p.rows_per_tile ? (int)rem : p.rows_per_tile;
-        const uintptr_t a = reinterpret_cast<uintptr_t>(p.X + row0 * c_in);
-        const uintptr_t a16 = a & ~(uintptr_t)15;
-        lead = (int)((a - a16) >> 2);
-        bytes = (uint32_t)(((a - a16) + (uintptr_t)valid * c_in * 4 + 15) & ~(uintptr_t)15);
-        return reinterpret_cast<const void *>(a16);
-    };
-
-    // ---- one-time setup: zero activations and stage, then TMA the weight image and the first tile
+    // ---- one-time setup: zero activations, then TMA the weight image and the first tile
     // (every activation / adjoint buffer is fully rewritten each tile before it is read, except
     // the upper 8 features of dZ_{L-1}, which must stay zero)
     for (uint8_t *z = smem + LY::dz_off(L - 1, L, K0P) + tid * 16; z < smem + act_bytes; z += TILE * 16) *reinterpret_cast<uint4 *>(z) = make_uint4(0, 0, 0, 0);
-    // A_0: only the slabs holding live features are rewritten per tile; its padding must be zero
+    // A_0: only the slabs holding live features are rewritten per tile; its K padding, which the layer-0 MMA reads from
+    // shared memory, must be zero
     for (uint8_t *z = smem + tid * 16; z < smem + (fwd_only ? LY::fwd_slabs(K0P) * SLAB : LY::a_off(1, K0P)); z += TILE * 16) *reinterpret_cast<uint4 *>(z) = make_uint4(0, 0, 0, 0);
-    for (uint8_t *z = reinterpret_cast<uint8_t *>(stage) + tid * 16; z < reinterpret_cast<uint8_t *>(tailp); z += TILE * 16)
-        *reinterpret_cast<uint4 *>(z) = make_uint4(0, 0, 0, 0);
     if (tid == 0) {
         mbar_init(bar_mma, 1);
         mbar_init(bar_x, 1);
@@ -425,7 +692,7 @@ __global__ void __launch_bounds__(TILE, FWD ? (HP == 64 ? 4 : 8) : 1) fused_v1_k
             const uint32_t a0 = smem_u32(smem + (fwd_only ? 0 : LY::a_off(l, K0P))), b0 = smem_u32(Wbase + LY::w_off(l, L, K0P));
             prog[l] = StageRec{smem_desc(a0, SLAB, 128), smem_desc(b0, Np * 16, 128), (uint32_t)(2 * SLAB) >> 4, (uint32_t)(2 * Np * 16) >> 4,
                                instr_desc(128, Np, 0, 0), 0u, (uint32_t)(Kp / 16), 0u, 0u, 0u};
-            if (fwd_only && l > 0) { prog[l].a = (uint64_t)HP; prog[l].inc_a = 8u; prog[l].pad0 = 1u; }   // A from TMEM, 8 columns per K-step
+            if (fwd_only && l > 0) { prog[l].a = (uint64_t)HP; prog[l].inc_a = 8u; prog[l].a_tmem = 1u; }   // A from TMEM, 8 columns per K-step
         }
         for (int l = 1; l < L; ++l) {          // dH_l[128 x Kp] = dZ_l[128 x Np] * W_l^T (same W bytes, MN-major)
             const int Np = LY::np(l, L), Kp = LY::kp(l, K0P);
@@ -436,7 +703,7 @@ __global__ void __launch_bounds__(TILE, FWD ? (HP == 64 ? 4 : 8) : 1) fused_v1_k
         {                                      // dW: [all A]^T [all dZ], K = 128 samples, both MN-major
             const uint32_t a0 = smem_u32(smem), b0 = smem_u32(smem + LY::dz_off(0, L, K0P));
             prog[2 * L] = StageRec{smem_desc(a0, 128, SLAB), smem_desc(b0, 128, SLAB), 256u >> 4, 256u >> 4,
-                                   instr_desc(128, LY::ndw(L), 1, 1), (uint32_t)HP, (uint32_t)(TILE / 16), 2u, 0u, 0u};
+                                   instr_desc(128, LY::ndw(L), 1, 1), (uint32_t)HP, (uint32_t)(TILE / 16), 0u, 0u, 0u};
         }
     }
     if (warp == 0) tmem_alloc(smem_u32(tmem_slot), LY::tmem_cols(L, !FWD));
@@ -446,16 +713,16 @@ __global__ void __launch_bounds__(TILE, FWD ? (HP == 64 ? 4 : 8) : 1) fused_v1_k
     tc_fence_after();
     // Programmatic dependent launch: everything above (shared-memory zeroing, barrier init, TMEM
     // allocation, the MMA program) overlaps the tail of the previous kernel in the stream; from here
-    // on we read what it produced (weight image, tile counter, step counter).  No-op without PDL.
-    asm volatile("griddepcontrol.wait;" ::: "memory");
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+    // on we read what it produced (weight image, tile counter, step counter).
+    pdl_wait();
+    pdl_trigger();
     if (tid == 0) {
         const uint32_t wb = (uint32_t)LY::wimg_bytes(L, K0P);
         mbar_expect_tx(bar_w, wb);
         bulk_g2s(smem_u32(Wbase), p.wimg, wb, bar_w);
         if (!RAYS) {
             int lead; uint32_t bytes;
-            const void *src = x_src(blockIdx.x, lead, bytes);
+            const void *src = x_src(p, blockIdx.x, c_in, lead, bytes);
             mbar_expect_tx(bar_x, bytes);
             bulk_g2s(smem_u32(stage), src, bytes, bar_x);
         }
@@ -471,27 +738,8 @@ __global__ void __launch_bounds__(TILE, FWD ? (HP == 64 ? 4 : 8) : 1) fused_v1_k
     auto a_buf = [&](int l) { return smem + (fwd_only ? 0 : LY::a_off(l, K0P)); };
     auto dz_buf = [&](int l) { return smem + LY::dz_off(l, L, K0P); };
     auto row_ptr = [&](uint8_t *buf, int slab) { return reinterpret_cast<uint4 *>(buf + slab * SLAB + tid * 16); };
-    // issue one stage of the MMA program (thread 0 only)
-    auto issue_stage = [&](int stage_id) {
-        const uint4 r0 = *reinterpret_cast<const uint4 *>(prog + stage_id);
-        const uint4 r1 = *(reinterpret_cast<const uint4 *>(prog + stage_id) + 1);
-        const uint4 r2 = *(reinterpret_cast<const uint4 *>(prog + stage_id) + 2);
-        uint32_t alo = r0.x, blo = r0.z;
-        const uint32_t ahi = r0.y, bhi = r0.w;
-        uint32_t acc = r2.y == 2u ? (dw_started ? 1u : 0u) : r2.y;
-        const uint32_t d = tmem + r1.w;
-        if (FWD && r2.z) {               // A operand in tensor memory
-            for (uint32_t k = 0; k < r2.x; ++k) {
-                umma_bf16_ts(d, tmem + alo, ((uint64_t)bhi << 32) | blo, r1.z, acc);
-                alo += r1.x; blo += r1.y; acc = 1u;
-            }
-            return;
-        }
-        for (uint32_t k = 0; k < r2.x; ++k) {
-            umma_bf16(d, ((uint64_t)ahi << 32) | alo, ((uint64_t)bhi << 32) | blo, r1.z, acc);
-            alo += r1.x; blo += r1.y; acc = 1u;
-        }
-    };
+    // issue all K-steps of one stage of the MMA program (thread 0 only); the weight gradient accumulates across tiles
+    auto issue_stage = [&](int stage_id, uint32_t acc) { issue_steps<FWD>(prog + stage_id, tmem, 0u, 64u, acc); };
     auto commit_and_wait = [&]() {
         if (tid == 0) umma_commit(bar_mma);
         if (FWD) mbar_wait_tight(bar_mma, phase);
@@ -524,130 +772,28 @@ __global__ void __launch_bounds__(TILE, FWD ? (HP == 64 ? 4 : 8) : 1) fused_v1_k
         const int ray0 = tile * p.G;      // = row0 / S: a tile holds G whole rays (R is an int)
         CLK(15);
         const bool live = tid < rays_here * S;
-        // early, latency-tolerant loads for this tile (consumed after the MLP forward)
-        float my_dist = 0.0f, tg0 = 0.0f, tg1 = 0.0f, tg2 = 0.0f;
-        if (p.head == LNB_HEAD_NERF && live) {
-            if (!RAYS) my_dist = __ldg(p.dists + row0 + tid);
-            if (p.target && smp == 0) {
-                const float *tg = p.target + (size_t)(ray0 + ray_l) * 3;
-                tg0 = __ldg(tg); tg1 = __ldg(tg + 1); tg2 = __ldg(tg + 2);
-            }
-        }
+        float x[3], my_dist, tg[3];
+        sample_inputs<RAYS>(p, row0, ray0, tid, smp, ray_l, live, x, my_dist, tg);
+        auto store_a0 = [&](int c8, uint4 q) { *row_ptr(a_buf(0), c8) = q; };
+        const int a0s = (c_in + 8) >> 3;   // slabs holding features 0..c_in (the ones column included)
         if (RAYS) {
-            // ---- features from rays: pts = o + d t (train_nerf.py:289-299), PE (pos_encoding.py:38-70),
-            // dist = t[s+1] - t[s], last 1e8 (train_nerf.py:306-311); written straight into A_0
-            float x[3] = {0.f, 0.f, 0.f};
-            if (live && p.cam_mode) {
-                // ray of pixel q and depth of sample smp straight from the pose (get_rays, train_nerf.py:23-62; linspace /
-                // stratified depths, train_nerf.py:289-311): no per-ray or per-sample input at all
-                const CamF32 &c = p.cam;
-                const long long ray = ray0 + ray_l;
-                const long long q = c.pixels ? (long long)__ldg(c.pixels + ray) : c.first_pixel + ray;
-                // q / width by the 64-bit reciprocal the launcher computed (exact for every 32-bit q)
-                const unsigned uq = (unsigned)q, row = c.width == 1 ? uq : (unsigned)__umul64hi((unsigned long long)uq, c.w_magic), col = uq - row * (unsigned)c.width;
-                const float fi = col == (unsigned)c.width - 1 ? 1.0f : (float)col * c.step, fj = row == (unsigned)c.width - 1 ? 1.0f : (float)row * c.step;
-                const float dx = (fi - c.cx) * c.inv_fx, dy = (c.cy - fj) * c.inv_fy;
-                float tt, tn;
-                if (c.stratified) {
-                    tt = fmaf((float)smp + (float)lnb_uniform_bits(c.seed, q, smp) * (1.0f / 16777216.0f), c.dt_str, c.near);
-                    tn = fmaf((float)(smp + 1) + (float)lnb_uniform_bits(c.seed, q, smp + 1) * (1.0f / 16777216.0f), c.dt_str, c.near);
-                } else {
-                    tt = smp == S - 1 && S > 1 ? c.far : fmaf((float)smp, c.dt_lin, c.near);
-                    tn = smp + 1 == S - 1 ? c.far : fmaf((float)(smp + 1), c.dt_lin, c.near);
-                }
-                my_dist = smp + 1 < S ? tn - tt : 1e8f;
-#pragma unroll
-                for (int k = 0; k < 3; ++k) {
-                    const float dk = fmaf(dx, c.c2w[4 * k], fmaf(dy, c.c2w[4 * k + 1], 0.0f - c.c2w[4 * k + 2]));
-                    x[k] = fmaf(dk, tt, c.c2w[4 * k + 3]);
-                }
-            } else if (live) {
-                const long long ray = ray0 + ray_l, smpl = row0 + tid;
-                if (p.ray_f64) {
-                    const double *o = reinterpret_cast<const double *>(p.rays_o) + ray * 3;
-                    const double *d = reinterpret_cast<const double *>(p.rays_d) + ray * 3;
-                    const double *tv = reinterpret_cast<const double *>(p.tvals) + smpl;
-                    const double tt = __ldg(tv);
-                    my_dist = smp + 1 < S ? (float)(__ldg(tv + 1) - tt) : 1e8f;
-#pragma unroll
-                    for (int c = 0; c < 3; ++c) x[c] = (float)(__ldg(o + c) + __ldg(d + c) * tt);
-                } else {
-                    const float *o = reinterpret_cast<const float *>(p.rays_o) + ray * 3;
-                    const float *d = reinterpret_cast<const float *>(p.rays_d) + ray * 3;
-                    const float *tv = reinterpret_cast<const float *>(p.tvals) + smpl;
-                    const float tt = __ldg(tv);
-                    my_dist = smp + 1 < S ? __ldg(tv + 1) - tt : 1e8f;
-#pragma unroll
-                    for (int c = 0; c < 3; ++c) x[c] = fmaf(__ldg(d + c), tt, __ldg(o + c));
-                }
-            }
+            // ---- features from rays: the positional encoding, written straight into A_0
             float sn[3], cs[3];
 #pragma unroll
             for (int c = 0; c < 3; ++c) pe_sincos(x[c], &sn[c], &cs[c]);
             if (dw_pending) { mbar_wait(bar_dw, dwphase); dwphase ^= 1; dw_pending = false; tc_fence_after(); }
             CLK(12);
-            // feature f = 3 * slot + coord: x0 x1 | x2 s0 | s1 s2 | c0 c1 | c2 s0' | ... as bf16 pairs (pair j = features 2j, 2j+1);
-            // band i fills pairs 1+3i .. 3+3i and leaves its last cosine pending; the ones column (feature 3 + 6E, odd) closes the
-            // pending pair.  Four pairs make this row's 16 bytes of a slab, stored as soon as they are complete.
-            {
-                uint8_t *const a0 = a_buf(0);
-                const int live_slabs = (c_in + 8) >> 3;
-                uint32_t q4[4] = {pack_bf16(x[0], x[1]), 0u, 0u, 0u};
-                float pend = x[2];
-                bool closed = false;
-                auto put = [&](int j, uint32_t v) {            // j is a compile-time constant at every call site
-                    q4[j & 3] = v;
-                    if ((j & 3) == 3) { if ((j >> 2) < live_slabs) *row_ptr(a0, j >> 2) = make_uint4(q4[0], q4[1], q4[2], q4[3]); q4[0] = q4[1] = q4[2] = q4[3] = 0u; }
-                };
-                // warp-uniform branches: the bands that are off cost nothing
-#pragma unroll
-                for (int i = 0; i < 10; ++i) {
-                    if (i < p.pe_bands) {
-                        put(1 + 3 * i, pack_bf16(pend, sn[0]));
-                        put(2 + 3 * i, pack_bf16(sn[1], sn[2]));
-                        put(3 + 3 * i, pack_bf16(cs[0], cs[1]));
-                        pend = cs[2];
-#pragma unroll
-                        for (int c = 0; c < 3; ++c) {
-                            const float s2 = 2.0f * sn[c] * cs[c], c2 = fmaf(-2.0f * sn[c], sn[c], 1.0f);
-                            sn[c] = s2; cs[c] = c2;
-                        }
-                    } else {
-                        if (closed && ((1 + 3 * i) >> 2) >= live_slabs) break;   // no live slab left to store (slab 7 then is not live either)
-                        put(1 + 3 * i, closed ? 0u : pack_bf16(pend, 1.0f));
-                        put(2 + 3 * i, 0u);
-                        put(3 + 3 * i, 0u);
-                        closed = true;
-                    }
-                }
-                put(31, closed ? 0u : pack_bf16(pend, 1.0f));
-            }
+            pack_pe(x, sn, cs, p.pe_bands, a0s, store_a0);
         } else {
-            // ---- features: wait for the TMA, convert this thread's row to bf16 slabs.  Columns beyond
-            // c_in read the following floats of `stage` (finite: next row / zeroed slack) and meet zero
-            // weights; column c_in is then patched to 1 (the bias-gradient feature).
+            // ---- features: wait for the TMA, convert this thread's row to bf16 slabs
             int lead; uint32_t bytes;
-            (void)x_src(tile, lead, bytes);
+            (void)x_src(p, tile, c_in, lead, bytes);
             mbar_wait(bar_x, xphase);
             xphase ^= 1;
             CLK(0);
             if (dw_pending) { mbar_wait(bar_dw, dwphase); dwphase ^= 1; dw_pending = false; tc_fence_after(); }
             CLK(12);
-            uint8_t *a0 = a_buf(0);
-            const float *xr = stage + lead + tid * c_in;
-            const int live_slabs = (c_in + 8) >> 3; // slabs containing features 0..c_in (incl. the ones column)
-            if (tid < valid) {
-                for (int c8 = 0; c8 < live_slabs; ++c8) {
-                    float f[8];
-#pragma unroll
-                    for (int j = 0; j < 8; ++j) f[j] = xr[c8 * 8 + j];
-                    *row_ptr(a0, c8) = make_uint4(pack_bf16(f[0], f[1]), pack_bf16(f[2], f[3]), pack_bf16(f[4], f[5]), pack_bf16(f[6], f[7]));
-                }
-            } else {
-                for (int c8 = 0; c8 < live_slabs; ++c8) *row_ptr(a0, c8) = make_uint4(0, 0, 0, 0);
-            }
-            __syncwarp();
-            reinterpret_cast<__nv_bfloat16 *>(a0)[(c_in >> 3) * (TILE * 8) + tid * 8 + (c_in & 7)] = __float2bfloat16_rn(1.0f);
+            pack_features(stage + lead + tid * c_in, c_in, tid < valid, store_a0);
         }
         publish_smem(); // also: every thread is done reading `stage`
         CLK(1);
@@ -658,7 +804,7 @@ __global__ void __launch_bounds__(TILE, FWD ? (HP == 64 ? 4 : 8) : 1) fused_v1_k
             *next_tile_s = nt;
             if (!RAYS && nt < p.n_tiles) {
                 int lead; uint32_t bytes;
-                const void *src = x_src(nt, lead, bytes);
+                const void *src = x_src(p, nt, c_in, lead, bytes);
                 mbar_expect_tx(bar_x, bytes);
                 bulk_g2s(smem_u32(stage), src, bytes, bar_x);
             }
@@ -666,12 +812,8 @@ __global__ void __launch_bounds__(TILE, FWD ? (HP == 64 ? 4 : 8) : 1) fused_v1_k
         // ---- forward
         float hz[4];
         for (int l = 0; l < L; ++l) {
-            if (tid == 0) issue_stage(l);
+            if (tid == 0) issue_stage(l, 0u);
             CLK(2);
-#ifdef LNB_TC_ISSUE_TWICE
-            if (tid == 0) issue_stage(l);
-            CLK(6);
-#endif
             commit_and_wait();
             CLK(3);
             const float *bl = bias_s + l * HP;
@@ -697,7 +839,7 @@ __global__ void __launch_bounds__(TILE, FWD ? (HP == 64 ? 4 : 8) : 1) fused_v1_k
                 }
                 CLK(4);
                 if (FWD) {              // nothing went to shared memory: the activations are in tensor memory
-                    tmem_st_wait_();
+                    tmem_st_wait();
                     tc_fence_before();
                     __syncthreads();
                     tc_fence_after();
@@ -714,119 +856,16 @@ __global__ void __launch_bounds__(TILE, FWD ? (HP == 64 ? 4 : 8) : 1) fused_v1_k
         }
         CLK(16);
         // ---- head + loss + adjoint of the head's pre-activation (unit seed)
-        float dz[4] = {0.f, 0.f, 0.f, 0.f};
-        if (p.head == LNB_HEAD_SIGMOID) {
-            // mlp_fit: row r <-> target row (scripts/mlp_fit.py:121-145)
-            if (tid < valid && row0 + tid < p.R) {
-                const float *tg = p.target + (row0 + tid) * p.Wt;
-                for (int c = 0; c < p.Wt && c < 4; ++c) {
-                    float y = sigmoid_f(hz[c]);
-                    float d = y - __ldg(tg + c);
-                    loss_acc = fmaf(d, d, loss_acc);
-                    dz[c] = 2.0f * d * (y * (1.0f - y));
-                }
-            }
-        } else {
-            // Compositing with one thread per sample (thread r <-> sample r of the tile): segmented
-            // warp-shuffle scans inside each warp, carries across the 4 warps through shared
-            // memory.  scripts/nerf.py:176-288 and its reverse (SURVEY.md Appendix B).
-            const float cr = sigmoid_f(hz[0]), cg = sigmoid_f(hz[1]), cb = sigmoid_f(hz[2]);
-            const float sg = fmaxf(hz[3], 0.0f);
-            const float e = __expf((0.0f - sg) * my_dist);
-            const float a = 1.0f - e;
-            const float qv = live ? (1.0f - a) + 1e-10f : 1.0f;
-            float pr = qv;                                   // segmented inclusive product
-#pragma unroll
-            for (int d = 1; d < 32; d <<= 1) {
-                float o = __shfl_up_sync(0xffffffffu, pr, d);
-                if (lane >= d && smp >= d) pr *= o;
-            }
-            if (lane == 31) { tailp[warp] = pr; tail_s[warp] = smp; }
-            if (lane == 0) headq[warp] = qv;
-            if (live && smp == 0) {
-                color_s[ray_l * 3] = 0.f; color_s[ray_l * 3 + 1] = 0.f; color_s[ray_l * 3 + 2] = 0.f;
-                tgt_s[ray_l * 3] = tg0; tgt_s[ray_l * 3 + 1] = tg1; tgt_s[ray_l * 3 + 2] = tg2;
-            }
-            CLK(17);
-            __syncthreads();
-            CLK(18);
-            float carry = 1.0f;                              // product of this ray's samples in earlier warps
-            if (smp > lane) {
-                for (int w2 = warp - 1; w2 >= 0; --w2) {
-                    carry *= tailp[w2];
-                    if (tail_s[w2] < 32) break;              // that warp's last segment started inside it
-                }
-            }
-            const float Cpre = pr * carry;                   // true inclusive product prod_{k<=s} q_k
-            const float T = (smp == 0) ? 1.0f : Cpre;
-            const float wgt = a * T;
-            {   // colour: segmented inclusive sums, one shared-memory atomic per (warp, ray) segment
-                float s0 = live ? wgt * cr : 0.f, s1 = live ? wgt * cg : 0.f, s2 = live ? wgt * cb : 0.f;
-#pragma unroll
-                for (int d = 1; d < 32; d <<= 1) {
-                    float o0 = __shfl_up_sync(0xffffffffu, s0, d), o1 = __shfl_up_sync(0xffffffffu, s1, d), o2 = __shfl_up_sync(0xffffffffu, s2, d);
-                    if (lane >= d && smp >= d) { s0 += o0; s1 += o1; s2 += o2; }
-                }
-                if (live && (lane == 31 || smp == S - 1)) {
-                    atomicAdd(color_s + ray_l * 3, s0); atomicAdd(color_s + ray_l * 3 + 1, s1); atomicAdd(color_s + ray_l * 3 + 2, s2);
-                }
-            }
-            CLK(19);
-            __syncthreads();
-            CLK(20);
-            float dc0 = 0.f, dc1 = 0.f, dc2 = 0.f;
-            if (live) {
-                const float c0 = color_s[ray_l * 3], c1 = color_s[ray_l * 3 + 1], c2 = color_s[ray_l * 3 + 2];
-                if (smp == 0 && p.color) {
-                    float *co = p.color + (size_t)(ray0 + ray_l) * 3;
-                    co[0] = c0; co[1] = c1; co[2] = c2;
-                }
-                if (p.target) {
-                    const float d0 = c0 - tgt_s[ray_l * 3], d1 = c1 - tgt_s[ray_l * 3 + 1], d2 = c2 - tgt_s[ray_l * 3 + 2];
-                    if (smp == 0) loss_acc += d0 * d0 + d1 * d1 + d2 * d2;
-                    dc0 = 2.0f * d0; dc1 = 2.0f * d1; dc2 = 2.0f * d2;
-                }
-            }
-            if (!FWD && p.target) {
-                // G_s = dT_s + q_{s+1} G_{s+1}: suffix scan of affine maps; B = 0 at a ray's last sample
-                const float d_w = cr * dc0 + cg * dc1 + cb * dc2;
-                const float dT = (smp == 0 || !live) ? 0.0f : d_w * a;
-                float qn = __shfl_down_sync(0xffffffffu, qv, 1);
-                if (lane == 31) qn = warp < 3 ? headq[warp + 1] : 0.0f;
-                float Aa = dT, Bb = (live && smp + 1 < S) ? qn : 0.0f;
-#pragma unroll
-                for (int d = 1; d < 32; d <<= 1) {
-                    float A2 = __shfl_down_sync(0xffffffffu, Aa, d);
-                    float B2 = __shfl_down_sync(0xffffffffu, Bb, d);
-                    if (lane + d < 32) { Aa = fmaf(Bb, A2, Aa); Bb = Bb * B2; }
-                }
-                if (lane == 0) { headA[warp] = Aa; headB[warp] = Bb; }
-                CLK(21);
-                __syncthreads();
-                CLK(22);
-                float Gn = 0.0f;                             // G at lane 0 of the next warp
-                for (int w2 = 3; w2 > warp; --w2) Gn = fmaf(headB[w2], Gn, headA[w2]);
-                const float Gv = fmaf(Bb, Gn, Aa);
-                float Cm1 = __shfl_up_sync(0xffffffffu, Cpre, 1);
-                if (lane == 0) Cm1 = carry;
-                if (smp == 0) Cm1 = 1.0f;
-                const float d_alpha = d_w * T - Cm1 * Gv;
-                if (live) {
-                    dz[0] = (wgt * dc0) * (cr * (1.0f - cr));
-                    dz[1] = (wgt * dc1) * (cg * (1.0f - cg));
-                    dz[2] = (wgt * dc2) * (cb * (1.0f - cb));
-                    dz[3] = sg > 0.0f ? d_alpha * e * my_dist : 0.0f;
-                }
-            }
-        }
-        CLK(23);
+        float dz[4];
+        head_and_composite<!FWD>(p, scratch, 0, hz, my_dist, tg, row0, ray0, valid, tid, smp, ray_l, live, loss_acc, dz);
+        CLK(17);
         if (FWD) { __syncthreads(); tile = *next_tile_s; continue; }
         // ---- backward.  dZ_{L-1}: 4 live features, the rest of the 16 stay zero
         *row_ptr(dz_buf(L - 1), 0) = make_uint4(pack_bf16(dz[0], dz[1]), pack_bf16(dz[2], dz[3]), 0u, 0u);
         publish_smem();
         CLK(7);
         for (int l = L - 1; l >= 1; --l) {
-            if (tid == 0) issue_stage(L + l);
+            if (tid == 0) issue_stage(L + l, 0u);
             CLK(8);
             commit_and_wait();
             CLK(9);
@@ -838,25 +877,17 @@ __global__ void __launch_bounds__(TILE, FWD ? (HP == 64 ? 4 : 8) : 1) fused_v1_k
 #pragma unroll
             for (int c8 = 0; c8 < HP / 8; ++c8) hm[c8] = *row_ptr(al, c8);
             tmem_ld_wait();
+            uint4 oz[HP / 8];
+            relu_adjoint<HP>(v, hm, oz);
 #pragma unroll
-            for (int c8 = 0; c8 < HP / 8; ++c8) {
-                // ReLU mask: bf16 post-ReLU values are >= 0, so positive <=> non-zero halfword
-                const uint32_t hw[4] = {hm[c8].x, hm[c8].y, hm[c8].z, hm[c8].w};
-                uint32_t o[4];
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    const int e = (c8 & 1) * 8 + 2 * j;
-                    o[j] = pack_bf16(__uint_as_float(v[c8 >> 1][e]), __uint_as_float(v[c8 >> 1][e + 1])) & gt0_mask_bf16x2(hw[j]);
-                }
-                *row_ptr(dzn, c8) = make_uint4(o[0], o[1], o[2], o[3]);
-            }
+            for (int c8 = 0; c8 < HP / 8; ++c8) *row_ptr(dzn, c8) = oz[c8];
             CLK(10);
             publish_smem();
             CLK(11);
         }
         // all dZ_l are in shared memory: the weight-gradient MMAs run in the background; their
         // completion is awaited only before A_0 is overwritten by the next tile (or at the end)
-        if (tid == 32) { issue_stage(2 * L); umma_commit(bar_dw); } // warp 1 issues; warp 0 moves on
+        if (tid == 32) { issue_stage(2 * L, dw_started ? 1u : 0u); umma_commit(bar_dw); } // warp 1 issues; warp 0 moves on
         dw_pending = true;
         CLK(13);
         tile = *next_tile_s; // written before this tile's forward; several block barriers ago
@@ -916,24 +947,6 @@ __global__ void __launch_bounds__(TILE, FWD ? (HP == 64 ? 4 : 8) : 1) fused_v1_k
 }
 
 #include "fused_mg.cuh"
-
-// image offset (bytes) of weight (l, k, j) / the fp32 bias region, mirroring tc_prep_kernel
-struct ImgMap {
-    int L, HP, K0P;
-    int dims[MAXL + 1];
-    __device__ int np(int l) const { return l < L - 1 ? HP : 16; }
-    __device__ int kp(int l) const { return l == 0 ? K0P : HP; }
-    __device__ int w_off(int l) const { int o = 0; for (int i = 0; i < l; ++i) o += np(i) * kp(i) * 2; return o; }
-    __device__ void put_w(uint8_t *img, int l, int k, int j, float v) const
-    {
-        reinterpret_cast<__nv_bfloat16 *>(img + w_off(l))[(k >> 3) * (np(l) * 8) + j * 8 + (k & 7)] = __float2bfloat16_rn(v);
-    }
-    __device__ void put_b(uint8_t *img, int l, int j, float v) const
-    {
-        if (l < L - 1) put_w(img, l, dims[l], j, v);                          // hidden layers: bias row of the MMA operand
-        else reinterpret_cast<float *>(img + w_off(L))[l * HP + j] = v;     // head: fp32
-    }
-};
 
 struct AdamArgs {
     float *param, *m, *v;
@@ -998,6 +1011,19 @@ __device__ __forceinline__ unsigned ld_acquire_sys(const unsigned *p)
     return v;
 }
 
+// element e0 of a partial's gradient block (the loss before it not counted): layer l, input row k (k == dims[l]: the
+// bias), output column j, and its index `off` in the padded ws block (is_w) or bs block
+struct PartElem { int l, k, j; bool is_w; long long off; };
+__device__ __forceinline__ PartElem part_elem(const TcParams &p, int e0)
+{
+    int e = e0 + 1, l = 0;
+    while (l + 1 < p.L && e >= p.part_off[l + 1]) ++l;
+    e -= p.part_off[l];
+    const int out_l = p.dims[l + 1], k = e / out_l, j = e % out_l;
+    const bool is_w = k < p.dims[l];
+    return PartElem{l, k, j, is_w, is_w ? ((long long)l * p.max_in + k) * p.max_out + j : (long long)l * p.max_out + j};
+}
+
 // reduce the per-CTA partials in a fixed order; apply the seed; accumulate into (or overwrite) the
 // caller's buffers; optionally apply Adam to the parameter and refresh the bf16 weight image
 __global__ void __launch_bounds__(1024) tc_reduce_kernel(const float *__restrict__ part, int n_part, int part_stride, TcParams p,
@@ -1007,8 +1033,8 @@ __global__ void __launch_bounds__(1024) tc_reduce_kernel(const float *__restrict
 {
     __shared__ float sloss;
     __shared__ AdamScalars s_adam;
-    asm volatile("griddepcontrol.wait;" ::: "memory");              // the fused kernel's partials are complete
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); // the next step may start its prologue
+    pdl_wait();      // the fused kernel's partials are complete
+    pdl_trigger();   // the next step may start its prologue
     // Three things run side by side, one barrier at the end: warp 31 sums the loss partials (every block itself, same order
     // everywhere, so the seed needs no second pass), one thread of warp 30 derives the Adam scalars (two double-precision
     // pow()), warps 0-29 gather the gradient partials: 32 consecutive elements per block (one coalesced 128 B line per
@@ -1019,20 +1045,14 @@ __global__ void __launch_bounds__(1024) tc_reduce_kernel(const float *__restrict
     const int e_glob = blockIdx.x * 32 + el;
     // the element this thread of warp 0 will update: its parameter and moments are fetched now, under the gather
     const bool mine_el = grp == 0 && e_glob < n_el && d_ws;
-    int ml = 0, mk = 0, mj = 0;
-    bool m_is_w = false;
+    PartElem me{};
     long long m_pi = 0;
     float *m_dst = nullptr;
     float pf_p = 0.0f, pf_m = 0.0f, pf_v = 0.0f, pf_d = 0.0f;
     if (mine_el) {
-        int e = e_glob + 1;
-        while (ml + 1 < p.L && e >= p.part_off[ml + 1]) ++ml;
-        e -= p.part_off[ml];
-        const int out_l = p.dims[ml + 1];
-        mk = e / out_l; mj = e % out_l;
-        m_is_w = mk < p.dims[ml];
-        m_dst = m_is_w ? d_ws + ((size_t)ml * p.max_in + mk) * p.max_out + mj : d_bs + (size_t)ml * p.max_out + mj;
-        m_pi = m_is_w ? ((long long)ml * p.max_in + mk) * p.max_out + mj : ad.n_w + (long long)ml * p.max_out + mj;
+        me = part_elem(p, e_glob);
+        m_dst = (me.is_w ? d_ws : d_bs) + me.off;
+        m_pi = me.is_w ? me.off : ad.n_w + me.off;
         if (!overwrite) pf_d = *m_dst;
         if (fuse_adam) { pf_p = ad.param[m_pi]; if (!ad.sgd) { pf_m = ad.m[m_pi]; pf_v = ad.v[m_pi]; } }
     }
@@ -1141,7 +1161,7 @@ __global__ void __launch_bounds__(1024) tc_reduce_kernel(const float *__restrict
         *m_dst = g;
         if (fuse_adam) {
             const float pn = adam_one(ad, m_pi, g, s_adam, pf_p, pf_m, pf_v);
-            if (ad.wimg) { if (m_is_w) im.put_w(ad.wimg, ml, mk, mj, pn); else im.put_b(ad.wimg, ml, mj, pn); }
+            if (ad.wimg) { if (me.is_w) im.put_w(ad.wimg, me.l, me.k, me.j, pn); else im.put_b(ad.wimg, me.l, me.j, pn); }
         }
     }
 }
@@ -1151,26 +1171,26 @@ __global__ void tc_adam_img_kernel(TcParams p, const float *__restrict__ grad, A
 {
     const int e0 = blockIdx.x * blockDim.x + threadIdx.x;
     if (e0 >= n_el) return;
-    int e = e0 + 1, l = 0;
-    while (l + 1 < p.L && e >= p.part_off[l + 1]) ++l;
-    e -= p.part_off[l];
-    const int out_l = p.dims[l + 1], k = e / out_l, j = e % out_l;
-    const bool is_w = k < p.dims[l];
-    const long long pi = is_w ? ((long long)l * p.max_in + k) * p.max_out + j : ad.n_w + (long long)l * p.max_out + j;
+    const PartElem me = part_elem(p, e0);
+    const long long pi = me.is_w ? me.off : ad.n_w + me.off;
     const float pn = adam_one(ad, pi, grad[pi], adam_scalars(ad), ad.param[pi], ad.sgd ? 0.0f : ad.m[pi], ad.sgd ? 0.0f : ad.v[pi]);
-    if (ad.wimg) { if (is_w) im.put_w(ad.wimg, l, k, j, pn); else im.put_b(ad.wimg, l, j, pn); }
+    if (ad.wimg) { if (me.is_w) im.put_w(ad.wimg, me.l, me.k, me.j, pn); else im.put_b(ad.wimg, me.l, me.j, pn); }
 }
 
-int tc_pick(const lnb_mlp *mlp, int *HP, int *K0P)
+// the padded widths of the fused kernels for this MLP: HP (hidden width + the ones feature, 16 / 32 / 64) and K0P (input
+// width + the ones feature, a multiple of 16).  Returns NULL, or why the MLP does not fit the fused kernels.
+const char *tc_pick(const lnb_mlp *mlp, int *HP, int *K0P)
 {
     const int L = mlp->n_layers;
-    if (L < 2 || L > MAXL) return 0;
+    if (L < 2 || L > MAXL) return "needs 2..4 layers";
     int hw = 0;
     for (int l = 1; l < L; ++l) hw = mlp->dims[l] > hw ? mlp->dims[l] : hw;
     *HP = hw + 1 <= 16 ? 16 : (hw + 1 <= 32 ? 32 : (hw + 1 <= 64 ? 64 : 0));
     *K0P = (mlp->dims[0] + 1 + 15) / 16 * 16;
-    if (!*HP || *K0P > 64 || mlp->dims[L] > 16) return 0;
-    return 1;
+    if (!*HP) return "hidden width + 1 must be <= 64";
+    if (*K0P > 64) return "input width + 1 must be <= 64";
+    if (mlp->dims[L] > 16) return "more than 16 output channels";
+    return nullptr;
 }
 
 void fill_layout(TcParams &p, const lnb_mlp *mlp, int K0P)
@@ -1185,30 +1205,44 @@ void fill_layout(TcParams &p, const lnb_mlp *mlp, int K0P)
     p.part_stride = off;
 }
 
+ImgMap img_map(const lnb_mlp *mlp, int HP, int K0P)
+{
+    ImgMap im{mlp->n_layers, HP, K0P, {}};
+    for (int l = 0; l <= mlp->n_layers; ++l) im.dims[l] = mlp->dims[l];
+    return im;
+}
+
+// f(std::integral_constant<int, HP>()) for a padded hidden width HP of 16, 32 or 64: the kernels and their layouts are
+// compiled per width
+template <class F>
+auto with_hp(int HP, F &&f)
+{
+    if (HP == 16) return f(std::integral_constant<int, 16>());
+    if (HP == 32) return f(std::integral_constant<int, 32>());
+    return f(std::integral_constant<int, 64>());
+}
+
 } // namespace
 
 // Returns LNB_ERR_UNSUPPORTED when the problem does not fit the fused tensor-core kernel.
 int lnb_tc_layout(const lnb_mlp *mlp, int *HP, int *K0P, int *wimg_bytes)
 {
     int hp = 0, k0p = 0;
-    if (!tc_pick(mlp, &hp, &k0p)) return 0;
-    const int L = mlp->n_layers;
+    if (tc_pick(mlp, &hp, &k0p)) return 0;
     if (HP) *HP = hp;
     if (K0P) *K0P = k0p;
-    if (wimg_bytes) *wimg_bytes = hp == 16 ? TcLayout<16>::wimg_bytes(L, k0p) : (hp == 32 ? TcLayout<32>::wimg_bytes(L, k0p) : TcLayout<64>::wimg_bytes(L, k0p));
+    if (wimg_bytes) *wimg_bytes = img_map(mlp, hp, k0p).bytes();
     return 1;
 }
 
 int lnb_tc_prep(lnb_ctx *ctx, const lnb_mlp *mlp, const float *ws, const float *bs, void *wimg)
 {
     int HP = 0, K0P = 0;
-    if (!tc_pick(mlp, &HP, &K0P)) { ctx->err = "fused tensor-core path: MLP shape not supported"; return LNB_ERR_UNSUPPORTED; }
+    if (tc_pick(mlp, &HP, &K0P)) { ctx->err = "fused tensor-core path: MLP shape not supported"; return LNB_ERR_UNSUPPORTED; }
     TcParams p{};
     fill_layout(p, mlp, K0P);
     p.ws = ws; p.bs = bs;
-    if (HP == 16) tc_prep_kernel<16><<<1, 256, 0, ctx->stream>>>(p, (uint8_t *)wimg);
-    else if (HP == 32) tc_prep_kernel<32><<<1, 256, 0, ctx->stream>>>(p, (uint8_t *)wimg);
-    else tc_prep_kernel<64><<<1, 256, 0, ctx->stream>>>(p, (uint8_t *)wimg);
+    tc_prep_kernel<<<1, 256, 0, ctx->stream>>>(p, img_map(mlp, HP, K0P), (uint8_t *)wimg);
     LNB_CHECK_LAUNCH();
     return LNB_OK;
 }
@@ -1217,14 +1251,12 @@ int lnb_tc_adam_img(lnb_ctx *ctx, const lnb_mlp *mlp, float *param, const float 
                     const int *t_dev, double lr, double b1, double b2, double eps, void *wimg)
 {
     int HP = 0, K0P = 0;
-    if (!tc_pick(mlp, &HP, &K0P)) { ctx->err = "fused tensor-core path: MLP shape not supported"; return LNB_ERR_UNSUPPORTED; }
+    if (tc_pick(mlp, &HP, &K0P)) { ctx->err = "fused tensor-core path: MLP shape not supported"; return LNB_ERR_UNSUPPORTED; }
     TcParams p{};
     fill_layout(p, mlp, K0P);
     AdamArgs ad{param, m, v, t_dev, lr, b1, b2, eps, (uint8_t *)wimg, (long long)mlp->n_layers * mlp->max_in * mlp->max_out, m == nullptr};
-    ImgMap im{mlp->n_layers, HP, K0P, {}};
-    for (int l = 0; l <= mlp->n_layers; ++l) im.dims[l] = mlp->dims[l];
     const int n_el = p.part_stride - 1;
-    tc_adam_img_kernel<<<(n_el + 255) / 256, 256, 0, ctx->stream>>>(p, grad, ad, im, n_el);
+    tc_adam_img_kernel<<<(n_el + 255) / 256, 256, 0, ctx->stream>>>(p, grad, ad, img_map(mlp, HP, K0P), n_el);
     LNB_CHECK_LAUNCH();
     return LNB_OK;
 }
@@ -1236,14 +1268,8 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
         ctx->err = std::string("fused tensor-core path: ") + why;
         return LNB_ERR_UNSUPPORTED;
     };
-    if (L < 2 || L > MAXL) return unsupported("needs 2..4 layers");
-    int hw = 0;
-    for (int l = 1; l < L; ++l) hw = mlp->dims[l] > hw ? mlp->dims[l] : hw;
-    const int HP = hw + 1 <= 16 ? 16 : (hw + 1 <= 32 ? 32 : (hw + 1 <= 64 ? 64 : 0));
-    if (!HP) return unsupported("hidden width + 1 must be <= 64");
-    const int K0P = (mlp->dims[0] + 1 + 15) / 16 * 16;
-    if (K0P > 64) return unsupported("input width + 1 must be <= 64");
-    if (mlp->dims[L] > 16) return unsupported("more than 16 output channels");
+    int HP = 0, K0P = 0;
+    if (const char *why = tc_pick(mlp, &HP, &K0P)) return unsupported(why);
     if (a->inter || a->rgba || a->alpha || a->cumprod || a->weights || a->d_X || a->d_target || a->d_dists ||
         a->d_color || a->d_inter)
         return unsupported("only loss, colour, d_ws and d_bs are produced (use the fp32 path for the rest)");
@@ -1263,6 +1289,7 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
     if (cudaSetDevice(ctx->device) != cudaSuccess) return LNB_ERR_CUDA;
 
     TcParams p{};
+    fill_layout(p, mlp, K0P);
     p.X = a->X; p.dists = a->dists; p.target = a->target; p.ws = a->ws; p.bs = a->bs;
     p.rays_o = a->rays_o; p.rays_d = a->rays_d; p.tvals = a->t; p.ray_f64 = a->ray_dtype == LNB_RAY_F64; p.pe_bands = a->pe_bands;
     if (cam) {
@@ -1280,14 +1307,7 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
     p.G = nerf ? TILE / S : TILE;
     p.rows_per_tile = p.G * S;
     p.n_tiles = (int)((N + p.rows_per_tile - 1) / p.rows_per_tile);
-    p.L = L;
-    for (int l = 0; l <= L; ++l) p.dims[l] = mlp->dims[l];
-    p.max_in = mlp->max_in; p.max_out = mlp->max_out;
-    p.K0P = K0P;
     p.head = mlp->head; p.want_grad = a->want_grad; p.Wt = a->target_w > 0 ? a->target_w : 3;
-    int off = 1;
-    for (int l = 0; l < L; ++l) { p.part_off[l] = off; off += (mlp->dims[l] + 1) * mlp->dims[l + 1]; }
-    p.part_stride = off;
 
     const int c_in = mlp->dims[0];
     const bool grad = a->want_grad != 0;
@@ -1299,25 +1319,26 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
         if (K0P / 8 + (L - 1) * (HP / 8) > 16) return unsupported("input + hidden widths exceed 128 features in total");
         if ((L - 1) * HP + 16 > 256) return unsupported("hidden widths exceed 256 gradient columns");
     }
+    void (*const kern)(TcParams) = with_hp(HP, [&](auto hp) -> void (*)(TcParams) {
+        constexpr int H = decltype(hp)::value;
+        if (mg) return rays ? fused_mg_kernel<true, H> : fused_mg_kernel<false, H>;
+        if (grad) return rays ? fused_v1_kernel<true, H, false> : fused_v1_kernel<false, H, false>;
+        return rays ? fused_v1_kernel<true, H, true> : fused_v1_kernel<false, H, true>;
+    });
     size_t smem = 0;
     int grid = 0, ng = 1;
-    const void *mg_fn = nullptr;
     if (mg) {
-#define LNB_MG_PICK(HPV)                                                                                         \
-    do {                                                                                                         \
-        mg_fn = rays ? (const void *)fused_mg_kernel<true, HPV> : (const void *)fused_mg_kernel<false, HPV>;     \
-        ng = mg_max_groups<HPV>();                                                                               \
-        while (ng > 1 && (MgLayout<HPV>::total(L, c_in, K0P, rays, ng) > 232448 || MgLayout<HPV>::tmem_need(L, K0P, ng) > 512)) --ng; \
-    } while (0)
-        if (HP == 16) LNB_MG_PICK(16);
-        else if (HP == 32) LNB_MG_PICK(32);
-        else LNB_MG_PICK(64);
-#undef LNB_MG_PICK
+        ng = with_hp(HP, [&](auto hp) {
+            using MG = MgLayout<decltype(hp)::value>;
+            int n = mg_max_groups<decltype(hp)::value>();
+            while (n > 1 && (MG::total(L, c_in, K0P, rays, n) > 232448 || MG::tmem_need(L, K0P, n) > 512)) --n;
+            return n;
+        });
         static int mg_regs[2][3] = {{0, 0, 0}, {0, 0, 0}};    // registers per thread of each instantiation, asked once
-        int &regs = mg_regs[rays ? 1 : 0][HP == 16 ? 0 : (HP == 32 ? 1 : 2)];
+        int &regs = mg_regs[rays ? 1 : 0][HP / 32];
         if (regs == 0) {
             cudaFuncAttributes fa;
-            LNB_CUDA(cudaFuncGetAttributes(&fa, mg_fn));
+            LNB_CUDA(cudaFuncGetAttributes(&fa, kern));
             regs = fa.numRegs;
         }
         while (ng > 1 && (long long)ng * TILE * ((regs + 7) / 8 * 8) > 65536) --ng;
@@ -1327,11 +1348,15 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
         grid = (p.n_tiles + ng - 1) / ng;
         if (grid > ctx->sm_count) grid = ctx->sm_count;
         if (grid < 1) grid = 1;
-        smem = HP == 16 ? MgLayout<16>::total(L, c_in, K0P, rays, ng) : (HP == 32 ? MgLayout<32>::total(L, c_in, K0P, rays, ng) : MgLayout<64>::total(L, c_in, K0P, rays, ng));
+        smem = with_hp(HP, [&](auto hp) { return MgLayout<decltype(hp)::value>::total(L, c_in, K0P, rays, ng); });
         if (smem > 232448) return unsupported("shared memory");
     } else {
-        smem = (HP == 16 ? TcLayout<16>::total(L, K0P, c_in, rays, grad) : (HP == 32 ? TcLayout<32>::total(L, K0P, c_in, rays, grad) : TcLayout<64>::total(L, K0P, c_in, rays, grad)));
-        const int tmem_cols = (int)(HP == 16 ? TcLayout<16>::tmem_cols(L, grad) : (HP == 32 ? TcLayout<32>::tmem_cols(L, grad) : TcLayout<64>::tmem_cols(L, grad)));
+        int tmem_cols = 0;
+        with_hp(HP, [&](auto hp) {
+            using LY = TcLayout<decltype(hp)::value>;
+            smem = LY::total(L, K0P, c_in, rays, grad);
+            tmem_cols = (int)LY::tmem_cols(L, grad);
+        });
         int per_sm = 512 / tmem_cols;
         int by_smem = (int)((228 * 1024) / (smem + 1024));
         if (by_smem < per_sm) per_sm = by_smem;
@@ -1341,7 +1366,8 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
         if (grid > p.n_tiles) grid = p.n_tiles;
         if (grid < 1) grid = 1;
     }
-    const int wimg_bytes = HP == 16 ? TcLayout<16>::wimg_bytes(L, K0P) : (HP == 32 ? TcLayout<32>::wimg_bytes(L, K0P) : TcLayout<64>::wimg_bytes(L, K0P));
+    const ImgMap im = img_map(mlp, HP, K0P);
+    const int wimg_bytes = im.bytes();
     LNB_TRY(lnb_arena_reserve(ctx, (size_t)grid * p.part_stride * sizeof(float) + wimg_bytes + 8192));
     p.part = (float *)lnb_arena_take(ctx, (size_t)grid * p.part_stride * sizeof(float));
     uint8_t *wimg = (uint8_t *)lnb_arena_take(ctx, wimg_bytes);
@@ -1364,36 +1390,21 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
     pdl_attr[0].val.programmaticStreamSerializationAllowed = 1;
     const bool use_pdl = getenv("LNB_NO_PDL") == nullptr;
     if (N > 0) {
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(mg ? ng * TILE : TILE); cfg.dynamicSmemBytes = smem; cfg.stream = ctx->stream;
-    cfg.attrs = pdl_attr; cfg.numAttrs = use_pdl ? 1 : 0;
-#define LNB_LAUNCH(KERNEL)                                                                        \
-    do {                                                                                         \
-        static size_t smem_set[64] = {};   /* per expansion = per kernel instantiation, per device: raise the limit only when it grows */ \
-        size_t &lim = smem_set[ctx->device & 63];                                                 \
-        if (smem > lim || ctx->device > 63) { LNB_CUDA(cudaFuncSetAttribute(KERNEL, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); lim = smem; } \
-        LNB_CUDA(cudaLaunchKernelEx(&cfg, KERNEL, p));                                           \
-    } while (0)
-#define LNB_TC(HPV)                                                                              \
-    do {                                                                                         \
-        if (mg) { if (rays) LNB_LAUNCH((fused_mg_kernel<true, HPV>)); else LNB_LAUNCH((fused_mg_kernel<false, HPV>)); } \
-        else if (grad) { if (rays) LNB_LAUNCH((fused_v1_kernel<true, HPV, false>)); else LNB_LAUNCH((fused_v1_kernel<false, HPV, false>)); } \
-        else { if (rays) LNB_LAUNCH((fused_v1_kernel<true, HPV, true>)); else LNB_LAUNCH((fused_v1_kernel<false, HPV, true>)); } \
-    } while (0)
+        cudaLaunchConfig_t cfg{};
+        cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(mg ? ng * TILE : TILE); cfg.dynamicSmemBytes = smem; cfg.stream = ctx->stream;
+        cfg.attrs = pdl_attr; cfg.numAttrs = use_pdl ? 1 : 0;
         if (!(ex && ex->wimg)) {
-            if (HP == 16) tc_prep_kernel<16><<<1, 256, 0, ctx->stream>>>(p, wimg);
-            else if (HP == 32) tc_prep_kernel<32><<<1, 256, 0, ctx->stream>>>(p, wimg);
-            else tc_prep_kernel<64><<<1, 256, 0, ctx->stream>>>(p, wimg);
+            tc_prep_kernel<<<1, 256, 0, ctx->stream>>>(p, im, wimg);
             LNB_CHECK_LAUNCH();
         }
+        // the dynamic shared-memory limit of each kernel instantiation (kind, input, HP) on each device: raised only when it grows
+        static size_t smem_set[3][2][3][64] = {};
+        size_t &lim = smem_set[mg ? 0 : (grad ? 1 : 2)][rays ? 1 : 0][HP / 32][ctx->device & 63];
+        if (smem > lim || ctx->device > 63) { LNB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); lim = smem; }
         lnb_prof_begin(ctx, mg ? (rays ? "fused_mg_kernel<rays>" : "fused_mg_kernel<features>")
                               : (rays ? "fused_v1_kernel<rays>" : "fused_v1_kernel<features>"));      // the symbols ncu lists
-        if (HP == 16) LNB_TC(16);
-        else if (HP == 32) LNB_TC(32);
-        else LNB_TC(64);
+        LNB_CUDA(cudaLaunchKernelEx(&cfg, kern, p));
         lnb_prof_end(ctx);
-#undef LNB_TC
-#undef LNB_LAUNCH
         LNB_CHECK_LAUNCH();
     } else {
         grid = 0;
@@ -1426,9 +1437,9 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
         } else if (++calls % 150 == 20) {
             double acc[24] = {0};
             for (int b = 0; b < grid; ++b) for (int i = 0; i < 24; ++i) acc[i] += h[(size_t)b * 24 + i];
-            const char *nm[24] = {"wait X", "convert+publish", "issue fwd", "wait fwd mma", "fwd epilogue", "fwd publish", "issue fwd AGAIN (experiment)", "dz publish",
+            const char *nm[24] = {"wait X", "convert+publish", "issue fwd", "wait fwd mma", "fwd epilogue", "fwd publish", "", "dz publish",
                                   "issue bwd", "wait bwd mma", "bwd epilogue", "bwd publish", "wait dW", "issue dW + final epilogue", "prologue", "loop top",
-                                  "head ld+bias", "comp: act+prodscan", "comp: sync1", "comp: carry+colour", "comp: sync2", "comp: dcol+affine", "comp: sync3", "comp: finish"};
+                                  "head ld+bias", "compositing", "", "", "", "", "", ""};
             double tot = 0; for (int i = 0; i < 24; ++i) tot += acc[i];
             fprintf(stderr, "[tc clk] grid %d tiles %d: cycles per tile (thread 0), total %.0f\n", grid, p.n_tiles, tot / p.n_tiles);
             {
@@ -1450,8 +1461,6 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
     const float seed_val = seed_is_loss ? 1.0f : a->seed;
     int blocks = a->want_grad ? (n_el + 31) / 32 : 1;
     AdamArgs ad{};
-    ImgMap im{L, HP, K0P, {}};
-    for (int l = 0; l <= L; ++l) im.dims[l] = mlp->dims[l];
     const int fuse = ex && ex->fuse_adam && a->want_grad;
     if (fuse) ad = AdamArgs{ex->param, ex->m, ex->v, ex->t_dev, ex->lr, ex->b1, ex->b2, ex->eps, (uint8_t *)ex->wimg_out,
                             (long long)L * mlp->max_in * mlp->max_out, ex->m == nullptr};

@@ -25,6 +25,7 @@
 #include <stdlib.h>
 
 #include "lnb_internal.h"
+#include "tc_ptx.cuh"
 
 namespace {
 
@@ -34,8 +35,6 @@ constexpr int GEMM_THREADS = 320; // warp 0 TMA, warp 1 MMA, warps 2..9 epilogue
                                   // scheduler cannot hide its own ALU latency, and the epilogue is the long pole)
 constexpr int DW_THREADS = 192;   // weight-gradient kernel: warp 0 TMA, warp 1 MMA, warps 2..5 column sums + epilogue
 
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) { asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count)); }
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity)
 {
     uint32_t done = 0;
@@ -54,7 +53,6 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity)
     }
 }
 __device__ __forceinline__ void mbar_arrive(uint32_t bar) { asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory"); }
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) { asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory"); }
 __device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap *map, int c0, int c1, uint32_t bar)
 {
     asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
@@ -79,21 +77,6 @@ __device__ __forceinline__ void tma_store_2d(const CUtensorMap *map, uint32_t sr
 }
 __device__ __forceinline__ void tma_store_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 __device__ __forceinline__ void tma_store_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tmem_alloc(uint32_t smem_dst, uint32_t cols)
-{
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_dst), "r"(cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t cols) { asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory"); }
-__device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate)
-{
-    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-                 ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) { asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory"); }
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32])
 {
     asm volatile(
@@ -105,21 +88,8 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32])
           "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
         : "r"(taddr) : "memory");
 }
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&v)[16])
-{
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
-          "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-        : "r"(taddr) : "memory");
-}
-// Programmatic dependent launch: a kernel launched with the attribute may start while its predecessor
-// drains; everything it reads that the predecessor wrote must come after pdl_wait().  Every kernel here
-// triggers its own dependents only AFTER its wait, so data from two or more launches back (weights,
-// biases) may be fetched before the wait.  Both are no-ops in a plain launch.
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+// Programmatic dependent launch (pdl_wait / pdl_trigger): every kernel here triggers its own dependents only AFTER its
+// wait, so data from two or more launches back (weights, biases) may be fetched before the wait.
 
 // UMMA shared-memory descriptor for a 128-byte-swizzled tile whose rows are 128 B (64 bf16) apart and
 // whose 8-row swizzle atoms are 1024 B apart (what a TMA box {64, rows} with SWIZZLE_128B writes).
@@ -131,16 +101,6 @@ __device__ __forceinline__ uint64_t sw128_desc(uint32_t addr, uint32_t lbo_bytes
 {
     return (uint64_t)((addr >> 4) & 0x3FFF) | ((uint64_t)((lbo_bytes >> 4) & 0x3FFF) << 16) |
            ((uint64_t)((sbo_bytes >> 4) & 0x3FFF) << 32) | (1ull << 46) | (2ull << 61);
-}
-__device__ __forceinline__ uint32_t instr_desc(int M, int N, int a_mn_major, int b_mn_major)
-{
-    return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)a_mn_major << 15) | ((uint32_t)b_mn_major << 16) |
-           ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-__device__ __forceinline__ uint32_t pack_bf16(float a, float b)
-{
-    __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
-    return *reinterpret_cast<uint32_t *>(&h);
 }
 
 enum { EPI_RELU_BF16 = 0,   // C = bf16(relu(acc + bias)), optionally + the ReLU pattern as bits

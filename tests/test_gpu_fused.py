@@ -59,6 +59,15 @@ def nerf_step(ctx, torch, case, path, seed=1.0, grad=True, outputs=("color", "lo
     return {k: host(v) for k, v in box["out"].items()}
 
 
+def rays_step(ctx, torch, case, grad=True):
+    out = ctx.nerf_step_rays([int(v) for v in case["dims"]], dev(torch, case["rays_o"], np.float64), dev(torch, case["rays_d"], np.float64),
+                             dev(torch, case["t"], np.float64), int(case["E"]), dev(torch, case["ws"]), dev(torch, case["bs"]),
+                             dev(torch, case["target"]) if grad else None, grad=grad, seed=1.0,
+                             outputs=("color", "loss") if grad else ("color",), path="tc")
+    ctx.synchronize()
+    return {k: host(v) for k, v in out.items()}
+
+
 # ------------------------------------------------------------------------------------------------
 # fused exact kernel
 # ------------------------------------------------------------------------------------------------
@@ -191,3 +200,7 @@ def test_multi_group_kernel_agrees_with_the_one_tile_per_cta_kernel(ctx, torch_c
         assert np.array_equal(o["color"], ref["color"]), ng
         assert rel_err(o["loss"][0], ref["loss"][0]) <= 1e-6
         assert rel_err(o["d_ws"], ref["d_ws"]) <= 1e-5 and rel_err(o["d_bs"], ref["d_bs"]) <= 1e-5, ng
+    # the forward-only (render) kernel computes the train step's colours to the bit, from features and from rays
+    fwd = nerf_step(ctx, torch, case, "tc", grad=False, outputs=("color",), expect_kernel="fused_v1_kernel")
+    assert np.array_equal(fwd["color"], ref["color"])
+    assert np.array_equal(rays_step(ctx, torch, case, grad=False)["color"], rays_step(ctx, torch, case)["color"])

@@ -4,8 +4,8 @@ Every forward MMA takes its A operand from tensor memory, the layer-0 one includ
 written as zeros).  These shapes reach what the shapes of test_gpu_fused.py do not: the widest first layer (63 input
 features + ones column, K0P = 64: all 32 A columns of a group live; seven groups and 496 of 512 tensor-memory columns from
 rays) and four layers at the 32-column width.  Each runs from features and from rays, against the float64 restatement
-within the bf16 bounds of test_gpu_fused.py, and its colours must be bit-equal to the one-tile-per-CTA kernel
-(LNB_TC_V1=1, A_0 from shared memory) wherever that kernel takes the shape.
+within the bf16 bounds of test_gpu_fused.py, and its colours must be bit-equal to the forward-only (render) kernel and to the
+one-tile-per-CTA train kernel (LNB_TC_V1=1, A_0 from shared memory) wherever that kernel takes the shape.
 """
 import os
 
@@ -13,7 +13,7 @@ import numpy as np
 import pytest
 
 from oracle import oracle as O
-from test_gpu_fused import dev, host, nerf_step, tc_check
+from test_gpu_fused import nerf_step, rays_step, tc_check
 
 pytestmark = pytest.mark.gpu
 
@@ -31,14 +31,6 @@ def ctx(torch_cuda):
     c = api.Context(0)
     yield c
     c.close()
-
-
-def rays_step(ctx, torch, case):
-    out = ctx.nerf_step_rays([int(v) for v in case["dims"]], dev(torch, case["rays_o"], np.float64), dev(torch, case["rays_d"], np.float64),
-                             dev(torch, case["t"], np.float64), int(case["E"]), dev(torch, case["ws"]), dev(torch, case["bs"]),
-                             dev(torch, case["target"]), grad=True, seed=1.0, outputs=("color", "loss"), path="tc")
-    ctx.synchronize()
-    return {k: host(v) for k, v in out.items()}
 
 
 def one_tile_per_cta(fn):
@@ -63,6 +55,9 @@ def test_multi_group_operands_against_f64_and_the_one_tile_per_cta_kernel(ctx, t
     tc_check(o, f)
     orays = rays_step(ctx, torch, case)
     tc_check(orays, f)
+    # the forward-only (render) kernel computes the train step's colours to the bit
+    assert np.array_equal(nerf_step(ctx, torch, case, "tc", grad=False, outputs=("color",))["color"], o["color"])
+    assert np.array_equal(rays_step(ctx, torch, case, grad=False)["color"], orays["color"])
     if v1:
         ref = one_tile_per_cta(lambda: nerf_step(ctx, torch, case, "tc"))
         ref_rays = one_tile_per_cta(lambda: rays_step(ctx, torch, case))
