@@ -13,8 +13,8 @@
 //                    tiles through all layers, the layer's weights in shared memory, the activations handed from
 //                    layer to layer through L2; tcgen05.mma (M = 128, N <= 256, K = 16) into
 //                    two TMEM accumulators, 16 epilogue warps (tcgen05.ld -> bias / ReLU + bit pattern / mask ->
-//                    bf16 -> swizzled staging -> TMA store).  The default.
-//   gemm_tc_kernel   the same GEMM + epilogues as one launch per layer (tests, ray slabs, LNB_WIDE_NO_CHAIN).
+//                    bf16 -> swizzled staging -> TMA store; or fp32 straight from registers on the last layer).
+//                    A chain of one layer is a single GEMM (the unit-test hooks, LNB_WIDE_NO_CHAIN).
 //   dw_tc_kernel     the weight gradient: the row-major bf16 activations read as MN-major operands (features
 //                    contiguous), a 256 x N product accumulated in TMEM over the CTA's share of the samples, the
 //                    column sums of dZ (the bias gradient) added up by the otherwise idle epilogue warps.
@@ -31,8 +31,6 @@ namespace {
 
 constexpr int BM = 128;     // rows (samples) per tile
 constexpr int BK = 64;      // K elements per pipeline stage = one 128-byte swizzle atom of bf16
-constexpr int GEMM_THREADS = 320; // warp 0 TMA, warp 1 MMA, warps 2..9 epilogue (two per TMEM lane quadrant: one warp per
-                                  // scheduler cannot hide its own ALU latency, and the epilogue is the long pole)
 constexpr int DW_THREADS = 192;   // weight-gradient kernel: warp 0 TMA, warp 1 MMA, warps 2..5 column sums + epilogue
 
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity)
@@ -105,219 +103,11 @@ __device__ __forceinline__ uint64_t sw128_desc(uint32_t addr, uint32_t lbo_bytes
 
 enum { EPI_RELU_BF16 = 0,   // C = bf16(relu(acc + bias)), optionally + the ReLU pattern as bits
        EPI_MASK_BF16 = 1,   // C = bf16(bit ? acc : 0)                 (ReLU adjoint, pattern from the forward pass)
-       EPI_HEAD_F32 = 2,    // C[row][0..3] = nerf/sigmoid head of (acc + bias), fp32 [M][4]
-       EPI_NONE_F32 = 3 };  // C = acc (+ bias) as fp32 [M][ldc]        (tests)
+       EPI_HEAD_F32 = 2,    // C[row][0..3] = nerf/sigmoid head of (acc + bias), fp32 [M][ldc]   (last layer only)
+       EPI_NONE_F32 = 3 };  // C = acc (+ bias) as fp32 [M][ldc]         (last layer only; the GEMM test hook)
 
 constexpr int MAX_A_STAGES = 8;
 constexpr int A_STAGE_BYTES = BM * BK * 2;   // 16 KB
-
-struct GemmParams {
-    int M, N, K;            // N multiple of 16 (<= 256), K multiple of 64 (<= 256)
-    const float *bias;      // [N] or NULL
-    // ReLU pattern, one bit per element, [M][ldbits] words; word w covers columns 32w .. 32w+31 and column
-    // 32w + 8g + 2j + p sits at bit 16p + 4g + j, so that the two flags of a packed bf16 pair are 16 bits
-    // apart: ((word >> (4g + j)) & 0x00010001) * 0xFFFF is the pair's AND-mask
-    const uint32_t *bits_in;   // EPI_MASK_BF16
-    uint32_t *bits_out;        // EPI_RELU_BF16: optional: which outputs are > 0
-    int ldbits;
-    void *C; int ldc;       // elements
-    int epi, head, a_stages;
-    int reverse;            // walk the tiles from the last to the first (see lnb_wide_tc_step: serpentine order)
-    int l2_hints;           // bit 0: A loads evict-first (read once), bit 1: C stores evict-last (the next kernel reads them)
-};
-
-// D[M x N] = A[M x K] * B[N x K]^T, A and B bf16 row-major (K contiguous), fp32 accumulation in TMEM.
-// B (a layer's weights, <= 128 KB) is loaded ONCE per CTA and stays in shared memory; everything
-// else is a ring of 16 KB A stages, so all TMA bytes in flight are HBM reads of activations.
-__global__ void __launch_bounds__(GEMM_THREADS, 1)
-gemm_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB,
-               const __grid_constant__ CUtensorMap mapC, const GemmParams p)
-{
-    extern __shared__ __align__(1024) uint8_t smem[];
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int b_bytes = p.N * BK * 2, b_stride = (b_bytes + 1023) / 1024 * 1024;
-    const int n_tiles = (p.M + BM - 1) / BM, kb_count = p.K / BK;
-    const int AS = p.a_stages;
-    uint8_t *sB = smem, *sA = smem + kb_count * b_stride;
-    // epilogue staging: per epilogue warp one 32-row x 128-byte box (128B-swizzled, as TMA expects)
-    uint8_t *sC = sA + AS * A_STAGE_BYTES;
-    uint64_t *bars = reinterpret_cast<uint64_t *>(sC + 8 * 4096);
-    const uint32_t full0 = smem_u32(bars), empty0 = smem_u32(bars + MAX_A_STAGES), tfull0 = smem_u32(bars + 2 * MAX_A_STAGES),
-                   tempty0 = smem_u32(bars + 2 * MAX_A_STAGES + 2), bfull = smem_u32(bars + 2 * MAX_A_STAGES + 4);
-    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(bars + 2 * MAX_A_STAGES + 5);
-    float *sBias = reinterpret_cast<float *>(bars + 2 * MAX_A_STAGES + 8);
-    for (int i = threadIdx.x; i < p.N; i += GEMM_THREADS) sBias[i] = p.bias ? __ldg(p.bias + i) : 0.0f;
-    const uint32_t acc_cols = p.N <= 32 ? 32 : (p.N <= 64 ? 64 : (p.N <= 128 ? 128 : 256));
-
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < AS; ++s) { mbar_init(full0 + 8 * s, 1); mbar_init(empty0 + 8 * s, 1); }
-        for (int a = 0; a < 2; ++a) { mbar_init(tfull0 + 8 * a, 1); mbar_init(tempty0 + 8 * a, 256); }
-        mbar_init(bfull, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 1) tmem_alloc(smem_u32(tmem_slot), 2 * acc_cols);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem = *tmem_slot;
-
-    if (warp == 0) {
-        // ---- TMA producer
-        if (lane == 0) {
-            mbar_expect_tx(bfull, (uint32_t)(kb_count * b_bytes));
-            for (int kb = 0; kb < kb_count; ++kb) tma_load_2d(smem_u32(sB + kb * b_stride), &mapB, kb * BK, 0, bfull);
-            pdl_wait();      // the activations below are the previous kernel's output
-            pdl_trigger();
-            uint32_t stage = 0, phase = 0;
-            for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-                const int at = p.reverse ? n_tiles - 1 - tile : tile;
-                for (int kb = 0; kb < kb_count; ++kb) {
-                    mbar_wait(empty0 + 8 * stage, phase ^ 1);
-                    mbar_expect_tx(full0 + 8 * stage, (uint32_t)A_STAGE_BYTES);
-                    if (p.l2_hints & 1) tma_load_2d_hint(smem_u32(sA + stage * A_STAGE_BYTES), &mapA, kb * BK, at * BM, full0 + 8 * stage, L2_EVICT_FIRST);
-                    else tma_load_2d(smem_u32(sA + stage * A_STAGE_BYTES), &mapA, kb * BK, at * BM, full0 + 8 * stage);
-                    if (++stage == (uint32_t)AS) { stage = 0; phase ^= 1; }
-                }
-            }
-        }
-    } else if (warp == 1) {
-        // ---- MMA issuer
-        if (lane == 0) {
-            const uint32_t idesc = instr_desc(128, p.N, 0, 0);
-            uint32_t stage = 0, phase = 0, acc = 0, acc_phase = 0;
-            mbar_wait(bfull, 0);
-            for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-                mbar_wait(tempty0 + 8 * acc, acc_phase ^ 1);
-                tc_fence_after();
-                for (int kb = 0; kb < kb_count; ++kb) {
-                    mbar_wait(full0 + 8 * stage, phase);
-                    tc_fence_after();
-                    const uint32_t a0 = smem_u32(sA + stage * A_STAGE_BYTES), b0 = smem_u32(sB + kb * b_stride);
-#pragma unroll
-                    for (int k = 0; k < BK / 16; ++k)
-                        umma_bf16(tmem + acc * acc_cols, sw128_desc(a0 + k * 32, 16, 1024), sw128_desc(b0 + k * 32, 16, 1024), idesc,
-                                  (kb > 0 || k > 0) ? 1u : 0u);
-                    umma_commit(empty0 + 8 * stage);   // frees the A stage when these MMAs retire
-                    if (++stage == (uint32_t)AS) { stage = 0; phase ^= 1; }
-                }
-                umma_commit(tfull0 + 8 * acc);          // accumulator ready for the epilogue
-                if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-            }
-        }
-    } else {
-        // ---- epilogue warps 2..9: warp w may touch TMEM lanes 32*(w%4) .. +31; the two warps of a quadrant
-        // take alternate 64-column chunks
-        const int q = warp & 3, half = (warp - 2) >> 2;
-        uint32_t acc = 0, acc_phase = 0;
-        pdl_wait();          // bits_in is the previous kernels' output; stores must not overtake its reads
-        for (int tile_i = blockIdx.x; tile_i < n_tiles; tile_i += gridDim.x) {
-            const int tile = p.reverse ? n_tiles - 1 - tile_i : tile_i;
-            const long long row = (long long)tile * BM + q * 32 + lane;
-            const bool live = row < p.M;
-            uint32_t mw[8];
-            if (p.epi == EPI_MASK_BF16) {   // this row's ReLU pattern, fetched while the MMAs of the tile still run
-#pragma unroll
-                for (int w = 0; w < 8; ++w) mw[w] = (live && w < p.ldbits) ? __ldg(p.bits_in + row * p.ldbits + w) : 0u;
-            }
-            mbar_wait(tfull0 + 8 * acc, acc_phase);
-            tc_fence_after();
-            const uint32_t tbase = tmem + acc * acc_cols + ((uint32_t)(q * 32) << 16);
-            if (p.epi == EPI_HEAD_F32) {
-                if (half == 0) {
-                uint32_t v[16];
-                tmem_ld16(tbase, v);
-                tmem_ld_wait();
-                if (live) {
-                    float z[4];
-#pragma unroll
-                    for (int j = 0; j < 4; ++j) z[j] = __uint_as_float(v[j]) + sBias[j];
-                    float4 o;
-                    o.x = 1.0f / (1.0f + __expf(-z[0])); o.y = 1.0f / (1.0f + __expf(-z[1])); o.z = 1.0f / (1.0f + __expf(-z[2]));
-                    o.w = p.head == LNB_HEAD_NERF ? fmaxf(z[3], 0.0f) : 1.0f / (1.0f + __expf(-z[3]));
-                    reinterpret_cast<float4 *>(p.C)[row] = o;
-                }
-                }
-            } else if (p.epi == EPI_NONE_F32) {
-                for (int c0 = half * 32; c0 < p.N; c0 += 64) {
-                    uint32_t v[32];
-                    if (p.N - c0 >= 32) tmem_ld32(tbase + c0, v);
-                    else tmem_ld16(tbase + c0, reinterpret_cast<uint32_t (&)[16]>(v));
-                    tmem_ld_wait();
-                    const int nc = p.N - c0 >= 32 ? 32 : 16;
-                    if (!live) continue;
-                    float *o = reinterpret_cast<float *>(p.C) + row * p.ldc + c0;
-                    for (int j = 0; j < nc; ++j) o[j] = __uint_as_float(v[j]) + sBias[c0 + j];
-                }
-            } else {
-                // bf16 outputs, 64 columns (one 128-byte row segment) at a time: registers -> this warp's
-                // swizzled staging box -> TMA store (coalesced 128 B rows in global memory).
-                uint8_t *buf = sC + (warp - 2) * 4096;
-                for (int c0 = half * 64; c0 < p.N; c0 += 128) {
-                    const int nc = p.N - c0 >= 64 ? 64 : p.N - c0;   // 64, 32 or 16 live columns
-                    uint32_t lo = 0, hi = 0;
-                    if (p.epi == EPI_MASK_BF16) {
-                        switch (c0 >> 6) {
-                        case 0: lo = mw[0]; hi = mw[1]; break;
-                        case 1: lo = mw[2]; hi = mw[3]; break;
-                        case 2: lo = mw[4]; hi = mw[5]; break;
-                        default: lo = mw[6]; hi = mw[7]; break;
-                        }
-                    }
-                    uint32_t v[64];
-                    tmem_ld32(tbase + c0, reinterpret_cast<uint32_t (&)[32]>(v[0]));
-                    if (nc > 32) tmem_ld32(tbase + c0 + 32, reinterpret_cast<uint32_t (&)[32]>(v[32]));
-                    tmem_ld_wait();
-                    tma_store_wait_read0();                          // this warp's previous store has left the buffer
-                    __syncwarp();
-#pragma unroll
-                    for (int g = 0; g < 8; ++g) {                    // eight 16-byte chunks of this row
-                        if (g * 8 >= nc) break;
-                        uint4 *slot = reinterpret_cast<uint4 *>(buf + lane * 128 + ((g ^ (lane & 7)) << 4));
-                        uint32_t pk[4];
-                        if (p.epi == EPI_RELU_BF16) {
-                            uint32_t b8 = 0;
-#pragma unroll
-                            const float4 bA = *reinterpret_cast<const float4 *>(sBias + c0 + g * 8), bB = *reinterpret_cast<const float4 *>(sBias + c0 + g * 8 + 4);
-                            const float bv[8] = {bA.x, bA.y, bA.z, bA.w, bB.x, bB.y, bB.z, bB.w};
-#pragma unroll
-                            for (int j = 0; j < 4; ++j) {
-                                const float r0 = fmaxf(__uint_as_float(v[g * 8 + 2 * j]) + bv[2 * j], 0.0f);
-                                const float r1 = fmaxf(__uint_as_float(v[g * 8 + 2 * j + 1]) + bv[2 * j + 1], 0.0f);
-                                pk[j] = pack_bf16(r0, r1);
-                                // a non-negative bf16 half is non-zero iff adding 0x7FFF carries into its top bit
-                                b8 |= ((((pk[j] & 0x7FFF7FFFu) + 0x7FFF7FFFu) >> (15 - j)) & (0x00010001u << j));
-                            }
-                            if (g < 4) lo |= b8 << (g * 4);
-                            else hi |= b8 << ((g - 4) * 4);
-                        } else {
-                            const uint32_t b8 = (g < 4 ? lo : hi) >> ((g & 3) * 4);
-#pragma unroll
-                            for (int j = 0; j < 4; ++j)
-                                pk[j] = pack_bf16(__uint_as_float(v[g * 8 + 2 * j]), __uint_as_float(v[g * 8 + 2 * j + 1])) &
-                                        (((b8 >> j) & 0x00010001u) * 0xFFFFu);
-                        }
-                        *slot = make_uint4(pk[0], pk[1], pk[2], pk[3]);
-                    }
-                    if (p.epi == EPI_RELU_BF16 && p.bits_out && live)
-                        *reinterpret_cast<uint2 *>(p.bits_out + row * p.ldbits + (c0 >> 5)) = make_uint2(lo, hi);
-                    fence_async_smem();
-                    __syncwarp();
-                    if (lane == 0) {
-                        if (p.l2_hints & 2) tma_store_2d_hint(&mapC, smem_u32(buf), c0, (int)(tile * BM + q * 32), L2_EVICT_LAST);
-                        else tma_store_2d(&mapC, smem_u32(buf), c0, (int)(tile * BM + q * 32));
-                    }
-                }
-            }
-            tc_fence_before();
-            mbar_arrive(tempty0 + 8 * acc);
-            if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-        }
-    }
-    if (warp >= 2) tma_store_wait_all();
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 1) tmem_dealloc(tmem, 2 * acc_cols);
-}
 
 // ---------------------------------------------------------------------------------------------
 // Chain of layers in ONE persistent launch.  Tile t of layer l+1 needs only tile t of layer l (the
@@ -327,7 +117,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
 // G x 9.5 MB over the chip, stored evict-last) is still in L2 when layer l+1 reads it a few
 // microseconds later, so HBM sees every activation tensor written once and never read back; the
 // weights are reloaded from L2 once per layer per block (128 KB / G tiles), chunk by chunk as the
-// previous layer's last MMAs release them.  Same warp roles, rings and epilogues as gemm_tc_kernel.
+// previous layer's last MMAs release them.
 // ---------------------------------------------------------------------------------------------
 #ifdef LNB_WIDE_CLK
 // debug build (LNB_WIDE_CLK=1 python -m loma_nerf_b200.build): where the chain kernel's MMA and epilogue warps wait
@@ -346,10 +136,13 @@ constexpr int CHAIN_MAX_G = 8;
 constexpr int CHAIN_THREADS = 576;   // warp 0 TMA, warp 1 MMA, warps 2..17 epilogue: the epilogue is the long pole of the chain
 struct ChainLayer {
     const float *bias;         // [N] or NULL
+    // ReLU pattern, one bit per element, [M][ldbits] words; word w covers columns 32w .. 32w+31 and column
+    // 32w + 8g + 2j + p sits at bit 16p + 4g + j, so that the two flags of a packed bf16 pair are 16 bits
+    // apart: ((word >> (4g + j)) & 0x00010001) * 0xFFFF is the pair's AND-mask
     const uint32_t *bits_in;   // EPI_MASK_BF16
     uint32_t *bits_out;        // EPI_RELU_BF16 (optional)
-    float *head_out;           // EPI_HEAD_F32: [M][4]
-    int ldbits, N, K, epi;
+    float *out_f32;            // EPI_HEAD_F32, EPI_NONE_F32: [M][ldc]
+    int ldbits, N, K, epi, ldc;
 };
 struct ChainParams {
     int M, n_layers, G, a_stages, head, l2_hints, b_region;
@@ -495,7 +288,7 @@ chain_tc_kernel(const __grid_constant__ ChainMaps maps, const __grid_constant__ 
                 const ChainLayer &Ly = p.layer[li];
                 const int N = Ly.N, epi = Ly.epi, c0 = k * 64;
                 const bool signal = li < p.n_layers - 1;
-                const int n_groups = (epi != EPI_HEAD_F32 && c0 < N) ? 2 : 0;   // TMA stores this warp issues per tile
+                const int n_groups = ((epi == EPI_RELU_BF16 || epi == EPI_MASK_BF16) && c0 < N) ? 2 : 0;   // TMA stores this warp issues per tile
                 asm volatile("bar.sync 1, 512;" ::: "memory");
                 if (et < N) sBias[et] = Ly.bias ? __ldg(Ly.bias + et) : 0.0f;
                 asm volatile("bar.sync 1, 512;" ::: "memory");
@@ -511,19 +304,27 @@ chain_tc_kernel(const __grid_constant__ ChainMaps maps, const __grid_constant__ 
                     const long long t_epi = clock64();
 #endif
                     const uint32_t tbase = tmem + acc * acc_cols + ((uint32_t)(q * 32) << 16);
-                    if (epi == EPI_HEAD_F32) {
-                        if (k == 0) {
+                    if (epi == EPI_HEAD_F32 || epi == EPI_NONE_F32) {
+                        // fp32 out of registers, 16 columns at a time: acc + bias, or the head's four outputs
+                        for (int c = c0; c < N && c < c0 + 64; c += 16) {
                             uint32_t v[16];
-                            tmem_ld16(tbase, v);
+                            tmem_ld16(tbase + c, v);
                             tmem_ld_wait();
-                            if (live) {
+                            if (!live) continue;
+                            float4 *o = reinterpret_cast<float4 *>(Ly.out_f32 + row * Ly.ldc + c);
+                            if (epi == EPI_HEAD_F32) {
                                 float z[4];
 #pragma unroll
-                                for (int c = 0; c < 4; ++c) z[c] = __uint_as_float(v[c]) + sBias[c];
-                                float4 o;
-                                o.x = 1.0f / (1.0f + __expf(-z[0])); o.y = 1.0f / (1.0f + __expf(-z[1])); o.z = 1.0f / (1.0f + __expf(-z[2]));
-                                o.w = p.head == LNB_HEAD_NERF ? fmaxf(z[3], 0.0f) : 1.0f / (1.0f + __expf(-z[3]));
-                                reinterpret_cast<float4 *>(Ly.head_out)[row] = o;
+                                for (int j = 0; j < 4; ++j) z[j] = __uint_as_float(v[j]) + sBias[j];
+                                float4 h;
+                                h.x = 1.0f / (1.0f + __expf(-z[0])); h.y = 1.0f / (1.0f + __expf(-z[1])); h.z = 1.0f / (1.0f + __expf(-z[2]));
+                                h.w = p.head == LNB_HEAD_NERF ? fmaxf(z[3], 0.0f) : 1.0f / (1.0f + __expf(-z[3]));
+                                o[0] = h;
+                            } else {
+#pragma unroll
+                                for (int j = 0; j < 4; ++j)
+                                    o[j] = make_float4(__uint_as_float(v[4 * j]) + sBias[c + 4 * j], __uint_as_float(v[4 * j + 1]) + sBias[c + 4 * j + 1],
+                                                       __uint_as_float(v[4 * j + 2]) + sBias[c + 4 * j + 2], __uint_as_float(v[4 * j + 3]) + sBias[c + 4 * j + 3]);
                             }
                         }
                     } else if (c0 < N && !WIDE_DEBUG_SKIP(16)) {
@@ -640,20 +441,6 @@ void pdl_config(cudaLaunchConfig_t *cfg, cudaLaunchAttribute *attr, int grid, in
     cfg->gridDim = dim3((unsigned)grid); cfg->blockDim = dim3((unsigned)block); cfg->dynamicSmemBytes = smem; cfg->stream = stream;
     cfg->attrs = attr; cfg->numAttrs = use_pdl ? 1 : 0;
 }
-
-int gemm_a_stages(int N, int K)
-{
-    const size_t b_stride = ((size_t)N * BK * 2 + 1023) / 1024 * 1024;
-    const long long room = 232448LL - 2048 - 8 * 4096 - (long long)(K / BK) * (long long)b_stride;
-    long long st = room / A_STAGE_BYTES;
-    return (int)(st > MAX_A_STAGES ? MAX_A_STAGES : st);
-}
-size_t gemm_smem(int N, int K, int a_stages)
-{
-    const size_t b_stride = ((size_t)N * BK * 2 + 1023) / 1024 * 1024;
-    return (size_t)(K / BK) * b_stride + (size_t)a_stages * A_STAGE_BYTES + 8 * 4096 + (2 * MAX_A_STAGES + 8) * 8 + 1024 + 16;
-}
-
 
 // ---------------------------------------------------------------------------------------------
 // Weight gradient dW[in x out] = H^T dZ, contraction over samples.  H [rows][in_pad] and dZ
@@ -786,53 +573,22 @@ dw_tc_kernel(const __grid_constant__ CUtensorMap mapH, const __grid_constant__ C
     if (warp == 1) tmem_dealloc(tmem, tcols);
 }
 
-// d_w[k*ldw + j] += scale * sum_z partial[z][k][j] for k < in_dim, j < out_dim.  A block covers 128
-// consecutive padded elements (32 lanes x float4) with 8 groups of partials in parallel; each group
+// dst[k*ldw + j] += scale * sum_z partial[z][k][j] for k < in_dim, j < out_dim, for every job in ONE launch (a step
+// keeps all its partials: a weight job and a bias job per layer): job j covers blocks [first_block[j], first_block[j+1]).
+// A block covers 128 consecutive padded elements (32 lanes x float4) with 8 groups of partials in parallel; each group
 // adds its partials in index order and the groups are combined in order, so the result is fixed.
-__global__ void __launch_bounds__(256) wide_dw_reduce_kernel(const float *__restrict__ partial, int n_part, int in_pad, int out_pad, int in_dim,
-                                                             int out_dim, float *__restrict__ d_w, int ldw, float seed_value,
-                                                             const float *__restrict__ seed_dev)
-{
-    __shared__ float4 acc[8][32];
-    const int lane = threadIdx.x & 31, grp = threadIdx.x >> 5;
-    const int e = (blockIdx.x * 32 + lane) * 4;                 // first of four consecutive padded elements
-    const size_t stride = (size_t)in_pad * out_pad;
-    float4 s0 = make_float4(0.f, 0.f, 0.f, 0.f), s1 = s0;
-    if (e < in_pad * out_pad) {
-        int z = grp;
-        for (; z + 8 < n_part; z += 16) {
-            const float4 a = *reinterpret_cast<const float4 *>(partial + (size_t)z * stride + e);
-            const float4 b = *reinterpret_cast<const float4 *>(partial + (size_t)(z + 8) * stride + e);
-            s0.x += a.x; s0.y += a.y; s0.z += a.z; s0.w += a.w;
-            s1.x += b.x; s1.y += b.y; s1.z += b.z; s1.w += b.w;
-        }
-        if (z < n_part) {
-            const float4 a = *reinterpret_cast<const float4 *>(partial + (size_t)z * stride + e);
-            s0.x += a.x; s0.y += a.y; s0.z += a.z; s0.w += a.w;
-        }
-    }
-    acc[grp][lane] = make_float4(s0.x + s1.x, s0.y + s1.y, s0.z + s1.z, s0.w + s1.w);
-    __syncthreads();
-    if (grp == 0 && e < in_pad * out_pad) {
-        float4 s = acc[0][lane];
-        for (int g = 1; g < 8; ++g) { s.x += acc[g][lane].x; s.y += acc[g][lane].y; s.z += acc[g][lane].z; s.w += acc[g][lane].w; }
-        const float scale = seed_value * (seed_dev ? __ldg(seed_dev) : 1.0f);
-        const int k = e / out_pad, j = e % out_pad;
-        if (k < in_dim) {
-            const float v[4] = {s.x, s.y, s.z, s.w};
-            for (int i = 0; i < 4; ++i)
-                if (j + i < out_dim) d_w[(size_t)k * ldw + j + i] += scale * v[i];
-        }
-    }
-}
-
-// The same reduction for every layer of a step in ONE launch (the step's partials are all kept):
-// job j covers blocks [first_block[j], first_block[j+1]); a weight job and a bias job per layer.
 struct ReduceJob {
     const float *partial; float *dst;
     int in_pad, out_pad, in_dim, out_dim, ldw, first_block;
 };
 struct ReduceJobs { ReduceJob job[2 * LNB_MAX_LAYERS]; int n_jobs, n_part; float seed_value; const float *seed_dev; };
+
+// appends the job of partials [n_part][in_pad][out_pad]; blocks counts the launch's grid
+void add_reduce_job(ReduceJobs &jobs, int &blocks, const float *partial, float *dst, int in_pad, int out_pad, int in_dim, int out_dim, int ldw)
+{
+    jobs.job[jobs.n_jobs++] = ReduceJob{partial, dst, in_pad, out_pad, in_dim, out_dim, ldw, blocks};
+    blocks += (in_pad * out_pad + 127) / 128;
+}
 
 __global__ void __launch_bounds__(256) wide_reduce_all_kernel(const __grid_constant__ ReduceJobs jobs)
 {
@@ -910,49 +666,10 @@ size_t dw_smem(int in_pad, int out_pad)
 
 } // namespace
 
-// C = epilogue(A[M x K] * B[N x K]^T): A, B bf16 device pointers, row pitches lda / ldb elements
-// (multiples of 8), K multiple of 64 (<= 256), N multiple of 16 and <= 256.
-int lnb_wide_gemm(lnb_ctx *ctx, const void *A, int lda, const void *B, int ldb, long long M, int N, int K, const float *bias,
-                  const uint32_t *bits_in, uint32_t *bits_out, int ldbits, void *C, int ldc, int epi, int head, int reverse)
-{
-    LNB_ARG(M >= 0 && N >= 16 && N <= 256 && N % 16 == 0 && K >= 64 && K <= 256 && K % 64 == 0, "wide gemm: shape");
-    LNB_ARG(lda % 8 == 0 && ldb % 8 == 0, "wide gemm: row pitches must be multiples of 8 elements");
-    if (M == 0) return LNB_OK;
-    if (cudaSetDevice(ctx->device) != cudaSuccess) return LNB_ERR_CUDA;
-    CUtensorMap mapA, mapB, mapC;
-    LNB_TRY(make_map(ctx, &mapA, A, M, K, lda, BM));
-    LNB_TRY(make_map(ctx, &mapB, B, N, K, ldb, N));
-    mapC = mapA; // placeholder when unused
-    if (epi == EPI_RELU_BF16 || epi == EPI_MASK_BF16) {
-        LNB_ARG(ldc % 8 == 0 && ldc >= ((N + 63) / 64) * 64, "wide gemm: bf16 output pitch must cover whole 64-column boxes");
-        LNB_TRY(make_map(ctx, &mapC, C, M, ((N + 63) / 64) * 64, ldc, 32));
-        LNB_ARG((epi != EPI_MASK_BF16 || bits_in) && (!(bits_in || bits_out) || (ldbits % 2 == 0 && ldbits * 32 >= ((N + 63) / 64) * 64 && ldbits <= 8)),
-                "wide gemm: ReLU bit pattern needs two words per 64 columns");
-    }
-    GemmParams p{};
-    p.M = (int)M; p.N = N; p.K = K; p.bias = bias; p.bits_in = bits_in; p.bits_out = bits_out; p.ldbits = ldbits; p.C = C; p.ldc = ldc;
-    p.epi = epi; p.head = head; p.reverse = reverse;
-    static const int l2_hints = [] { const char *e = getenv("LNB_WIDE_L2_HINTS"); return e ? atoi(e) : 2; }();
-    p.l2_hints = l2_hints;
-    p.a_stages = gemm_a_stages(N, K);
-    LNB_ARG(p.a_stages >= 2, "wide gemm: shared memory");
-    const size_t smem = gemm_smem(N, K, p.a_stages);
-    LNB_CUDA(cudaFuncSetAttribute(gemm_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));   // per device: set every time
-    const int n_tiles = (int)((M + BM - 1) / BM);
-    const int grid = n_tiles < ctx->sm_count ? n_tiles : ctx->sm_count;
-    cudaLaunchConfig_t cfg{};
-    cudaLaunchAttribute attr[1];
-    pdl_config(&cfg, attr, grid, GEMM_THREADS, smem, ctx->stream);
-    lnb_prof_begin(ctx, "gemm_tc_kernel");
-    LNB_CUDA(cudaLaunchKernelEx(&cfg, gemm_tc_kernel, mapA, mapB, mapC, p));
-    lnb_prof_end(ctx);
-    LNB_CHECK_LAUNCH();
-    return LNB_OK;
-}
-
 // One launch for a chain of layers (chain_tc_kernel): layer i computes epilogue_i(A_i B_i^T) where A_{i+1}
-// is the bf16 tensor layer i wrote.  All layers share M; K, N multiples of 64 (the last may have N = 16
-// with the head epilogue).
+// is the bf16 tensor layer i wrote.  All layers share M; K multiples of 64 (<= 256), row pitches multiples
+// of 8 elements; bf16 layers are multiples of 64 wide, and the last layer may instead write fp32 (the head,
+// or acc + bias) with N a multiple of 16.
 struct ChainDesc {
     const void *A; int lda;
     const void *B; int ldb;
@@ -982,11 +699,13 @@ int lnb_wide_chain(lnb_ctx *ctx, const ChainDesc *d, int n, long long M, int hea
             LNB_ARG((c.epi != EPI_MASK_BF16 || c.bits_in) && (!(c.bits_in || c.bits_out) || (c.ldbits * 32 >= c.N && c.ldbits <= 8)), "wide chain: ReLU bits");
             LNB_TRY(make_map(ctx, &maps.C[i], c.C, M, c.N, c.ldc, 32, 32));
         } else {
-            LNB_ARG(c.epi == EPI_HEAD_F32 && i == n - 1, "wide chain: only the last layer may be the head");
+            LNB_ARG((c.epi == EPI_HEAD_F32 || c.epi == EPI_NONE_F32) && i == n - 1, "wide chain: only the last layer may write fp32");
+            LNB_ARG(c.ldc % 4 == 0 && c.ldc >= (c.epi == EPI_HEAD_F32 ? 4 : c.N), "wide chain: fp32 output pitch");
         }
         ChainLayer &l = p.layer[i];
-        l.bias = c.bias; l.bits_in = c.bits_in; l.bits_out = c.bits_out; l.head_out = c.epi == EPI_HEAD_F32 ? (float *)c.C : nullptr;
-        l.ldbits = c.ldbits; l.N = c.N; l.K = c.K; l.epi = c.epi;
+        l.bias = c.bias; l.bits_in = c.bits_in; l.bits_out = c.bits_out;
+        l.out_f32 = (c.epi == EPI_HEAD_F32 || c.epi == EPI_NONE_F32) ? (float *)c.C : nullptr;
+        l.ldbits = c.ldbits; l.N = c.N; l.K = c.K; l.epi = c.epi; l.ldc = c.ldc;
         const size_t chunk = 256 * BK * 2, rows = c.N;   // chunks 32 KB apart
         const size_t need = (size_t)(c.K / BK - 1) * chunk + ((rows * BK * 2 + 1023) / 1024 * 1024);
         b_region = need > b_region ? need : b_region;
@@ -1013,22 +732,24 @@ int lnb_wide_chain(lnb_ctx *ctx, const ChainDesc *d, int n, long long M, int hea
     return LNB_OK;
 }
 
-// test hook (tests/test_gpu_wide.py): fp32 C = A * B^T (+ bias) from bf16 operands
+// test hook (tests/test_gpu_wide.py), a one-layer chain: fp32 C = A * B^T (+ bias) from bf16 operands
 extern "C" LNB_API int lnb_test_wide_gemm(lnb_ctx *ctx, const void *A, const void *B, long long M, int N, int K, const float *bias,
                                           float *C)
 {
     if (!ctx) return LNB_ERR_ARG;
-    return lnb_wide_gemm(ctx, A, K, B, K, M, N, K, bias, nullptr, nullptr, 0, C, N, EPI_NONE_F32, 0, (int)(M & 1));
+    const ChainDesc d{A, K, B, K, N, K, bias, nullptr, nullptr, 0, C, N, EPI_NONE_F32};
+    return lnb_wide_chain(ctx, &d, 1, M, 0);
 }
 
-// test hook: bf16 C = relu(A B^T + bias) (+ its ReLU bit pattern into bits_out), or, when bits_in != NULL,
-// C = A B^T where the bit is set and 0 elsewhere.  Bit rows are N/32 words.
+// test hook, a one-layer chain: bf16 C = relu(A B^T + bias) (+ its ReLU bit pattern into bits_out), or, when
+// bits_in != NULL, C = A B^T where the bit is set and 0 elsewhere.  N a multiple of 64; bit rows are N/32 words.
 extern "C" LNB_API int lnb_test_wide_gemm_bf16(lnb_ctx *ctx, const void *A, const void *B, long long M, int N, int K, const float *bias,
                                                const void *bits_in, void *bits_out, void *C)
 {
     if (!ctx) return LNB_ERR_ARG;
-    return lnb_wide_gemm(ctx, A, K, B, K, M, N, K, bias, (const uint32_t *)bits_in, (uint32_t *)bits_out, ((N + 63) / 64) * 2, C, N,
-                         bits_in ? EPI_MASK_BF16 : EPI_RELU_BF16, 0, (int)(M & 1));
+    const ChainDesc d{A, K, B, K, N, K, bias, (const uint32_t *)bits_in, (uint32_t *)bits_out, N / 32, C, N,
+                      bits_in ? EPI_MASK_BF16 : EPI_RELU_BF16};
+    return lnb_wide_chain(ctx, &d, 1, M, 0);
 }
 
 // dW partials of one layer ([n_part][in_pad][out_pad] fp32) and, if colsum != NULL, the column sums of
@@ -1067,27 +788,23 @@ extern "C" LNB_API int lnb_test_wide_dw(lnb_ctx *ctx, const void *H, int in_pad,
     float *partial = (float *)lnb_arena_take(ctx, (size_t)n_part * in_pad * out_pad * sizeof(float));
     float *bpartial = (float *)lnb_arena_take(ctx, (size_t)n_part * out_pad * sizeof(float));
     LNB_TRY(lnb_wide_dw(ctx, H, in_pad, in_pad, dZ, out_pad, out_pad, rows, partial, db ? bpartial : nullptr, n_part, (int)(rows & 1)));
+    ReduceJobs jobs{};
+    int blocks = 0;
+    add_reduce_job(jobs, blocks, partial, dW, in_pad, out_pad, in_pad, out_pad, out_pad);
+    if (db) add_reduce_job(jobs, blocks, bpartial, db, 1, out_pad, 1, out_pad, out_pad);
+    jobs.n_part = n_part;
+    jobs.seed_value = 1.0f;
+    // the reduction adds into dW / db
     LNB_CUDA(cudaMemsetAsync(dW, 0, (size_t)in_pad * out_pad * sizeof(float), ctx->stream));
-    wide_dw_reduce_kernel<<<(in_pad * out_pad + 127) / 128, 256, 0, ctx->stream>>>(partial, n_part, in_pad, out_pad, in_pad, out_pad, dW, out_pad, 1.0f, nullptr);
+    if (db) LNB_CUDA(cudaMemsetAsync(db, 0, (size_t)out_pad * sizeof(float), ctx->stream));
+    wide_reduce_all_kernel<<<blocks, 256, 0, ctx->stream>>>(jobs);
     LNB_CHECK_LAUNCH();
-    if (db) {
-        LNB_CUDA(cudaMemsetAsync(db, 0, (size_t)out_pad * sizeof(float), ctx->stream));
-        wide_dw_reduce_kernel<<<(out_pad + 127) / 128, 256, 0, ctx->stream>>>(bpartial, n_part, 1, out_pad, 1, out_pad, db, out_pad, 1.0f, nullptr);
-        LNB_CHECK_LAUNCH();
-    }
     return LNB_OK;
 }
 
 // ---------------------------------------------------------------------------------------------
 // The wide-MLP step: layerwise on the tensor cores (see the header of this file).  Produces what
 // the fused kernel produces: loss, colour, d_ws, d_bs.  Returns LNB_ERR_UNSUPPORTED otherwise.
-//
-// The whole batch normally goes through each kernel in one launch.  LNB_WIDE_SLAB_WAVES=k splits it
-// into slabs of whole rays (k waves of tiles over the SMs) that run forward, adjoint chain and weight
-// gradients one after another, each slab with its own set of per-CTA partials: an experiment in
-// keeping a layer's activations in L2 for the next layer.  Measured slower at every size (C5: 3.33 ms
-// whole, 3.50 / 3.70 / 3.88 ms for 2 / 3 / 4 slabs: every extra launch costs ~4.5 us of weight reload,
-// pipeline fill and tail), so the default is one slab.
 // ---------------------------------------------------------------------------------------------
 static int pad64(int v) { return (v + 63) / 64 * 64; }
 
@@ -1122,15 +839,6 @@ int lnb_wide_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, b
     for (int l = 0; l < L; ++l) { in_pad[l] = pad64(mlp->dims[l]); out_pad[l] = pad64(mlp->dims[l + 1]); }
     const int n_part = ctx->sm_count;
 
-    // ---- slab of rays: k waves of 128-sample tiles over the SMs (LNB_WIDE_SLAB_WAVES, 0 = whole batch)
-    static const int slab_waves = [] { const char *e = getenv("LNB_WIDE_SLAB_WAVES"); return e ? atoi(e) : 0; }();
-    int slab_rays = R;
-    if (slab_waves > 0 && S > 0) {
-        const long long r = (long long)slab_waves * ctx->sm_count * BM / S;
-        slab_rays = (int)(r < 1 ? 1 : (r > R ? R : r));
-    }
-    const int n_slabs = R > 0 ? (R + slab_rays - 1) / slab_rays : 1;
-
     // ---- arena plan
     size_t need = 1 << 16;
     auto add = [&](size_t bytes) { need += (bytes + 255) / 256 * 256 + 256; };
@@ -1146,7 +854,7 @@ int lnb_wide_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, b
     if (rays) add((size_t)R * S * 4);
     for (int l = 0; l < L; ++l) { add((size_t)in_pad[l] * out_pad[l] * 2); add((size_t)in_pad[l] * out_pad[l] * 2); add((size_t)out_pad[l] * 4); }
     if (grad)
-        for (int l = 0; l < L; ++l) { add((size_t)n_slabs * n_part * in_pad[l] * out_pad[l] * 4); add((size_t)n_slabs * n_part * out_pad[l] * 4); }
+        for (int l = 0; l < L; ++l) { add((size_t)n_part * in_pad[l] * out_pad[l] * 4); add((size_t)n_part * out_pad[l] * 4); }
     add((size_t)R * 4 + 16); add((size_t)R * 12 + 16); add(64);
     if (grad && a->d_dists) add((size_t)N * 4);
     if (grad && (a->d_color || a->d_target)) add((size_t)R * 12 + 16);
@@ -1182,8 +890,8 @@ int lnb_wide_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, b
     }
     float *partial[LNB_MAX_LAYERS], *bpartial[LNB_MAX_LAYERS];
     for (int l = 0; l < L; ++l) {
-        partial[l] = grad ? (float *)take((size_t)n_slabs * n_part * in_pad[l] * out_pad[l] * 4) : nullptr;
-        bpartial[l] = grad ? (float *)take((size_t)n_slabs * n_part * out_pad[l] * 4) : nullptr;
+        partial[l] = grad ? (float *)take((size_t)n_part * in_pad[l] * out_pad[l] * 4) : nullptr;
+        bpartial[l] = grad ? (float *)take((size_t)n_part * out_pad[l] * 4) : nullptr;
     }
     float *ray_sse = (float *)take((size_t)R * 4 + 16);
     float *color = a->color ? a->color : (float *)take((size_t)R * 12 + 16);
@@ -1211,102 +919,68 @@ int lnb_wide_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, b
         LNB_CHECK_LAUNCH();
     }
 
-    // ---- forward and adjoint chain, slab by slab (unit seed; the seed scales d_ws / d_bs at the end).
-    // Serpentine order: every GEMM / dW launch walks the samples in the direction opposite to the
-    // launch before it, so it starts on the part of its input that the previous kernel touched last
-    // and that is still in the 126 MB L2 (LNB_WIDE_NO_SERPENTINE=1 turns it off).
-    static const bool serpentine = getenv("LNB_WIDE_NO_SERPENTINE") == nullptr;
-    // one persistent launch per chain of layers (chain_tc_kernel) when the batch is one slab and every hidden width
-    // is a multiple of 64 after padding (always); LNB_WIDE_NO_CHAIN=1 keeps one launch per layer
-    static const bool chain_on = getenv("LNB_WIDE_NO_CHAIN") == nullptr;
-    const bool chain = chain_on && n_slabs == 1;
-    ReduceJobs jobs{};
-    int blocks = 0;
-    for (int r0 = 0; r0 < R; r0 += slab_rays) {
-        const int Rs = R - r0 < slab_rays ? R - r0 : slab_rays;
-        const long long n0 = (long long)r0 * S, Ns = (long long)Rs * S;
-        const int slab = r0 / slab_rays;
-        int dir = 0;                                             // the conversion kernels write front to back
-        auto next_dir = [&] { dir = serpentine ? !dir : 0; return dir; };
-        if (!rays) {
-            const long long n = Ns * (in_pad[0] / 8);
-            f32_to_bf16_rows_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(X + n0 * c_in, c_in, c_in, Ns, H[0] + n0 * in_pad[0], in_pad[0]);
-            LNB_CHECK_LAUNCH();
-        }
-        if (chain) {
-            ChainDesc cd[LNB_MAX_LAYERS];
-            for (int l = 0; l < L - 1; ++l)
-                cd[l] = ChainDesc{H[l], in_pad[l], Wf[l], in_pad[l], out_pad[l], in_pad[l], biasP[l], nullptr, grad ? bits[l + 1] : nullptr, in_pad[l + 1] / 32,
-                                  H[l + 1], out_pad[l], EPI_RELU_BF16};
-            cd[L - 1] = ChainDesc{H[L - 1], in_pad[L - 1], Wf[L - 1], in_pad[L - 1], 16, in_pad[L - 1], biasP[L - 1], nullptr, nullptr, 0, head, 4, EPI_HEAD_F32};
-            LNB_TRY(lnb_wide_chain(ctx, cd, L, N, mlp->head));
-        } else {
+    // ---- forward and adjoint chain (unit seed; the seed scales d_ws / d_bs at the end): one chain_tc_kernel launch per
+    // pass, or with LNB_WIDE_NO_CHAIN=1 one per layer, where no activations are handed over inside the kernel
+    static const bool per_layer = getenv("LNB_WIDE_NO_CHAIN") != nullptr;
+    auto run_chain = [&](const ChainDesc *cd, int n, int head_kind) {
+        if (!per_layer) return lnb_wide_chain(ctx, cd, n, N, head_kind);
+        for (int i = 0; i < n; ++i) LNB_TRY(lnb_wide_chain(ctx, cd + i, 1, N, head_kind));
+        return (int)LNB_OK;
+    };
+    if (!rays) {
+        const long long n = N * (in_pad[0] / 8);
+        f32_to_bf16_rows_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(X, c_in, c_in, N, H[0], in_pad[0]);
+        LNB_CHECK_LAUNCH();
+    }
+    {
+        ChainDesc cd[LNB_MAX_LAYERS];
         for (int l = 0; l < L - 1; ++l)
-            LNB_TRY(lnb_wide_gemm(ctx, H[l] + n0 * in_pad[l], in_pad[l], Wf[l], in_pad[l], Ns, out_pad[l], in_pad[l], biasP[l], nullptr,
-                                  grad ? bits[l + 1] + n0 * (in_pad[l + 1] / 32) : nullptr, in_pad[l + 1] / 32, H[l + 1] + n0 * out_pad[l], out_pad[l],
-                                  EPI_RELU_BF16, 0, next_dir()));
-        LNB_TRY(lnb_wide_gemm(ctx, H[L - 1] + n0 * in_pad[L - 1], in_pad[L - 1], Wf[L - 1], in_pad[L - 1], Ns, 16, in_pad[L - 1], biasP[L - 1],
-                              nullptr, nullptr, 0, head + n0 * 4, 4, EPI_HEAD_F32, mlp->head, next_dir()));
-        }
-        if (nerf) {
-            LNB_TRY(lnb_launch_composite_fwd(ctx, head + n0 * 4, 4, dists + n0, a->target ? a->target + (size_t)r0 * 3 : nullptr, Rs, S,
-                                             a->rgba ? a->rgba + n0 * 4 : nullptr, a->alpha ? a->alpha + n0 : nullptr, a->cumprod ? a->cumprod + n0 : nullptr,
-                                             a->weights ? a->weights + n0 : nullptr, color + (size_t)r0 * 3, 0, ray_sse + r0));
-        } else if (a->target) {   // mlp_fit: the prediction is the sigmoid head itself, SSE over target_w channels (mlp_fit.py:140-145)
-            LNB_TRY(lnb_launch_fit_loss(ctx, head + n0 * 4, 4, a->target + (size_t)r0 * a->target_w, Rs, a->target_w, ray_sse + r0));
-        }
-        if (!grad) continue;
+            cd[l] = ChainDesc{H[l], in_pad[l], Wf[l], in_pad[l], out_pad[l], in_pad[l], biasP[l], nullptr, grad ? bits[l + 1] : nullptr, in_pad[l + 1] / 32,
+                              H[l + 1], out_pad[l], EPI_RELU_BF16};
+        cd[L - 1] = ChainDesc{H[L - 1], in_pad[L - 1], Wf[L - 1], in_pad[L - 1], 16, in_pad[L - 1], biasP[L - 1], nullptr, nullptr, 0, head, 4, EPI_HEAD_F32};
+        LNB_TRY(run_chain(cd, L, mlp->head));
+    }
+    if (nerf)
+        LNB_TRY(lnb_launch_composite_fwd(ctx, head, 4, dists, a->target, R, S, a->rgba, a->alpha, a->cumprod, a->weights, color, 0, ray_sse));
+    else if (a->target)   // mlp_fit: the prediction is the sigmoid head itself, SSE over target_w channels (mlp_fit.py:140-145)
+        LNB_TRY(lnb_launch_fit_loss(ctx, head, 4, a->target, R, a->target_w, ray_sse));
+    if (grad) {
         if (nerf)
-            LNB_TRY(lnb_launch_composite_bwd(ctx, head + n0 * 4, 4, dists + n0, a->target + (size_t)r0 * 3, color + (size_t)r0 * 3, Rs, S, dzh + n0 * 4, 4, 4,
-                                             d_dists_u ? d_dists_u + n0 : nullptr, d_color_u ? d_color_u + (size_t)r0 * 3 : nullptr));
+            LNB_TRY(lnb_launch_composite_bwd(ctx, head, 4, dists, a->target, color, R, S, dzh, 4, 4, d_dists_u, d_color_u));
         else
-            LNB_TRY(lnb_launch_fit_head_bwd(ctx, head + n0 * 4, 4, a->target + (size_t)r0 * a->target_w, Rs, a->target_w, Rs, 4, dzh + n0 * 4, 4, nullptr));
-        {
-            const long long n = Ns * (out_pad[L - 1] / 8);
-            f32_to_bf16_rows_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(dzh + n0 * 4, 4, 4, Ns, dZ[L - 1] + n0 * out_pad[L - 1], out_pad[L - 1]);
-            LNB_CHECK_LAUNCH();
-        }
-        dir = 0;
-        if (chain) {
-            // the adjoint chain dZ_{L-1} -> ... -> dZ_0 in one launch, then the weight gradients, first the layers whose
-            // adjoints were written last
-            ChainDesc cd[LNB_MAX_LAYERS];
-            int n = 0;
-            for (int l = L - 1; l >= 1; --l)
-                cd[n++] = ChainDesc{dZ[l], out_pad[l], Wb[l], out_pad[l], in_pad[l], out_pad[l], nullptr, bits[l], nullptr, in_pad[l] / 32, dZ[l - 1], in_pad[l],
-                                    EPI_MASK_BF16};
-            if (n) LNB_TRY(lnb_wide_chain(ctx, cd, n, N, 0));
-            for (int l = 0; l < L; ++l)
-                LNB_TRY(lnb_wide_dw(ctx, H[l], in_pad[l], in_pad[l], dZ[l], out_pad[l], out_pad[l], N, partial[l], bpartial[l], n_part, next_dir()));
-        } else
-        for (int l = L - 1; l >= 0; --l) {
-            // the weight gradient of layer l (this slab's share: its own set of per-CTA partials) runs right here,
-            // between the kernel that wrote dZ_l and the one that reads it again
-            LNB_TRY(lnb_wide_dw(ctx, H[l] + n0 * in_pad[l], in_pad[l], in_pad[l], dZ[l] + n0 * out_pad[l], out_pad[l], out_pad[l], Ns,
-                                partial[l] + (size_t)slab * n_part * in_pad[l] * out_pad[l], bpartial[l] + (size_t)slab * n_part * out_pad[l], n_part,
-                                next_dir()));
-            if (l >= 1)   // dZ_{l-1} = (dZ_l W_l^T) where H_l > 0
-                LNB_TRY(lnb_wide_gemm(ctx, dZ[l] + n0 * out_pad[l], out_pad[l], Wb[l], out_pad[l], Ns, in_pad[l], out_pad[l], nullptr,
-                                      bits[l] + n0 * (in_pad[l] / 32), nullptr, in_pad[l] / 32, dZ[l - 1] + n0 * in_pad[l], in_pad[l], EPI_MASK_BF16, 0,
-                                      next_dir()));
-        }
+            LNB_TRY(lnb_launch_fit_head_bwd(ctx, head, 4, a->target, R, a->target_w, R, 4, dzh, 4, nullptr));
+        const long long n = N * (out_pad[L - 1] / 8);
+        f32_to_bf16_rows_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(dzh, 4, 4, N, dZ[L - 1], out_pad[L - 1]);
+        LNB_CHECK_LAUNCH();
+        // the adjoint chain dZ_{L-1} -> ... -> dZ_0, then the weight gradients, first the layers whose adjoints were
+        // written last
+        ChainDesc cd[LNB_MAX_LAYERS];
+        int nc = 0;
+        for (int l = L - 1; l >= 1; --l)
+            cd[nc++] = ChainDesc{dZ[l], out_pad[l], Wb[l], out_pad[l], in_pad[l], out_pad[l], nullptr, bits[l], nullptr, in_pad[l] / 32, dZ[l - 1], in_pad[l],
+                                 EPI_MASK_BF16};
+        LNB_TRY(run_chain(cd, nc, 0));
+        // serpentine order: each dW launch walks the samples in the direction opposite to the launch before it, so it
+        // starts on the part of its input that the previous kernel touched last and that is still in the 126 MB L2
+        // (LNB_WIDE_NO_SERPENTINE=1 turns it off)
+        static const bool serpentine = getenv("LNB_WIDE_NO_SERPENTINE") == nullptr;
+        for (int l = 0; l < L; ++l)
+            LNB_TRY(lnb_wide_dw(ctx, H[l], in_pad[l], in_pad[l], dZ[l], out_pad[l], out_pad[l], N, partial[l], bpartial[l], n_part,
+                                serpentine && l % 2 == 0));
     }
     if (a->target) LNB_TRY(lnb_launch_sum(ctx, ray_sse, R, loss));
     else if (a->loss) LNB_TRY(lnb_launch_fill(ctx, loss, 1, 0.0f));
     if (!grad) return LNB_OK;
 
-    // ---- weight and bias gradients: per layer one dW kernel (+ column sums) over the whole batch (above, or
-    // here when the chain ran in slabs), then one launch that reduces every layer's partials into d_ws / d_bs
+    // ---- weight and bias gradients: one launch reduces every layer's partials into d_ws / d_bs
+    ReduceJobs jobs{};
+    int blocks = 0;
     for (int l = L - 1; l >= 0; --l) {
-        ReduceJob &w = jobs.job[jobs.n_jobs++];
-        w = ReduceJob{partial[l], a->d_ws + (size_t)l * mlp->max_in * mlp->max_out, in_pad[l], out_pad[l], mlp->dims[l], mlp->dims[l + 1],
-                      mlp->max_out, blocks};
-        blocks += (in_pad[l] * out_pad[l] + 127) / 128;
-        ReduceJob &bj = jobs.job[jobs.n_jobs++];
-        bj = ReduceJob{bpartial[l], a->d_bs + (size_t)l * mlp->max_out, 1, out_pad[l], 1, mlp->dims[l + 1], mlp->max_out, blocks};
-        blocks += (out_pad[l] + 127) / 128;
+        add_reduce_job(jobs, blocks, partial[l], a->d_ws + (size_t)l * mlp->max_in * mlp->max_out, in_pad[l], out_pad[l], mlp->dims[l],
+                       mlp->dims[l + 1], mlp->max_out);
+        add_reduce_job(jobs, blocks, bpartial[l], a->d_bs + (size_t)l * mlp->max_out, 1, out_pad[l], 1, mlp->dims[l + 1], mlp->max_out);
     }
-    jobs.n_part = n_part * n_slabs;
+    jobs.n_part = n_part;
     jobs.seed_value = a->seed_mode == LNB_SEED_LOSS ? 1.0f : a->seed;
     jobs.seed_dev = a->seed_mode == LNB_SEED_LOSS ? loss : nullptr;
     wide_reduce_all_kernel<<<blocks, 256, 0, ctx->stream>>>(jobs);

@@ -1,6 +1,7 @@
-"""Wide-MLP tensor-core path (wide_tc.cu): the TMA-fed, 128B-swizzled tcgen05 GEMM and the weight-
-gradient kernel against fp32 matrix products of the same bf16-rounded operands (torch is only the
-checker here), then the whole layerwise step against the reference golden vectors of the 8x256 net."""
+"""Wide-MLP tensor-core path (wide_tc.cu): the TMA-fed tcgen05 chain kernel run as a one-layer GEMM, and the
+weight-gradient kernel with the step's reduction, against fp32 matrix products of the same bf16-rounded operands
+(torch is only the checker here), then the whole layerwise step against the reference golden vectors of the 8x256
+net."""
 import ctypes
 
 import numpy as np
@@ -44,7 +45,7 @@ def test_wide_gemm_matches_fp32_product_of_bf16_operands(ctx, torch_cuda, M, N, 
 
 
 def _pack_bits(torch, positive):
-    """[M][N] bool -> [M][N/32] int32 in the kernel's ReLU-pattern layout (wide_tc.cu GemmParams): word w
+    """[M][N] bool -> [M][N/32] int32 in the kernel's ReLU-pattern layout (wide_tc.cu ChainLayer): word w
     covers columns 32w..32w+31, column 32w + 8g + 2j + p at bit 16p + 4g + j."""
     pos = positive.cpu().numpy().astype(np.uint64)
     M, N = pos.shape
@@ -229,11 +230,12 @@ def test_trainer_on_a_wide_mlp_follows_numpy_adam(ctx, torch_cuda):
 
 
 def test_chain_kernel_equals_one_launch_per_layer():
-    """chain_tc_kernel (all layers of a pass in one launch, activations handed over through L2) runs the very
-    same MMAs and epilogues as one gemm_tc_kernel launch per layer: loss and colour of a 345 600-sample step
-    must agree to the last printed digit, run after run (a lost hand-over would show up here); the gradients
-    go through differently ordered fp32 partial sums, so they are compared to 1e-5.  The switch is an
-    environment variable read once per process, hence the subprocesses."""
+    """chain_tc_kernel with all layers of a pass in one launch (activations handed over through L2) runs the very
+    same MMAs and epilogues as one one-layer launch per layer (LNB_WIDE_NO_CHAIN=1, no hand-over inside the
+    kernel), and as blocks of 3 or of single tiles (LNB_WIDE_CHAIN_G): loss and colour of a 345 600-sample step
+    must agree to the last printed digit, run after run (a lost hand-over would show up here); the gradient
+    checksums are compared to 1e-5.  The switches are environment variables read once per process, hence the
+    subprocesses."""
     import os, subprocess, sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 

@@ -1,4 +1,5 @@
-"""Times the wide-path kernels alone (wide_tc.cu) at the BASELINE config-5 layer shape."""
+"""Times the wide-path kernels alone (wide_tc.cu) at the BASELINE config-5 layer shape: one layer as a one-layer
+chain_tc_kernel launch, and dw_tc_kernel with the reduction of its partials."""
 import ctypes, sys
 sys.path.insert(0, ".")
 import torch
@@ -30,4 +31,4 @@ for (M, N, K) in [(786432, 256, 256), (786432, 256, 64), (113664, 256, 256)]:
         t0.record()
         for _ in range(10): f()
         t1.record(); torch.cuda.synchronize()
-        print(f"dW + colsum + both reduces rows={M} in={K} out={N}: {t0.elapsed_time(t1)*100:.1f} us per call", flush=True)
+        print(f"dW + colsum + reduce rows={M} in={K} out={N}: {t0.elapsed_time(t1)*100:.1f} us per call", flush=True)
