@@ -146,19 +146,28 @@ def make_fit_case(seed, N, E=5, width=16, n_layers=3):
 # ------------------------------------------------------------------------------------------------
 # float64 numpy restatement (SURVEY.md Appendix B)
 # ------------------------------------------------------------------------------------------------
+def head_f64(Z, head):
+    """The head's activation of the last layer's pre-activations Z: sigmoid, and for nerf ReLU on sigma."""
+    Y = 1.0 / (1.0 + np.exp(-Z))
+    if head == "nerf":
+        Y[:, 3] = np.maximum(Z[:, 3], 0.0)
+    return Y
+
+
+def head_adjoint_f64(Y, dY, head):
+    """Adjoint of the head's pre-activations from that of its outputs Y."""
+    dZ = dY * Y * (1.0 - Y)
+    if head == "nerf":
+        dZ[:, 3] = dY[:, 3] * (Y[:, 3] > 0)
+    return dZ
+
+
 def _mlp_f64(X, ws, bs, dims, head):
     L = len(dims) - 1
     H = [np.asarray(X, np.float64)]
     for l in range(L):
         Z = H[-1] @ ws[l, :dims[l], :dims[l + 1]].astype(np.float64) + bs[l, :dims[l + 1]]
-        if l < L - 1:
-            Z = np.maximum(Z, 0.0)
-        else:
-            Y = 1.0 / (1.0 + np.exp(-Z))
-            if head == "nerf":
-                Y[:, 3] = np.maximum(Z[:, 3], 0.0)
-            Z = Y
-        H.append(Z)
+        H.append(np.maximum(Z, 0.0) if l < L - 1 else head_f64(Z, head))
     return H  # H[0]=X, H[l+1] = post-activation output of layer l
 
 
@@ -170,13 +179,7 @@ def _mlp_back_f64(H, dY, ws, bs, dims, head):
     dZs = [None] * L
     dH = dY
     for l in range(L - 1, -1, -1):
-        Y = H[l + 1]
-        if l < L - 1:
-            dZ = dH * (Y > 0)
-        else:
-            dZ = dH * Y * (1.0 - Y)
-            if head == "nerf":
-                dZ[:, 3] = dH[:, 3] * (Y[:, 3] > 0)
+        dZ = dH * (H[l + 1] > 0) if l < L - 1 else head_adjoint_f64(H[l + 1], dH, head)
         dZs[l] = dZ
         d_ws[l, :dims[l], :dims[l + 1]] = H[l].T @ dZ
         d_bs[l, :dims[l + 1]] = dZ.sum(0)
@@ -184,12 +187,10 @@ def _mlp_back_f64(H, dY, ws, bs, dims, head):
     return d_ws, d_bs, dH, dZs
 
 
-def nerf_f64(X, ws, bs, dims, target, dists, R, S, g=None):
-    """Forward (+ backward when g is not None; g='loss' seeds with the loss as the reference host
-    does, train_nerf.py:477). Returns a dict of float64 arrays."""
-    dims = [int(v) for v in dims]
-    H = _mlp_f64(X, ws, bs, dims, "nerf")
-    out = H[-1].reshape(R, S, 4)
+def composite_f64(rgba, dists, target, R, S, g=None):
+    """Compositing and SSE loss of the head outputs rgba [R*S][4] (scripts/nerf.py:176-302) and, when g is not None, the
+    adjoints: dY (of rgba, seeded with g; g='loss' seeds with the loss), d_dists, d_acc, d_target."""
+    out = np.asarray(rgba, np.float64).reshape(R, S, 4)
     rgb, sigma = out[..., :3], out[..., 3]
     dist = np.asarray(dists, np.float64).reshape(R, S)
     e = np.exp(-sigma * dist)
@@ -201,8 +202,7 @@ def nerf_f64(X, ws, bs, dims, target, dists, R, S, g=None):
     w = alpha * T
     color = (w[..., None] * rgb).sum(1)
     loss = ((color - target) ** 2).sum()
-    res = dict(loss=loss, color=color, rgba=out, alpha=alpha, cumprod=T, weights=w,
-               inter=[h for h in H[1:]])
+    res = dict(loss=loss, color=color, rgba=out, alpha=alpha, cumprod=T, weights=w)
     if g is None:
         return res
     g = loss if isinstance(g, str) else float(g)
@@ -221,27 +221,49 @@ def nerf_f64(X, ws, bs, dims, target, dists, R, S, g=None):
     d_sigma = d_alpha * e * dist
     d_dists = d_alpha * e * sigma
     dY = np.concatenate([d_rgb, d_sigma[..., None]], -1).reshape(R * S, 4)
-    d_ws, d_bs, d_X, dZs = _mlp_back_f64(H, dY, ws, bs, dims, "nerf")
-    res.update(d_ws=d_ws, d_bs=d_bs, d_X=d_X, d_target=-d_color, d_dists=d_dists,
-               d_acc=d_color, d_inter=dZs, g=g)
+    res.update(dY=dY, d_target=-d_color, d_dists=d_dists, d_acc=d_color, g=g)
+    return res
+
+
+def fit_loss_f64(pred, target, g=None):
+    """SSE of the first target.shape[0] rows / target.shape[1] channels of pred (scripts/mlp_fit.py:140-145) and, when g is
+    not None, its adjoint dY (of pred, seeded with g; g='loss' seeds with the loss)."""
+    R, Wt = target.shape
+    diff = pred[:R, :Wt] - target
+    loss = (diff ** 2).sum()
+    res = dict(loss=loss, pred=pred)
+    if g is None:
+        return res
+    g = loss if isinstance(g, str) else float(g)
+    dY = np.zeros_like(pred)
+    dY[:R, :Wt] = 2.0 * g * diff
+    res.update(dY=dY, d_target=-dY[:R, :Wt], g=g)
+    return res
+
+
+def nerf_f64(X, ws, bs, dims, target, dists, R, S, g=None):
+    """Forward (+ backward when g is not None; g='loss' seeds with the loss as the reference host
+    does, train_nerf.py:477). Returns a dict of float64 arrays."""
+    dims = [int(v) for v in dims]
+    H = _mlp_f64(X, ws, bs, dims, "nerf")
+    res = composite_f64(H[-1], dists, target, R, S, g)
+    res["inter"] = [h for h in H[1:]]
+    if g is None:
+        return res
+    d_ws, d_bs, d_X, dZs = _mlp_back_f64(H, res.pop("dY"), ws, bs, dims, "nerf")
+    res.update(d_ws=d_ws, d_bs=d_bs, d_X=d_X, d_inter=dZs)
     return res
 
 
 def mlp_fit_f64(X, ws, bs, dims, target, g=None):
     dims = [int(v) for v in dims]
     H = _mlp_f64(X, ws, bs, dims, "sigmoid")
-    pred = H[-1]
-    R, Wt = target.shape
-    diff = pred[:R, :Wt] - target
-    loss = (diff ** 2).sum()
-    res = dict(loss=loss, pred=pred, inter=[h for h in H[1:]])
+    res = fit_loss_f64(H[-1], target, g)
+    res["inter"] = [h for h in H[1:]]
     if g is None:
         return res
-    g = loss if isinstance(g, str) else float(g)
-    dY = np.zeros_like(pred)
-    dY[:R, :Wt] = 2.0 * g * diff
-    d_ws, d_bs, d_X, dZs = _mlp_back_f64(H, dY, ws, bs, dims, "sigmoid")
-    res.update(d_ws=d_ws, d_bs=d_bs, d_X=d_X, d_target=-dY[:R, :Wt], d_inter=dZs, g=g)
+    d_ws, d_bs, d_X, dZs = _mlp_back_f64(H, res.pop("dY"), ws, bs, dims, "sigmoid")
+    res.update(d_ws=d_ws, d_bs=d_bs, d_X=d_X, d_inter=dZs)
     return res
 
 

@@ -1,6 +1,10 @@
 """Tensor-core path (LNB_PATH_TC, fused_tc.cu): bf16 operands, fp32 accumulation in TMEM.
 Compared with the reference golden vectors and the float64 restatement under the bf16 bound stated
-in DESIGN.md: norm-wise relative error <= TC_TOL on loss, colour and weight gradients."""
+in DESIGN.md 2.2: norm-wise relative error <= TC_TOL on loss, colour and weight gradients (measured
+7e-5 .. 2e-3 on loss, 1e-3 .. 2e-2 on gradients).  These bounds check the semantics and absorb the
+whole bf16 error; the kernels' own arithmetic is held 100x tighter in test_gpu_tc_model.py, against
+the bf16-faithful model oracle/tc_model.py (4e-4 on colour, 6e-5 on gradients for the fused kernels,
+measured on one B200 at 1000 W: DESIGN.md 2.2)."""
 import os
 
 import numpy as np
