@@ -147,7 +147,9 @@ typedef struct {
  * stratified == 1: t_s = near + (s + u)(far - near) / S with u = lnb_uniform(seed, q, s) in [0, 1), the counter-based
  * generator documented at lnb_uniform below (SURVEY.md 8d's synthetic sampling; the reference has the jitter commented
  * out).  dists = t[s+1] - t[s], last 1e8.  The exact path forms every value in float64 like numpy does and rounds
- * once to float32; the tensor-core path computes in float32. */
+ * once to float32; the tensor-core path computes in float32.
+ * With VIEW DIRECTIONS (dims[0] even, see pe_bands in lnb_step_args) the direction of ray r is dir / |dir|, dir as above
+ * (what lnb_camera_rays returns as rays_d). */
 typedef struct {
     double c2w[12];
     double fx, fy, cx, cy;        /* normalized_K[0][0], [1][1], [0][2], [1][2] */
@@ -202,7 +204,15 @@ typedef struct {
     const void *rays_o, *rays_d; /* [R][3]                                                      */
     const void *t;            /* [R][S] sample depths along each ray                            */
     int ray_dtype;            /* LNB_RAY_F64 (the reference's get_rays/linspace dtype) or F32   */
-    int pe_bands;             /* E; dims[0] must equal 3 + 6E                                   */
+    int pe_bands;             /* E.  dims[0] selects the input form (rays and camera mode alike): */
+    /*   dims[0] == 3 + 6E (odd): X = PE(pts, E), positions only.                                 */
+    /*   dims[0] == (3 + 6E) + (3 + 6 E_d), E_d >= 0 (even): X = [PE(pts, E) | PE(u, E_d)] with   */
+    /*   the unit view direction u = d / |d|, d = rays_d[r] (camera mode: the generated direction),*/
+    /*   the same for all S samples of a ray; E_d = (dims[0] - 6 - 6E) / 6.  PE is                 */
+    /*   positional_encoding_3d (slot 0 identity, slots 2i+1 / 2i+2 sin / cos(2^i .), feature =    */
+    /*   3 * slot + coord).  The exact path forms |d| = sqrt((d0^2 + d1^2) + d2^2) in float64 with */
+    /*   every operation rounded (no FMA), divides, encodes in float64 and rounds once to float32. */
+    /*   Any other width is LNB_ERR_ARG.                                                          */
     /* CAMERA MODE (selected when X == NULL, rays_o == NULL and cam != NULL): see lnb_camera.      */
     /* `cam` is always a HOST pointer (a few bytes, passed to the kernels by value).               */
     const lnb_camera *cam;
@@ -253,6 +263,11 @@ LNB_API int lnb_pos_encoding(lnb_ctx *ctx, const double *x, long long n, int F, 
  * rays_o, rays_d [R][3] float64, t [R][S] float64. Device pointers. */
 LNB_API int lnb_sample_encode(lnb_ctx *ctx, const double *rays_o, const double *rays_d, const double *t,
                       int R, int S, int E, float *X, float *dists);
+/* The same with the view direction (E_dir >= 0): X [R*S][(3+6E) + (3+6E_dir)] = [PE(pts, E) | PE(u, E_dir)], u the unit
+ * direction of rays_d as rays mode defines it (pe_bands in lnb_step_args).  The input a features-mode step of a net with
+ * view directions expects.  Device pointers. */
+LNB_API int lnb_sample_encode_dirs(lnb_ctx *ctx, const double *rays_o, const double *rays_d, const double *t,
+                                   int R, int S, int E, int E_dir, float *X, float *dists);
 
 /* The rays and sample depths camera mode generates, written out (any pointer may be NULL): rays_o, rays_d [R][3], t [R][S]
  * float64.  Device pointers (cam itself is a host pointer). */

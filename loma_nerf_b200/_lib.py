@@ -98,6 +98,8 @@ def load():
     lib.lnb_pos_encoding.argtypes = [c_void_p, c_void_p, c_longlong, c_int, c_int, c_void_p]
     lib.lnb_sample_encode.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
                                       c_void_p, c_void_p]
+    lib.lnb_sample_encode_dirs.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int,
+                                           c_void_p, c_void_p]
     lib.lnb_camera_rays.argtypes = [c_void_p, P(LnbCamera), c_int, c_int, c_void_p, c_void_p, c_void_p]
     lib.lnb_color_to_u8.argtypes = [c_void_p, c_void_p, c_longlong, c_void_p]
     lib.lnb_uniform.argtypes = [ctypes.c_ulonglong, c_longlong, c_int]

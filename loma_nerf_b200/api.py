@@ -49,6 +49,26 @@ def make_camera(c2w, normalized_K, width, height=None, near=2.0, far=6.0, first_
     return c
 
 
+def rays_input_width(pe_bands, dir_bands=None):
+    """dims[0] of a net fed in rays or camera mode: 3 + 6E for positions only, (3 + 6E) + (3 + 6E_d) with the view
+    direction encoded in E_d = dir_bands bands (include/loma_nerf_b200.h, lnb_step_args.pe_bands)."""
+    E = int(pe_bands)
+    if E < 0 or (dir_bands is not None and int(dir_bands) < 0):
+        raise ValueError("pe_bands and dir_bands must be >= 0")
+    return 3 + 6 * E + (0 if dir_bands is None else 3 + 6 * int(dir_bands))
+
+
+def check_rays_width(dims0, pe_bands, dir_bands=None):
+    """ValueError unless dims[0] is the input width of (pe_bands, dir_bands): the library reads the input form off dims[0]
+    alone, so the caller states it and a net of the other form is refused before anything is launched."""
+    want = rays_input_width(pe_bands, dir_bands)
+    if int(dims0) != want:
+        form = "positions only" if dir_bands is None else "positions and %d direction bands" % int(dir_bands)
+        raise ValueError("dims[0] = %d, but %d position bands with %s need %d inputs%s"
+                         % (int(dims0), int(pe_bands), form, want,
+                            " (pass dir_bands for a net with view directions)" if dir_bands is None else ""))
+
+
 def make_mlp(dims, ws_shape, head):
     m = L.LnbMlp()
     dims = [int(d) for d in dims]
@@ -196,7 +216,9 @@ class Context:
 
     # -------------------------------------------------------------------------------------------
     def _step(self, nerf, dims, X, ws, bs, target, dists, R, S, grad, seed, outputs, out, rows,
-              path, inter_accumulate, color_accumulate, head, rays=None, pe_bands=0, camera=None):
+              path, inter_accumulate, color_accumulate, head, rays=None, pe_bands=0, camera=None, dir_bands=None):
+        if rays is not None or camera is not None:
+            check_rays_width(dims[0], pe_bands, dir_bands)
         dev = _is_cuda(ws)
         mlp = make_mlp(dims, ws.shape, head)
         Ln, mi, mo = mlp.n_layers, mlp.max_in, mlp.max_out
@@ -270,22 +292,24 @@ class Context:
                           rows, path, inter_accumulate, color_accumulate, L.HEAD_NERF)
 
     def nerf_step_rays(self, dims, rays_o, rays_d, t, pe_bands, ws, bs, target=None, grad=False, seed=1.0,
-                       outputs=("color", "loss"), out=None, path="f32"):
+                       outputs=("color", "loss"), out=None, path="f32", dir_bands=None):
         """The same step starting from rays: the sample positions o + d*t, their positional encoding
         and the dists are computed on the device (train_nerf.py:289-311, pos_encoding.py:38-70) --
         fused into the first layer on the tensor-core path.  rays_o, rays_d [R][3], t [R][S], all
-        float64 (the reference's dtype) or all float32."""
+        float64 (the reference's dtype) or all float32.  dir_bands=E_d: the net also takes the unit view
+        direction in E_d bands (dims[0] = 3 + 6 pe_bands + 3 + 6 E_d, rays_input_width)."""
         R, S = int(t.shape[0]), int(t.shape[1])
         return self._step(True, dims, None, ws, bs, target, None, R, S, grad, seed, outputs, out, None, path,
-                          False, False, L.HEAD_NERF, rays=(rays_o, rays_d, t), pe_bands=pe_bands)
+                          False, False, L.HEAD_NERF, rays=(rays_o, rays_d, t), pe_bands=pe_bands, dir_bands=dir_bands)
 
     def nerf_step_camera(self, dims, camera, R, S, pe_bands, ws, bs, target=None, grad=False, seed=1.0,
-                         outputs=("color", "loss"), out=None, path="f32"):
+                         outputs=("color", "loss"), out=None, path="f32", dir_bands=None):
         """The same step with rays AND sample depths generated on the device from a pose (`make_camera`): the
         device-side get_rays (train_nerf.py:23-62) and linspace / stratified depths (train_nerf.py:289-311).
-        Nothing per ray or per sample is read: R rays of S samples through pixels first_pixel .. (or `pixels`)."""
+        Nothing per ray or per sample is read: R rays of S samples through pixels first_pixel .. (or `pixels`).
+        dir_bands as in nerf_step_rays."""
         return self._step(True, dims, None, ws, bs, target, None, int(R), int(S), grad, seed, outputs, out, None, path,
-                          False, False, L.HEAD_NERF, pe_bands=pe_bands, camera=camera)
+                          False, False, L.HEAD_NERF, pe_bands=pe_bands, camera=camera, dir_bands=dir_bands)
 
     def camera_rays(self, camera, R, S):
         """(rays_o, rays_d, t) float64 cuda tensors camera mode generates (for checks / hosts that want them)."""
@@ -322,14 +346,20 @@ class Context:
         self._check(self.lib.lnb_pos_encoding(self.h, x.data_ptr(), n, F, int(E), o.data_ptr()))
         return o
 
-    def sample_encode(self, rays_o, rays_d, t, E):
-        """train_nerf.py:289-311 + pos_encoding_3d: returns X [R*S][3+6E] f32 and dists [R][S]."""
+    def sample_encode(self, rays_o, rays_d, t, E, dir_bands=None):
+        """train_nerf.py:289-311 + pos_encoding_3d: returns X [R*S][3+6E] f32 and dists [R][S].  dir_bands=E_d appends
+        the unit view direction's encoding: X [R*S][rays_input_width(E, E_d)], what rays mode feeds such a net."""
         assert all(_is_cuda(v) and v.dtype == torch.float64 and v.is_contiguous() for v in (rays_o, rays_d, t))
         R, S = int(t.shape[0]), int(t.shape[1])
-        X = torch.empty((R * S, 3 + 6 * E), dtype=torch.float32, device=t.device)
+        X = torch.empty((R * S, rays_input_width(E, dir_bands)), dtype=torch.float32, device=t.device)
         dists = torch.empty((R, S), dtype=torch.float32, device=t.device)
-        self._check(self.lib.lnb_sample_encode(self.h, rays_o.data_ptr(), rays_d.data_ptr(),
-                                               t.data_ptr(), R, S, int(E), X.data_ptr(), dists.data_ptr()))
+        if dir_bands is None:
+            rc = self.lib.lnb_sample_encode(self.h, rays_o.data_ptr(), rays_d.data_ptr(),
+                                            t.data_ptr(), R, S, int(E), X.data_ptr(), dists.data_ptr())
+        else:
+            rc = self.lib.lnb_sample_encode_dirs(self.h, rays_o.data_ptr(), rays_d.data_ptr(), t.data_ptr(), R, S, int(E),
+                                                 int(dir_bands), X.data_ptr(), dists.data_ptr())
+        self._check(rc)
         return X, dists
 
     def mult_a_b(self, a, b, c):
@@ -377,9 +407,12 @@ class Trainer:
             self.lib.lnb_trainer_destroy(self.h)
             self.h = None
 
-    def _batch(self, X=None, dists=None, target=None, rays=None, pe_bands=0, R=None, S=None, path="tc", seed=1.0, camera=None):
+    def _batch(self, X=None, dists=None, target=None, rays=None, pe_bands=0, R=None, S=None, path="tc", seed=1.0, camera=None,
+               dir_bands=None):
         a = L.LnbStepArgs()
         nerf = self.head == L.HEAD_NERF
+        if camera is not None or rays is not None:
+            check_rays_width(self.dims[0], pe_bands, dir_bands)   # dir_bands: the view direction's bands, as in nerf_step_rays
         if camera is not None:
             R, S = int(target.shape[0]) if R is None else int(R), int(S)
             a.cam, a.pe_bands = ctypes.pointer(camera), int(pe_bands)

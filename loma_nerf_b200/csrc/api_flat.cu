@@ -271,7 +271,8 @@ int validate(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf
     if (rays) {
         LNB_ARG(nerf, "rays mode is a nerf-path feature");
         LNB_ARG(cam || (a->rays_d && a->t), "rays mode needs rays_o, rays_d and t");
-        LNB_ARG(a->pe_bands >= 0 && d->c_in == 3 + 6 * a->pe_bands, "rays mode: dims[0] != 3 + 6*pe_bands");
+        LNB_ARG(lnb_rays_dir_bands(d->c_in, a->pe_bands) != LNB_DIRS_BAD,
+                "rays mode: dims[0] must be 3 + 6*pe_bands, or 6 + 6*pe_bands + 6*E_dir with view directions");
         LNB_ARG(a->ray_dtype == LNB_RAY_F64 || a->ray_dtype == LNB_RAY_F32, "ray_dtype");
         LNB_ARG(!a->d_X, "d_X is not available in rays mode");
     }
@@ -332,8 +333,9 @@ int step_layerwise(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, boo
     const float *X = a->X, *dists = a->dists;
     if (rays) {
         float *Xe = takef((size_t)N * d.c_in), *de = takef((size_t)R * S);
-        if (cam) LNB_TRY(lnb_launch_camera_encode(ctx, a->cam, R, S, a->pe_bands, Xe, de, nullptr, 0));
-        else LNB_TRY(lnb_launch_sample_encode(ctx, a->rays_o, a->rays_d, a->t, a->ray_dtype == LNB_RAY_F64, R, S, a->pe_bands, Xe, de));
+        const int Ed = lnb_rays_dir_bands(d.c_in, a->pe_bands);
+        if (cam) LNB_TRY(lnb_launch_camera_encode(ctx, a->cam, R, S, a->pe_bands, Ed, Xe, de, nullptr, 0));
+        else LNB_TRY(lnb_launch_sample_encode(ctx, a->rays_o, a->rays_d, a->t, a->ray_dtype == LNB_RAY_F64, R, S, a->pe_bands, Ed, Xe, de));
         X = Xe; dists = de;
     }
     // ---- forward
@@ -658,7 +660,16 @@ extern "C" int lnb_sample_encode(lnb_ctx *ctx, const double *rays_o, const doubl
     if (!ctx) return LNB_ERR_ARG;
     LNB_ARG(rays_o && rays_d && t && X && R >= 0 && S >= 1 && E >= 0, "sample_encode arguments");
     if (cudaSetDevice(ctx->device) != cudaSuccess) return LNB_ERR_CUDA;
-    return lnb_launch_sample_encode(ctx, rays_o, rays_d, t, 1, R, S, E, X, dists);
+    return lnb_launch_sample_encode(ctx, rays_o, rays_d, t, 1, R, S, E, LNB_DIRS_NONE, X, dists);
+}
+
+extern "C" int lnb_sample_encode_dirs(lnb_ctx *ctx, const double *rays_o, const double *rays_d,
+                                      const double *t, int R, int S, int E, int E_dir, float *X, float *dists)
+{
+    if (!ctx) return LNB_ERR_ARG;
+    LNB_ARG(rays_o && rays_d && t && X && R >= 0 && S >= 1 && E >= 0 && E_dir >= 0, "sample_encode_dirs arguments");
+    if (cudaSetDevice(ctx->device) != cudaSuccess) return LNB_ERR_CUDA;
+    return lnb_launch_sample_encode(ctx, rays_o, rays_d, t, 1, R, S, E, E_dir, X, dists);
 }
 
 extern "C" int lnb_mult_a_b(lnb_ctx *ctx, const float *a, int a_h, int a_w, const float *b, int b_w,

@@ -32,9 +32,48 @@ __global__ void pos_encoding_kernel(const double *__restrict__ x, long long n, i
     }
 }
 
+// slot 0 = v and slots 2i+1 / 2i+2 = sin / cos(2^i v), i < E, of one coordinate f: feature 3 * slot + f of the row at o.
+// fp32 features: float64 sin / cos, rounded once (pos_encoding.py:38-70).
+__device__ __forceinline__ void encode_coord(double v, int E, int f, float *o)
+{
+    o[f] = (float)v;
+    double freq = 1.0;
+    for (int i = 0; i < E; ++i) {
+        double sn, cs;
+        sincos(freq * v, &sn, &cs);
+        o[(2 * i + 1) * 3 + f] = (float)sn;
+        o[(2 * i + 2) * 3 + f] = (float)cs;
+        freq *= 2.0;
+    }
+}
+// the wide tensor-core path's bf16 operand: the float value rounded once more
+__device__ __forceinline__ void encode_coord(double v, int E, int f, __nv_bfloat16 *o)
+{
+    o[f] = __float2bfloat16_rn((float)v);
+    double freq = 1.0;
+    for (int i = 0; i < E; ++i) {
+        // the argument is formed in double and rounded once (error <= 2^-24 * |arg|, far below the bf16 step of
+        // the result); fp32 sincosf with full range reduction instead of the double one: B200's fp64 rate is low
+        float sn, cs;
+        sincosf((float)(freq * v), &sn, &cs);
+        o[(2 * i + 1) * 3 + f] = __float2bfloat16_rn(sn);
+        o[(2 * i + 2) * 3 + f] = __float2bfloat16_rn(cs);
+        freq *= 2.0;
+    }
+}
+
+// coordinate f of the unit view direction d / |d|, |d| = sqrt((d0^2 + d1^2) + d2^2) in float64 with every operation
+// rounded (no FMA contraction): what numpy computes elementwise
+__device__ __forceinline__ double unit_coord(const double (&d)[3], int f)
+{
+    const double n2 = __dadd_rn(__dadd_rn(__dmul_rn(d[0], d[0]), __dmul_rn(d[1], d[1])), __dmul_rn(d[2], d[2]));
+    return __ddiv_rn(d[f], __dsqrt_rn(n2));
+}
+
+// one thread per (sample, coordinate).  Ed >= 0 appends the view direction's encoding PE(u, Ed) after PE(x, E).
 template <typename T, bool CAM>
 __global__ void sample_encode_kernel(const T *__restrict__ o, const T *__restrict__ d,
-                                     const T *__restrict__ t, const CamDev cam, int R, int S, int E,
+                                     const T *__restrict__ t, const CamDev cam, int R, int S, int E, int Ed,
                                      float *__restrict__ X, float *__restrict__ dists, __nv_bfloat16 *__restrict__ Xb, int ldb)
 {
     long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -42,11 +81,11 @@ __global__ void sample_encode_kernel(const T *__restrict__ o, const T *__restric
     long long smp = e / 3;
     int f = (int)(e % 3);
     int r = (int)(smp / S), s = (int)(smp % S);
-    const int C = 3 * (1 + 2 * E);
-    double tt, tnext = 0.0, v;
+    const int P = 3 * (1 + 2 * E), C = P + (Ed >= 0 ? 3 * (1 + 2 * Ed) : 0);
+    double tt, tnext = 0.0, v, dd[3];
     if (CAM) {   // rays and depths from the pose (camera.cuh): float64 values in get_rays' / linspace's operation order
         const long long q = cam_pixel(cam, r);
-        double oo[3], dd[3];
+        double oo[3];
         cam_ray_f64(cam, q, oo, dd);
         tt = cam_t_f64(cam, q, s, S);
         if (s + 1 < S) tnext = cam_t_f64(cam, q, s + 1, S);
@@ -55,34 +94,19 @@ __global__ void sample_encode_kernel(const T *__restrict__ o, const T *__restric
         tt = (double)t[smp];
         if (s + 1 < S) tnext = (double)t[smp + 1];
         v = (double)o[r * 3 + f] + (double)d[r * 3 + f] * tt;
+        if (Ed >= 0)
+            for (int k = 0; k < 3; ++k) dd[k] = (double)d[r * 3 + k];
     }
     if (Xb) {
-        // the wide tensor-core path's operand layout: bf16 rows of ldb columns, the float value rounded once more
         __nv_bfloat16 *x = Xb + smp * ldb;
-        x[f] = __float2bfloat16_rn((float)v);
-        double freq = 1.0;
-        for (int i = 0; i < E; ++i) {
-            // the argument is formed in double and rounded once (error <= 2^-24 * |arg|, far below the bf16 step of
-            // the result); fp32 sincosf with full range reduction instead of the double one: B200's fp64 rate is low
-            float sn, cs;
-            sincosf((float)(freq * v), &sn, &cs);
-            x[(2 * i + 1) * 3 + f] = __float2bfloat16_rn(sn);
-            x[(2 * i + 2) * 3 + f] = __float2bfloat16_rn(cs);
-            freq *= 2.0;
-        }
+        encode_coord(v, E, f, x);
+        if (Ed >= 0) encode_coord(unit_coord(dd, f), Ed, f, x + P);
         if (f == 0)
             for (int c = C; c < ldb; ++c) x[c] = __float2bfloat16_rn(0.0f);
     } else {
-    float *x = X + smp * C;
-    x[f] = (float)v;
-    double freq = 1.0;
-    for (int i = 0; i < E; ++i) {
-        double sn, cs;
-        sincos(freq * v, &sn, &cs);
-        x[(2 * i + 1) * 3 + f] = (float)sn;
-        x[(2 * i + 2) * 3 + f] = (float)cs;
-        freq *= 2.0;
-    }
+        float *x = X + smp * C;
+        encode_coord(v, E, f, x);
+        if (Ed >= 0) encode_coord(unit_coord(dd, f), Ed, f, x + P);
     }
     if (f == 0 && dists) dists[smp] = (s + 1 < S) ? (float)(tnext - tt) : (float)1e8;
 }
@@ -99,33 +123,34 @@ int lnb_launch_pos_encoding(lnb_ctx *ctx, const double *x, long long n, int F, i
 }
 
 int lnb_launch_sample_encode(lnb_ctx *ctx, const void *o, const void *d, const void *t, int f64,
-                             int R, int S, int E, float *X, float *dists)
+                             int R, int S, int E, int Ed, float *X, float *dists)
 {
-    return lnb_launch_sample_encode_bf16(ctx, o, d, t, f64, R, S, E, X, dists, nullptr, 0);
+    return lnb_launch_sample_encode_bf16(ctx, o, d, t, f64, R, S, E, Ed, X, dists, nullptr, 0);
 }
 
-// the same, writing either fp32 features X [N][3+6E] or (Xb != NULL) bf16 rows Xb [N][ldb], zero beyond 3+6E
+// the same, writing either fp32 features X [N][C] or (Xb != NULL) bf16 rows Xb [N][ldb], zero beyond C
+// (C = 3+6E, plus 3+6Ed with directions)
 int lnb_launch_sample_encode_bf16(lnb_ctx *ctx, const void *o, const void *d, const void *t, int f64,
-                                  int R, int S, int E, float *X, float *dists, void *Xb, int ldb)
+                                  int R, int S, int E, int Ed, float *X, float *dists, void *Xb, int ldb)
 {
     long long tot = (long long)R * S * 3;
     if (tot <= 0) return LNB_OK;
     const unsigned blocks = (unsigned)((tot + 255) / 256);
     if (f64)
-        sample_encode_kernel<double, false><<<blocks, 256, 0, ctx->stream>>>((const double *)o, (const double *)d, (const double *)t, CamDev{}, R, S, E, X, dists, (__nv_bfloat16 *)Xb, ldb);
+        sample_encode_kernel<double, false><<<blocks, 256, 0, ctx->stream>>>((const double *)o, (const double *)d, (const double *)t, CamDev{}, R, S, E, Ed, X, dists, (__nv_bfloat16 *)Xb, ldb);
     else
-        sample_encode_kernel<float, false><<<blocks, 256, 0, ctx->stream>>>((const float *)o, (const float *)d, (const float *)t, CamDev{}, R, S, E, X, dists, (__nv_bfloat16 *)Xb, ldb);
+        sample_encode_kernel<float, false><<<blocks, 256, 0, ctx->stream>>>((const float *)o, (const float *)d, (const float *)t, CamDev{}, R, S, E, Ed, X, dists, (__nv_bfloat16 *)Xb, ldb);
     LNB_CHECK_LAUNCH();
     return LNB_OK;
 }
 
 // camera mode: the same outputs with rays and depths generated from the pose (lnb_camera)
-int lnb_launch_camera_encode(lnb_ctx *ctx, const lnb_camera *cam, int R, int S, int E, float *X, float *dists, void *Xb, int ldb)
+int lnb_launch_camera_encode(lnb_ctx *ctx, const lnb_camera *cam, int R, int S, int E, int Ed, float *X, float *dists, void *Xb, int ldb)
 {
     long long tot = (long long)R * S * 3;
     if (tot <= 0) return LNB_OK;
     const unsigned blocks = (unsigned)((tot + 255) / 256);
-    sample_encode_kernel<double, true><<<blocks, 256, 0, ctx->stream>>>(nullptr, nullptr, nullptr, make_cam_dev(*cam), R, S, E, X, dists, (__nv_bfloat16 *)Xb, ldb);
+    sample_encode_kernel<double, true><<<blocks, 256, 0, ctx->stream>>>(nullptr, nullptr, nullptr, make_cam_dev(*cam), R, S, E, Ed, X, dists, (__nv_bfloat16 *)Xb, ldb);
     LNB_CHECK_LAUNCH();
     return LNB_OK;
 }

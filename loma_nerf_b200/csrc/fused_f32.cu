@@ -545,8 +545,9 @@ int lnb_fused_f32_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a,
     p.X = a->X; p.dists = a->dists;
     if (rays) {
         float *Xe = (float *)lnb_arena_take(ctx, (size_t)N * c_in * sizeof(float)), *de = (float *)lnb_arena_take(ctx, (size_t)R * S * sizeof(float));
-        if (cam) LNB_TRY(lnb_launch_camera_encode(ctx, a->cam, R, S, a->pe_bands, Xe, de, nullptr, 0));
-        else LNB_TRY(lnb_launch_sample_encode(ctx, a->rays_o, a->rays_d, a->t, a->ray_dtype == LNB_RAY_F64, R, S, a->pe_bands, Xe, de));
+        const int Ed = lnb_rays_dir_bands(c_in, a->pe_bands);
+        if (cam) LNB_TRY(lnb_launch_camera_encode(ctx, a->cam, R, S, a->pe_bands, Ed, Xe, de, nullptr, 0));
+        else LNB_TRY(lnb_launch_sample_encode(ctx, a->rays_o, a->rays_d, a->t, a->ray_dtype == LNB_RAY_F64, R, S, a->pe_bands, Ed, Xe, de));
         p.X = Xe; p.dists = de;
     }
     p.x_vec4 = (reinterpret_cast<uintptr_t>(p.X) & 15) == 0 && ((long long)p.rows_per_tile * c_in) % 4 == 0;

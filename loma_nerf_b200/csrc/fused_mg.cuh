@@ -77,7 +77,7 @@ __device__ __forceinline__ void tmem_st4(uint32_t taddr, uint4 v)   // one 8-fea
 }
 template <int HP> constexpr int mg_max_groups() { return HP <= 32 ? MG_MAX_GROUPS : 4; }   // registers: 64 K / (groups x 128 threads)
 
-template <bool RAYS, int HP>
+template <bool RAYS, int HP, bool DIRS = false>
 __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel(const TcParams p)
 {
     using LY = TcLayout<HP>;
@@ -245,11 +245,14 @@ __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel
             const int nxt = tile + (int)gridDim.x * NG;
             if (nxt < p.n_tiles) { const void *src = x_src(p, nxt, c_in, lead, bytes); bulk_prefetch_l2(src, bytes); }
         }
-        float x[3], my_dist, tg[3];
-        sample_inputs<RAYS>(p, row0, tile * p.G, tid, smp, ray_l, live, x, my_dist, tg);
+        float x[3], my_dist, tg[3], u[3];
+        sample_inputs<RAYS, DIRS>(p, row0, tile * p.G, tid, smp, ray_l, live, x, my_dist, tg, u);
         // A_0 goes to shared memory (for the weight gradient, MN-major) and to TMEM (the layer-0 MMA's A operand)
         auto store_a0 = [&](int c8, uint4 q) { *row_ptr(a_buf(0), c8) = q; tmem_st4(a_tm + (uint32_t)c8 * 4u, q); };
-        if (RAYS) {
+        if (DIRS) {
+            // ---- features from rays with the view direction
+            pack_pe_dirs(x, u, p.pe_bands, p.dir_bands, store_a0);
+        } else if (RAYS) {
             // ---- features from rays: the positional encoding, written straight into A_0
             float sn[3], cs[3];
 #pragma unroll

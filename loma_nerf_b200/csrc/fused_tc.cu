@@ -68,6 +68,7 @@ struct TcParams {
     // rays mode (X == NULL): features are computed in the kernel from rays and sample depths
     const void *rays_o, *rays_d, *tvals; // [R][3], [R][3], [R][S]; float64 when ray_f64 else float32
     int ray_f64, pe_bands;
+    int dir_bands;     // view-direction bands E_d of a DIRS instantiation (dims[0] == 6 + 6 pe_bands + 6 E_d)
     int cam_mode;      // rays and depths generated from `cam` instead of read from rays_o / rays_d / tvals
     CamF32 cam;
     int *t_dev;        // optimiser step counter, incremented once per launch (or NULL)
@@ -334,10 +335,10 @@ __device__ __forceinline__ const void *x_src(const TcParams &p, int tile, int c_
 // This row's inputs other than its features, loaded early (latency-tolerant, consumed after the MLP forward): the sample
 // spacing `dist` and, at a ray's first sample, the ray's target colour.  From rays (RAYS) also the sample point x:
 // pts = o + d t (train_nerf.py:289-299), dist = t[s+1] - t[s], last 1e8 (train_nerf.py:306-311).  x and dist stay 0 in a
-// row past the tile's live samples.
-template <bool RAYS>
+// row past the tile's live samples.  DIRS: also the ray's unit direction u = d / |d| (0 in a row that is not live).
+template <bool RAYS, bool DIRS>
 __device__ __forceinline__ void sample_inputs(const TcParams &p, long long row0, int ray0, int tid, int smp, int ray_l, bool live,
-                                              float (&x)[3], float &dist, float (&tg)[3])
+                                              float (&x)[3], float &dist, float (&tg)[3], float (&u)[3])
 {
     const int S = p.S;
     dist = 0.0f;
@@ -350,6 +351,7 @@ __device__ __forceinline__ void sample_inputs(const TcParams &p, long long row0,
         }
     }
     x[0] = x[1] = x[2] = 0.0f;
+    if (DIRS) u[0] = u[1] = u[2] = 0.0f;
     if (!RAYS || !live) return;
     const long long ray = ray0 + ray_l;
     if (p.cam_mode) {
@@ -374,6 +376,7 @@ __device__ __forceinline__ void sample_inputs(const TcParams &p, long long row0,
         for (int k = 0; k < 3; ++k) {
             const float dk = fmaf(dx, c.c2w[4 * k], fmaf(dy, c.c2w[4 * k + 1], 0.0f - c.c2w[4 * k + 2]));
             x[k] = fmaf(dk, tt, c.c2w[4 * k + 3]);
+            if (DIRS) u[k] = dk;
         }
     } else if (p.ray_f64) {
         const double *o = reinterpret_cast<const double *>(p.rays_o) + ray * 3;
@@ -383,6 +386,8 @@ __device__ __forceinline__ void sample_inputs(const TcParams &p, long long row0,
         dist = smp + 1 < S ? (float)(__ldg(tv + 1) - tt) : 1e8f;
 #pragma unroll
         for (int c = 0; c < 3; ++c) x[c] = (float)(__ldg(o + c) + __ldg(d + c) * tt);
+        if (DIRS)
+            for (int c = 0; c < 3; ++c) u[c] = (float)__ldg(d + c);
     } else {
         const float *o = reinterpret_cast<const float *>(p.rays_o) + ray * 3;
         const float *d = reinterpret_cast<const float *>(p.rays_d) + ray * 3;
@@ -391,6 +396,13 @@ __device__ __forceinline__ void sample_inputs(const TcParams &p, long long row0,
         dist = smp + 1 < S ? __ldg(tv + 1) - tt : 1e8f;
 #pragma unroll
         for (int c = 0; c < 3; ++c) x[c] = fmaf(__ldg(d + c), tt, __ldg(o + c));
+        if (DIRS)
+            for (int c = 0; c < 3; ++c) u[c] = __ldg(d + c);
+    }
+    if (DIRS) {
+        const float inv = rsqrtf(fmaf(u[0], u[0], fmaf(u[1], u[1], u[2] * u[2])));
+#pragma unroll
+        for (int c = 0; c < 3; ++c) u[c] *= inv;
     }
 }
 
@@ -435,6 +447,64 @@ __device__ __forceinline__ void pack_pe(const float (&x)[3], float (&sn)[3], flo
         }
     }
     put(31, closed ? 0u : pack_bf16(pend, 1.0f));
+}
+
+// The same with the view direction (rays / camera mode with dims[0] = (3 + 6E) + (3 + 6E_d)): the stream of 3-vectors
+// x, its 2E band slots, u, its 2E_d band slots, then the ones column, into this row's first (dims[0] + 8) / 8 slabs of A_0.
+// x starts a pair, so its bands leave their last cosine pending as in pack_pe; the position part is odd-long, so u starts
+// mid-pair (pend, u0) (u1, u2) and its bands pair up without a pending element; the ones column (feature dims[0], even)
+// opens a pair.  The pair index depends on E, so the four pairs of a slab are selected at run time.  u = d rsqrt(d.d) in
+// fp32 is within ~1e-7 of the float64 unit vector, and |u| <= 1 keeps pe_sincos at its base error (~2^-21) without
+// range reduction; angle doubling amplifies that by 2^(E_d - 1) <= 8 for E_d <= 4: ~1e-6, far below the bf16 step.
+template <class Store>
+__device__ __forceinline__ void pack_pe_dirs(const float (&x)[3], const float (&u)[3], int pe_bands, int dir_bands, Store &&store)
+{
+    uint32_t q4[4] = {0u, 0u, 0u, 0u};
+    int j = 0;                                     // the next pair (features 2j, 2j+1)
+    auto put = [&](uint32_t v) {
+        const int k = j & 3;
+        q4[0] = k == 0 ? v : q4[0];
+        q4[1] = k == 1 ? v : q4[1];
+        q4[2] = k == 2 ? v : q4[2];
+        q4[3] = k == 3 ? v : q4[3];
+        if (k == 3) {
+            store(j >> 2, make_uint4(q4[0], q4[1], q4[2], q4[3]));
+            q4[0] = q4[1] = q4[2] = q4[3] = 0u;
+        }
+        ++j;
+    };
+    float sn[3], cs[3];
+#pragma unroll
+    for (int c = 0; c < 3; ++c) pe_sincos(x[c], &sn[c], &cs[c]);
+    put(pack_bf16(x[0], x[1]));
+    float pend = x[2];
+    for (int i = 0; i < pe_bands; ++i) {
+        put(pack_bf16(pend, sn[0]));
+        put(pack_bf16(sn[1], sn[2]));
+        put(pack_bf16(cs[0], cs[1]));
+        pend = cs[2];
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+            const float s2 = 2.0f * sn[c] * cs[c], c2 = fmaf(-2.0f * sn[c], sn[c], 1.0f);
+            sn[c] = s2; cs[c] = c2;
+        }
+    }
+#pragma unroll
+    for (int c = 0; c < 3; ++c) pe_sincos(u[c], &sn[c], &cs[c]);
+    put(pack_bf16(pend, u[0]));
+    put(pack_bf16(u[1], u[2]));
+    for (int i = 0; i < dir_bands; ++i) {
+        put(pack_bf16(sn[0], sn[1]));
+        put(pack_bf16(sn[2], cs[0]));
+        put(pack_bf16(cs[1], cs[2]));
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+            const float s2 = 2.0f * sn[c] * cs[c], c2 = fmaf(-2.0f * sn[c], sn[c], 1.0f);
+            sn[c] = s2; cs[c] = c2;
+        }
+    }
+    put(pack_bf16(1.0f, 0.0f));
+    while (j & 3) put(0u);
 }
 
 // Features mode: this row's c_in fp32 features (xr) -> its first (c_in + 8) / 8 slabs of A_0, through store(slab, its
@@ -639,7 +709,7 @@ __device__ __forceinline__ void relu_adjoint(const uint32_t (&v)[HP / 16][16], c
 // FWD: the forward-only (render) form, compiled separately: nothing of the backward pass in its register budget.  Its
 // launch bounds are the CTAs per SM that tensor memory admits (512 columns / 64 per CTA = 8; 4 for the 64-wide form), not
 // more: a ninth CTA could never allocate its columns and the tighter register budget only bought a spill.
-template <bool RAYS, int HP, bool FWD>
+template <bool RAYS, int HP, bool FWD, bool DIRS = false>
 __global__ void __launch_bounds__(TILE, FWD ? (HP == 64 ? 4 : 8) : 1) fused_v1_kernel(const TcParams p)
 {
     using LY = TcLayout<HP>;
@@ -772,18 +842,21 @@ __global__ void __launch_bounds__(TILE, FWD ? (HP == 64 ? 4 : 8) : 1) fused_v1_k
         const int ray0 = tile * p.G;      // = row0 / S: a tile holds G whole rays (R is an int)
         CLK(15);
         const bool live = tid < rays_here * S;
-        float x[3], my_dist, tg[3];
-        sample_inputs<RAYS>(p, row0, ray0, tid, smp, ray_l, live, x, my_dist, tg);
+        float x[3], my_dist, tg[3], u[3];
+        sample_inputs<RAYS, DIRS>(p, row0, ray0, tid, smp, ray_l, live, x, my_dist, tg, u);
         auto store_a0 = [&](int c8, uint4 q) { *row_ptr(a_buf(0), c8) = q; };
         const int a0s = (c_in + 8) >> 3;   // slabs holding features 0..c_in (the ones column included)
         if (RAYS) {
             // ---- features from rays: the positional encoding, written straight into A_0
             float sn[3], cs[3];
+            if (!DIRS) {
 #pragma unroll
-            for (int c = 0; c < 3; ++c) pe_sincos(x[c], &sn[c], &cs[c]);
+                for (int c = 0; c < 3; ++c) pe_sincos(x[c], &sn[c], &cs[c]);
+            }
             if (dw_pending) { mbar_wait(bar_dw, dwphase); dwphase ^= 1; dw_pending = false; tc_fence_after(); }
             CLK(12);
-            pack_pe(x, sn, cs, p.pe_bands, a0s, store_a0);
+            if (DIRS) pack_pe_dirs(x, u, p.pe_bands, p.dir_bands, store_a0);
+            else pack_pe(x, sn, cs, p.pe_bands, a0s, store_a0);
         } else {
             // ---- features: wait for the TMA, convert this thread's row to bf16 slabs
             int lead; uint32_t bytes;
@@ -1279,8 +1352,10 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
     if (nerf && (S > TILE || N != (long long)R * S)) return unsupported("needs S <= 128 and n_rows == R*S");
     const bool cam = a->X == nullptr && a->rays_o == nullptr && a->cam != nullptr;
     const bool rays = a->X == nullptr && (a->rays_o != nullptr || cam);
-    if (rays && (!nerf || (!cam && (!a->rays_d || !a->t)) || mlp->dims[0] != 3 + 6 * a->pe_bands))
-        return unsupported("rays mode needs rays_o, rays_d, t (or a camera) and dims[0] == 3 + 6 * pe_bands");
+    const int dir_bands = rays ? lnb_rays_dir_bands(mlp->dims[0], a->pe_bands) : LNB_DIRS_NONE;
+    if (rays && (!nerf || (!cam && (!a->rays_d || !a->t)) || dir_bands == LNB_DIRS_BAD))
+        return unsupported("rays mode needs rays_o, rays_d, t (or a camera) and dims[0] == 3 + 6 * pe_bands (+ 3 + 6 * E_dir)");
+    const bool dirs = dir_bands >= 0;
     if (cam && (long long)a->cam->width * a->cam->height >= (1ll << 31)) return unsupported("camera: more than 2^31 pixels");
     if (!nerf && N != R) return unsupported("needs n_rows == R");
     if (a->rows > N) return unsupported("rows > n_rows");
@@ -1292,6 +1367,7 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
     fill_layout(p, mlp, K0P);
     p.X = a->X; p.dists = a->dists; p.target = a->target; p.ws = a->ws; p.bs = a->bs;
     p.rays_o = a->rays_o; p.rays_d = a->rays_d; p.tvals = a->t; p.ray_f64 = a->ray_dtype == LNB_RAY_F64; p.pe_bands = a->pe_bands;
+    p.dir_bands = dirs ? dir_bands : 0;
     if (cam) {
         const lnb_camera &c = *a->cam;
         p.cam_mode = 1;
@@ -1321,9 +1397,9 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
     }
     void (*const kern)(TcParams) = with_hp(HP, [&](auto hp) -> void (*)(TcParams) {
         constexpr int H = decltype(hp)::value;
-        if (mg) return rays ? fused_mg_kernel<true, H> : fused_mg_kernel<false, H>;
-        if (grad) return rays ? fused_v1_kernel<true, H, false> : fused_v1_kernel<false, H, false>;
-        return rays ? fused_v1_kernel<true, H, true> : fused_v1_kernel<false, H, true>;
+        if (mg) return dirs ? fused_mg_kernel<true, H, true> : rays ? fused_mg_kernel<true, H> : fused_mg_kernel<false, H>;
+        if (grad) return dirs ? fused_v1_kernel<true, H, false, true> : rays ? fused_v1_kernel<true, H, false> : fused_v1_kernel<false, H, false>;
+        return dirs ? fused_v1_kernel<true, H, true, true> : rays ? fused_v1_kernel<true, H, true> : fused_v1_kernel<false, H, true>;
     });
     size_t smem = 0;
     int grid = 0, ng = 1;
@@ -1334,8 +1410,8 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
             while (n > 1 && (MG::total(L, c_in, K0P, rays, n) > 232448 || MG::tmem_need(L, K0P, n) > 512)) --n;
             return n;
         });
-        static int mg_regs[2][3] = {{0, 0, 0}, {0, 0, 0}};    // registers per thread of each instantiation, asked once
-        int &regs = mg_regs[rays ? 1 : 0][HP / 32];
+        static int mg_regs[3][3] = {};    // registers per thread of each instantiation (features, rays, rays + directions), asked once
+        int &regs = mg_regs[dirs ? 2 : (rays ? 1 : 0)][HP / 32];
         if (regs == 0) {
             cudaFuncAttributes fa;
             LNB_CUDA(cudaFuncGetAttributes(&fa, kern));
@@ -1398,8 +1474,8 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
             LNB_CHECK_LAUNCH();
         }
         // the dynamic shared-memory limit of each kernel instantiation (kind, input, HP) on each device: raised only when it grows
-        static size_t smem_set[3][2][3][64] = {};
-        size_t &lim = smem_set[mg ? 0 : (grad ? 1 : 2)][rays ? 1 : 0][HP / 32][ctx->device & 63];
+        static size_t smem_set[3][3][3][64] = {};
+        size_t &lim = smem_set[mg ? 0 : (grad ? 1 : 2)][dirs ? 2 : (rays ? 1 : 0)][HP / 32][ctx->device & 63];
         if (smem > lim || ctx->device > 63) { LNB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); lim = smem; }
         lnb_prof_begin(ctx, mg ? (rays ? "fused_mg_kernel<rays>" : "fused_mg_kernel<features>")
                               : (rays ? "fused_v1_kernel<rays>" : "fused_v1_kernel<features>"));      // the symbols ncu lists

@@ -187,13 +187,25 @@ int lnb_fused_f32_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a,
 int lnb_step_f32_fused(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf, int overwrite);   // validated (api_flat.cu)
 
 // ---- encode.cu / optim.cu ---------------------------------------------------------------------
+// Rays and camera mode: the input form the MLP's input width selects (include/loma_nerf_b200.h).  Returns the direction
+// band count E_d >= 0 when c_in == (3 + 6E) + (3 + 6E_d), LNB_DIRS_NONE when c_in == 3 + 6E (positions only), and
+// LNB_DIRS_BAD for any other width.  One width is odd, the other even: they cannot be confused.
+constexpr int LNB_DIRS_NONE = -1, LNB_DIRS_BAD = -2;
+inline int lnb_rays_dir_bands(int c_in, int E)
+{
+    if (E < 0) return LNB_DIRS_BAD;
+    const int rest = c_in - (3 + 6 * E);
+    if (rest == 0) return LNB_DIRS_NONE;
+    return rest >= 3 && (rest - 3) % 6 == 0 ? (rest - 3) / 6 : LNB_DIRS_BAD;
+}
+// Ed: direction bands (LNB_DIRS_NONE: positions only); rows are [PE(x, E) | PE(u, Ed)]
 int lnb_launch_pos_encoding(lnb_ctx *ctx, const double *x, long long n, int F, int E, float *out);
 int lnb_launch_sample_encode(lnb_ctx *ctx, const void *o, const void *d, const void *t, int f64,
-                             int R, int S, int E, float *X, float *dists);
+                             int R, int S, int E, int Ed, float *X, float *dists);
 int lnb_launch_sample_encode_bf16(lnb_ctx *ctx, const void *o, const void *d, const void *t, int f64,
-                                  int R, int S, int E, float *X, float *dists, void *Xb, int ldb);
+                                  int R, int S, int E, int Ed, float *X, float *dists, void *Xb, int ldb);
 // camera mode (lnb_camera): features / dists (or the wide path's bf16 rows) straight from the pose
-int lnb_launch_camera_encode(lnb_ctx *ctx, const lnb_camera *cam, int R, int S, int E, float *X, float *dists, void *Xb, int ldb);
+int lnb_launch_camera_encode(lnb_ctx *ctx, const lnb_camera *cam, int R, int S, int E, int Ed, float *X, float *dists, void *Xb, int ldb);
 int lnb_launch_adam(lnb_ctx *ctx, float *p, const float *g, float *m, float *v, long long n, int t,
                     double lr, double b1, double b2, double eps);
 int lnb_launch_adam_dev(lnb_ctx *ctx, float *p, const float *g, float *m, float *v, long long n,

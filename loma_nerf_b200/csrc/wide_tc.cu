@@ -872,12 +872,13 @@ int lnb_wide_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, b
     float *dzh = grad ? (float *)take((size_t)N * 16) : nullptr;
     float *head = (float *)take((size_t)N * 16);
     const float *X = a->X, *dists = a->dists;
-    if (rays) {   // sample positions and positional encoding straight into the bf16 operand of layer 0
+    if (rays) {   // sample positions (and view directions) and their encoding straight into the bf16 operand of layer 0
         float *de = (float *)take((size_t)R * S * 4);
+        const int Ed = lnb_rays_dir_bands(c_in, a->pe_bands);
         if (N > 0 && cam)
-            LNB_TRY(lnb_launch_camera_encode(ctx, a->cam, R, S, a->pe_bands, nullptr, de, H[0], in_pad[0]));
+            LNB_TRY(lnb_launch_camera_encode(ctx, a->cam, R, S, a->pe_bands, Ed, nullptr, de, H[0], in_pad[0]));
         else if (N > 0)
-            LNB_TRY(lnb_launch_sample_encode_bf16(ctx, a->rays_o, a->rays_d, a->t, a->ray_dtype == LNB_RAY_F64, R, S, a->pe_bands, nullptr, de, H[0],
+            LNB_TRY(lnb_launch_sample_encode_bf16(ctx, a->rays_o, a->rays_d, a->t, a->ray_dtype == LNB_RAY_F64, R, S, a->pe_bands, Ed, nullptr, de, H[0],
                                                   in_pad[0]));
         dists = de;
     }

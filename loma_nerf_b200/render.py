@@ -27,10 +27,10 @@ def compute_psnr(img1, img2, max_val=1.0):
         return 20 * np.log10(max_val / np.sqrt(mse))
 
 
-def render_rays(ctx, dims, ws, bs, rays_o, rays_d, t, pe_bands, path="tc", rays_per_call=1 << 18):
+def render_rays(ctx, dims, ws, bs, rays_o, rays_d, t, pe_bands, path="tc", rays_per_call=1 << 18, dir_bands=None):
     """Colours [R][3] (numpy float32) of R rays; rays_o/rays_d [R][3] and t [R][S] numpy (float64 as
     the reference makes them, or float32).  Host buffers in, host buffer out, chunked so the device
-    staging stays bounded."""
+    staging stays bounded.  dir_bands: the net also takes the view direction (Context.nerf_step_rays)."""
     R = rays_o.shape[0]
     out = np.empty((R, 3), np.float32)
     ws = np.ascontiguousarray(ws, np.float32)
@@ -39,21 +39,22 @@ def render_rays(ctx, dims, ws, bs, rays_o, rays_d, t, pe_bands, path="tc", rays_
         r1 = min(R, r0 + rays_per_call)
         res = ctx.nerf_step_rays(dims, np.ascontiguousarray(rays_o[r0:r1]), np.ascontiguousarray(rays_d[r0:r1]),
                                  np.ascontiguousarray(t[r0:r1]), pe_bands, ws, bs, target=None, grad=False,
-                                 outputs=("color",), path=path)
+                                 outputs=("color",), path=path, dir_bands=dir_bands)
         out[r0:r1] = res["color"]
     return out
 
 
 def render_frame(ctx, dims, ws, bs, height, width, normalized_K, c2w_pose, n_samples, pe_bands, near=2.0, far=6.0,
-                 path="tc"):
+                 path="tc", dir_bands=None):
     """One H x W frame: t = linspace(near, far, S) for every ray (train_nerf.py:589-605)."""
     o, d = get_rays(height, width, normalized_K, c2w_pose)
     t = np.broadcast_to(np.linspace(near, far, n_samples)[None, :], (o.shape[0], n_samples))
-    return render_rays(ctx, dims, ws, bs, o, d, np.ascontiguousarray(t), pe_bands, path=path).reshape(height, width, 3)
+    return render_rays(ctx, dims, ws, bs, o, d, np.ascontiguousarray(t), pe_bands, path=path,
+                       dir_bands=dir_bands).reshape(height, width, 3)
 
 
 def render_frame_device(ctx, dims, ws_dev, bs_dev, height, width, normalized_K, c2w_pose, n_samples, pe_bands, near=2.0, far=6.0,
-                        path="tc", out_u8=None, color=None, rays_per_call=None):
+                        path="tc", out_u8=None, color=None, rays_per_call=None, dir_bands=None):
     """One frame with NOTHING per ray crossing the bus: the pose goes in (camera mode: rays and the linspace depths of
     train_nerf.py:589-605 are generated inside the kernels), a uint8 H x W x 3 frame (torch cuda tensor) comes out.
     ws_dev / bs_dev are cuda tensors in the padded layout."""
@@ -67,7 +68,7 @@ def render_frame_device(ctx, dims, ws_dev, bs_dev, height, width, normalized_K, 
         r1 = min(n, r0 + step)
         cam = api.make_camera(c2w_pose, normalized_K, width, height, near=near, far=far, first_pixel=r0)
         ctx.nerf_step_camera(dims, cam, r1 - r0, n_samples, pe_bands, ws_dev, bs_dev, target=None, grad=False,
-                             outputs=("color",), out={"color": color[r0:r1]}, path=path)
+                             outputs=("color",), out={"color": color[r0:r1]}, path=path, dir_bands=dir_bands)
     return ctx.color_to_u8(color, out_u8).reshape(height, width, 3)
 
 
@@ -135,7 +136,7 @@ def write_mjpeg_avi(path, frames, fps=30, quality=90):
 
 
 def render_video(ctx, dims, ws, bs, height, width, normalized_K, poses, n_samples, pe_bands, out_dir=None, near=2.0, far=6.0,
-                 path="tc", ground_truth=None, fps=30, frame_fn=None):
+                 path="tc", ground_truth=None, fps=30, frame_fn=None, dir_bands=None):
     """What make_nerf_video.py is named for but does not do (it stitches ground-truth PNGs): render one frame per
     camera pose with the trained weights, optionally score each against its ground-truth image
     (train_nerf.py:163-183) and write frame_%04d.png, an animated orbit.gif and a Motion-JPEG orbit.avi into out_dir (PIL
@@ -145,7 +146,8 @@ def render_video(ctx, dims, ws, bs, height, width, normalized_K, poses, n_sample
     frames, psnr = [], ([] if ground_truth is not None else None)
     for i, pose in enumerate(poses):
         img = frame_fn(i, pose) if frame_fn else render_frame(ctx, dims, ws, bs, height, width, normalized_K, np.asarray(pose, np.float64),
-                                                            n_samples, pe_bands, near=near, far=far, path=path)
+                                                            n_samples, pe_bands, near=near, far=far, path=path,
+                                                            dir_bands=dir_bands)
         img = np.clip(np.asarray(img, np.float32), 0.0, 1.0)
         if ground_truth is not None:
             psnr.append(float(compute_psnr(img, ground_truth[i])))
