@@ -164,6 +164,32 @@ typedef struct {
  * (z ^= z >> 30; z *= 0xBF58476D1CE4E5B9; z ^= z >> 27; z *= 0x94D049BB133111EB; z ^= z >> 31).  Host-callable. */
 LNB_API double lnb_uniform(unsigned long long seed, long long pixel, int s);
 
+/* HIERARCHICAL SAMPLING (the NeRF paper's sample_pdf): importance sampling of fine depths from a coarse pass's compositing
+ * weights, device pointers, float64 arithmetic.  t [R][S] float64 (the coarse depths), w [R][S] float32 (the coarse pass's
+ * weights_samples: lnb_step_args.weights, or lnb_trainer_step_weights), out [R][S + n_fine] float64.  Row r:
+ *   bins      m_k = 0.5 * (t_k + t_{k+1}), k = 0 .. S-2;
+ *   weights   v_j = (double)w_{j+1} + 1e-5, j = 0 .. S-3 (the first and last weights are dropped, as in the paper);
+ *   cdf       c_0 = 0, c_{j+1} = c_j + v_j summed sequentially in j, cdf_k = c_k / c_{S-2} (cdf_0 = 0, cdf_{S-2} = 1
+ *             exactly; the paper normalises before it sums, the same mathematically);
+ *   positions u_i, i = 0 .. n_fine-1: stratified == 0: np.linspace(0.0, 1.0, n_fine) bit for bit (i * (1 / (n_fine-1)),
+ *             the last value exactly 1; [0.0] for n_fine = 1); stratified != 0: u_i = (i + xi_i) / n_fine with
+ *             xi_i = lnb_uniform(seed, ray0 + r, i);
+ *   ind       = the number of k with cdf_k <= u_i (numpy's searchsorted(side="right")),
+ *             below = max(ind-1, 0), above = min(ind, S-2);
+ *   d         = cdf_above - cdf_below, d = 1 when d < 1e-5;  tau = (u_i - cdf_below) / d;
+ *   x_i       = m_below + tau * (m_above - m_below);
+ *   out row r = the S + n_fine values {t_k} U {x_i} in ascending order (np.sort of the concatenation; only the values are
+ *             defined, so ties need no rule).
+ * Every operation is float64 and rounded, with no FMA contraction: the rows are bit-equal to that numpy statement.  The
+ * weights are constants (no gradient flows through the sampled depths, as in the paper) and are expected >= 0.  ray0 makes
+ * a chunked or sharded call reproduce the whole-batch call bit for bit (for contiguous camera chunks: first_pixel).
+ * LNB_ERR_ARG for null pointers, S < 3 (no interior weights), n_fine < 1 or S + n_fine > 4096; R = 0 is a no-op (the
+ * pointers of an empty batch may be NULL).
+ * Camera mode on the tensor-core path forms its depths in float32, while lnb_camera_rays returns the float64 ones this
+ * sampler bins: the two differ by at most one float32 ulp, far below the bf16 error of those kernels. */
+LNB_API int lnb_sample_pdf(lnb_ctx *ctx, const double *t, const float *w, int R, int S, int n_fine,
+                           int stratified, unsigned long long seed, long long ray0, double *out);
+
 /* One forward(+backward) problem in the reference's layout.  N = R*S samples.  Pointers are
  * DEVICE pointers for lnb_nerf_step / lnb_fit_step and HOST pointers for the *_host variants.
  * Any output pointer may be NULL (not produced).  Accumulating outputs (+=) are marked. */
@@ -310,6 +336,11 @@ LNB_API int lnb_trainer_create(lnb_ctx *ctx, const lnb_mlp *mlp, const float *ws
                        int optimizer, double lr, double beta1, double beta2, double eps, lnb_trainer **out);
 LNB_API void lnb_trainer_destroy(lnb_trainer *t);
 LNB_API int lnb_trainer_step(lnb_trainer *t, const lnb_step_args *batch, int nerf);
+/* lnb_trainer_step, and also writes this step's forward compositing weights w_s = alpha_s * T_s (at the
+ * pre-update parameters) into weights [R][S] (device, overwritten).  nerf batches only.  On the tensor-core path the fused
+ * train kernel or the wide path writes them, whichever the step runs on; the fused exact kernel writes none, so an
+ * exact-path step with weights runs on the layerwise fp32 kernels (the same arithmetic to <= 1e-5). */
+LNB_API int lnb_trainer_step_weights(lnb_trainer *t, const lnb_step_args *batch, int nerf, float *weights);
 /* the same step with the batch in HOST memory (pinned buffers are copied from directly): stages
  * host->device, steps, returns the loss through *loss_out; synchronous */
 LNB_API int lnb_trainer_step_host(lnb_trainer *t, const lnb_step_args *batch, int nerf, float *loss_out);

@@ -104,6 +104,8 @@ def load():
     lib.lnb_color_to_u8.argtypes = [c_void_p, c_void_p, c_longlong, c_void_p]
     lib.lnb_uniform.argtypes = [ctypes.c_ulonglong, c_longlong, c_int]
     lib.lnb_uniform.restype = c_double
+    lib.lnb_sample_pdf.argtypes = [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, ctypes.c_ulonglong,
+                                   c_longlong, c_void_p]
     lib.lnb_mult_a_b.argtypes = [c_void_p, c_void_p, c_int, c_int, c_void_p, c_int, c_void_p]
     lib.lnb_adam_step.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_longlong,
                                   c_int, c_double, c_double, c_double, c_double]
@@ -116,6 +118,7 @@ def load():
     lib.lnb_trainer_destroy.restype = None
     for name in ("lnb_trainer_step", "lnb_trainer_grad"):
         getattr(lib, name).argtypes = [c_void_p, P(LnbStepArgs), c_int]
+    lib.lnb_trainer_step_weights.argtypes = [c_void_p, P(LnbStepArgs), c_int, c_void_p]
     lib.lnb_trainer_step_host.argtypes = [c_void_p, P(LnbStepArgs), c_int, P(c_float)]
     lib.lnb_trainer_submit_host.argtypes = [c_void_p, P(LnbStepArgs), c_int]
     lib.lnb_trainer_wait.argtypes = [c_void_p, P(c_float), c_int, P(c_int)]

@@ -311,15 +311,43 @@ class Context:
         return self._step(True, dims, None, ws, bs, target, None, int(R), int(S), grad, seed, outputs, out, None, path,
                           False, False, L.HEAD_NERF, pe_bands=pe_bands, camera=camera, dir_bands=dir_bands)
 
-    def camera_rays(self, camera, R, S):
-        """(rays_o, rays_d, t) float64 cuda tensors camera mode generates (for checks / hosts that want them)."""
+    def camera_rays(self, camera, R, S, out=None):
+        """(rays_o, rays_d, t) float64 cuda tensors camera mode generates (for checks / hosts that want them).
+        out=(rays_o, rays_d, t): contiguous [R][3], [R][3], [R][S] float64 cuda tensors to write instead of new ones."""
         dev = torch.device("cuda", self.device)
-        o = torch.empty((R, 3), dtype=torch.float64, device=dev)
-        d = torch.empty((R, 3), dtype=torch.float64, device=dev)
-        t = torch.empty((R, S), dtype=torch.float64, device=dev)
+        if out is None:
+            out = (torch.empty((R, 3), dtype=torch.float64, device=dev), torch.empty((R, 3), dtype=torch.float64, device=dev),
+                   torch.empty((R, S), dtype=torch.float64, device=dev))
+        o, d, t = out
+        if not all(_is_cuda(v) and v.dtype == torch.float64 and v.is_contiguous() and tuple(v.shape) == sh
+                   for v, sh in zip(out, ((R, 3), (R, 3), (R, S)))):
+            raise ValueError("camera_rays: out must be contiguous [R][3], [R][3], [R][S] float64 CUDA tensors")
         self.order_after_torch()
         self._check(self.lib.lnb_camera_rays(self.h, ctypes.byref(camera), int(R), int(S), o.data_ptr(), d.data_ptr(), t.data_ptr()))
         return o, d, t
+
+    def sample_pdf(self, t, weights, n_fine, stratified=False, seed=0, ray0=0, out=None):
+        """Hierarchical sampling (lnb_sample_pdf): n_fine depths per ray drawn by inverse transform from the piecewise-
+        constant PDF of a coarse pass's compositing weights, merged with the coarse depths and sorted.  t [R][S] float64,
+        weights [R][S] float32, CUDA tensors; returns out [R][S + n_fine] float64.  Row r of a stratified draw uses
+        lnb_uniform(seed, ray0 + r, i), so a chunk passed with its first ray's index reproduces the whole-batch call."""
+        if not (_is_cuda(t) and t.dtype == torch.float64 and t.dim() == 2 and t.is_contiguous()):
+            raise ValueError("t must be a contiguous [R][S] float64 CUDA tensor")
+        R, S = int(t.shape[0]), int(t.shape[1])
+        if not (_is_cuda(weights) and weights.dtype == torch.float32 and weights.is_contiguous()
+                and tuple(weights.shape) == (R, S)):
+            raise ValueError("weights must be a contiguous [%d][%d] float32 CUDA tensor" % (R, S))
+        n_fine = int(n_fine)
+        if out is None:
+            out = torch.empty((R, S + max(n_fine, 0)), dtype=torch.float64, device=t.device)
+        elif not (_is_cuda(out) and out.dtype == torch.float64 and out.is_contiguous()
+                  and tuple(out.shape) == (R, S + n_fine)):
+            raise ValueError("out must be a contiguous [%d][%d] float64 CUDA tensor" % (R, S + n_fine))
+        self.order_after_torch()
+        self._hold(t, weights, out)
+        self._check(self.lib.lnb_sample_pdf(self.h, t.data_ptr(), weights.data_ptr(), R, S, n_fine, int(bool(stratified)),
+                                            int(seed) & 0xFFFFFFFFFFFFFFFF, int(ray0), out.data_ptr()))
+        return out
 
     def color_to_u8(self, rgb, out=None):
         """uint8 image bytes of float colours, clamp(rgb, 0, 1) * 255 rounded (train_nerf.py:686-700), on the device."""
@@ -461,6 +489,20 @@ class Trainer:
         self._order(batch)
         self.ctx._check(self.lib.lnb_trainer_step(self.h, ctypes.byref(a), nerf))
 
+    def step_weights(self, weights, prepared=None, **batch):
+        """step(), and also writes this step's forward compositing weights w_s = alpha_s T_s (at the parameters before
+        the update) into weights, a [R][S] float32 CUDA tensor (lnb_trainer_step_weights).  nerf batches only."""
+        if prepared is not None:
+            a, nerf, batch = prepared.args, prepared.nerf, prepared.batch
+        else:
+            a, nerf = self._batch(**batch)
+        if not (_is_cuda(weights) and weights.dtype == torch.float32 and weights.is_contiguous()
+                and tuple(weights.shape) == (a.R, a.S)):
+            raise ValueError("weights must be a contiguous [%d][%d] float32 CUDA tensor" % (a.R, a.S))
+        self._order(batch)
+        self.ctx._hold(weights)
+        self.ctx._check(self.lib.lnb_trainer_step_weights(self.h, ctypes.byref(a), nerf, weights.data_ptr()))
+
     def step_host(self, prepared=None, **batch):
         """step() with the batch in host memory (numpy arrays / pinned CPU tensors): the C library
         stages it to the device, steps, and returns the loss.  Synchronous."""
@@ -534,6 +576,65 @@ class Trainer:
         loss = np.empty(1, np.float32)
         self.ctx._check(self.lib.lnb_trainer_read(self.h, ws.ctypes.data, bs.ctypes.data, loss.ctypes.data))
         return ws, bs, float(loss[0])
+
+
+class CoarseFine:
+    """Hierarchical sampling in training (the NeRF paper's coarse-to-fine step), on the device.  One step():
+      1. camera batch: the rays and the S coarse depths (lnb_camera_rays) into buffers this object owns;
+      2. a coarse Trainer.step_weights on the batch (a camera batch stays in camera mode);
+      3. sample_pdf: n_fine depths from the coarse weights, merged with the coarse ones (S + n_fine, sorted);
+      4. a fine Trainer.step in rays mode on (rays_o, rays_d, t_fine).
+    Both nets train on their own colour loss.  Nothing is synchronised with the host and, after the first step of a
+    shape, nothing is allocated: a run of steps can be captured in one CUDA graph.  The two nets may differ in shape;
+    each runs on the path its shape and sample count select.  Not for a trainer with the peer all-reduce attached."""
+
+    def __init__(self, coarse, fine, n_fine, stratified=True):
+        if coarse.head != L.HEAD_NERF or fine.head != L.HEAD_NERF:
+            raise ValueError("CoarseFine needs two nerf trainers")
+        self.coarse, self.fine, self.n_fine, self.stratified = coarse, fine, int(n_fine), bool(stratified)
+        self.ctx = coarse.ctx
+        self._buf, self._key = None, None
+
+    def _buffers(self, R, S, device):
+        key = (R, S, str(device))
+        if self._key != key:
+            f64 = dict(dtype=torch.float64, device=device)
+            self._buf = dict(o=torch.empty((R, 3), **f64), d=torch.empty((R, 3), **f64), t=torch.empty((R, S), **f64),
+                             w=torch.empty((R, S), dtype=torch.float32, device=device),
+                             t_fine=torch.empty((R, S + self.n_fine), **f64))
+            self._key = key
+        return self._buf
+
+    def step(self, camera=None, rays=None, S=None, pe_bands=0, dir_bands=None, target=None, path="tc", seed=None):
+        """One coarse-to-fine train step on a camera batch (camera=make_camera(...), S coarse depths, R = len(target))
+        or a rays batch (rays=(rays_o, rays_d, t), float64 CUDA tensors).  seed: the stratified fine draw's seed
+        (default: the camera's seed; 0 for a rays batch).  Returns the buffers of this step: o, d, t (coarse depths),
+        w (coarse weights) and t_fine."""
+        if (camera is None) == (rays is None):
+            raise ValueError("pass exactly one of camera= and rays=")
+        if target is None:
+            raise ValueError("a train step needs a target")
+        ctx = self.ctx
+        R = int(target.shape[0])
+        if camera is not None:
+            S = int(S)
+            b = self._buffers(R, S, target.device)
+            o, d, t = ctx.camera_rays(camera, R, S, out=(b["o"], b["d"], b["t"]))
+            self.coarse.step_weights(b["w"], camera=camera, R=R, S=S, pe_bands=pe_bands, dir_bands=dir_bands,
+                                     target=target, path=path)
+            seed = camera.seed if seed is None else seed
+            ray0 = camera.first_pixel if not camera.pixels else 0
+        else:
+            o, d, t = rays
+            if not all(_is_cuda(v) and v.dtype == torch.float64 for v in (o, d, t)):
+                raise ValueError("a rays batch must be float64 CUDA tensors (the sampler bins float64 depths)")
+            S = int(t.shape[1])
+            b = self._buffers(R, S, target.device)
+            self.coarse.step_weights(b["w"], rays=(o, d, t), pe_bands=pe_bands, dir_bands=dir_bands, target=target, path=path)
+            seed, ray0 = (0 if seed is None else seed), 0
+        ctx.sample_pdf(t, b["w"], self.n_fine, stratified=self.stratified, seed=seed, ray0=ray0, out=b["t_fine"])
+        self.fine.step(rays=(o, d, b["t_fine"]), pe_bands=pe_bands, dir_bands=dir_bands, target=target, path=path)
+        return dict(o=o, d=d, t=t, w=b["w"], t_fine=b["t_fine"])
 
 
 class PreparedBatch:

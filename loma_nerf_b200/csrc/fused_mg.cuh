@@ -77,7 +77,7 @@ __device__ __forceinline__ void tmem_st4(uint32_t taddr, uint4 v)   // one 8-fea
 }
 template <int HP> constexpr int mg_max_groups() { return HP <= 32 ? MG_MAX_GROUPS : 4; }   // registers: 64 K / (groups x 128 threads)
 
-template <bool RAYS, int HP, bool DIRS = false>
+template <bool RAYS, int HP, bool DIRS = false, bool WGT = false>
 __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel(const TcParams p)
 {
     using LY = TcLayout<HP>;
@@ -311,7 +311,7 @@ __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel
         }
         // ---- head + loss + adjoint of the head's pre-activation (unit seed)
         float dz[4];
-        head_and_composite<true>(p, scratch, g + 1, hz, my_dist, tg, row0, tile * p.G, valid, tid, smp, ray_l, live, loss_acc, dz);
+        head_and_composite<true, WGT>(p, scratch, g + 1, hz, my_dist, tg, row0, tile * p.G, valid, tid, smp, ray_l, live, loss_acc, dz);
         // ---- backward.  dZ_{L-1}: 4 live features of its one slab
         {
             const uint32_t o[8] = {pack_bf16(dz[0], dz[1]), pack_bf16(dz[2], dz[3]), 0u, 0u, 0u, 0u, 0u, 0u};

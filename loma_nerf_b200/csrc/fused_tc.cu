@@ -59,7 +59,7 @@ struct CamF32 {
     int width, stratified;
 };
 
-struct TcParams {
+struct alignas(16) TcParams {   // 16: the kernel parameters after it keep their alignment
     const float *X, *dists, *target, *ws, *bs;
     float *color;      // [R][3] or NULL
     float *part;       // [grid][part_stride]
@@ -80,6 +80,7 @@ struct TcParams {
     int head, want_grad, Wt;
     int part_stride;
     int part_off[MAXL]; // offset of layer l's [(in_l+1) x out_l] block inside a partial
+    float *weights;     // [R][S] compositing weights of a train step (lnb_trainer_step_weights), or NULL
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -548,8 +549,10 @@ struct CompScratch {
 };
 
 // The head on the last layer's pre-activations hz, the loss (added to loss_acc) and, with GRAD, dz = the adjoint of hz
-// (unit seed).  `bar` is the tile's named barrier (bar_tile).
-template <bool GRAD>
+// (unit seed).  `bar` is the tile's named barrier (bar_tile).  WGT (train kernels of lnb_trainer_step_weights): the
+// compositing weights of live rows go to p.weights; a separate instantiation, so the plain train and render kernels stay as
+// they were.
+template <bool GRAD, bool WGT = false>
 __device__ __forceinline__ void head_and_composite(const TcParams &p, const CompScratch &s, int bar, const float (&hz)[4], float dist,
                                                    const float (&tg)[3], long long row0, int ray0, int valid, int tid, int smp,
                                                    int ray_l, bool live, float &loss_acc, float (&dz)[4])
@@ -600,6 +603,7 @@ __device__ __forceinline__ void head_and_composite(const TcParams &p, const Comp
     const float Cpre = pr * carry;                   // true inclusive product prod_{k<=s} q_k
     const float T = (smp == 0) ? 1.0f : Cpre;
     const float wgt = a * T;
+    if (WGT && live) p.weights[row0 + tid] = wgt;
     {   // colour: segmented inclusive sums, one shared-memory atomic per (warp, ray) segment
         float s0 = live ? wgt * cr : 0.f, s1 = live ? wgt * cg : 0.f, s2 = live ? wgt * cb : 0.f;
 #pragma unroll
@@ -709,7 +713,7 @@ __device__ __forceinline__ void relu_adjoint(const uint32_t (&v)[HP / 16][16], c
 // FWD: the forward-only (render) form, compiled separately: nothing of the backward pass in its register budget.  Its
 // launch bounds are the CTAs per SM that tensor memory admits (512 columns / 64 per CTA = 8; 4 for the 64-wide form), not
 // more: a ninth CTA could never allocate its columns and the tighter register budget only bought a spill.
-template <bool RAYS, int HP, bool FWD, bool DIRS = false>
+template <bool RAYS, int HP, bool FWD, bool DIRS = false, bool WGT = false>
 __global__ void __launch_bounds__(TILE, FWD ? (HP == 64 ? 4 : 8) : 1) fused_v1_kernel(const TcParams p)
 {
     using LY = TcLayout<HP>;
@@ -930,7 +934,7 @@ __global__ void __launch_bounds__(TILE, FWD ? (HP == 64 ? 4 : 8) : 1) fused_v1_k
         CLK(16);
         // ---- head + loss + adjoint of the head's pre-activation (unit seed)
         float dz[4];
-        head_and_composite<!FWD>(p, scratch, 0, hz, my_dist, tg, row0, ray0, valid, tid, smp, ray_l, live, loss_acc, dz);
+        head_and_composite<!FWD, WGT>(p, scratch, 0, hz, my_dist, tg, row0, ray0, valid, tid, smp, ray_l, live, loss_acc, dz);
         CLK(17);
         if (FWD) { __syncthreads(); tile = *next_tile_s; continue; }
         // ---- backward.  dZ_{L-1}: 4 live features, the rest of the 16 stay zero
@@ -1391,13 +1395,17 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
     // Train steps run on the multi-group kernel (fused_mg.cuh: one CTA per SM, up to seven 128-thread groups, adjoints in
     // place); forward-only launches and LNB_TC_V1=1 on the one-tile-per-CTA kernel above.
     const bool mg = grad && getenv("LNB_TC_V1") == nullptr && (!nerf || S >= 2);
+    const bool wgt = grad && nerf && ex && ex->weights;   // lnb_trainer_step_weights
     if (grad && !mg) {   // the one-tile-per-CTA kernel computes all weight gradients with ONE concatenated M = 128 MMA per K-step
         if (K0P / 8 + (L - 1) * (HP / 8) > 16) return unsupported("input + hidden widths exceed 128 features in total");
         if ((L - 1) * HP + 16 > 256) return unsupported("hidden widths exceed 256 gradient columns");
     }
     void (*const kern)(TcParams) = with_hp(HP, [&](auto hp) -> void (*)(TcParams) {
         constexpr int H = decltype(hp)::value;
+        if (mg && wgt) return dirs ? fused_mg_kernel<true, H, true, true> : rays ? fused_mg_kernel<true, H, false, true> : fused_mg_kernel<false, H, false, true>;
         if (mg) return dirs ? fused_mg_kernel<true, H, true> : rays ? fused_mg_kernel<true, H> : fused_mg_kernel<false, H>;
+        if (grad && wgt)
+            return dirs ? fused_v1_kernel<true, H, false, true, true> : rays ? fused_v1_kernel<true, H, false, false, true> : fused_v1_kernel<false, H, false, false, true>;
         if (grad) return dirs ? fused_v1_kernel<true, H, false, true> : rays ? fused_v1_kernel<true, H, false> : fused_v1_kernel<false, H, false>;
         return dirs ? fused_v1_kernel<true, H, true, true> : rays ? fused_v1_kernel<true, H, true> : fused_v1_kernel<false, H, true>;
     });
@@ -1410,8 +1418,8 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
             while (n > 1 && (MG::total(L, c_in, K0P, rays, n) > 232448 || MG::tmem_need(L, K0P, n) > 512)) --n;
             return n;
         });
-        static int mg_regs[3][3] = {};    // registers per thread of each instantiation (features, rays, rays + directions), asked once
-        int &regs = mg_regs[dirs ? 2 : (rays ? 1 : 0)][HP / 32];
+        static int mg_regs[2][3][3] = {}; // registers per thread of each instantiation ([weights] (features, rays, rays + directions)), asked once
+        int &regs = mg_regs[wgt][dirs ? 2 : (rays ? 1 : 0)][HP / 32];
         if (regs == 0) {
             cudaFuncAttributes fa;
             LNB_CUDA(cudaFuncGetAttributes(&fa, kern));
@@ -1449,6 +1457,7 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
     uint8_t *wimg = (uint8_t *)lnb_arena_take(ctx, wimg_bytes);
     p.wimg = (ex && ex->wimg) ? ex->wimg : wimg;
     p.t_dev = ex ? ex->t_dev : nullptr;
+    p.weights = wgt ? ex->weights : nullptr;
     if (!ctx->tc_counter) {
         LNB_CUDA(cudaMalloc((void **)&ctx->tc_counter, 256));
         LNB_CUDA(cudaMemsetAsync(ctx->tc_counter, 0, 256, ctx->stream));

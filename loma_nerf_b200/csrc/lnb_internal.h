@@ -165,6 +165,7 @@ struct lnb_tc_extra {
     int *t_dev = nullptr;                               // incremented by the fused kernel
     double lr = 0, b1 = 0, b2 = 0, eps = 0;
     void *wimg_out = nullptr;
+    float *weights = nullptr;                           // train kernels: [R][S] compositing weights w_s = alpha_s T_s
 };
 int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf,
                       const lnb_tc_extra *ex);

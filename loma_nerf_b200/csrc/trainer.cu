@@ -118,7 +118,8 @@ static int comm_failed(lnb_trainer *t, float *loss_out)
     return LNB_ERR_CUDA;
 }
 
-static int trainer_run(lnb_trainer *t, const lnb_step_args *batch, int nerf, bool fuse_update)
+// weights: [R][S] compositing weights of this step's forward pass (lnb_trainer_step_weights), or NULL
+static int trainer_run(lnb_trainer *t, const lnb_step_args *batch, int nerf, bool fuse_update, float *weights = nullptr)
 {
     lnb_ctx *ctx = t->ctx;
     LNB_ARG(batch, "trainer: null batch");
@@ -131,7 +132,7 @@ static int trainer_run(lnb_trainer *t, const lnb_step_args *batch, int nerf, boo
     a.inter = a.rgba = a.alpha = a.cumprod = a.weights = nullptr;
     if (a.path == LNB_PATH_TC && t->tc_ok) {
         lnb_tc_extra ex;
-        ex.wimg = t->wimg; ex.overwrite_grads = 1; ex.t_dev = t->t_dev;
+        ex.wimg = t->wimg; ex.overwrite_grads = 1; ex.t_dev = t->t_dev; ex.weights = weights;
         if (fuse_update) {
             if (t->comm.world > 1) ex.comm = &t->comm;
             ex.fuse_adam = 1; ex.param = t->params; ex.m = t->opt == LNB_OPT_ADAM ? t->m : nullptr; ex.v = t->v;
@@ -151,6 +152,8 @@ static int trainer_run(lnb_trainer *t, const lnb_step_args *batch, int nerf, boo
                    "exchange gradients in-kernel; use lnb_trainer_grad + an all-reduce of lnb_trainer_grad_buffer + lnb_trainer_apply";
         return LNB_ERR_UNSUPPORTED;
     }
+    // the fused exact kernel writes no weights: a step that asks for them runs on the layerwise kernels
+    a.weights = weights;
     int rc = LNB_ERR_UNSUPPORTED;
     if (a.path == LNB_PATH_F32 && !getenv("LNB_F32_NO_FUSED")) {
         // fused exact kernel writing the (zero-padded, never otherwise touched) gradient buffer: no memset
@@ -176,6 +179,14 @@ extern "C" int lnb_trainer_step(lnb_trainer *t, const lnb_step_args *batch, int 
 {
     if (!t) return LNB_ERR_ARG;
     return trainer_run(t, batch, nerf, true);
+}
+
+extern "C" int lnb_trainer_step_weights(lnb_trainer *t, const lnb_step_args *batch, int nerf, float *weights)
+{
+    if (!t) return LNB_ERR_ARG;
+    lnb_ctx *ctx = t->ctx;
+    LNB_ARG(nerf && weights, "trainer_step_weights: a nerf batch and a weights buffer");
+    return trainer_run(t, batch, nerf, true, weights);
 }
 
 extern "C" int lnb_trainer_apply(lnb_trainer *t)
