@@ -280,6 +280,35 @@ LNB_API int lnb_fit_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *
 LNB_API int lnb_nerf_step_host(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *args);
 LNB_API int lnb_fit_step_host(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *args);
 
+/* COMPOSITING EXTRAS of a nerf step: opacity and depth maps, and compositing onto a background colour (the NeRF paper's
+ * acc_map, depth_map and white-background renders).  With w_s the compositing weight of sample s (weights_samples,
+ * nerf.py:270: w_s = alpha_s T_s, inclusive transmittance) and t_s its depth (lnb_step_args.t in rays mode, the depth
+ * lnb_camera defines in camera mode):
+ *   acc_r   = sum_s w_s                       (opacity)
+ *   depth_r = sum_s w_s t_s                   (expected depth, NOT divided by acc_r, like the paper's depth_map; rays and
+ *                                              camera mode only: features mode has no depths)
+ *   color_r = sum_s w_s rgb_s + (1 - acc_r) bg   when background == 1 (overwritten, or added to the caller's colour under
+ *                                              color_accumulate); the loss, d_color and d_target use this colour.
+ * The reference's inclusive transmittance gives sum_s w_s <= 1 + O(1e-10) (the 1e-10 added to every 1 - alpha), so
+ * 1 - acc_r is the light that reaches the background under the same model.
+ * Backward: the one change is d_w_s = sum_c (rgb_{s,c} - bg_c) dcol_c; the transmittance scan, d_alpha, d_sigma, d_dists
+ * and the MLP adjoint follow from d_w_s as without a background.  bg is a constant (no gradient); acc and depth are
+ * forward outputs only (no gradient flows into them).
+ * A NULL lnb_composite, or one that asks for nothing (background 0, acc and depth NULL), is exactly lnb_nerf_step: the
+ * same kernels, the same bits.  Otherwise: LNB_PATH_TC runs the fused kernels' extras instantiations (or the wide path);
+ * the exact path runs on the layerwise fp32 kernels (the fused exact kernel has no extras).  LNB_ERR_ARG for depth in
+ * features mode, background not 0 or 1, or a non-finite bg.  The compat symbols keep the reference's compositing. */
+typedef struct {
+    int background;      /* 0: none (the reference's compositing); 1: composite onto bg */
+    float bg[3];
+    float *acc;          /* [R] overwritten, or NULL (device pointer; host pointer for the *_host call) */
+    float *depth;        /* [R] overwritten, or NULL (rays / camera mode only)                           */
+} lnb_composite;
+LNB_API int lnb_nerf_step_composite(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *args, const lnb_composite *comp);
+LNB_API int lnb_nerf_step_composite_host(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *args, const lnb_composite *comp);
+/* Fills out[0..n) with {sizeof(lnb_composite), offsetof background, bg, acc, depth}; returns how many values exist. */
+LNB_API int lnb_composite_layout(int *out, int n);
+
 /* Positional encoding, pos_encoding.py:4-70: x [n][F] float64 -> out [n][F*(1+2E)] float32,
  * feature = slot*F + coord, slot 0 identity, 2i+1 sin(2^i x), 2i+2 cos(2^i x); float64 range
  * reduction so the result matches the reference's float64-then-cast values. Device pointers. */
@@ -354,6 +383,11 @@ LNB_API int lnb_trainer_step_host(lnb_trainer *t, const lnb_step_args *batch, in
 LNB_API int lnb_trainer_submit_host(lnb_trainer *t, const lnb_step_args *batch, int nerf);
 LNB_API int lnb_trainer_wait(lnb_trainer *t, float *losses, int max_losses, int *n_out);
 LNB_API int lnb_trainer_grad(lnb_trainer *t, const lnb_step_args *batch, int nerf);
+/* Composite every later nerf step of this trainer (step, step_weights, step_host, submit_host, grad) onto the background
+ * colour rgb (3 floats; see lnb_composite), whichever kernels the step runs on; NULL restores the reference's compositing
+ * (a trainer that never had a background set runs exactly as before).  The term is per ray, so the peer all-reduce is
+ * unaffected, but every rank of a data-parallel run must set the same background.  LNB_ERR_ARG for a non-finite value. */
+LNB_API int lnb_trainer_set_background(lnb_trainer *t, const float *rgb);
 LNB_API int lnb_trainer_apply(lnb_trainer *t);
 LNB_API float *lnb_trainer_grad_buffer(lnb_trainer *t, long long *n_floats);
 LNB_API float *lnb_trainer_params(lnb_trainer *t, long long *n_w, long long *n_b);

@@ -55,6 +55,12 @@ class LnbStepArgs(Structure):
     ]
 
 
+class LnbComposite(Structure):
+    """Mirror of lnb_composite (compositing extras: background colour, opacity and depth maps); checked against
+    lnb_composite_layout."""
+    _fields_ = [("background", c_int), ("bg", c_float * 3), ("acc", c_void_p), ("depth", c_void_p)]
+
+
 class LibraryMissing(RuntimeError):
     pass
 
@@ -95,6 +101,12 @@ def load():
         fn = getattr(lib, name)
         fn.argtypes = [c_void_p, P(LnbMlp), P(LnbStepArgs)]
         fn.restype = c_int
+    for name in ("lnb_nerf_step_composite", "lnb_nerf_step_composite_host"):
+        fn = getattr(lib, name)
+        fn.argtypes = [c_void_p, P(LnbMlp), P(LnbStepArgs), P(LnbComposite)]
+        fn.restype = c_int
+    lib.lnb_composite_layout.argtypes = [P(c_int), c_int]
+    lib.lnb_composite_layout.restype = c_int
     lib.lnb_pos_encoding.argtypes = [c_void_p, c_void_p, c_longlong, c_int, c_int, c_void_p]
     lib.lnb_sample_encode.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
                                       c_void_p, c_void_p]
@@ -118,6 +130,8 @@ def load():
     lib.lnb_trainer_destroy.restype = None
     for name in ("lnb_trainer_step", "lnb_trainer_grad"):
         getattr(lib, name).argtypes = [c_void_p, P(LnbStepArgs), c_int]
+    lib.lnb_trainer_set_background.argtypes = [c_void_p, P(c_float)]
+    lib.lnb_trainer_set_background.restype = c_int
     lib.lnb_trainer_step_weights.argtypes = [c_void_p, P(LnbStepArgs), c_int, c_void_p]
     lib.lnb_trainer_step_host.argtypes = [c_void_p, P(LnbStepArgs), c_int, P(c_float)]
     lib.lnb_trainer_submit_host.argtypes = [c_void_p, P(LnbStepArgs), c_int]

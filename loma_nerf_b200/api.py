@@ -22,6 +22,21 @@ except Exception:  # pragma: no cover
 
 FWD_OUTPUTS = ("inter", "rgba", "alpha", "cumprod", "weights", "color", "loss")
 GRAD_OUTPUTS = ("d_ws", "d_bs", "d_X", "d_target", "d_dists", "d_color", "d_inter")
+COMPOSITE_OUTPUTS = ("acc", "depth")   # [R] float32, through lnb_composite
+
+
+def make_composite(background=None):
+    """An lnb_composite: background=None (the reference's compositing) or 3 finite floats.  acc / depth are set by the
+    caller."""
+    c = L.LnbComposite()
+    if background is not None:
+        bg = [float(v) for v in np.asarray(background, np.float64).reshape(-1)]
+        if len(bg) != 3 or not all(np.isfinite(bg)):
+            raise ValueError("background must be 3 finite floats, got %r" % (background,))
+        c.background = 1
+        for i in range(3):
+            c.bg[i] = bg[i]
+    return c
 PATHS = {"f32": L.PATH_F32, "tc": L.PATH_TC, "f32_layerwise": L.PATH_F32_LAYERWISE}
 
 
@@ -216,9 +231,17 @@ class Context:
 
     # -------------------------------------------------------------------------------------------
     def _step(self, nerf, dims, X, ws, bs, target, dists, R, S, grad, seed, outputs, out, rows,
-              path, inter_accumulate, color_accumulate, head, rays=None, pe_bands=0, camera=None, dir_bands=None):
+              path, inter_accumulate, color_accumulate, head, rays=None, pe_bands=0, camera=None, dir_bands=None,
+              background=None):
         if rays is not None or camera is not None:
             check_rays_width(dims[0], pe_bands, dir_bands)
+        outputs = tuple(outputs)
+        extras = [k for k in COMPOSITE_OUTPUTS if k in outputs]
+        if (extras or background is not None) and not nerf:
+            raise ValueError("background, acc and depth are nerf-step features")
+        if "depth" in extras and rays is None and camera is None:
+            raise ValueError("the depth map needs rays or camera mode: features mode has no sample depths")
+        comp = make_composite(background) if (background is not None or extras) else None
         dev = _is_cuda(ws)
         mlp = make_mlp(dims, ws.shape, head)
         Ln, mi, mo = mlp.n_layers, mlp.max_in, mlp.max_out
@@ -253,7 +276,7 @@ class Context:
                       d_color=(R, Wt), d_inter=(Ln, M, mo))
         res = {}
         out = out or {}
-        want = list(outputs)
+        want = [k for k in outputs if k not in COMPOSITE_OUTPUTS]
         if grad:
             want += [k for k in ("d_ws", "d_bs") if k not in want]
         for k in want:
@@ -271,45 +294,63 @@ class Context:
                 assert tuple(buf.shape) == tuple(shapes[k]), (k, tuple(buf.shape), shapes[k])
             res[k] = buf
             setattr(a, k, _ptr(buf))
-        fn = {(True, True): self.lib.lnb_nerf_step, (True, False): self.lib.lnb_nerf_step_host,
-              (False, True): self.lib.lnb_fit_step, (False, False): self.lib.lnb_fit_step_host}[(nerf, dev)]
+        for k in extras:   # acc / depth [R]: through the lnb_composite extras
+            buf = out.get(k)
+            if buf is None:
+                buf = torch.zeros((int(R),), dtype=torch.float32, device=ws.device) if dev else np.zeros((int(R),), np.float32)
+            else:
+                assert tuple(buf.shape) == (int(R),), (k, tuple(buf.shape), (int(R),))
+            res[k] = buf
+            setattr(comp, k, _ptr(buf))
         if dev:
             # the zero fills above and whatever produced the inputs ran on torch's current stream
             self.order_after_torch()
             self._hold(X, ws, bs, target, dists, *(rays or ()), *res.values())
+        if comp is not None:   # only a step that uses an extra calls the composite entry
+            fn = self.lib.lnb_nerf_step_composite if dev else self.lib.lnb_nerf_step_composite_host
+            self._check(fn(self.h, ctypes.byref(mlp), ctypes.byref(a), ctypes.byref(comp)))
+            return res
+        fn = {(True, True): self.lib.lnb_nerf_step, (True, False): self.lib.lnb_nerf_step_host,
+              (False, True): self.lib.lnb_fit_step, (False, False): self.lib.lnb_fit_step_host}[(nerf, dev)]
         self._check(fn(self.h, ctypes.byref(mlp), ctypes.byref(a)))
         return res
 
     def nerf_step(self, dims, X, ws, bs, dists, target=None, R=None, S=None, grad=False, seed=1.0,
                   outputs=("color", "loss"), out=None, rows=None, path="f32",
-                  inter_accumulate=False, color_accumulate=False):
+                  inter_accumulate=False, color_accumulate=False, background=None):
         """MLP -> compositing -> SSE loss [-> gradients] (scripts/nerf.py:67-306).
         X [R*S][C_in] features, dists [R][S], target [R][3]; returns {name: buffer}.  Gradient
-        outputs ACCUMULATE into buffers passed through `out` (the reference's += semantics)."""
+        outputs ACCUMULATE into buffers passed through `out` (the reference's += semantics).
+        background=(r, g, b) composites onto that colour (colour += (1 - acc) bg; the loss and the gradients follow);
+        outputs may also name "acc" ([R] opacity, sum of the compositing weights) and, in rays / camera mode, "depth"
+        ([R] sum of weight x sample depth).  See lnb_composite in include/loma_nerf_b200.h."""
         R = int(dists.shape[0]) if R is None else R
         S = int(dists.shape[1]) if S is None else S
         return self._step(True, dims, X, ws, bs, target, dists, R, S, grad, seed, outputs, out,
-                          rows, path, inter_accumulate, color_accumulate, L.HEAD_NERF)
+                          rows, path, inter_accumulate, color_accumulate, L.HEAD_NERF, background=background)
 
     def nerf_step_rays(self, dims, rays_o, rays_d, t, pe_bands, ws, bs, target=None, grad=False, seed=1.0,
-                       outputs=("color", "loss"), out=None, path="f32", dir_bands=None):
+                       outputs=("color", "loss"), out=None, path="f32", dir_bands=None, background=None):
         """The same step starting from rays: the sample positions o + d*t, their positional encoding
         and the dists are computed on the device (train_nerf.py:289-311, pos_encoding.py:38-70) --
         fused into the first layer on the tensor-core path.  rays_o, rays_d [R][3], t [R][S], all
         float64 (the reference's dtype) or all float32.  dir_bands=E_d: the net also takes the unit view
-        direction in E_d bands (dims[0] = 3 + 6 pe_bands + 3 + 6 E_d, rays_input_width)."""
+        direction in E_d bands (dims[0] = 3 + 6 pe_bands + 3 + 6 E_d, rays_input_width).  background and the "acc" /
+        "depth" outputs as in nerf_step (depth = sum of w_s t_s)."""
         R, S = int(t.shape[0]), int(t.shape[1])
         return self._step(True, dims, None, ws, bs, target, None, R, S, grad, seed, outputs, out, None, path,
-                          False, False, L.HEAD_NERF, rays=(rays_o, rays_d, t), pe_bands=pe_bands, dir_bands=dir_bands)
+                          False, False, L.HEAD_NERF, rays=(rays_o, rays_d, t), pe_bands=pe_bands, dir_bands=dir_bands,
+                          background=background)
 
     def nerf_step_camera(self, dims, camera, R, S, pe_bands, ws, bs, target=None, grad=False, seed=1.0,
-                         outputs=("color", "loss"), out=None, path="f32", dir_bands=None):
+                         outputs=("color", "loss"), out=None, path="f32", dir_bands=None, background=None):
         """The same step with rays AND sample depths generated on the device from a pose (`make_camera`): the
         device-side get_rays (train_nerf.py:23-62) and linspace / stratified depths (train_nerf.py:289-311).
         Nothing per ray or per sample is read: R rays of S samples through pixels first_pixel .. (or `pixels`).
-        dir_bands as in nerf_step_rays."""
+        dir_bands, background and the "acc" / "depth" outputs as in nerf_step_rays (the depths are the camera's)."""
         return self._step(True, dims, None, ws, bs, target, None, int(R), int(S), grad, seed, outputs, out, None, path,
-                          False, False, L.HEAD_NERF, pe_bands=pe_bands, camera=camera, dir_bands=dir_bands)
+                          False, False, L.HEAD_NERF, pe_bands=pe_bands, camera=camera, dir_bands=dir_bands,
+                          background=background)
 
     def camera_rays(self, camera, R, S, out=None):
         """(rays_o, rays_d, t) float64 cuda tensors camera mode generates (for checks / hosts that want them).
@@ -414,10 +455,11 @@ class Context:
 class Trainer:
     """Device-resident weights + optimiser state (lnb_trainer): the reference hosts' per-chunk
     "grad call, then Adam / SGD on the padded arrays" loop (train_nerf.py:395-499,
-    fit_img.py:468-513) without host round trips.  Batches are torch CUDA tensors."""
+    fit_img.py:468-513) without host round trips.  Batches are torch CUDA tensors.
+    background=(r, g, b): every nerf step composites onto that colour (set_background)."""
 
     def __init__(self, ctx, dims, ws, bs, head=L.HEAD_NERF, optimizer="adam", lr=5e-4, beta1=0.9, beta2=0.999,
-                 eps=1e-8):
+                 eps=1e-8, background=None):
         self.ctx, self.lib = ctx, ctx.lib
         ws = np.ascontiguousarray(ws, np.float32)
         bs = np.ascontiguousarray(bs, np.float32)
@@ -429,6 +471,22 @@ class Trainer:
         ctx._check(self.lib.lnb_trainer_create(ctx.h, ctypes.byref(self.mlp), ws.ctypes.data, bs.ctypes.data, opt,
                                                lr, beta1, beta2, eps, ctypes.byref(h)))
         self.h = h
+        self.background = None
+        if background is not None:
+            self.set_background(background)
+
+    def set_background(self, rgb):
+        """Composite every later nerf step (step, step_weights, step_host, submit_host, grad) onto the colour rgb
+        (3 floats): colour += (1 - acc) rgb before the loss, on whichever path the step runs (lnb_trainer_set_background).
+        None restores the reference's compositing.  With the peer all-reduce every rank must set the same colour."""
+        if rgb is None:
+            self.ctx._check(self.lib.lnb_trainer_set_background(self.h, None))
+            self.background = None
+            return
+        bg = make_composite(rgb).bg
+        arr = (ctypes.c_float * 3)(bg[0], bg[1], bg[2])
+        self.ctx._check(self.lib.lnb_trainer_set_background(self.h, arr))
+        self.background = (float(bg[0]), float(bg[1]), float(bg[2]))
 
     def close(self):
         if getattr(self, "h", None):
@@ -586,7 +644,9 @@ class CoarseFine:
       4. a fine Trainer.step in rays mode on (rays_o, rays_d, t_fine).
     Both nets train on their own colour loss.  Nothing is synchronised with the host and, after the first step of a
     shape, nothing is allocated: a run of steps can be captured in one CUDA graph.  The two nets may differ in shape;
-    each runs on the path its shape and sample count select.  Not for a trainer with the peer all-reduce attached."""
+    each runs on the path its shape and sample count select.  Not for a trainer with the peer all-reduce attached.
+    Backgrounds need nothing here: each trainer composites onto its own (Trainer(..., background=) / set_background), so a
+    white-background run gives both trainers background=(1, 1, 1)."""
 
     def __init__(self, coarse, fine, n_fine, stratified=True):
         if coarse.head != L.HEAD_NERF or fine.head != L.HEAD_NERF:

@@ -90,6 +90,39 @@ extern "C" int lnb_struct_layout(int *out, int n)
     return k;
 }
 
+extern "C" int lnb_composite_layout(int *out, int n)
+{
+    const int v[] = {(int)sizeof(lnb_composite), (int)offsetof(lnb_composite, background), (int)offsetof(lnb_composite, bg),
+                     (int)offsetof(lnb_composite, acc), (int)offsetof(lnb_composite, depth)};
+    const int k = (int)(sizeof(v) / sizeof(v[0]));
+    for (int i = 0; i < k && i < n; ++i) out[i] = v[i];
+    return k;
+}
+
+int lnb_comp_resolve(lnb_ctx *ctx, const lnb_step_args *a, bool nerf, const lnb_composite *comp, lnb_comp_args *out,
+                     const lnb_comp_args **resolved)
+{
+    *resolved = nullptr;
+    if (!comp) return LNB_OK;
+    LNB_ARG(comp->background == 0 || comp->background == 1, "composite: background must be 0 or 1");
+    if (comp->background)
+        for (int c = 0; c < 3; ++c) LNB_ARG(isfinite(comp->bg[c]), "composite: non-finite background colour");
+    if (!comp->background && !comp->acc && !comp->depth) return LNB_OK;   // asks for nothing: the plain step
+    LNB_ARG(nerf, "composite: a nerf-step feature");
+    const bool cam = !a->X && !a->rays_o && a->cam;
+    const bool rays = !a->X && (a->rays_o || cam);
+    LNB_ARG(!comp->depth || rays, "composite: depth needs rays or camera mode (features mode has no sample depths)");
+    *out = lnb_comp_args{};
+    out->background = comp->background;
+    for (int c = 0; c < 3; ++c) out->bg[c] = comp->background ? comp->bg[c] : 0.0f;
+    out->acc = comp->acc;
+    out->depth = comp->depth;
+    if (cam) out->cam = a->cam;
+    else if (rays) { out->t = a->t; out->t_f64 = a->ray_dtype == LNB_RAY_F64; }
+    *resolved = out;
+    return LNB_OK;
+}
+
 extern "C" int lnb_device_count(void)
 {
     int n = 0;
@@ -296,7 +329,7 @@ int validate(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf
     return LNB_OK;
 }
 
-int step_layerwise(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf)
+int step_layerwise(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf, const lnb_comp_args *cx)
 {
     StepDims d;
     LNB_TRY(validate(ctx, mlp, a, nerf, &d));
@@ -379,7 +412,7 @@ int step_layerwise(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, boo
     if (nerf) {
         LNB_TRY(lnb_launch_composite_fwd(ctx, head, ldh, dists, a->target, R, S, a->rgba,
                                          a->alpha, a->cumprod, a->weights, color, color_acc,
-                                         ray_sse));
+                                         ray_sse, cx));
     } else if (a->target) {
         LNB_TRY(lnb_launch_fit_loss(ctx, head, ldh, a->target, R, d.Wt, ray_sse));
     }
@@ -397,7 +430,7 @@ int step_layerwise(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, boo
     int ldz = d.out_last;
     if (nerf) {
         LNB_TRY(lnb_launch_composite_bwd(ctx, head, ldh, dists, a->target, color, R, S, dZa, ldz,
-                                         d.out_last, a->d_dists ? d_dists_u : nullptr, d_color_u));
+                                         d.out_last, a->d_dists ? d_dists_u : nullptr, d_color_u, cx));
         if (a->d_dists)
             LNB_TRY(lnb_launch_axpy2d(ctx, a->d_dists, S, d_dists_u, S, R, S, 1.0f, seed_val, seed_dev));
     } else {
@@ -441,28 +474,34 @@ int step_layerwise(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, boo
 } // namespace
 
 
-static int step_dispatch(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf, const lnb_tc_extra *ex = nullptr)
+// comp: the compositing extras (lnb_composite), resolved here against the (device-pointer) step; one that asks for nothing
+// leaves the step exactly as it is without
+static int step_dispatch(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf, const lnb_tc_extra *ex = nullptr,
+                         const lnb_composite *comp = nullptr)
 {
     if (!ctx) return LNB_ERR_ARG;
     LNB_ARG(a, "null args");
-    if (a->path == LNB_PATH_F32_LAYERWISE) return step_layerwise(ctx, mlp, a, nerf);
+    lnb_comp_args cxa;
+    const lnb_comp_args *cx = nullptr;
+    LNB_TRY(lnb_comp_resolve(ctx, a, nerf, comp, &cxa, &cx));
+    if (a->path == LNB_PATH_F32_LAYERWISE) return step_layerwise(ctx, mlp, a, nerf, cx);
     if (a->path == LNB_PATH_F32) {
         // same arithmetic type and tolerance either way: the fused kernel when the problem and the outputs asked for fit
         // it (loss, colour, d_ws, d_bs of a 2-3 layer network of the reference's widths), else the layerwise kernels
         StepDims d;
         LNB_TRY(validate(ctx, mlp, a, nerf, &d));
-        const int rc = getenv("LNB_F32_NO_FUSED") ? LNB_ERR_UNSUPPORTED : lnb_fused_f32_step(ctx, mlp, a, nerf, 0);
+        const int rc = getenv("LNB_F32_NO_FUSED") ? LNB_ERR_UNSUPPORTED : lnb_fused_f32_step(ctx, mlp, a, nerf, 0, cx);
         if (rc != LNB_ERR_UNSUPPORTED) return rc;
-        return step_layerwise(ctx, mlp, a, nerf);
+        return step_layerwise(ctx, mlp, a, nerf, cx);
     }
     if (a->path == LNB_PATH_TC) {
         StepDims d;
         LNB_TRY(validate(ctx, mlp, a, nerf, &d));
-        int rc = lnb_fused_tc_step(ctx, mlp, a, nerf, ex); // never silently changes arithmetic
+        int rc = lnb_fused_tc_step(ctx, mlp, a, nerf, ex, cx); // never silently changes arithmetic
         if (rc == LNB_ERR_UNSUPPORTED && !ex) {
             // wide MLPs: layerwise tensor-core path (same operand precision, same outputs)
             const std::string why = ctx->err;
-            rc = lnb_wide_tc_step(ctx, mlp, a, nerf);
+            rc = lnb_wide_tc_step(ctx, mlp, a, nerf, cx);
             if (rc == LNB_ERR_UNSUPPORTED) ctx->err = why + "; " + ctx->err;
         }
         return rc;
@@ -480,9 +519,10 @@ int lnb_step_f32_fused(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a,
     return lnb_fused_f32_step(ctx, mlp, a, nerf, overwrite);
 }
 
-int lnb_step_ex(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf, const lnb_tc_extra *ex)
+int lnb_step_ex(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf, const lnb_tc_extra *ex,
+                const lnb_composite *comp)
 {
-    return step_dispatch(ctx, mlp, a, nerf, ex);
+    return step_dispatch(ctx, mlp, a, nerf, ex, comp);
 }
 
 extern "C" int lnb_nerf_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *args)
@@ -492,6 +532,10 @@ extern "C" int lnb_nerf_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_ar
 extern "C" int lnb_fit_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *args)
 {
     return step_dispatch(ctx, mlp, args, false);
+}
+extern "C" int lnb_nerf_step_composite(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *args, const lnb_composite *comp)
+{
+    return step_dispatch(ctx, mlp, args, true, nullptr, comp);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -520,7 +564,7 @@ bool is_pinned(const void *p)
     return at.type == cudaMemoryTypeHost;
 }
 
-int step_host(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf)
+int step_host(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf, const lnb_composite *comp = nullptr)
 {
     if (!ctx) return LNB_ERR_ARG;
     StepDims d;
@@ -564,6 +608,12 @@ int step_host(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool ner
         OUT_(cumprod, R * S);
         OUT_(weights, R * S);
         if (a->color) reg(a->color, a->color, R * 3, a->color_accumulate ? BUF_INOUT : BUF_OUT, (void **)&dev.color);
+    }
+    lnb_composite comp_dev;   // the compositing extras: acc / depth are staged like colour
+    if (comp) {
+        comp_dev = *comp;
+        if (nerf && comp->acc) reg(nullptr, comp->acc, R, BUF_OUT, (void **)&comp_dev.acc);
+        if (nerf && comp->depth) reg(nullptr, comp->depth, R, BUF_OUT, (void **)&comp_dev.depth);
     }
     OUT_(loss, 1);
     if (a->want_grad) {
@@ -610,7 +660,7 @@ int step_host(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool ner
             LNB_CUDA(cudaMemsetAsync(dptr, 0, b.bytes, ctx->stream));
         }
     }
-    int rc = step_dispatch(ctx, mlp, &dev, nerf);
+    int rc = step_dispatch(ctx, mlp, &dev, nerf, nullptr, comp ? &comp_dev : nullptr);
     if (rc != LNB_OK) return rc;
     // D2H
     for (auto &b : bufs) {
@@ -641,6 +691,10 @@ extern "C" int lnb_nerf_step_host(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_st
 extern "C" int lnb_fit_step_host(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *args)
 {
     return step_host(ctx, mlp, args, false);
+}
+extern "C" int lnb_nerf_step_composite_host(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *args, const lnb_composite *comp)
+{
+    return step_host(ctx, mlp, args, true, comp);
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -495,13 +495,15 @@ __global__ void __launch_bounds__(1024) fused_f32_reduce_kernel(const float *__r
 // LNB_ERR_UNSUPPORTED when the problem does not fit the fused exact kernel (the caller then runs the layerwise kernels).
 // Rays and camera batches are encoded first (float64 sample positions and sin / cos like the reference host, encode.cu).
 // overwrite != 0: d_ws / d_bs are written (=) instead of accumulated (+=), live entries only (the trainer's buffer).
-int lnb_fused_f32_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf, int overwrite)
+int lnb_fused_f32_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf, int overwrite,
+                       const lnb_comp_args *cx)
 {
     const int L = mlp->n_layers;
     auto unsupported = [&](const char *why) {
         ctx->err = std::string("fused fp32 path: ") + why;
         return LNB_ERR_UNSUPPORTED;
     };
+    if (cx) return unsupported("no compositing extras (background, acc, depth): the layerwise kernels have them");
     if (L < 2 || L > 3) return unsupported("needs 2 or 3 layers");
     if (mlp->dims[0] + 1 > K0) return unsupported("input width + 1 must be <= 36");
     for (int l = 1; l < L; ++l)

@@ -77,7 +77,10 @@ __device__ __forceinline__ void tmem_st4(uint32_t taddr, uint4 v)   // one 8-fea
 }
 template <int HP> constexpr int mg_max_groups() { return HP <= 32 ? MG_MAX_GROUPS : 4; }   // registers: 64 K / (groups x 128 threads)
 
-template <bool RAYS, int HP, bool DIRS = false, bool WGT = false>
+// EXT: the extras instantiation (head_and_composite: weights, acc / depth, background), the one lnb_trainer_step_weights and
+// a step with compositing extras run.  Its acc / depth scratch is the slot's dZ_{L-1} slab, dead until the head's adjoint
+// is written into it (the previous tile's weight-gradient MMA that read it has been awaited in the backward loop).
+template <bool RAYS, int HP, bool DIRS = false, bool EXT = false>
 __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel(const TcParams p)
 {
     using LY = TcLayout<HP>;
@@ -113,7 +116,7 @@ __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel
     const uint32_t bar_mma = smem_u32(bar_p), bar_x = smem_u32(bar_p + 1), bar_dw = smem_u32(bar_p + 2);
     const uint32_t bar_w = smem_u32(globals);
     uint32_t *const tmem_slot = reinterpret_cast<uint32_t *>(globals + 8);
-    const CompScratch scratch{color_s, tgt_s, tailp, tail_s, headq, headA, headB};
+    const CompScratch scratch{color_s, tgt_s, reinterpret_cast<float *>(slot + MG::dzl_off(A0S)), tailp, tail_s, headq, headA, headB};
     StageRec *const prog = reinterpret_cast<StageRec *>(misc + 1728);   // fwd l | dH l (L + l) | dW l (2L + l)
 
     auto a_buf = [&](int l) { return slot + MG::a_off(l, A0S); };
@@ -311,7 +314,7 @@ __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel
         }
         // ---- head + loss + adjoint of the head's pre-activation (unit seed)
         float dz[4];
-        head_and_composite<true, WGT>(p, scratch, g + 1, hz, my_dist, tg, row0, tile * p.G, valid, tid, smp, ray_l, live, loss_acc, dz);
+        head_and_composite<true, EXT>(p, scratch, g + 1, hz, my_dist, tg, row0, tile * p.G, valid, tid, smp, ray_l, live, loss_acc, dz);
         // ---- backward.  dZ_{L-1}: 4 live features of its one slab
         {
             const uint32_t o[8] = {pack_bf16(dz[0], dz[1]), pack_bf16(dz[2], dz[3]), 0u, 0u, 0u, 0u, 0u, 0u};

@@ -81,6 +81,10 @@ struct alignas(16) TcParams {   // 16: the kernel parameters after it keep their
     int part_stride;
     int part_off[MAXL]; // offset of layer l's [(in_l+1) x out_l] block inside a partial
     float *weights;     // [R][S] compositing weights of a train step (lnb_trainer_step_weights), or NULL
+    // compositing extras (lnb_composite), read by the EXT instantiations only
+    float *acc, *depth; // [R] opacity / expected depth, or NULL
+    int background;     // 1: colour += (1 - acc) bg
+    float bg[3];
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -543,16 +547,31 @@ __device__ __forceinline__ void pack_features(const float *xr, int c_in, bool ro
 // shared-memory scratch of the head and compositing stage of one tile
 struct CompScratch {
     float *color, *tgt;             // [rays of the tile][3]: colour sums, targets
+    float *ext;                     // EXT: [rays of the tile][2]: acc and depth sums
     float *tailp;                   // [4] inclusive product at lane 31 of each warp
     int *tail_s;                    // [4] sample index at lane 31
     float *headq, *headA, *headB;   // [5] q at lane 0 of each warp; the affine suffix scan's head of each warp
 };
 
+// Depth t_s of sample smp of ray `ray` (row `row` of the batch) for the depth map: re-loaded (rays mode) or re-derived from
+// the camera exactly as sample_inputs forms it, at the compositing stage rather than held in a register across the MMAs.
+__device__ __forceinline__ float tile_sample_depth(const TcParams &p, long long ray, int smp, long long row)
+{
+    if (p.cam_mode) {
+        const CamF32 &c = p.cam;
+        const long long q = c.pixels ? (long long)__ldg(c.pixels + ray) : c.first_pixel + ray;
+        if (c.stratified) return fmaf((float)smp + (float)lnb_uniform_bits(c.seed, q, smp) * (1.0f / 16777216.0f), c.dt_str, c.near);
+        return smp == p.S - 1 && p.S > 1 ? c.far : fmaf((float)smp, c.dt_lin, c.near);
+    }
+    return p.ray_f64 ? (float)__ldg(reinterpret_cast<const double *>(p.tvals) + row) : __ldg(reinterpret_cast<const float *>(p.tvals) + row);
+}
+
 // The head on the last layer's pre-activations hz, the loss (added to loss_acc) and, with GRAD, dz = the adjoint of hz
-// (unit seed).  `bar` is the tile's named barrier (bar_tile).  WGT (train kernels of lnb_trainer_step_weights): the
-// compositing weights of live rows go to p.weights; a separate instantiation, so the plain train and render kernels stay as
-// they were.
-template <bool GRAD, bool WGT = false>
+// (unit seed).  `bar` is the tile's named barrier (bar_tile).  EXT (the extras instantiations): the compositing weights of
+// live rows go to p.weights when it is set (lnb_trainer_step_weights), acc and depth ride in the segmented colour sum as
+// two more channels (p.acc / p.depth), and with p.background the colour gets (1 - acc) bg before the loss, the weight
+// adjoint uses rgb - bg.  A separate instantiation, so the plain train and render kernels stay as they were.
+template <bool GRAD, bool EXT = false>
 __device__ __forceinline__ void head_and_composite(const TcParams &p, const CompScratch &s, int bar, const float (&hz)[4], float dist,
                                                    const float (&tg)[3], long long row0, int ray0, int valid, int tid, int smp,
                                                    int ray_l, bool live, float &loss_acc, float (&dz)[4])
@@ -590,6 +609,7 @@ __device__ __forceinline__ void head_and_composite(const TcParams &p, const Comp
     if (lane == 0) s.headq[warp] = qv;
     if (live && smp == 0) {
         s.color[ray_l * 3] = 0.f; s.color[ray_l * 3 + 1] = 0.f; s.color[ray_l * 3 + 2] = 0.f;
+        if (EXT) { s.ext[ray_l * 2] = 0.f; s.ext[ray_l * 2 + 1] = 0.f; }
         s.tgt[ray_l * 3] = tg[0]; s.tgt[ray_l * 3 + 1] = tg[1]; s.tgt[ray_l * 3 + 2] = tg[2];
     }
     bar_tile(bar);
@@ -603,7 +623,7 @@ __device__ __forceinline__ void head_and_composite(const TcParams &p, const Comp
     const float Cpre = pr * carry;                   // true inclusive product prod_{k<=s} q_k
     const float T = (smp == 0) ? 1.0f : Cpre;
     const float wgt = a * T;
-    if (WGT && live) p.weights[row0 + tid] = wgt;
+    if (EXT && live && p.weights) p.weights[row0 + tid] = wgt;
     {   // colour: segmented inclusive sums, one shared-memory atomic per (warp, ray) segment
         float s0 = live ? wgt * cr : 0.f, s1 = live ? wgt * cg : 0.f, s2 = live ? wgt * cb : 0.f;
 #pragma unroll
@@ -614,11 +634,29 @@ __device__ __forceinline__ void head_and_composite(const TcParams &p, const Comp
         if (live && (lane == 31 || smp == S - 1)) {
             atomicAdd(s.color + ray_l * 3, s0); atomicAdd(s.color + ray_l * 3 + 1, s1); atomicAdd(s.color + ray_l * 3 + 2, s2);
         }
+        if (EXT) {   // acc = sum w, depth = sum w t: the same segmented sum
+            float s3 = live ? wgt : 0.f, s4 = (live && p.depth) ? wgt * tile_sample_depth(p, ray0 + ray_l, smp, row0 + tid) : 0.f;
+#pragma unroll
+            for (int d = 1; d < 32; d <<= 1) {
+                float o3 = __shfl_up_sync(0xffffffffu, s3, d), o4 = __shfl_up_sync(0xffffffffu, s4, d);
+                if (lane >= d && smp >= d) { s3 += o3; s4 += o4; }
+            }
+            if (live && (lane == 31 || smp == S - 1)) { atomicAdd(s.ext + ray_l * 2, s3); atomicAdd(s.ext + ray_l * 2 + 1, s4); }
+        }
     }
     bar_tile(bar);
     float dc0 = 0.f, dc1 = 0.f, dc2 = 0.f;
     if (live) {
-        const float c0 = s.color[ray_l * 3], c1 = s.color[ray_l * 3 + 1], c2 = s.color[ray_l * 3 + 2];
+        float c0 = s.color[ray_l * 3], c1 = s.color[ray_l * 3 + 1], c2 = s.color[ray_l * 3 + 2];
+        if (EXT) {
+            const float acc = s.ext[ray_l * 2];
+            if (p.background) {
+                const float tr = 1.0f - acc;   // the light that reaches the background
+                c0 = fmaf(tr, p.bg[0], c0); c1 = fmaf(tr, p.bg[1], c1); c2 = fmaf(tr, p.bg[2], c2);
+            }
+            if (smp == 0 && p.acc) p.acc[ray0 + ray_l] = acc;
+            if (smp == 0 && p.depth) p.depth[ray0 + ray_l] = s.ext[ray_l * 2 + 1];
+        }
         if (smp == 0 && p.color) {
             float *co = p.color + (size_t)(ray0 + ray_l) * 3;
             co[0] = c0; co[1] = c1; co[2] = c2;
@@ -632,7 +670,8 @@ __device__ __forceinline__ void head_and_composite(const TcParams &p, const Comp
     }
     if (!GRAD) return;
     // G_s = dT_s + q_{s+1} G_{s+1}: suffix scan of affine maps; B = 0 at a ray's last sample
-    const float d_w = cr * dc0 + cg * dc1 + cb * dc2;
+    const float d_w = (EXT && p.background) ? (cr - p.bg[0]) * dc0 + (cg - p.bg[1]) * dc1 + (cb - p.bg[2]) * dc2
+                                            : cr * dc0 + cg * dc1 + cb * dc2;
     const float dT = (smp == 0 || !live) ? 0.0f : d_w * a;
     float qn = __shfl_down_sync(0xffffffffu, qv, 1);
     if (lane == 31) qn = warp < 3 ? s.headq[warp + 1] : 0.0f;
@@ -713,7 +752,8 @@ __device__ __forceinline__ void relu_adjoint(const uint32_t (&v)[HP / 16][16], c
 // FWD: the forward-only (render) form, compiled separately: nothing of the backward pass in its register budget.  Its
 // launch bounds are the CTAs per SM that tensor memory admits (512 columns / 64 per CTA = 8; 4 for the 64-wide form), not
 // more: a ninth CTA could never allocate its columns and the tighter register budget only bought a spill.
-template <bool RAYS, int HP, bool FWD, bool DIRS = false, bool WGT = false>
+// EXT: the extras instantiations (head_and_composite); its acc / depth scratch follows the colour / target scratch.
+template <bool RAYS, int HP, bool FWD, bool DIRS = false, bool EXT = false>
 __global__ void __launch_bounds__(TILE, FWD ? (HP == 64 ? 4 : 8) : 1) fused_v1_kernel(const TcParams p)
 {
     using LY = TcLayout<HP>;
@@ -744,7 +784,9 @@ __global__ void __launch_bounds__(TILE, FWD ? (HP == 64 ? 4 : 8) : 1) fused_v1_k
     uint64_t *const bar_p = reinterpret_cast<uint64_t *>(tailp + 48);
     uint32_t *const tmem_slot = reinterpret_cast<uint32_t *>(bar_p + 4);
     const uint32_t bar_mma = smem_u32(bar_p), bar_x = smem_u32(bar_p + 1), bar_w = smem_u32(bar_p + 2), bar_dw = smem_u32(bar_p + 3);
-    const CompScratch scratch{color_s, tgt_s, tailp, tail_s, headq, headA, headB};
+    // EXT: [TILE][2] more floats: colour, target and these fill the forward form's two scratch slabs exactly, and the train
+    // form's dZ region (>= 4 slabs) has room to spare
+    const CompScratch scratch{color_s, tgt_s, tgt_s + TILE * 3, tailp, tail_s, headq, headA, headB};
     StageRec *const prog = reinterpret_cast<StageRec *>(reinterpret_cast<uint8_t *>(bar_p) + 64);   // the MMA program
 
     // ---- one-time setup: zero activations, then TMA the weight image and the first tile
@@ -934,7 +976,7 @@ __global__ void __launch_bounds__(TILE, FWD ? (HP == 64 ? 4 : 8) : 1) fused_v1_k
         CLK(16);
         // ---- head + loss + adjoint of the head's pre-activation (unit seed)
         float dz[4];
-        head_and_composite<!FWD, WGT>(p, scratch, 0, hz, my_dist, tg, row0, ray0, valid, tid, smp, ray_l, live, loss_acc, dz);
+        head_and_composite<!FWD, EXT>(p, scratch, 0, hz, my_dist, tg, row0, ray0, valid, tid, smp, ray_l, live, loss_acc, dz);
         CLK(17);
         if (FWD) { __syncthreads(); tile = *next_tile_s; continue; }
         // ---- backward.  dZ_{L-1}: 4 live features, the rest of the 16 stay zero
@@ -1338,7 +1380,8 @@ int lnb_tc_adam_img(lnb_ctx *ctx, const lnb_mlp *mlp, float *param, const float 
     return LNB_OK;
 }
 
-int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf, const lnb_tc_extra *ex)
+int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf, const lnb_tc_extra *ex,
+                      const lnb_comp_args *cx)
 {
     const int L = mlp->n_layers;
     auto unsupported = [&](const char *why) {
@@ -1395,18 +1438,21 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
     // Train steps run on the multi-group kernel (fused_mg.cuh: one CTA per SM, up to seven 128-thread groups, adjoints in
     // place); forward-only launches and LNB_TC_V1=1 on the one-tile-per-CTA kernel above.
     const bool mg = grad && getenv("LNB_TC_V1") == nullptr && (!nerf || S >= 2);
-    const bool wgt = grad && nerf && ex && ex->weights;   // lnb_trainer_step_weights
+    // the extras instantiations: lnb_trainer_step_weights, and any step with compositing extras (lnb_composite)
+    const bool ext = nerf && ((grad && ex && ex->weights) || cx);
     if (grad && !mg) {   // the one-tile-per-CTA kernel computes all weight gradients with ONE concatenated M = 128 MMA per K-step
         if (K0P / 8 + (L - 1) * (HP / 8) > 16) return unsupported("input + hidden widths exceed 128 features in total");
         if ((L - 1) * HP + 16 > 256) return unsupported("hidden widths exceed 256 gradient columns");
     }
     void (*const kern)(TcParams) = with_hp(HP, [&](auto hp) -> void (*)(TcParams) {
         constexpr int H = decltype(hp)::value;
-        if (mg && wgt) return dirs ? fused_mg_kernel<true, H, true, true> : rays ? fused_mg_kernel<true, H, false, true> : fused_mg_kernel<false, H, false, true>;
+        if (mg && ext) return dirs ? fused_mg_kernel<true, H, true, true> : rays ? fused_mg_kernel<true, H, false, true> : fused_mg_kernel<false, H, false, true>;
         if (mg) return dirs ? fused_mg_kernel<true, H, true> : rays ? fused_mg_kernel<true, H> : fused_mg_kernel<false, H>;
-        if (grad && wgt)
+        if (grad && ext)
             return dirs ? fused_v1_kernel<true, H, false, true, true> : rays ? fused_v1_kernel<true, H, false, false, true> : fused_v1_kernel<false, H, false, false, true>;
         if (grad) return dirs ? fused_v1_kernel<true, H, false, true> : rays ? fused_v1_kernel<true, H, false> : fused_v1_kernel<false, H, false>;
+        if (ext)
+            return dirs ? fused_v1_kernel<true, H, true, true, true> : rays ? fused_v1_kernel<true, H, true, false, true> : fused_v1_kernel<false, H, true, false, true>;
         return dirs ? fused_v1_kernel<true, H, true, true> : rays ? fused_v1_kernel<true, H, true> : fused_v1_kernel<false, H, true>;
     });
     size_t smem = 0;
@@ -1418,8 +1464,8 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
             while (n > 1 && (MG::total(L, c_in, K0P, rays, n) > 232448 || MG::tmem_need(L, K0P, n) > 512)) --n;
             return n;
         });
-        static int mg_regs[2][3][3] = {}; // registers per thread of each instantiation ([weights] (features, rays, rays + directions)), asked once
-        int &regs = mg_regs[wgt][dirs ? 2 : (rays ? 1 : 0)][HP / 32];
+        static int mg_regs[2][3][3] = {}; // registers per thread of each instantiation ([extras] (features, rays, rays + directions)), asked once
+        int &regs = mg_regs[ext][dirs ? 2 : (rays ? 1 : 0)][HP / 32];
         if (regs == 0) {
             cudaFuncAttributes fa;
             LNB_CUDA(cudaFuncGetAttributes(&fa, kern));
@@ -1457,7 +1503,11 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
     uint8_t *wimg = (uint8_t *)lnb_arena_take(ctx, wimg_bytes);
     p.wimg = (ex && ex->wimg) ? ex->wimg : wimg;
     p.t_dev = ex ? ex->t_dev : nullptr;
-    p.weights = wgt ? ex->weights : nullptr;
+    p.weights = (ext && ex) ? ex->weights : nullptr;
+    if (cx) {
+        p.acc = cx->acc; p.depth = cx->depth; p.background = cx->background;
+        for (int c = 0; c < 3; ++c) p.bg[c] = cx->bg[c];
+    }
     if (!ctx->tc_counter) {
         LNB_CUDA(cudaMalloc((void **)&ctx->tc_counter, 256));
         LNB_CUDA(cudaMemsetAsync(ctx->tc_counter, 0, 256, ctx->stream));
@@ -1483,11 +1533,14 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
             LNB_CHECK_LAUNCH();
         }
         // the dynamic shared-memory limit of each kernel instantiation (kind, input, HP) on each device: raised only when it grows
-        static size_t smem_set[3][3][3][64] = {};
-        size_t &lim = smem_set[mg ? 0 : (grad ? 1 : 2)][dirs ? 2 : (rays ? 1 : 0)][HP / 32][ctx->device & 63];
+        static size_t smem_set[2][3][3][3][64] = {};
+        size_t &lim = smem_set[ext][mg ? 0 : (grad ? 1 : 2)][dirs ? 2 : (rays ? 1 : 0)][HP / 32][ctx->device & 63];
         if (smem > lim || ctx->device > 63) { LNB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); lim = smem; }
-        lnb_prof_begin(ctx, mg ? (rays ? "fused_mg_kernel<rays>" : "fused_mg_kernel<features>")
-                              : (rays ? "fused_v1_kernel<rays>" : "fused_v1_kernel<features>"));      // the symbols ncu lists
+        // the symbols ncu lists; "+extras": an extras instantiation (weights / acc / depth / background)
+        static const char *const names[2][2][2] = {{{"fused_v1_kernel<features>", "fused_v1_kernel<rays>"}, {"fused_mg_kernel<features>", "fused_mg_kernel<rays>"}},
+                                                   {{"fused_v1_kernel<features>+extras", "fused_v1_kernel<rays>+extras"},
+                                                    {"fused_mg_kernel<features>+extras", "fused_mg_kernel<rays>+extras"}}};
+        lnb_prof_begin(ctx, names[ext][mg][rays]);
         LNB_CUDA(cudaLaunchKernelEx(&cfg, kern, p));
         lnb_prof_end(ctx);
         LNB_CHECK_LAUNCH();

@@ -7,6 +7,7 @@
 // scripts/mlp_fit.py:39-147 and their reverse (loma_public/reverse_diff.py:576-951).
 #include <stdint.h>
 
+#include "camera.cuh"
 #include "lnb_internal.h"
 
 namespace {
@@ -442,17 +443,36 @@ __device__ __forceinline__ float warp_incl_prod(float p, int lane)
     return p;
 }
 
+// The compositing extras (lnb_composite) as the EXT instantiations of the kernels below take them (by value): the
+// background, the acc / depth outputs and the depth source of sample s of ray r (sample_depth)
+struct CompK {
+    int background;
+    float bg0, bg1, bg2;
+    float *acc, *depth;
+    const void *t;
+    int t_f64, cam_mode;
+    CamDev cam;
+};
+__device__ __forceinline__ float sample_depth(const CompK &k, int ray, int s, int S)
+{
+    if (k.cam_mode) return (float)cam_t_f64(k.cam, cam_pixel(k.cam, ray), s, S);
+    const size_t i = (size_t)ray * S + s;
+    return k.t_f64 ? (float)__ldg(reinterpret_cast<const double *>(k.t) + i) : __ldg(reinterpret_cast<const float *>(k.t) + i);
+}
+
+// EXT: with the extras of `k` (acc = sum w, depth = sum w t, colour += (1 - acc) bg before the caller's colour is added)
+template <bool EXT>
 __global__ void __launch_bounds__(COMP_WARPS * 32)
 composite_fwd_kernel(const float *__restrict__ head, int ldh, const float *__restrict__ dists,
                      const float *__restrict__ target, int R, int S, float *__restrict__ rgba,
                      float *__restrict__ alpha, float *__restrict__ cumprod,
                      float *__restrict__ weights, float *__restrict__ color, int color_accumulate,
-                     float *__restrict__ ray_sse)
+                     float *__restrict__ ray_sse, const CompK k)
 {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int ray = blockIdx.x * COMP_WARPS + warp;
     if (ray >= R) return;
-    float carry = 1.0f, c0 = 0.0f, c1 = 0.0f, c2 = 0.0f;
+    float carry = 1.0f, c0 = 0.0f, c1 = 0.0f, c2 = 0.0f, c3 = 0.0f, c4 = 0.0f;   // c3, c4: acc, depth (EXT)
     for (int s0 = 0; s0 < S; s0 += 32) {
         const int s = s0 + lane;
         const bool valid = s < S;
@@ -475,6 +495,10 @@ composite_fwd_kernel(const float *__restrict__ head, int ldh, const float *__res
             if (cumprod) cumprod[i] = T;
             if (weights) weights[i] = w;
             c0 = fmaf(w, r, c0); c1 = fmaf(w, gch, c1); c2 = fmaf(w, b, c2);
+            if (EXT) {
+                c3 += w;
+                if (k.depth) c4 = fmaf(w, sample_depth(k, ray, s, S), c4);
+            }
         }
     }
 #pragma unroll
@@ -482,9 +506,21 @@ composite_fwd_kernel(const float *__restrict__ head, int ldh, const float *__res
         c0 += __shfl_xor_sync(0xffffffffu, c0, d);
         c1 += __shfl_xor_sync(0xffffffffu, c1, d);
         c2 += __shfl_xor_sync(0xffffffffu, c2, d);
+        if (EXT) {
+            c3 += __shfl_xor_sync(0xffffffffu, c3, d);
+            c4 += __shfl_xor_sync(0xffffffffu, c4, d);
+        }
     }
     if (lane == 0) {
         float *c = color + (size_t)ray * 3;
+        if (EXT) {
+            if (k.acc) k.acc[ray] = c3;
+            if (k.depth) k.depth[ray] = c4;
+            if (k.background) {
+                const float tr = 1.0f - c3;   // the light that reaches the background
+                c0 = fmaf(tr, k.bg0, c0); c1 = fmaf(tr, k.bg1, c1); c2 = fmaf(tr, k.bg2, c2);
+            }
+        }
         if (color_accumulate) { c0 += c[0]; c1 += c[1]; c2 += c[2]; }
         c[0] = c0; c[1] = c1; c[2] = c2;
         float sse = 0.0f;
@@ -502,11 +538,13 @@ composite_fwd_kernel(const float *__restrict__ head, int ldh, const float *__res
 //   d_alpha_s = d_w_s T_s - dq_s;  dT_s = d_w_s alpha_s (s >= 1), dT_0 = 0
 //   G_s = dT_s + q_{s+1} G_{s+1}  (G_S = 0);  dq_s = Cpre_{s-1} G_s, Cpre_{-1} = 1
 //   e = expf(-sigma dist); d_sigma = d_alpha e dist; d_dist = d_alpha e sigma
+// EXT with a background: d_w_s = <rgb_s - bg, dcol> (the background term's adjoint; bg itself gets none)
+template <bool EXT>
 __global__ void __launch_bounds__(COMP_WARPS * 32)
 composite_bwd_kernel(const float *__restrict__ head, int ldh, const float *__restrict__ dists,
                      const float *__restrict__ target, const float *__restrict__ color, int R,
                      int S, float *__restrict__ dZ, int ldz, int out_dim,
-                     float *__restrict__ d_dists_u, float *__restrict__ d_color_u)
+                     float *__restrict__ d_dists_u, float *__restrict__ d_color_u, const CompK k)
 {
     __shared__ float carry_in[COMP_WARPS][COMP_MAX_CHUNKS];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -559,7 +597,8 @@ composite_bwd_kernel(const float *__restrict__ head, int ldh, const float *__res
         const float Cpre = warp_incl_prod(q, lane) * cin; // true inclusive product
         const float T = (s == 0) ? 1.0f : Cpre;
         const float w = a * T;
-        const float d_w = r * dc0 + gch * dc1 + b * dc2;
+        const float d_w = (EXT && k.background) ? (r - k.bg0) * dc0 + (gch - k.bg1) * dc1 + (b - k.bg2) * dc2
+                                                : r * dc0 + gch * dc1 + b * dc2;
         const float dT = (s == 0 || !valid) ? 0.0f : d_w * a;
         // affine suffix scan: G_s = A_s + B_s * G_next
         float qn = __shfl_down_sync(0xffffffffu, q, 1);
@@ -738,27 +777,41 @@ int lnb_launch_dw_reduce(lnb_ctx *ctx, const float *partial, int n_chunks, int i
     return LNB_OK;
 }
 
+static CompK comp_k(const lnb_comp_args *cx)
+{
+    CompK k{};
+    if (!cx) return k;
+    k.background = cx->background;
+    k.bg0 = cx->bg[0]; k.bg1 = cx->bg[1]; k.bg2 = cx->bg[2];
+    k.acc = cx->acc; k.depth = cx->depth;
+    k.t = cx->t; k.t_f64 = cx->t_f64;
+    if (cx->cam) { k.cam_mode = 1; k.cam = make_cam_dev(*cx->cam); }
+    return k;
+}
+
 int lnb_launch_composite_fwd(lnb_ctx *ctx, const float *head, int ldh, const float *dists,
                              const float *target, int R, int S, float *rgba, float *alpha,
                              float *cumprod, float *weights, float *color, int color_accumulate,
-                             float *ray_sse)
+                             float *ray_sse, const lnb_comp_args *cx)
 {
     if (R <= 0) return LNB_OK;
-    composite_fwd_kernel<<<(R + COMP_WARPS - 1) / COMP_WARPS, COMP_WARPS * 32, 0, ctx->stream>>>(
+    auto kern = cx ? composite_fwd_kernel<true> : composite_fwd_kernel<false>;
+    kern<<<(R + COMP_WARPS - 1) / COMP_WARPS, COMP_WARPS * 32, 0, ctx->stream>>>(
         head, ldh, dists, target, R, S, rgba, alpha, cumprod, weights, color, color_accumulate,
-        ray_sse);
+        ray_sse, comp_k(cx));
     LNB_CHECK_LAUNCH();
     return LNB_OK;
 }
 
 int lnb_launch_composite_bwd(lnb_ctx *ctx, const float *head, int ldh, const float *dists,
                              const float *target, const float *color, int R, int S, float *dZ_head,
-                             int ldz, int out_dim, float *d_dists_u, float *d_color_u)
+                             int ldz, int out_dim, float *d_dists_u, float *d_color_u, const lnb_comp_args *cx)
 {
     if (R <= 0) return LNB_OK;
     LNB_ARG(S <= 32 * COMP_MAX_CHUNKS, "samples per ray > 2048");
-    composite_bwd_kernel<<<(R + COMP_WARPS - 1) / COMP_WARPS, COMP_WARPS * 32, 0, ctx->stream>>>(
-        head, ldh, dists, target, color, R, S, dZ_head, ldz, out_dim, d_dists_u, d_color_u);
+    auto kern = (cx && cx->background) ? composite_bwd_kernel<true> : composite_bwd_kernel<false>;
+    kern<<<(R + COMP_WARPS - 1) / COMP_WARPS, COMP_WARPS * 32, 0, ctx->stream>>>(
+        head, ldh, dists, target, color, R, S, dZ_head, ldz, out_dim, d_dists_u, d_color_u, comp_k(cx));
     LNB_CHECK_LAUNCH();
     return LNB_OK;
 }

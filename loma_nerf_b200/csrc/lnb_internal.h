@@ -113,10 +113,12 @@ int lnb_launch_dw_reduce(lnb_ctx *ctx, const float *partial, int n_chunks, int i
 // compositing forward: one warp per ray (scripts/nerf.py:176-288). ray_sse[r] = sum_c (col-t)^2
 // (0 when target == NULL).  Any of rgba/alpha/cumprod/weights may be NULL.  color is read first
 // when color_accumulate (nerf.py:284-286 adds onto the caller's buffer).
+// cx (NULL: the reference's compositing) adds the extras of lnb_composite: the background term, acc / depth outputs.
+struct lnb_comp_args;
 int lnb_launch_composite_fwd(lnb_ctx *ctx, const float *head, int ldh, const float *dists,
                              const float *target, int R, int S, float *rgba, float *alpha,
                              float *cumprod, float *weights, float *color, int color_accumulate,
-                             float *ray_sse);
+                             float *ray_sse, const lnb_comp_args *cx = nullptr);
 // compositing backward with UNIT seed (the caller scales): from head (post-activation), dists,
 // the final colour and target writes dZ_head[i][0..3] = adjoint of the head's PRE-activation
 // (sigmoid'/ReLU mask applied), and when non-NULL d_dists_u [R][S], d_color_u [R][3]
@@ -124,7 +126,7 @@ int lnb_launch_composite_fwd(lnb_ctx *ctx, const float *head, int ldh, const flo
 int lnb_launch_composite_bwd(lnb_ctx *ctx, const float *head, int ldh, const float *dists,
                              const float *target, const float *color, int R, int S,
                              float *dZ_head, int ldz, int out_dim, float *d_dists_u,
-                             float *d_color_u);
+                             float *d_color_u, const lnb_comp_args *cx = nullptr);
 // out[0] = sum_i v[i]  (fixed order, one block)
 int lnb_launch_sum(lnb_ctx *ctx, const float *v, long long n, float *out);
 // mlp_fit loss terms: ray_sse[r] = sum_{c<Wt} (pred[r][c]-t[r][c])^2 (scripts/mlp_fit.py:140-145)
@@ -139,6 +141,21 @@ int lnb_launch_fill(lnb_ctx *ctx, float *p, size_t n, float v);
 int lnb_launch_axpy2d(lnb_ctx *ctx, float *dst, long long ldd, const float *src, long long lds,
                       long long rows, int cols, float sign, float seed_value,
                       const float *seed_dev);
+
+// The compositing extras (lnb_composite) of one step as the kernels take them.  The depths are the ones the encoder used:
+// rays mode t (float64 or float32), camera mode the camera (its depths re-derived per sample), features mode none.
+struct lnb_comp_args {
+    int background = 0;
+    float bg[3] = {0.f, 0.f, 0.f};
+    float *acc = nullptr, *depth = nullptr;
+    const void *t = nullptr;       // rays mode: [R][S] sample depths
+    int t_f64 = 0;
+    const lnb_camera *cam = nullptr; // camera mode (host pointer; its pixel list is a device pointer)
+};
+// NULL when comp asks for nothing (the step is then exactly lnb_nerf_step), else comp with the depth source of step a
+// filled in; LNB_ERR_ARG for the cases lnb_composite lists (api_flat.cu)
+int lnb_comp_resolve(lnb_ctx *ctx, const lnb_step_args *a, bool nerf, const lnb_composite *comp, lnb_comp_args *out,
+                     const lnb_comp_args **resolved);
 
 // ---- fused_tc.cu ---------------------------------------------------------------------------
 // Optional extras of the fused tensor-core step, used by the trainer (trainer.cu):
@@ -167,12 +184,14 @@ struct lnb_tc_extra {
     void *wimg_out = nullptr;
     float *weights = nullptr;                           // train kernels: [R][S] compositing weights w_s = alpha_s T_s
 };
+// cx: the compositing extras (lnb_comp_resolve), or NULL
 int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf,
-                      const lnb_tc_extra *ex);
-// validated dispatch of one step with tensor-core extras (api_flat.cu)
-int lnb_step_ex(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf, const lnb_tc_extra *ex);
+                      const lnb_tc_extra *ex, const lnb_comp_args *cx = nullptr);
+// validated dispatch of one step with tensor-core extras and / or compositing extras (api_flat.cu)
+int lnb_step_ex(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf, const lnb_tc_extra *ex,
+                const lnb_composite *comp = nullptr);
 // layerwise tensor-core step for wide MLPs (wide_tc.cu); LNB_ERR_UNSUPPORTED when it does not apply
-int lnb_wide_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf);
+int lnb_wide_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf, const lnb_comp_args *cx = nullptr);
 // padded widths of the fused kernel for this MLP, 0 when unsupported; bytes of its weight image
 int lnb_tc_layout(const lnb_mlp *mlp, int *HP, int *K0P, int *wimg_bytes);
 // build the weight image from fp32 padded weights (one small kernel)
@@ -184,7 +203,9 @@ int lnb_tc_adam_img(lnb_ctx *ctx, const lnb_mlp *mlp, float *param, const float 
 
 // ---- fused_f32.cu: the fused exact (fp32 CUDA-core) step for the reference's own network shapes; LNB_ERR_UNSUPPORTED
 // when the problem (or the outputs asked for) does not fit it
-int lnb_fused_f32_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf, int overwrite);
+// (it has no compositing extras: a step with cx != NULL is LNB_ERR_UNSUPPORTED there and runs on the layerwise kernels)
+int lnb_fused_f32_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf, int overwrite,
+                       const lnb_comp_args *cx = nullptr);
 int lnb_step_f32_fused(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf, int overwrite);   // validated (api_flat.cu)
 
 // ---- encode.cu / optim.cu ---------------------------------------------------------------------

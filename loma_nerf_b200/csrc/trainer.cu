@@ -7,6 +7,7 @@
 //     fused forward+backward kernel  ->  reduce partials + optimiser update + weight-image refresh
 // For multi-GPU data parallelism the step splits at the gradient buffer:
 //     lnb_trainer_grad -> (caller: NCCL all-reduce of lnb_trainer_grad_buffer) -> lnb_trainer_apply
+#include <math.h>
 #include <stdlib.h>
 #include <string.h>
 
@@ -25,6 +26,7 @@ struct lnb_trainer {
     void *wimg = nullptr;    // tensor-core weight image, kept in sync with params
     bool tc_ok = false;
     bool t_bumped = false;   // the last lnb_trainer_grad already incremented *t_dev
+    lnb_composite comp{};    // lnb_trainer_set_background: background 0 = the reference's compositing
     // peer-memory all-reduce (lnb_trainer_comm_*): header [status | pad] + receive slots for 8 senders
     char *comm_buf = nullptr;
     size_t comm_bytes = 0;
@@ -130,6 +132,7 @@ static int trainer_run(lnb_trainer *t, const lnb_step_args *batch, int nerf, boo
     a.d_ws = t->grads; a.d_bs = t->grads + t->n_w; a.loss = t->grads + t->n_w + t->n_b;
     a.d_X = a.d_target = a.d_dists = a.d_color = a.d_inter = nullptr;
     a.inter = a.rgba = a.alpha = a.cumprod = a.weights = nullptr;
+    const lnb_composite *comp = (nerf && t->comp.background) ? &t->comp : nullptr;   // every route below composites onto it
     if (a.path == LNB_PATH_TC && t->tc_ok) {
         lnb_tc_extra ex;
         ex.wimg = t->wimg; ex.overwrite_grads = 1; ex.t_dev = t->t_dev; ex.weights = weights;
@@ -138,7 +141,7 @@ static int trainer_run(lnb_trainer *t, const lnb_step_args *batch, int nerf, boo
             ex.fuse_adam = 1; ex.param = t->params; ex.m = t->opt == LNB_OPT_ADAM ? t->m : nullptr; ex.v = t->v;
             ex.lr = t->lr; ex.b1 = t->b1; ex.b2 = t->b2; ex.eps = t->eps; ex.wimg_out = t->wimg;
         }
-        const int rc = lnb_step_ex(ctx, &t->mlp, &a, nerf != 0, &ex);
+        const int rc = lnb_step_ex(ctx, &t->mlp, &a, nerf != 0, &ex, comp);
         if (rc == LNB_OK) { t->t_bumped = !fuse_update; return LNB_OK; }
         // the MLP fits the fused kernel but this batch does not (e.g. S > 128): the layerwise
         // tensor-core kernels below take it, exactly as lnb_nerf_step would
@@ -152,17 +155,18 @@ static int trainer_run(lnb_trainer *t, const lnb_step_args *batch, int nerf, boo
                    "exchange gradients in-kernel; use lnb_trainer_grad + an all-reduce of lnb_trainer_grad_buffer + lnb_trainer_apply";
         return LNB_ERR_UNSUPPORTED;
     }
-    // the fused exact kernel writes no weights: a step that asks for them runs on the layerwise kernels
+    // the fused exact kernel writes no weights and has no background: a step that asks for either runs on the layerwise
+    // kernels
     a.weights = weights;
     int rc = LNB_ERR_UNSUPPORTED;
-    if (a.path == LNB_PATH_F32 && !getenv("LNB_F32_NO_FUSED")) {
+    if (a.path == LNB_PATH_F32 && !comp && !getenv("LNB_F32_NO_FUSED")) {
         // fused exact kernel writing the (zero-padded, never otherwise touched) gradient buffer: no memset
         rc = lnb_step_f32_fused(ctx, &t->mlp, &a, nerf != 0, 1);
         if (rc != LNB_OK && rc != LNB_ERR_UNSUPPORTED) return rc;
     }
     if (rc == LNB_ERR_UNSUPPORTED) {
         LNB_CUDA(cudaMemsetAsync(t->grads, 0, (size_t)(t->n_w + t->n_b + 1) * 4, ctx->stream));
-        LNB_TRY(nerf ? lnb_nerf_step(ctx, &t->mlp, &a) : lnb_fit_step(ctx, &t->mlp, &a));
+        LNB_TRY(nerf ? lnb_step_ex(ctx, &t->mlp, &a, true, nullptr, comp) : lnb_fit_step(ctx, &t->mlp, &a));
     }
     t->t_bumped = false;
     if (fuse_update) return lnb_trainer_apply(t);
@@ -173,6 +177,18 @@ extern "C" int lnb_trainer_grad(lnb_trainer *t, const lnb_step_args *batch, int 
 {
     if (!t) return LNB_ERR_ARG;
     return trainer_run(t, batch, nerf, false);
+}
+
+extern "C" int lnb_trainer_set_background(lnb_trainer *t, const float *rgb)
+{
+    if (!t) return LNB_ERR_ARG;
+    lnb_ctx *ctx = t->ctx;
+    if (!rgb) { t->comp = lnb_composite{}; return LNB_OK; }
+    for (int c = 0; c < 3; ++c) LNB_ARG(isfinite(rgb[c]), "trainer_set_background: non-finite colour");
+    t->comp = lnb_composite{};
+    t->comp.background = 1;
+    for (int c = 0; c < 3; ++c) t->comp.bg[c] = rgb[c];
+    return LNB_OK;
 }
 
 extern "C" int lnb_trainer_step(lnb_trainer *t, const lnb_step_args *batch, int nerf)

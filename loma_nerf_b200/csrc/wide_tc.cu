@@ -808,7 +808,7 @@ extern "C" LNB_API int lnb_test_wide_dw(lnb_ctx *ctx, const void *H, int in_pad,
 // ---------------------------------------------------------------------------------------------
 static int pad64(int v) { return (v + 63) / 64 * 64; }
 
-int lnb_wide_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf)
+int lnb_wide_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf, const lnb_comp_args *cx)
 {
     auto unsupported = [&](const char *why) {
         ctx->err = std::string("wide tensor-core path: ") + why;
@@ -942,12 +942,12 @@ int lnb_wide_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, b
         LNB_TRY(run_chain(cd, L, mlp->head));
     }
     if (nerf)
-        LNB_TRY(lnb_launch_composite_fwd(ctx, head, 4, dists, a->target, R, S, a->rgba, a->alpha, a->cumprod, a->weights, color, 0, ray_sse));
+        LNB_TRY(lnb_launch_composite_fwd(ctx, head, 4, dists, a->target, R, S, a->rgba, a->alpha, a->cumprod, a->weights, color, 0, ray_sse, cx));
     else if (a->target)   // mlp_fit: the prediction is the sigmoid head itself, SSE over target_w channels (mlp_fit.py:140-145)
         LNB_TRY(lnb_launch_fit_loss(ctx, head, 4, a->target, R, a->target_w, ray_sse));
     if (grad) {
         if (nerf)
-            LNB_TRY(lnb_launch_composite_bwd(ctx, head, 4, dists, a->target, color, R, S, dzh, 4, 4, d_dists_u, d_color_u));
+            LNB_TRY(lnb_launch_composite_bwd(ctx, head, 4, dists, a->target, color, R, S, dzh, 4, 4, d_dists_u, d_color_u, cx));
         else
             LNB_TRY(lnb_launch_fit_head_bwd(ctx, head, 4, a->target, R, a->target_w, R, 4, dzh, 4, nullptr));
         const long long n = N * (out_pad[L - 1] / 8);

@@ -27,10 +27,12 @@ def compute_psnr(img1, img2, max_val=1.0):
         return 20 * np.log10(max_val / np.sqrt(mse))
 
 
-def render_rays(ctx, dims, ws, bs, rays_o, rays_d, t, pe_bands, path="tc", rays_per_call=1 << 18, dir_bands=None):
+def render_rays(ctx, dims, ws, bs, rays_o, rays_d, t, pe_bands, path="tc", rays_per_call=1 << 18, dir_bands=None,
+                background=None):
     """Colours [R][3] (numpy float32) of R rays; rays_o/rays_d [R][3] and t [R][S] numpy (float64 as
     the reference makes them, or float32).  Host buffers in, host buffer out, chunked so the device
-    staging stays bounded.  dir_bands: the net also takes the view direction (Context.nerf_step_rays)."""
+    staging stays bounded.  dir_bands: the net also takes the view direction (Context.nerf_step_rays).
+    background=(r, g, b): composited onto that colour (e.g. (1, 1, 1) for a net trained on white)."""
     R = rays_o.shape[0]
     out = np.empty((R, 3), np.float32)
     ws = np.ascontiguousarray(ws, np.float32)
@@ -39,15 +41,16 @@ def render_rays(ctx, dims, ws, bs, rays_o, rays_d, t, pe_bands, path="tc", rays_
         r1 = min(R, r0 + rays_per_call)
         res = ctx.nerf_step_rays(dims, np.ascontiguousarray(rays_o[r0:r1]), np.ascontiguousarray(rays_d[r0:r1]),
                                  np.ascontiguousarray(t[r0:r1]), pe_bands, ws, bs, target=None, grad=False,
-                                 outputs=("color",), path=path, dir_bands=dir_bands)
+                                 outputs=("color",), path=path, dir_bands=dir_bands, background=background)
         out[r0:r1] = res["color"]
     return out
 
 
 def render_frame(ctx, dims, ws, bs, height, width, normalized_K, c2w_pose, n_samples, pe_bands, near=2.0, far=6.0,
-                 path="tc", dir_bands=None, fine=None):
+                 path="tc", dir_bands=None, fine=None, background=None):
     """One H x W frame: t = linspace(near, far, S) for every ray (train_nerf.py:589-605).  fine=(dims_f, ws_f, bs_f,
-    n_fine): hierarchical sampling, the frame render_frame_device(fine=...) makes, as float colours."""
+    n_fine): hierarchical sampling, the frame render_frame_device(fine=...) makes, as float colours.  background as in
+    render_rays."""
     if fine is not None:
         import torch
         dev = torch.device("cuda", ctx.device)
@@ -55,29 +58,44 @@ def render_frame(ctx, dims, ws, bs, height, width, normalized_K, c2w_pose, n_sam
         color = torch.empty((height * width, 3), dtype=torch.float32, device=dev)
         dims_f, ws_f, bs_f, n_fine = fine
         render_frame_device(ctx, dims, cv(ws), cv(bs), height, width, normalized_K, c2w_pose, n_samples, pe_bands, near=near,
-                            far=far, path=path, color=color, dir_bands=dir_bands, fine=(dims_f, cv(ws_f), cv(bs_f), n_fine))
+                            far=far, path=path, color=color, dir_bands=dir_bands, fine=(dims_f, cv(ws_f), cv(bs_f), n_fine),
+                            background=background)
         ctx.order_torch_after()
         return color.cpu().numpy().reshape(height, width, 3)
     o, d = get_rays(height, width, normalized_K, c2w_pose)
     t = np.broadcast_to(np.linspace(near, far, n_samples)[None, :], (o.shape[0], n_samples))
     return render_rays(ctx, dims, ws, bs, o, d, np.ascontiguousarray(t), pe_bands, path=path,
-                       dir_bands=dir_bands).reshape(height, width, 3)
+                       dir_bands=dir_bands, background=background).reshape(height, width, 3)
 
 
 def render_frame_device(ctx, dims, ws_dev, bs_dev, height, width, normalized_K, c2w_pose, n_samples, pe_bands, near=2.0, far=6.0,
-                        path="tc", out_u8=None, color=None, rays_per_call=None, dir_bands=None, fine=None):
+                        path="tc", out_u8=None, color=None, rays_per_call=None, dir_bands=None, fine=None, background=None,
+                        acc=None, depth=None):
     """One frame with NOTHING per ray crossing the bus: the pose goes in (camera mode: rays and the linspace depths of
     train_nerf.py:589-605 are generated inside the kernels), a uint8 H x W x 3 frame (torch cuda tensor) comes out.
     ws_dev / bs_dev are cuda tensors in the padded layout.
     fine=(dims_f, ws_f, bs_f, n_fine) renders with hierarchical sampling: per chunk of rays, the camera's rays and S
     coarse depths (lnb_camera_rays), a forward-only coarse pass for the compositing weights, a deterministic sample_pdf
-    of n_fine more depths, and the fine net's colour at all S + n_fine of them (rays mode)."""
+    of n_fine more depths, and the fine net's colour at all S + n_fine of them (rays mode).
+    background=(r, g, b) composites the colour onto that background; acc= / depth= ([H*W] float32 CUDA tensors) receive
+    the opacity and the expected-depth maps (sum of w_s, sum of w_s t_s), filled chunk by chunk in the same kernels as
+    the colour (under fine=, from the fine pass)."""
     import torch
     from . import api
     n = height * width
     dev = ws_dev.device
     color = torch.empty((n, 3), dtype=torch.float32, device=dev) if color is None else color
     step = n if rays_per_call is None else int(rays_per_call)
+    for name, m in (("acc", acc), ("depth", depth)):
+        if m is not None and not (api._is_cuda(m) and m.dtype == torch.float32 and m.is_contiguous() and tuple(m.shape) == (n,)):
+            raise ValueError("%s must be a contiguous [%d] float32 CUDA tensor" % (name, n))
+
+    def maps(r0, r1):   # the colour and whichever maps were asked for, for rays r0 .. r1
+        outs, bufs = ("color",), {"color": color[r0:r1]}
+        for name, m in (("acc", acc), ("depth", depth)):
+            if m is not None:
+                outs, bufs[name] = outs + (name,), m[r0:r1]
+        return outs, bufs
     if fine is not None:
         dims_f, ws_f, bs_f, n_fine = fine
         m = min(step, n)
@@ -88,9 +106,10 @@ def render_frame_device(ctx, dims, ws_dev, bs_dev, height, width, normalized_K, 
     for r0 in range(0, n, step):
         r1 = min(n, r0 + step)
         cam = api.make_camera(c2w_pose, normalized_K, width, height, near=near, far=far, first_pixel=r0)
+        outs, bufs = maps(r0, r1)
         if fine is None:
             ctx.nerf_step_camera(dims, cam, r1 - r0, n_samples, pe_bands, ws_dev, bs_dev, target=None, grad=False,
-                                 outputs=("color",), out={"color": color[r0:r1]}, path=path, dir_bands=dir_bands)
+                                 outputs=outs, out=bufs, path=path, dir_bands=dir_bands, background=background)
             continue
         k = r1 - r0
         ck, dk, tk, wk, tfk = o[:k], d[:k], t[:k], w[:k], t_fine[:k]
@@ -98,8 +117,8 @@ def render_frame_device(ctx, dims, ws_dev, bs_dev, height, width, normalized_K, 
         ctx.nerf_step_camera(dims, cam, k, n_samples, pe_bands, ws_dev, bs_dev, target=None, grad=False,
                              outputs=("weights",), out={"weights": wk}, path=path, dir_bands=dir_bands)
         ctx.sample_pdf(tk, wk, n_fine, stratified=False, ray0=r0, out=tfk)
-        ctx.nerf_step_rays(dims_f, ck, dk, tfk, pe_bands, ws_f, bs_f, target=None, grad=False, outputs=("color",),
-                           out={"color": color[r0:r1]}, path=path, dir_bands=dir_bands)
+        ctx.nerf_step_rays(dims_f, ck, dk, tfk, pe_bands, ws_f, bs_f, target=None, grad=False, outputs=outs,
+                           out=bufs, path=path, dir_bands=dir_bands, background=background)
     return ctx.color_to_u8(color, out_u8).reshape(height, width, 3)
 
 
@@ -167,19 +186,19 @@ def write_mjpeg_avi(path, frames, fps=30, quality=90):
 
 
 def render_video(ctx, dims, ws, bs, height, width, normalized_K, poses, n_samples, pe_bands, out_dir=None, near=2.0, far=6.0,
-                 path="tc", ground_truth=None, fps=30, frame_fn=None, dir_bands=None, fine=None):
+                 path="tc", ground_truth=None, fps=30, frame_fn=None, dir_bands=None, fine=None, background=None):
     """What make_nerf_video.py is named for but does not do (it stitches ground-truth PNGs): render one frame per
     camera pose with the trained weights, optionally score each against its ground-truth image
     (train_nerf.py:163-183) and write frame_%04d.png, an animated orbit.gif and a Motion-JPEG orbit.avi into out_dir (PIL
     only; an mp4 needs imageio/ffmpeg, which the hosts' environment may not have).  Returns (frames uint8 [F][H][W][3],
     psnr list | None).
     frame_fn(i, pose) -> float image may replace the device render (tests of the host side).  fine: hierarchical
-    sampling, as in render_frame."""
+    sampling and background, as in render_frame."""
     frames, psnr = [], ([] if ground_truth is not None else None)
     for i, pose in enumerate(poses):
         img = frame_fn(i, pose) if frame_fn else render_frame(ctx, dims, ws, bs, height, width, normalized_K, np.asarray(pose, np.float64),
                                                             n_samples, pe_bands, near=near, far=far, path=path,
-                                                            dir_bands=dir_bands, fine=fine)
+                                                            dir_bands=dir_bands, fine=fine, background=background)
         img = np.clip(np.asarray(img, np.float32), 0.0, 1.0)
         if ground_truth is not None:
             psnr.append(float(compute_psnr(img, ground_truth[i])))
