@@ -66,9 +66,18 @@ def allreduce_gradients(flat, group=None):
 
 
 def data_parallel_step(trainer, batch, group=None):
-    """One data-parallel train step on this rank's shard: gradients, all-reduce, optimiser."""
-    trainer.grad(**batch)
+    """One data-parallel train step on this rank's shard: gradients, all-reduce, optimiser.
+
+    Every rank applies the gradient of the whole batch.  With a numeric seed that is the sum of the shards' gradients.
+    With seed="loss" (train_nerf.py:477) the whole batch's gradient is (sum of the ranks' losses) x (sum of the ranks'
+    unit-seed gradients), not the sum of gradients each seeded with its own shard's loss: so the shards are
+    differentiated with seed 1, the buffer is summed, and then its gradient part is multiplied by the summed loss
+    buf[-1] -- the arithmetic of the fused peer exchange (tc_reduce_kernel)."""
+    loss_seed = isinstance(batch.get("seed"), str)   # Trainer: any string seed is the loss
+    trainer.grad(**(dict(batch, seed=1.0) if loss_seed else batch))
     trainer.ctx.order_torch_after()       # the collective runs behind torch's current stream
-    allreduce_gradients(trainer.grad_buffer(), group)
+    buf = allreduce_gradients(trainer.grad_buffer(), group)
+    if loss_seed:
+        buf[:-1] *= buf[-1]
     trainer.ctx.order_after_torch()       # ... and the optimiser behind the collective
     trainer.apply()
