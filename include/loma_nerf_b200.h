@@ -309,6 +309,56 @@ LNB_API int lnb_nerf_step_composite_host(lnb_ctx *ctx, const lnb_mlp *mlp, const
 /* Fills out[0..n) with {sizeof(lnb_composite), offsetof background, bg, acc, depth}; returns how many values exist. */
 LNB_API int lnb_composite_layout(int *out, int n);
 
+/* VIEWS MODE (nerf only): camera mode with a pose per ray, so that one batch can mix rays from every training view (the NeRF
+ * paper's "random rays from all images" batching) and a step's whole batch can be drawn on the device (lnb_views_draw).
+ * Ray r is camera mode's ray of pixel q = pixels[r] under the pose poses[view[r]]: direction, origin, linspace depths, dists
+ * and the view direction follow the lnb_camera rule unchanged, with c2w = poses[view[r]].  The stratified jitter is
+ * u = lnb_uniform(seed', g, s) with the 64-bit key g = view[r] * P + q (P = width * height) and seed' = *seed_dev when
+ * seed_dev is set, else seed.  So:
+ *   - with every ray on view 0, views mode is camera mode with that pose (pixels = the same list), bit for bit;
+ *   - with linspace depths that holds for any single view v.
+ * view[r] and pixels[r] are checked on the device: an index outside [0, n_views) or [0, P) makes that ray's colour, and so the
+ * loss, NaN (nothing outside the pose table is read).  LNB_ERR_ARG for NULL pointers when R > 0, n_views < 1, width < 2,
+ * height < 1, P >= 2^31, a zero focal length or S > 4096.  All pointers are device pointers; the struct itself is a host
+ * pointer (passed to the kernels by value). */
+typedef struct {
+    const double *poses;                 /* [n_views][12] c2w rows, as lnb_camera.c2w                          */
+    int n_views, width, height;          /* every view has the same pixel grid; P = width * height             */
+    double fx, fy, cx, cy, near, far;    /* shared normalised intrinsics and depth range, as lnb_camera        */
+    int stratified;
+    unsigned long long seed;             /* jitter seed ...                                                    */
+    const unsigned long long *seed_dev;  /* ... or, when non-NULL, read from device memory (lnb_views_draw's step_seed) */
+    const int *view, *pixels;            /* [R] per ray                                                        */
+} lnb_views;
+/* Fills out[0..n) with {sizeof(lnb_views), offsetof poses, n_views, fx, near, stratified, seed, seed_dev, view, pixels};
+ * returns how many values exist. */
+LNB_API int lnb_views_layout(int *out, int n);
+/* The step for a views batch: args has no X, rays or cam (LNB_ERR_ARG otherwise); comp is optional (lnb_composite, the depth
+ * being views mode's).  Device pointers, asynchronous on the context's stream. */
+LNB_API int lnb_nerf_step_views(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *args, const lnb_views *views,
+                                const lnb_composite *comp);
+/* The rays and sample depths views mode generates (any output may be NULL): rays_o, rays_d [R][3], t [R][S] float64.  A ray
+ * with an out-of-range index gets NaN.  Device pointers (views itself is a host pointer). */
+LNB_API int lnb_views_rays(lnb_ctx *ctx, const lnb_views *views, int R, int S, double *rays_o, double *rays_d, double *t);
+/* THE DRAW: one step's batch from a device-resident scene, images [n_views][P][3] float32.  It reads k = counter[0] and leaves
+ * counter[0] = k + 1 (counter[1] is the draw's own block ticket: 0 before the first call, left at 0), so every replay of a
+ * captured graph draws a new batch.  With z(k, i) = mix(seed + 0x9E3779B97F4A7C15 * (k * 2^32 + i + 1)) mod 2^64, mix the
+ * SplitMix64 finaliser of lnb_uniform, and umulhi(z, n) the high 64 bits of the 128-bit product z * n:
+ *   one_view == 0 (every view, the paper's batching): g_r = umulhi(z(k, r), n_views * P), view_r = g_r / P, pixels_r = g_r mod P;
+ *   one_view != 0 (one view per step, the paper's Blender protocol): v = umulhi(z(k, 2^32 - 1), n_views), view_r = v,
+ *                 pixels_r = umulhi(z(k, r), P);
+ *   *step_seed = z(k, 2^32 - 2) (the step's jitter seed: lnb_views.seed_dev = step_seed);
+ *   target_r   = images[view_r][pixels_r] (the bits copied).
+ * R < 2^32 - 2.  The draw never lets a dependent launch start early (no programmatic trigger): the fused train kernel builds
+ * its first tile's inputs before it waits for its predecessor, so a step launched right after the draw only starts once the
+ * batch is complete.  Device pointers. */
+LNB_API int lnb_views_draw(lnb_ctx *ctx, const float *images, int n_views, long long P, int R, int one_view,
+                           unsigned long long seed, unsigned long long *counter, int *view, int *pixels, float *target,
+                           unsigned long long *step_seed);
+/* umulhi(z(k, i), n) of the draw, host-callable (like lnb_uniform): the draw's rule without a GPU. */
+LNB_API unsigned long long lnb_views_pick(unsigned long long seed, unsigned long long k, unsigned long long i,
+                                          unsigned long long n);
+
 /* Positional encoding, pos_encoding.py:4-70: x [n][F] float64 -> out [n][F*(1+2E)] float32,
  * feature = slot*F + coord, slot 0 identity, 2i+1 sin(2^i x), 2i+2 cos(2^i x); float64 range
  * reduction so the result matches the reference's float64-then-cast values. Device pointers. */
@@ -388,6 +438,11 @@ LNB_API int lnb_trainer_grad(lnb_trainer *t, const lnb_step_args *batch, int ner
  * (a trainer that never had a background set runs exactly as before).  The term is per ray, so the peer all-reduce is
  * unaffected, but every rank of a data-parallel run must set the same background.  LNB_ERR_ARG for a non-finite value. */
 LNB_API int lnb_trainer_set_background(lnb_trainer *t, const float *rgb);
+/* Attach a views batch (lnb_views, copied; its buffers must live as long as it is attached): from then on a nerf batch with
+ * no X, rays or cam is a views batch on lnb_trainer_step, lnb_trainer_step_weights and lnb_trainer_grad (so the NCCL route
+ * works too).  lnb_trainer_step_host and lnb_trainer_submit_host refuse such a batch (the scene lives on the device).  NULL
+ * detaches it.  LNB_ERR_ARG for the cases lnb_views lists. */
+LNB_API int lnb_trainer_set_views(lnb_trainer *t, const lnb_views *views);
 LNB_API int lnb_trainer_apply(lnb_trainer *t);
 LNB_API float *lnb_trainer_grad_buffer(lnb_trainer *t, long long *n_floats);
 LNB_API float *lnb_trainer_params(lnb_trainer *t, long long *n_w, long long *n_b);

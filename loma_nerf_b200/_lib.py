@@ -61,6 +61,14 @@ class LnbComposite(Structure):
     _fields_ = [("background", c_int), ("bg", c_float * 3), ("acc", c_void_p), ("depth", c_void_p)]
 
 
+class LnbViews(Structure):
+    """Mirror of lnb_views (views mode: camera mode with a pose per ray); checked against lnb_views_layout."""
+    _fields_ = [("poses", c_void_p), ("n_views", c_int), ("width", c_int), ("height", c_int),
+                ("fx", c_double), ("fy", c_double), ("cx", c_double), ("cy", c_double), ("near", c_double), ("far", c_double),
+                ("stratified", c_int), ("seed", ctypes.c_ulonglong), ("seed_dev", c_void_p), ("view", c_void_p),
+                ("pixels", c_void_p)]
+
+
 class LibraryMissing(RuntimeError):
     pass
 
@@ -105,6 +113,17 @@ def load():
         fn = getattr(lib, name)
         fn.argtypes = [c_void_p, P(LnbMlp), P(LnbStepArgs), P(LnbComposite)]
         fn.restype = c_int
+    lib.lnb_nerf_step_views.argtypes = [c_void_p, P(LnbMlp), P(LnbStepArgs), P(LnbViews), P(LnbComposite)]
+    lib.lnb_nerf_step_views.restype = c_int
+    lib.lnb_views_layout.argtypes = [P(c_int), c_int]
+    lib.lnb_views_layout.restype = c_int
+    lib.lnb_views_rays.argtypes = [c_void_p, P(LnbViews), c_int, c_int, c_void_p, c_void_p, c_void_p]
+    lib.lnb_views_draw.argtypes = [c_void_p, c_void_p, c_int, c_longlong, c_int, c_int, ctypes.c_ulonglong, c_void_p, c_void_p,
+                                   c_void_p, c_void_p, c_void_p]
+    lib.lnb_views_pick.argtypes = [ctypes.c_ulonglong, ctypes.c_ulonglong, ctypes.c_ulonglong, ctypes.c_ulonglong]
+    lib.lnb_views_pick.restype = ctypes.c_ulonglong
+    lib.lnb_trainer_set_views.argtypes = [c_void_p, P(LnbViews)]
+    lib.lnb_trainer_set_views.restype = c_int
     lib.lnb_composite_layout.argtypes = [P(c_int), c_int]
     lib.lnb_composite_layout.restype = c_int
     lib.lnb_pos_encoding.argtypes = [c_void_p, c_void_p, c_longlong, c_int, c_int, c_void_p]

@@ -232,14 +232,14 @@ class Context:
     # -------------------------------------------------------------------------------------------
     def _step(self, nerf, dims, X, ws, bs, target, dists, R, S, grad, seed, outputs, out, rows,
               path, inter_accumulate, color_accumulate, head, rays=None, pe_bands=0, camera=None, dir_bands=None,
-              background=None):
-        if rays is not None or camera is not None:
+              background=None, views=None):
+        if rays is not None or camera is not None or views is not None:
             check_rays_width(dims[0], pe_bands, dir_bands)
         outputs = tuple(outputs)
         extras = [k for k in COMPOSITE_OUTPUTS if k in outputs]
         if (extras or background is not None) and not nerf:
             raise ValueError("background, acc and depth are nerf-step features")
-        if "depth" in extras and rays is None and camera is None:
+        if "depth" in extras and rays is None and camera is None and views is None:
             raise ValueError("the depth map needs rays or camera mode: features mode has no sample depths")
         comp = make_composite(background) if (background is not None or extras) else None
         dev = _is_cuda(ws)
@@ -261,6 +261,10 @@ class Context:
             a.ray_dtype, a.pe_bands = (L.RAY_F64 if f64 else L.RAY_F32), int(pe_bands)
         if camera is not None:
             a.cam, a.pe_bands = ctypes.pointer(camera), int(pe_bands)
+        if views is not None:
+            if not dev:
+                raise ValueError("a views step takes device buffers (the scene lives on the device)")
+            a.pe_bands = int(pe_bands)
         a.inter_rows, a.inter_ld = M, mo
         a.inter_accumulate, a.color_accumulate = int(inter_accumulate), int(color_accumulate)
         a.want_grad = int(bool(grad))
@@ -306,6 +310,10 @@ class Context:
             # the zero fills above and whatever produced the inputs ran on torch's current stream
             self.order_after_torch()
             self._hold(X, ws, bs, target, dists, *(rays or ()), *res.values())
+        if views is not None:
+            self._check(self.lib.lnb_nerf_step_views(self.h, ctypes.byref(mlp), ctypes.byref(a), ctypes.byref(views),
+                                                     ctypes.byref(comp) if comp is not None else None))
+            return res
         if comp is not None:   # only a step that uses an extra calls the composite entry
             fn = self.lib.lnb_nerf_step_composite if dev else self.lib.lnb_nerf_step_composite_host
             self._check(fn(self.h, ctypes.byref(mlp), ctypes.byref(a), ctypes.byref(comp)))
@@ -351,6 +359,32 @@ class Context:
         return self._step(True, dims, None, ws, bs, target, None, int(R), int(S), grad, seed, outputs, out, None, path,
                           False, False, L.HEAD_NERF, pe_bands=pe_bands, camera=camera, dir_bands=dir_bands,
                           background=background)
+
+    def nerf_step_views(self, dims, views, S, pe_bands, ws, bs, target=None, grad=False, seed=1.0,
+                        outputs=("color", "loss"), out=None, path="f32", dir_bands=None, background=None):
+        """The same step on a views batch (`Scene.batch(...)`, lnb_views): ray r is camera mode's ray of pixel
+        pixels[r] under the pose of view[r], S samples each.  target defaults to the batch's drawn target.  dir_bands,
+        background and the "acc" / "depth" outputs as in nerf_step_camera."""
+        target = views.target if target is None else target
+        return self._step(True, dims, None, ws, bs, target, None, views.R, int(S), grad, seed, outputs, out, None, path,
+                          False, False, L.HEAD_NERF, pe_bands=pe_bands, dir_bands=dir_bands, background=background,
+                          views=views.views)
+
+    def views_rays(self, views, S, out=None):
+        """(rays_o, rays_d, t) float64 cuda tensors views mode generates for a views batch (NaN for a ray with an
+        out-of-range index)."""
+        R, dev = views.R, torch.device("cuda", self.device)
+        if out is None:
+            out = (torch.empty((R, 3), dtype=torch.float64, device=dev), torch.empty((R, 3), dtype=torch.float64, device=dev),
+                   torch.empty((R, S), dtype=torch.float64, device=dev))
+        o, d, t = out
+        if not all(_is_cuda(v) and v.dtype == torch.float64 and v.is_contiguous() and tuple(v.shape) == sh
+                   for v, sh in zip(out, ((R, 3), (R, 3), (R, S)))):
+            raise ValueError("views_rays: out must be contiguous [R][3], [R][3], [R][S] float64 CUDA tensors")
+        self.order_after_torch()
+        self._check(self.lib.lnb_views_rays(self.h, ctypes.byref(views.views), int(R), int(S), o.data_ptr(), d.data_ptr(),
+                                            t.data_ptr()))
+        return o, d, t
 
     def camera_rays(self, camera, R, S, out=None):
         """(rays_o, rays_d, t) float64 cuda tensors camera mode generates (for checks / hosts that want them).
@@ -488,18 +522,29 @@ class Trainer:
         self.ctx._check(self.lib.lnb_trainer_set_background(self.h, arr))
         self.background = (float(bg[0]), float(bg[1]), float(bg[2]))
 
+    def set_views(self, batch):
+        """Attach a views batch (`Scene.batch(...)`; lnb_trainer_set_views): later nerf steps with no X, rays or camera
+        train on it.  step(views=b) attaches b itself; None detaches.  The host-buffer steps refuse such a batch."""
+        self.ctx._check(self.lib.lnb_trainer_set_views(self.h, None if batch is None else ctypes.byref(batch.views)))
+        self._views_keep = batch
+
     def close(self):
         if getattr(self, "h", None):
             self.lib.lnb_trainer_destroy(self.h)
             self.h = None
 
     def _batch(self, X=None, dists=None, target=None, rays=None, pe_bands=0, R=None, S=None, path="tc", seed=1.0, camera=None,
-               dir_bands=None):
+               dir_bands=None, views=None):
         a = L.LnbStepArgs()
         nerf = self.head == L.HEAD_NERF
-        if camera is not None or rays is not None:
+        if camera is not None or rays is not None or views is not None:
             check_rays_width(self.dims[0], pe_bands, dir_bands)   # dir_bands: the view direction's bands, as in nerf_step_rays
-        if camera is not None:
+        if views is not None:   # a views batch: no input of its own, the trainer reads the attached lnb_views
+            self.set_views(views)
+            target = views.target if target is None else target
+            R, S = views.R, int(S)
+            a.pe_bands = int(pe_bands)
+        elif camera is not None:
             R, S = int(target.shape[0]) if R is None else int(R), int(S)
             a.cam, a.pe_bands = ctypes.pointer(camera), int(pe_bands)
             self._cam_keep = camera
@@ -695,6 +740,74 @@ class CoarseFine:
         ctx.sample_pdf(t, b["w"], self.n_fine, stratified=self.stratified, seed=seed, ray0=ray0, out=b["t_fine"])
         self.fine.step(rays=(o, d, b["t_fine"]), pe_bands=pe_bands, dir_bands=dir_bands, target=target, path=path)
         return dict(o=o, d=d, t=t, w=b["w"], t_fine=b["t_fine"])
+
+
+class Scene:
+    """A training scene held on the device: poses [n_views][12] float64 (the 3 x 4 camera-to-world rows) and images
+    [n_views][P][3] float32, P = width * height, uploaded once.  batch() makes the per-step views batches drawn from it."""
+
+    def __init__(self, ctx, poses, images, normalized_K, near=2.0, far=6.0):
+        self.ctx = ctx
+        dev = torch.device("cuda", ctx.device)
+        images = torch.as_tensor(np.asarray(images, np.float32) if not isinstance(images, torch.Tensor) else images)
+        if images.dim() != 4 or images.shape[3] != 3:
+            raise ValueError("images must be [n_views][height][width][3], got %r" % (tuple(images.shape),))
+        self.n_views, self.height, self.width = int(images.shape[0]), int(images.shape[1]), int(images.shape[2])
+        pz = np.asarray(poses.cpu() if isinstance(poses, torch.Tensor) else poses, np.float64)
+        if pz.shape[0] != self.n_views or pz.shape[1:] not in ((3, 4), (4, 4)):
+            raise ValueError("poses must be [n_views][3 or 4][4], got %r" % (pz.shape,))
+        self.poses = torch.as_tensor(np.ascontiguousarray(pz[:, :3, :4].reshape(self.n_views, 12))).to(dev)
+        self.images = images.to(device=dev, dtype=torch.float32).reshape(self.n_views, self.width * self.height, 3).contiguous()
+        K = np.asarray(normalized_K, np.float64)
+        self.fx, self.fy, self.cx, self.cy = float(K[0, 0]), float(K[1, 1]), float(K[0, 2]), float(K[1, 2])
+        self.near, self.far = float(near), float(far)
+
+    @property
+    def P(self):
+        return self.width * self.height
+
+    @classmethod
+    def from_blender(cls, ctx, scene, near=2.0, far=6.0):
+        """Every frame of a dataset.BlenderScene (its white_background compositing included)."""
+        frames = [scene[i] for i in range(len(scene))]
+        return cls(ctx, np.stack([f["pose"] for f in frames]), np.stack([f["image"] for f in frames]), scene.normalized_K,
+                   near=near, far=far)
+
+    def batch(self, R, stratified=False, one_view=False, seed=0):
+        """A views batch of R rays drawn from this scene (ViewsBatch).  one_view=True: every ray of a step from one view
+        (the paper's Blender protocol); else from all views.  seed: the draw's seed."""
+        return ViewsBatch(self, R, stratified, one_view, seed)
+
+
+class ViewsBatch:
+    """The buffers of one step's views batch (view, pixels [R] int32, target [R][3] float32, the step's jitter seed and
+    the draw counter [2] int64 (counter[0] = the next draw's k), all on the device) and the lnb_views that points at them.
+    draw() writes a new batch and advances the counter (lnb_views_draw), so a captured graph of draw() + a step trains on a
+    new batch at every replay.  The stratified jitter seed is the drawn step seed (views.seed_dev)."""
+
+    def __init__(self, scene, R, stratified=False, one_view=False, seed=0):
+        self.scene, self.ctx, self.R = scene, scene.ctx, int(R)
+        self.one_view, self.seed = bool(one_view), int(seed) & 0xFFFFFFFFFFFFFFFF
+        dev = scene.images.device
+        self.view = torch.zeros(self.R, dtype=torch.int32, device=dev)
+        self.pixels = torch.zeros(self.R, dtype=torch.int32, device=dev)
+        self.target = torch.zeros((self.R, 3), dtype=torch.float32, device=dev)
+        self.step_seed = torch.zeros(1, dtype=torch.int64, device=dev)
+        self.counter = torch.zeros(2, dtype=torch.int64, device=dev)
+        v = L.LnbViews()
+        v.poses, v.n_views, v.width, v.height = scene.poses.data_ptr(), scene.n_views, scene.width, scene.height
+        v.fx, v.fy, v.cx, v.cy, v.near, v.far = scene.fx, scene.fy, scene.cx, scene.cy, scene.near, scene.far
+        v.stratified, v.seed, v.seed_dev = int(bool(stratified)), 0, self.step_seed.data_ptr()
+        v.view, v.pixels = self.view.data_ptr(), self.pixels.data_ptr()
+        self.views = v
+
+    def draw(self):
+        """Launch the draw on the context's stream."""
+        ctx, sc = self.ctx, self.scene
+        ctx.order_after_torch()
+        ctx._check(ctx.lib.lnb_views_draw(ctx.h, sc.images.data_ptr(), sc.n_views, sc.P, self.R, int(self.one_view), self.seed,
+                                          self.counter.data_ptr(), self.view.data_ptr(), self.pixels.data_ptr(),
+                                          self.target.data_ptr(), self.step_seed.data_ptr()))
 
 
 class PreparedBatch:

@@ -10,6 +10,7 @@
 #include <mutex>
 #include <vector>
 
+#include "camera.cuh"
 #include "lnb_internal.h"
 
 // ------------------------------------------------------------------------------------------------
@@ -99,26 +100,55 @@ extern "C" int lnb_composite_layout(int *out, int n)
     return k;
 }
 
-int lnb_comp_resolve(lnb_ctx *ctx, const lnb_step_args *a, bool nerf, const lnb_composite *comp, lnb_comp_args *out,
-                     const lnb_comp_args **resolved)
+extern "C" int lnb_views_layout(int *out, int n)
+{
+    const int v[] = {(int)sizeof(lnb_views), (int)offsetof(lnb_views, poses), (int)offsetof(lnb_views, n_views),
+                     (int)offsetof(lnb_views, fx), (int)offsetof(lnb_views, near), (int)offsetof(lnb_views, stratified),
+                     (int)offsetof(lnb_views, seed), (int)offsetof(lnb_views, seed_dev), (int)offsetof(lnb_views, view),
+                     (int)offsetof(lnb_views, pixels)};
+    const int k = (int)(sizeof(v) / sizeof(v[0]));
+    for (int i = 0; i < k && i < n; ++i) out[i] = v[i];
+    return k;
+}
+
+int lnb_views_check(lnb_ctx *ctx, const lnb_views *v, int R, int S)
+{
+    LNB_ARG(v, "views: null");
+    LNB_ARG(R == 0 || (v->poses && v->view && v->pixels), "views: poses, view and pixels are required");
+    LNB_ARG(v->n_views >= 1, "views: n_views >= 1");
+    LNB_ARG(v->width >= 2 && v->height >= 1, "views: width >= 2, height >= 1");
+    LNB_ARG((long long)v->width * v->height < (1ll << 31), "views: fewer than 2^31 pixels per view");
+    LNB_ARG(v->fx != 0.0 && v->fy != 0.0, "views: zero focal length");
+    LNB_ARG(S <= 4096, "views: at most 4096 samples per ray");
+    return LNB_OK;
+}
+
+int lnb_comp_resolve(lnb_ctx *ctx, const lnb_step_args *a, bool nerf, const lnb_composite *comp, const lnb_views *views,
+                     lnb_comp_args *out, const lnb_comp_args **resolved)
 {
     *resolved = nullptr;
-    if (!comp) return LNB_OK;
-    LNB_ARG(comp->background == 0 || comp->background == 1, "composite: background must be 0 or 1");
-    if (comp->background)
-        for (int c = 0; c < 3; ++c) LNB_ARG(isfinite(comp->bg[c]), "composite: non-finite background colour");
-    if (!comp->background && !comp->acc && !comp->depth) return LNB_OK;   // asks for nothing: the plain step
-    LNB_ARG(nerf, "composite: a nerf-step feature");
+    if (comp) {
+        LNB_ARG(comp->background == 0 || comp->background == 1, "composite: background must be 0 or 1");
+        if (comp->background)
+            for (int c = 0; c < 3; ++c) LNB_ARG(isfinite(comp->bg[c]), "composite: non-finite background colour");
+    }
+    const bool extras = comp && (comp->background || comp->acc || comp->depth);
+    if (!extras && !views) return LNB_OK;   // asks for nothing: the plain step
+    LNB_ARG(nerf, "composite / views: a nerf-step feature");
     const bool cam = !a->X && !a->rays_o && a->cam;
     const bool rays = !a->X && (a->rays_o || cam);
-    LNB_ARG(!comp->depth || rays, "composite: depth needs rays or camera mode (features mode has no sample depths)");
+    LNB_ARG(!extras || !comp->depth || rays, "composite: depth needs rays or camera mode (features mode has no sample depths)");
     *out = lnb_comp_args{};
-    out->background = comp->background;
-    for (int c = 0; c < 3; ++c) out->bg[c] = comp->background ? comp->bg[c] : 0.0f;
-    out->acc = comp->acc;
-    out->depth = comp->depth;
+    out->views = views;
     if (cam) out->cam = a->cam;
     else if (rays) { out->t = a->t; out->t_f64 = a->ray_dtype == LNB_RAY_F64; }
+    if (extras) {
+        out->extras = 1;
+        out->background = comp->background;
+        for (int c = 0; c < 3; ++c) out->bg[c] = comp->background ? comp->bg[c] : 0.0f;
+        out->acc = comp->acc;
+        out->depth = comp->depth;
+    }
     *resolved = out;
     return LNB_OK;
 }
@@ -367,7 +397,7 @@ int step_layerwise(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, boo
     if (rays) {
         float *Xe = takef((size_t)N * d.c_in), *de = takef((size_t)R * S);
         const int Ed = lnb_rays_dir_bands(d.c_in, a->pe_bands);
-        if (cam) LNB_TRY(lnb_launch_camera_encode(ctx, a->cam, R, S, a->pe_bands, Ed, Xe, de, nullptr, 0));
+        if (cam) LNB_TRY(lnb_launch_camera_encode(ctx, a->cam, lnb_cx_views(cx), R, S, a->pe_bands, Ed, Xe, de, nullptr, 0));
         else LNB_TRY(lnb_launch_sample_encode(ctx, a->rays_o, a->rays_d, a->t, a->ray_dtype == LNB_RAY_F64, R, S, a->pe_bands, Ed, Xe, de));
         X = Xe; dists = de;
     }
@@ -474,16 +504,38 @@ int step_layerwise(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, boo
 } // namespace
 
 
+// A views batch as the routes take it: the step with cam pointing at the views' shared camera fields (the per-ray poses
+// travel in lnb_comp_args).  LNB_ERR_ARG for a step that has its own input or a bad lnb_views.
+struct ViewsStep {
+    lnb_step_args a;
+    lnb_camera cam;
+};
+static int views_step(lnb_ctx *ctx, const lnb_step_args *a, const lnb_views *views, ViewsStep *vs)
+{
+    LNB_ARG(a, "null args");
+    LNB_ARG(!a->X && !a->rays_o && !a->cam, "views step: the batch must have no X, rays or cam");
+    LNB_TRY(lnb_views_check(ctx, views, a->R, a->S));
+    vs->a = *a;
+    vs->cam = views_camera(*views);
+    vs->a.cam = &vs->cam;
+    return LNB_OK;
+}
+
 // comp: the compositing extras (lnb_composite), resolved here against the (device-pointer) step; one that asks for nothing
-// leaves the step exactly as it is without
+// leaves the step exactly as it is without.  views: a views batch (lnb_views; a has no input of its own).
 static int step_dispatch(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf, const lnb_tc_extra *ex = nullptr,
-                         const lnb_composite *comp = nullptr)
+                         const lnb_composite *comp = nullptr, const lnb_views *views = nullptr)
 {
     if (!ctx) return LNB_ERR_ARG;
     LNB_ARG(a, "null args");
+    ViewsStep vs;
+    if (views) {
+        LNB_TRY(views_step(ctx, a, views, &vs));
+        a = &vs.a;
+    }
     lnb_comp_args cxa;
     const lnb_comp_args *cx = nullptr;
-    LNB_TRY(lnb_comp_resolve(ctx, a, nerf, comp, &cxa, &cx));
+    LNB_TRY(lnb_comp_resolve(ctx, a, nerf, comp, views, &cxa, &cx));
     if (a->path == LNB_PATH_F32_LAYERWISE) return step_layerwise(ctx, mlp, a, nerf, cx);
     if (a->path == LNB_PATH_F32) {
         // same arithmetic type and tolerance either way: the fused kernel when the problem and the outputs asked for fit
@@ -511,18 +563,26 @@ static int step_dispatch(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *
 }
 
 // validated entry to the fused exact kernel for the trainer (overwrite: gradients written, not accumulated)
-int lnb_step_f32_fused(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf, int overwrite)
+int lnb_step_f32_fused(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf, int overwrite, const lnb_views *views)
 {
     if (!ctx) return LNB_ERR_ARG;
+    ViewsStep vs;
+    if (views) {
+        LNB_TRY(views_step(ctx, a, views, &vs));
+        a = &vs.a;
+    }
+    lnb_comp_args cxa;
+    const lnb_comp_args *cx = nullptr;
+    LNB_TRY(lnb_comp_resolve(ctx, a, nerf, nullptr, views, &cxa, &cx));
     StepDims d;
     LNB_TRY(validate(ctx, mlp, a, nerf, &d));
-    return lnb_fused_f32_step(ctx, mlp, a, nerf, overwrite);
+    return lnb_fused_f32_step(ctx, mlp, a, nerf, overwrite, cx);
 }
 
 int lnb_step_ex(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf, const lnb_tc_extra *ex,
-                const lnb_composite *comp)
+                const lnb_composite *comp, const lnb_views *views)
 {
-    return step_dispatch(ctx, mlp, a, nerf, ex, comp);
+    return step_dispatch(ctx, mlp, a, nerf, ex, comp, views);
 }
 
 extern "C" int lnb_nerf_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *args)
@@ -536,6 +596,13 @@ extern "C" int lnb_fit_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_arg
 extern "C" int lnb_nerf_step_composite(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *args, const lnb_composite *comp)
 {
     return step_dispatch(ctx, mlp, args, true, nullptr, comp);
+}
+extern "C" int lnb_nerf_step_views(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *args, const lnb_views *views,
+                                   const lnb_composite *comp)
+{
+    if (!ctx) return LNB_ERR_ARG;
+    LNB_ARG(views, "nerf_step_views: null views");
+    return step_dispatch(ctx, mlp, args, true, nullptr, comp, views);
 }
 
 // ------------------------------------------------------------------------------------------------

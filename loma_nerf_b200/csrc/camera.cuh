@@ -13,6 +13,12 @@ struct CamDev {
     const int *pixels;
     unsigned long long seed;
     int width, height, stratified;
+    // views mode (lnb_views; poses == NULL: camera mode): pixels is the views' pixel list
+    const double *poses;
+    const int *view;
+    const unsigned long long *seed_dev;
+    long long P;
+    int n_views;
 };
 
 inline CamDev make_cam_dev(const lnb_camera &c)
@@ -27,6 +33,27 @@ inline CamDev make_cam_dev(const lnb_camera &c)
     return d;
 }
 
+// The camera fields a views batch shares with camera mode (c2w unused, pixels = the views' pixel list)
+inline lnb_camera views_camera(const lnb_views &v)
+{
+    lnb_camera c{};
+    c.fx = v.fx; c.fy = v.fy; c.cx = v.cx; c.cy = v.cy;
+    c.width = v.width; c.height = v.height;
+    c.pixels = v.pixels;
+    c.near = v.near; c.far = v.far;
+    c.stratified = v.stratified; c.seed = v.seed;
+    return c;
+}
+inline CamDev make_cam_dev(const lnb_camera &c, const lnb_views *v)
+{
+    CamDev d = make_cam_dev(c);
+    if (v) {
+        d.poses = v->poses; d.view = v->view; d.seed_dev = v->seed_dev;
+        d.P = (long long)v->width * v->height; d.n_views = v->n_views;
+    }
+    return d;
+}
+
 // SplitMix64 finaliser over (seed, pixel, sample): 24 uniform bits
 __host__ __device__ inline unsigned lnb_uniform_bits(unsigned long long seed, long long pixel, int s)
 {
@@ -38,6 +65,23 @@ __host__ __device__ inline unsigned lnb_uniform_bits(unsigned long long seed, lo
 }
 
 __device__ __forceinline__ long long cam_pixel(const CamDev &c, long long ray) { return c.pixels ? (long long)__ldg(c.pixels + ray) : c.first_pixel + ray; }
+
+// Views mode: camera mode's camera of ray r (its pose in c2w, its jitter seed seed') in cr, with its pixel q and jitter key
+// g = view[r] * P + q.  false when view[r] or pixels[r] is out of range (c2w is then the table's first pose: nothing outside
+// the table is read; the caller makes the ray NaN).
+__device__ __forceinline__ bool views_ray(const CamDev &c, long long r, CamDev &cr, long long &q, long long &g)
+{
+    const int v = __ldg(c.view + r), p = __ldg(c.pixels + r);
+    const bool ok = v >= 0 && v < c.n_views && p >= 0 && p < c.P;
+    const double *m = c.poses + 12 * (long long)(ok ? v : 0);
+    cr = c;
+#pragma unroll
+    for (int i = 0; i < 12; ++i) cr.c2w[i] = __ldg(m + i);
+    if (c.seed_dev) cr.seed = *c.seed_dev;
+    q = p;
+    g = (long long)v * c.P + p;
+    return ok;
+}
 
 // float64: the operation order of get_rays (linspace value, (i - cx) / fx, dirs @ R^T as a plain k-sum)
 __device__ __forceinline__ void cam_ray_f64(const CamDev &c, long long q, double o[3], double d[3])

@@ -71,7 +71,8 @@ __device__ __forceinline__ double unit_coord(const double (&d)[3], int f)
 }
 
 // one thread per (sample, coordinate).  Ed >= 0 appends the view direction's encoding PE(u, Ed) after PE(x, E).
-template <typename T, bool CAM>
+// CAM: 0 rays mode, 1 camera mode, 2 views mode (a pose per ray; a ray with an out-of-range index gets NaN features and dists)
+template <typename T, int CAM>
 __global__ void sample_encode_kernel(const T *__restrict__ o, const T *__restrict__ d,
                                      const T *__restrict__ t, const CamDev cam, int R, int S, int E, int Ed,
                                      float *__restrict__ X, float *__restrict__ dists, __nv_bfloat16 *__restrict__ Xb, int ldb)
@@ -83,7 +84,17 @@ __global__ void sample_encode_kernel(const T *__restrict__ o, const T *__restric
     int r = (int)(smp / S), s = (int)(smp % S);
     const int P = 3 * (1 + 2 * E), C = P + (Ed >= 0 ? 3 * (1 + 2 * Ed) : 0);
     double tt, tnext = 0.0, v, dd[3];
-    if (CAM) {   // rays and depths from the pose (camera.cuh): float64 values in get_rays' / linspace's operation order
+    if (CAM == 2) {   // views mode: camera mode's ray of pixels[r] under its own pose, jitter keyed by g
+        CamDev cr;
+        long long q, g;
+        const bool ok = views_ray(cam, r, cr, q, g);
+        double oo[3];
+        cam_ray_f64(cr, q, oo, dd);
+        tt = cam_t_f64(cr, g, s, S);
+        if (s + 1 < S) tnext = cam_t_f64(cr, g, s + 1, S);
+        if (!ok) tt = tnext = __longlong_as_double(0x7ff8000000000000ll);
+        v = oo[f] + dd[f] * tt;
+    } else if (CAM) {   // rays and depths from the pose (camera.cuh): float64 values in get_rays' / linspace's operation order
         const long long q = cam_pixel(cam, r);
         double oo[3];
         cam_ray_f64(cam, q, oo, dd);
@@ -108,7 +119,7 @@ __global__ void sample_encode_kernel(const T *__restrict__ o, const T *__restric
         encode_coord(v, E, f, x);
         if (Ed >= 0) encode_coord(unit_coord(dd, f), Ed, f, x + P);
     }
-    if (f == 0 && dists) dists[smp] = (s + 1 < S) ? (float)(tnext - tt) : (float)1e8;
+    if (f == 0 && dists) dists[smp] = (s + 1 < S || (CAM == 2 && tt != tt)) ? (float)(tnext - tt) : (float)1e8;
 }
 
 } // namespace
@@ -137,20 +148,24 @@ int lnb_launch_sample_encode_bf16(lnb_ctx *ctx, const void *o, const void *d, co
     if (tot <= 0) return LNB_OK;
     const unsigned blocks = (unsigned)((tot + 255) / 256);
     if (f64)
-        sample_encode_kernel<double, false><<<blocks, 256, 0, ctx->stream>>>((const double *)o, (const double *)d, (const double *)t, CamDev{}, R, S, E, Ed, X, dists, (__nv_bfloat16 *)Xb, ldb);
+        sample_encode_kernel<double, 0><<<blocks, 256, 0, ctx->stream>>>((const double *)o, (const double *)d, (const double *)t, CamDev{}, R, S, E, Ed, X, dists, (__nv_bfloat16 *)Xb, ldb);
     else
-        sample_encode_kernel<float, false><<<blocks, 256, 0, ctx->stream>>>((const float *)o, (const float *)d, (const float *)t, CamDev{}, R, S, E, Ed, X, dists, (__nv_bfloat16 *)Xb, ldb);
+        sample_encode_kernel<float, 0><<<blocks, 256, 0, ctx->stream>>>((const float *)o, (const float *)d, (const float *)t, CamDev{}, R, S, E, Ed, X, dists, (__nv_bfloat16 *)Xb, ldb);
     LNB_CHECK_LAUNCH();
     return LNB_OK;
 }
 
-// camera mode: the same outputs with rays and depths generated from the pose (lnb_camera)
-int lnb_launch_camera_encode(lnb_ctx *ctx, const lnb_camera *cam, int R, int S, int E, int Ed, float *X, float *dists, void *Xb, int ldb)
+// camera mode: the same outputs with rays and depths generated from the pose (lnb_camera); views mode with views != NULL
+int lnb_launch_camera_encode(lnb_ctx *ctx, const lnb_camera *cam, const lnb_views *views, int R, int S, int E, int Ed, float *X,
+                             float *dists, void *Xb, int ldb)
 {
     long long tot = (long long)R * S * 3;
     if (tot <= 0) return LNB_OK;
     const unsigned blocks = (unsigned)((tot + 255) / 256);
-    sample_encode_kernel<double, true><<<blocks, 256, 0, ctx->stream>>>(nullptr, nullptr, nullptr, make_cam_dev(*cam), R, S, E, Ed, X, dists, (__nv_bfloat16 *)Xb, ldb);
+    if (views)
+        sample_encode_kernel<double, 2><<<blocks, 256, 0, ctx->stream>>>(nullptr, nullptr, nullptr, make_cam_dev(*cam, views), R, S, E, Ed, X, dists, (__nv_bfloat16 *)Xb, ldb);
+    else
+        sample_encode_kernel<double, 1><<<blocks, 256, 0, ctx->stream>>>(nullptr, nullptr, nullptr, make_cam_dev(*cam), R, S, E, Ed, X, dists, (__nv_bfloat16 *)Xb, ldb);
     LNB_CHECK_LAUNCH();
     return LNB_OK;
 }
@@ -170,6 +185,23 @@ __global__ void camera_rays_kernel(const CamDev cam, int R, int S, double *__res
         for (int k = 0; k < 3; ++k) { if (o) o[r * 3 + k] = oo[k]; if (d) d[r * 3 + k] = dd[k]; }
     }
 }
+// views mode's rays and depths (lnb_views_rays); NaN for a ray with an out-of-range index
+__global__ void views_rays_kernel(const CamDev cam, int R, int S, double *__restrict__ o, double *__restrict__ d, double *__restrict__ t)
+{
+    const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= (long long)R * S) return;
+    const int r = (int)(e / S), s = (int)(e % S);
+    CamDev cr;
+    long long q, g;
+    const bool ok = views_ray(cam, r, cr, q, g);
+    const double nan = __longlong_as_double(0x7ff8000000000000ll);
+    if (t) t[e] = ok ? cam_t_f64(cr, g, s, S) : nan;
+    if (s == 0) {
+        double oo[3], dd[3];
+        cam_ray_f64(cr, q, oo, dd);
+        for (int k = 0; k < 3; ++k) { if (o) o[r * 3 + k] = ok ? oo[k] : nan; if (d) d[r * 3 + k] = ok ? dd[k] : nan; }
+    }
+}
 __global__ void color_to_u8_kernel(const float *__restrict__ rgb, long long n, unsigned char *__restrict__ out)
 {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -185,6 +217,19 @@ extern "C" int lnb_camera_rays(lnb_ctx *ctx, const lnb_camera *cam, int R, int S
     const long long tot = (long long)R * S;
     if (tot <= 0) return LNB_OK;
     camera_rays_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, ctx->stream>>>(make_cam_dev(*cam), R, S, rays_o, rays_d, t);
+    LNB_CHECK_LAUNCH();
+    return LNB_OK;
+}
+
+extern "C" int lnb_views_rays(lnb_ctx *ctx, const lnb_views *views, int R, int S, double *rays_o, double *rays_d, double *t)
+{
+    if (!ctx) return LNB_ERR_ARG;
+    LNB_ARG(views && R >= 0 && S >= 1, "views_rays arguments");
+    LNB_TRY(lnb_views_check(ctx, views, R, S));
+    if (cudaSetDevice(ctx->device) != cudaSuccess) return LNB_ERR_CUDA;
+    const long long tot = (long long)R * S;
+    if (tot <= 0) return LNB_OK;
+    views_rays_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, ctx->stream>>>(make_cam_dev(views_camera(*views), views), R, S, rays_o, rays_d, t);
     LNB_CHECK_LAUNCH();
     return LNB_OK;
 }

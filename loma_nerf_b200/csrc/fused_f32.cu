@@ -503,7 +503,7 @@ int lnb_fused_f32_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a,
         ctx->err = std::string("fused fp32 path: ") + why;
         return LNB_ERR_UNSUPPORTED;
     };
-    if (cx) return unsupported("no compositing extras (background, acc, depth): the layerwise kernels have them");
+    if (lnb_cx_extras(cx)) return unsupported("no compositing extras (background, acc, depth): the layerwise kernels have them");
     if (L < 2 || L > 3) return unsupported("needs 2 or 3 layers");
     if (mlp->dims[0] + 1 > K0) return unsupported("input width + 1 must be <= 36");
     for (int l = 1; l < L; ++l)
@@ -548,7 +548,7 @@ int lnb_fused_f32_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a,
     if (rays) {
         float *Xe = (float *)lnb_arena_take(ctx, (size_t)N * c_in * sizeof(float)), *de = (float *)lnb_arena_take(ctx, (size_t)R * S * sizeof(float));
         const int Ed = lnb_rays_dir_bands(c_in, a->pe_bands);
-        if (cam) LNB_TRY(lnb_launch_camera_encode(ctx, a->cam, R, S, a->pe_bands, Ed, Xe, de, nullptr, 0));
+        if (cam) LNB_TRY(lnb_launch_camera_encode(ctx, a->cam, lnb_cx_views(cx), R, S, a->pe_bands, Ed, Xe, de, nullptr, 0));
         else LNB_TRY(lnb_launch_sample_encode(ctx, a->rays_o, a->rays_d, a->t, a->ray_dtype == LNB_RAY_F64, R, S, a->pe_bands, Ed, Xe, de));
         p.X = Xe; p.dists = de;
     }

@@ -80,7 +80,8 @@ template <int HP> constexpr int mg_max_groups() { return HP <= 32 ? MG_MAX_GROUP
 // EXT: the extras instantiation (head_and_composite: weights, acc / depth, background), the one lnb_trainer_step_weights and
 // a step with compositing extras run.  Its acc / depth scratch is the slot's dZ_{L-1} slab, dead until the head's adjoint
 // is written into it (the previous tile's weight-gradient MMA that read it has been awaited in the backward loop).
-template <bool RAYS, int HP, bool DIRS = false, bool EXT = false>
+// RAYS: 0 features, 1 rays or camera mode, 2 views mode (sample_inputs).
+template <int RAYS, int HP, bool DIRS = false, bool EXT = false>
 __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel(const TcParams p)
 {
     using LY = TcLayout<HP>;
@@ -314,7 +315,7 @@ __global__ void __launch_bounds__(mg_max_groups<HP>() * TILE, 1) fused_mg_kernel
         }
         // ---- head + loss + adjoint of the head's pre-activation (unit seed)
         float dz[4];
-        head_and_composite<true, EXT>(p, scratch, g + 1, hz, my_dist, tg, row0, tile * p.G, valid, tid, smp, ray_l, live, loss_acc, dz);
+        head_and_composite<true, EXT, RAYS == 2>(p, scratch, g + 1, hz, my_dist, tg, row0, tile * p.G, valid, tid, smp, ray_l, live, loss_acc, dz);
         // ---- backward.  dZ_{L-1}: 4 live features of its one slab
         {
             const uint32_t o[8] = {pack_bf16(dz[0], dz[1]), pack_bf16(dz[2], dz[3]), 0u, 0u, 0u, 0u, 0u, 0u};

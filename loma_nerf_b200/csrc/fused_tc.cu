@@ -57,6 +57,12 @@ struct CamF32 {
     unsigned long long seed;
     unsigned long long w_magic;      // floor(2^64 / width) + 1 (width >= 2): q / width = umul64hi(q, w_magic) for every 32-bit q
     int width, stratified;
+    // views mode (the RAYS == 2 instantiations; lnb_views): pixels is the views' pixel list
+    const double *poses;
+    const int *view;
+    const unsigned long long *seed_dev;
+    long long P;
+    int n_views;
 };
 
 struct alignas(16) TcParams {   // 16: the kernel parameters after it keep their alignment
@@ -341,7 +347,9 @@ __device__ __forceinline__ const void *x_src(const TcParams &p, int tile, int c_
 // spacing `dist` and, at a ray's first sample, the ray's target colour.  From rays (RAYS) also the sample point x:
 // pts = o + d t (train_nerf.py:289-299), dist = t[s+1] - t[s], last 1e8 (train_nerf.py:306-311).  x and dist stay 0 in a
 // row past the tile's live samples.  DIRS: also the ray's unit direction u = d / |d| (0 in a row that is not live).
-template <bool RAYS, bool DIRS>
+// RAYS: 0 features, 1 rays or camera mode (p.cam_mode), 2 views mode (a separate instantiation, so that the camera prologue
+// of the others stays as it was).
+template <int RAYS, bool DIRS>
 __device__ __forceinline__ void sample_inputs(const TcParams &p, long long row0, int ray0, int tid, int smp, int ray_l, bool live,
                                               float (&x)[3], float &dist, float (&tg)[3], float (&u)[3])
 {
@@ -359,7 +367,36 @@ __device__ __forceinline__ void sample_inputs(const TcParams &p, long long row0,
     if (DIRS) u[0] = u[1] = u[2] = 0.0f;
     if (!RAYS || !live) return;
     const long long ray = ray0 + ray_l;
-    if (p.cam_mode) {
+    if (RAYS == 2) {
+        // views mode: camera mode's ray of pixel q = pixels[r] under the pose poses[view[r]] (rounded to float32 as camera
+        // mode rounds its c2w), the jitter keyed by g = view[r] * P + q under seed'.  An out-of-range index makes x and
+        // dist NaN (dist too, so the colour is NaN whatever the MLP makes of x) and reads the table's first pose.
+        const CamF32 &c = p.cam;
+        const int v = __ldg(c.view + ray), q = __ldg(c.pixels + ray);
+        const bool ok = (unsigned)v < (unsigned)c.n_views && (long long)(unsigned)q < c.P;
+        const double *m = c.poses + 12 * (ok ? v : 0);
+        const unsigned long long seed = c.seed_dev ? __ldg(c.seed_dev) : c.seed;
+        const long long g = (long long)v * c.P + q;
+        const unsigned uq = (unsigned)q, row = (unsigned)__umul64hi((unsigned long long)uq, c.w_magic), col = uq - row * (unsigned)c.width;
+        const float fi = col == (unsigned)c.width - 1 ? 1.0f : (float)col * c.step, fj = row == (unsigned)c.width - 1 ? 1.0f : (float)row * c.step;
+        const float dx = (fi - c.cx) * c.inv_fx, dy = (c.cy - fj) * c.inv_fy;
+        float tt, tn;
+        if (c.stratified) {
+            tt = fmaf((float)smp + (float)lnb_uniform_bits(seed, g, smp) * (1.0f / 16777216.0f), c.dt_str, c.near);
+            tn = fmaf((float)(smp + 1) + (float)lnb_uniform_bits(seed, g, smp + 1) * (1.0f / 16777216.0f), c.dt_str, c.near);
+        } else {
+            tt = smp == S - 1 && S > 1 ? c.far : fmaf((float)smp, c.dt_lin, c.near);
+            tn = smp + 1 == S - 1 ? c.far : fmaf((float)(smp + 1), c.dt_lin, c.near);
+        }
+        dist = smp + 1 < S ? tn - tt : 1e8f;
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+            const float dk = fmaf(dx, (float)__ldg(m + 4 * k), fmaf(dy, (float)__ldg(m + 4 * k + 1), 0.0f - (float)__ldg(m + 4 * k + 2)));
+            x[k] = fmaf(dk, tt, (float)__ldg(m + 4 * k + 3));
+            if (DIRS) u[k] = dk;
+        }
+        if (!ok) x[0] = x[1] = x[2] = dist = __int_as_float(0x7fc00000);
+    } else if (p.cam_mode) {
         // ray of pixel q and depth of sample smp straight from the pose (get_rays, train_nerf.py:23-62; linspace /
         // stratified depths, train_nerf.py:289-311): no per-ray or per-sample input at all
         const CamF32 &c = p.cam;
@@ -555,8 +592,16 @@ struct CompScratch {
 
 // Depth t_s of sample smp of ray `ray` (row `row` of the batch) for the depth map: re-loaded (rays mode) or re-derived from
 // the camera exactly as sample_inputs forms it, at the compositing stage rather than held in a register across the MMAs.
+template <bool VIEWS>
 __device__ __forceinline__ float tile_sample_depth(const TcParams &p, long long ray, int smp, long long row)
 {
+    if (VIEWS) {   // views mode: camera mode's depth under the ray's jitter key g = view * P + q and seed'
+        const CamF32 &c = p.cam;
+        if (!c.stratified) return smp == p.S - 1 && p.S > 1 ? c.far : fmaf((float)smp, c.dt_lin, c.near);
+        const long long g = (long long)__ldg(c.view + ray) * c.P + __ldg(c.pixels + ray);
+        const unsigned long long seed = c.seed_dev ? __ldg(c.seed_dev) : c.seed;
+        return fmaf((float)smp + (float)lnb_uniform_bits(seed, g, smp) * (1.0f / 16777216.0f), c.dt_str, c.near);
+    }
     if (p.cam_mode) {
         const CamF32 &c = p.cam;
         const long long q = c.pixels ? (long long)__ldg(c.pixels + ray) : c.first_pixel + ray;
@@ -571,7 +616,7 @@ __device__ __forceinline__ float tile_sample_depth(const TcParams &p, long long 
 // live rows go to p.weights when it is set (lnb_trainer_step_weights), acc and depth ride in the segmented colour sum as
 // two more channels (p.acc / p.depth), and with p.background the colour gets (1 - acc) bg before the loss, the weight
 // adjoint uses rgb - bg.  A separate instantiation, so the plain train and render kernels stay as they were.
-template <bool GRAD, bool EXT = false>
+template <bool GRAD, bool EXT = false, bool VIEWS = false>
 __device__ __forceinline__ void head_and_composite(const TcParams &p, const CompScratch &s, int bar, const float (&hz)[4], float dist,
                                                    const float (&tg)[3], long long row0, int ray0, int valid, int tid, int smp,
                                                    int ray_l, bool live, float &loss_acc, float (&dz)[4])
@@ -635,7 +680,7 @@ __device__ __forceinline__ void head_and_composite(const TcParams &p, const Comp
             atomicAdd(s.color + ray_l * 3, s0); atomicAdd(s.color + ray_l * 3 + 1, s1); atomicAdd(s.color + ray_l * 3 + 2, s2);
         }
         if (EXT) {   // acc = sum w, depth = sum w t: the same segmented sum
-            float s3 = live ? wgt : 0.f, s4 = (live && p.depth) ? wgt * tile_sample_depth(p, ray0 + ray_l, smp, row0 + tid) : 0.f;
+            float s3 = live ? wgt : 0.f, s4 = (live && p.depth) ? wgt * tile_sample_depth<VIEWS>(p, ray0 + ray_l, smp, row0 + tid) : 0.f;
 #pragma unroll
             for (int d = 1; d < 32; d <<= 1) {
                 float o3 = __shfl_up_sync(0xffffffffu, s3, d), o4 = __shfl_up_sync(0xffffffffu, s4, d);
@@ -753,7 +798,7 @@ __device__ __forceinline__ void relu_adjoint(const uint32_t (&v)[HP / 16][16], c
 // launch bounds are the CTAs per SM that tensor memory admits (512 columns / 64 per CTA = 8; 4 for the 64-wide form), not
 // more: a ninth CTA could never allocate its columns and the tighter register budget only bought a spill.
 // EXT: the extras instantiations (head_and_composite); its acc / depth scratch follows the colour / target scratch.
-template <bool RAYS, int HP, bool FWD, bool DIRS = false, bool EXT = false>
+template <int RAYS, int HP, bool FWD, bool DIRS = false, bool EXT = false>
 __global__ void __launch_bounds__(TILE, FWD ? (HP == 64 ? 4 : 8) : 1) fused_v1_kernel(const TcParams p)
 {
     using LY = TcLayout<HP>;
@@ -976,7 +1021,7 @@ __global__ void __launch_bounds__(TILE, FWD ? (HP == 64 ? 4 : 8) : 1) fused_v1_k
         CLK(16);
         // ---- head + loss + adjoint of the head's pre-activation (unit seed)
         float dz[4];
-        head_and_composite<!FWD, EXT>(p, scratch, 0, hz, my_dist, tg, row0, ray0, valid, tid, smp, ray_l, live, loss_acc, dz);
+        head_and_composite<!FWD, EXT, RAYS == 2>(p, scratch, 0, hz, my_dist, tg, row0, ray0, valid, tid, smp, ray_l, live, loss_acc, dz);
         CLK(17);
         if (FWD) { __syncthreads(); tile = *next_tile_s; continue; }
         // ---- backward.  dZ_{L-1}: 4 live features, the rest of the 16 stay zero
@@ -1404,6 +1449,7 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
         return unsupported("rays mode needs rays_o, rays_d, t (or a camera) and dims[0] == 3 + 6 * pe_bands (+ 3 + 6 * E_dir)");
     const bool dirs = dir_bands >= 0;
     if (cam && (long long)a->cam->width * a->cam->height >= (1ll << 31)) return unsupported("camera: more than 2^31 pixels");
+    const lnb_views *views = cam ? lnb_cx_views(cx) : nullptr;   // views mode: the RAYS == 2 instantiations
     if (!nerf && N != R) return unsupported("needs n_rows == R");
     if (a->rows > N) return unsupported("rows > n_rows");
     if (!nerf && (a->target_w > 4)) return unsupported("target wider than 4");
@@ -1424,6 +1470,10 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
         p.cam.dt_lin = (float)((c.far - c.near) / (double)(a->S > 1 ? a->S - 1 : 1)); p.cam.dt_str = (float)((c.far - c.near) / (double)a->S);
         p.cam.first_pixel = c.first_pixel; p.cam.pixels = c.pixels; p.cam.seed = c.seed; p.cam.width = c.width; p.cam.stratified = c.stratified;
         p.cam.w_magic = c.width >= 2 ? ~0ull / (unsigned long long)c.width + 1ull : 0ull;
+        if (views) {
+            p.cam.poses = views->poses; p.cam.view = views->view; p.cam.seed_dev = views->seed_dev;
+            p.cam.P = (long long)views->width * views->height; p.cam.n_views = views->n_views;
+        }
     }
     p.color = nerf ? a->color : nullptr;
     p.N = N; p.R = R; p.S = S;
@@ -1439,13 +1489,21 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
     // place); forward-only launches and LNB_TC_V1=1 on the one-tile-per-CTA kernel above.
     const bool mg = grad && getenv("LNB_TC_V1") == nullptr && (!nerf || S >= 2);
     // the extras instantiations: lnb_trainer_step_weights, and any step with compositing extras (lnb_composite)
-    const bool ext = nerf && ((grad && ex && ex->weights) || cx);
+    const bool ext = nerf && ((grad && ex && ex->weights) || lnb_cx_extras(cx));
+    if (views && grad && !mg) return unsupported("views mode trains on the multi-group kernel (S >= 2, LNB_TC_V1 unset)");
     if (grad && !mg) {   // the one-tile-per-CTA kernel computes all weight gradients with ONE concatenated M = 128 MMA per K-step
         if (K0P / 8 + (L - 1) * (HP / 8) > 16) return unsupported("input + hidden widths exceed 128 features in total");
         if ((L - 1) * HP + 16 > 256) return unsupported("hidden widths exceed 256 gradient columns");
     }
+    const int in_kind = views ? (dirs ? 4 : 3) : (dirs ? 2 : (rays ? 1 : 0));   // the input form, as mg_regs lists them
     void (*const kern)(TcParams) = with_hp(HP, [&](auto hp) -> void (*)(TcParams) {
         constexpr int H = decltype(hp)::value;
+        if (views) {
+            if (mg && ext) return dirs ? fused_mg_kernel<2, H, true, true> : fused_mg_kernel<2, H, false, true>;
+            if (mg) return dirs ? fused_mg_kernel<2, H, true> : fused_mg_kernel<2, H>;
+            if (ext) return dirs ? fused_v1_kernel<2, H, true, true, true> : fused_v1_kernel<2, H, true, false, true>;
+            return dirs ? fused_v1_kernel<2, H, true, true> : fused_v1_kernel<2, H, true>;
+        }
         if (mg && ext) return dirs ? fused_mg_kernel<true, H, true, true> : rays ? fused_mg_kernel<true, H, false, true> : fused_mg_kernel<false, H, false, true>;
         if (mg) return dirs ? fused_mg_kernel<true, H, true> : rays ? fused_mg_kernel<true, H> : fused_mg_kernel<false, H>;
         if (grad && ext)
@@ -1464,8 +1522,10 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
             while (n > 1 && (MG::total(L, c_in, K0P, rays, n) > 232448 || MG::tmem_need(L, K0P, n) > 512)) --n;
             return n;
         });
-        static int mg_regs[2][3][3] = {}; // registers per thread of each instantiation ([extras] (features, rays, rays + directions)), asked once
-        int &regs = mg_regs[ext][dirs ? 2 : (rays ? 1 : 0)][HP / 32];
+        // registers per thread of each instantiation ([extras] (features, rays, rays + directions, views, views + directions)),
+        // asked once
+        static int mg_regs[2][5][3] = {};
+        int &regs = mg_regs[ext][in_kind][HP / 32];
         if (regs == 0) {
             cudaFuncAttributes fa;
             LNB_CUDA(cudaFuncGetAttributes(&fa, kern));
@@ -1533,14 +1593,15 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
             LNB_CHECK_LAUNCH();
         }
         // the dynamic shared-memory limit of each kernel instantiation (kind, input, HP) on each device: raised only when it grows
-        static size_t smem_set[2][3][3][3][64] = {};
-        size_t &lim = smem_set[ext][mg ? 0 : (grad ? 1 : 2)][dirs ? 2 : (rays ? 1 : 0)][HP / 32][ctx->device & 63];
+        static size_t smem_set[2][3][5][3][64] = {};
+        size_t &lim = smem_set[ext][mg ? 0 : (grad ? 1 : 2)][in_kind][HP / 32][ctx->device & 63];
         if (smem > lim || ctx->device > 63) { LNB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); lim = smem; }
         // the symbols ncu lists; "+extras": an extras instantiation (weights / acc / depth / background)
-        static const char *const names[2][2][2] = {{{"fused_v1_kernel<features>", "fused_v1_kernel<rays>"}, {"fused_mg_kernel<features>", "fused_mg_kernel<rays>"}},
-                                                   {{"fused_v1_kernel<features>+extras", "fused_v1_kernel<rays>+extras"},
-                                                    {"fused_mg_kernel<features>+extras", "fused_mg_kernel<rays>+extras"}}};
-        lnb_prof_begin(ctx, names[ext][mg][rays]);
+        static const char *const names[2][2][3] = {{{"fused_v1_kernel<features>", "fused_v1_kernel<rays>", "fused_v1_kernel<views>"},
+                                                    {"fused_mg_kernel<features>", "fused_mg_kernel<rays>", "fused_mg_kernel<views>"}},
+                                                   {{"fused_v1_kernel<features>+extras", "fused_v1_kernel<rays>+extras", "fused_v1_kernel<views>+extras"},
+                                                    {"fused_mg_kernel<features>+extras", "fused_mg_kernel<rays>+extras", "fused_mg_kernel<views>+extras"}}};
+        lnb_prof_begin(ctx, names[ext][mg][views ? 2 : rays]);
         LNB_CUDA(cudaLaunchKernelEx(&cfg, kern, p));
         lnb_prof_end(ctx);
         LNB_CHECK_LAUNCH();

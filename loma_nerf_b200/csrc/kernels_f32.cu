@@ -453,15 +453,21 @@ struct CompK {
     int t_f64, cam_mode;
     CamDev cam;
 };
+template <bool VIEWS>
 __device__ __forceinline__ float sample_depth(const CompK &k, int ray, int s, int S)
 {
+    if (VIEWS) {   // views mode: camera mode's depth under the ray's jitter key g = view * P + q and seed'
+        CamDev c = k.cam;
+        if (c.seed_dev) c.seed = *c.seed_dev;
+        return (float)cam_t_f64(c, (long long)__ldg(c.view + ray) * c.P + __ldg(c.pixels + ray), s, S);
+    }
     if (k.cam_mode) return (float)cam_t_f64(k.cam, cam_pixel(k.cam, ray), s, S);
     const size_t i = (size_t)ray * S + s;
     return k.t_f64 ? (float)__ldg(reinterpret_cast<const double *>(k.t) + i) : __ldg(reinterpret_cast<const float *>(k.t) + i);
 }
 
 // EXT: with the extras of `k` (acc = sum w, depth = sum w t, colour += (1 - acc) bg before the caller's colour is added)
-template <bool EXT>
+template <bool EXT, bool VIEWS = false>   // VIEWS: the depths of a views batch (a separate instantiation)
 __global__ void __launch_bounds__(COMP_WARPS * 32)
 composite_fwd_kernel(const float *__restrict__ head, int ldh, const float *__restrict__ dists,
                      const float *__restrict__ target, int R, int S, float *__restrict__ rgba,
@@ -497,7 +503,7 @@ composite_fwd_kernel(const float *__restrict__ head, int ldh, const float *__res
             c0 = fmaf(w, r, c0); c1 = fmaf(w, gch, c1); c2 = fmaf(w, b, c2);
             if (EXT) {
                 c3 += w;
-                if (k.depth) c4 = fmaf(w, sample_depth(k, ray, s, S), c4);
+                if (k.depth) c4 = fmaf(w, sample_depth<VIEWS>(k, ray, s, S), c4);
             }
         }
     }
@@ -785,7 +791,7 @@ static CompK comp_k(const lnb_comp_args *cx)
     k.bg0 = cx->bg[0]; k.bg1 = cx->bg[1]; k.bg2 = cx->bg[2];
     k.acc = cx->acc; k.depth = cx->depth;
     k.t = cx->t; k.t_f64 = cx->t_f64;
-    if (cx->cam) { k.cam_mode = 1; k.cam = make_cam_dev(*cx->cam); }
+    if (cx->cam) { k.cam_mode = 1; k.cam = make_cam_dev(*cx->cam, cx->views); }
     return k;
 }
 
@@ -795,7 +801,7 @@ int lnb_launch_composite_fwd(lnb_ctx *ctx, const float *head, int ldh, const flo
                              float *ray_sse, const lnb_comp_args *cx)
 {
     if (R <= 0) return LNB_OK;
-    auto kern = cx ? composite_fwd_kernel<true> : composite_fwd_kernel<false>;
+    auto kern = lnb_cx_extras(cx) ? (cx->views ? composite_fwd_kernel<true, true> : composite_fwd_kernel<true>) : composite_fwd_kernel<false>;
     kern<<<(R + COMP_WARPS - 1) / COMP_WARPS, COMP_WARPS * 32, 0, ctx->stream>>>(
         head, ldh, dists, target, R, S, rgba, alpha, cumprod, weights, color, color_accumulate,
         ray_sse, comp_k(cx));

@@ -142,20 +142,27 @@ int lnb_launch_axpy2d(lnb_ctx *ctx, float *dst, long long ldd, const float *src,
                       long long rows, int cols, float sign, float seed_value,
                       const float *seed_dev);
 
-// The compositing extras (lnb_composite) of one step as the kernels take them.  The depths are the ones the encoder used:
-// rays mode t (float64 or float32), camera mode the camera (its depths re-derived per sample), features mode none.
+// The per-step carrier from the entry points to each route: the compositing extras (lnb_composite) of one step as the kernels
+// take them, and the per-ray poses of a views batch.  The depths are the ones the encoder used: rays mode t (float64 or
+// float32), camera and views mode the camera (its depths re-derived per sample), features mode none.
 struct lnb_comp_args {
+    int extras = 0;                // 1: background, acc or depth asked for (the extras kernels); 0: a plain views step
     int background = 0;
     float bg[3] = {0.f, 0.f, 0.f};
     float *acc = nullptr, *depth = nullptr;
     const void *t = nullptr;       // rays mode: [R][S] sample depths
     int t_f64 = 0;
-    const lnb_camera *cam = nullptr; // camera mode (host pointer; its pixel list is a device pointer)
+    const lnb_camera *cam = nullptr; // camera and views mode (host pointer; its pixel list is a device pointer)
+    const lnb_views *views = nullptr; // views mode (host pointer): the step's cam holds the views' shared fields (views_camera)
 };
-// NULL when comp asks for nothing (the step is then exactly lnb_nerf_step), else comp with the depth source of step a
-// filled in; LNB_ERR_ARG for the cases lnb_composite lists (api_flat.cu)
-int lnb_comp_resolve(lnb_ctx *ctx, const lnb_step_args *a, bool nerf, const lnb_composite *comp, lnb_comp_args *out,
-                     const lnb_comp_args **resolved);
+// NULL when comp asks for nothing and there is no views batch (the step is then exactly lnb_nerf_step), else the carrier with
+// the depth source of step a filled in; LNB_ERR_ARG for the cases lnb_composite lists (api_flat.cu)
+int lnb_comp_resolve(lnb_ctx *ctx, const lnb_step_args *a, bool nerf, const lnb_composite *comp, const lnb_views *views,
+                     lnb_comp_args *out, const lnb_comp_args **resolved);
+// a views batch of R rays, S samples: LNB_ERR_ARG for the cases lnb_views lists (api_flat.cu)
+int lnb_views_check(lnb_ctx *ctx, const lnb_views *v, int R, int S);
+inline bool lnb_cx_extras(const lnb_comp_args *cx) { return cx && cx->extras; }
+inline const lnb_views *lnb_cx_views(const lnb_comp_args *cx) { return cx ? cx->views : nullptr; }
 
 // ---- fused_tc.cu ---------------------------------------------------------------------------
 // Optional extras of the fused tensor-core step, used by the trainer (trainer.cu):
@@ -189,7 +196,7 @@ int lnb_fused_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, 
                       const lnb_tc_extra *ex, const lnb_comp_args *cx = nullptr);
 // validated dispatch of one step with tensor-core extras and / or compositing extras (api_flat.cu)
 int lnb_step_ex(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf, const lnb_tc_extra *ex,
-                const lnb_composite *comp = nullptr);
+                const lnb_composite *comp = nullptr, const lnb_views *views = nullptr);
 // layerwise tensor-core step for wide MLPs (wide_tc.cu); LNB_ERR_UNSUPPORTED when it does not apply
 int lnb_wide_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf, const lnb_comp_args *cx = nullptr);
 // padded widths of the fused kernel for this MLP, 0 when unsupported; bytes of its weight image
@@ -203,10 +210,11 @@ int lnb_tc_adam_img(lnb_ctx *ctx, const lnb_mlp *mlp, float *param, const float 
 
 // ---- fused_f32.cu: the fused exact (fp32 CUDA-core) step for the reference's own network shapes; LNB_ERR_UNSUPPORTED
 // when the problem (or the outputs asked for) does not fit it
-// (it has no compositing extras: a step with cx != NULL is LNB_ERR_UNSUPPORTED there and runs on the layerwise kernels)
+// (it has no compositing extras: a step with lnb_cx_extras(cx) is LNB_ERR_UNSUPPORTED there and runs on the layerwise kernels)
 int lnb_fused_f32_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf, int overwrite,
                        const lnb_comp_args *cx = nullptr);
-int lnb_step_f32_fused(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf, int overwrite);   // validated (api_flat.cu)
+int lnb_step_f32_fused(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, bool nerf, int overwrite,
+                       const lnb_views *views = nullptr);   // validated (api_flat.cu)
 
 // ---- encode.cu / optim.cu ---------------------------------------------------------------------
 // Rays and camera mode: the input form the MLP's input width selects (include/loma_nerf_b200.h).  Returns the direction
@@ -226,8 +234,10 @@ int lnb_launch_sample_encode(lnb_ctx *ctx, const void *o, const void *d, const v
                              int R, int S, int E, int Ed, float *X, float *dists);
 int lnb_launch_sample_encode_bf16(lnb_ctx *ctx, const void *o, const void *d, const void *t, int f64,
                                   int R, int S, int E, int Ed, float *X, float *dists, void *Xb, int ldb);
-// camera mode (lnb_camera): features / dists (or the wide path's bf16 rows) straight from the pose
-int lnb_launch_camera_encode(lnb_ctx *ctx, const lnb_camera *cam, int R, int S, int E, int Ed, float *X, float *dists, void *Xb, int ldb);
+// camera mode (lnb_camera): features / dists (or the wide path's bf16 rows) straight from the pose; views mode (lnb_views)
+// when views != NULL, cam then holding its shared fields
+int lnb_launch_camera_encode(lnb_ctx *ctx, const lnb_camera *cam, const lnb_views *views, int R, int S, int E, int Ed, float *X,
+                             float *dists, void *Xb, int ldb);
 int lnb_launch_adam(lnb_ctx *ctx, float *p, const float *g, float *m, float *v, long long n, int t,
                     double lr, double b1, double b2, double eps);
 int lnb_launch_adam_dev(lnb_ctx *ctx, float *p, const float *g, float *m, float *v, long long n,

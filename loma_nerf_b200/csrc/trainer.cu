@@ -27,6 +27,8 @@ struct lnb_trainer {
     bool tc_ok = false;
     bool t_bumped = false;   // the last lnb_trainer_grad already incremented *t_dev
     lnb_composite comp{};    // lnb_trainer_set_background: background 0 = the reference's compositing
+    lnb_views views{};       // lnb_trainer_set_views: a nerf batch with no input of its own is a views batch
+    bool has_views = false;
     // peer-memory all-reduce (lnb_trainer_comm_*): header [status | pad] + receive slots for 8 senders
     char *comm_buf = nullptr;
     size_t comm_bytes = 0;
@@ -133,6 +135,7 @@ static int trainer_run(lnb_trainer *t, const lnb_step_args *batch, int nerf, boo
     a.d_X = a.d_target = a.d_dists = a.d_color = a.d_inter = nullptr;
     a.inter = a.rgba = a.alpha = a.cumprod = a.weights = nullptr;
     const lnb_composite *comp = (nerf && t->comp.background) ? &t->comp : nullptr;   // every route below composites onto it
+    const lnb_views *views = (nerf && t->has_views && !a.X && !a.rays_o && !a.cam) ? &t->views : nullptr;
     if (a.path == LNB_PATH_TC && t->tc_ok) {
         lnb_tc_extra ex;
         ex.wimg = t->wimg; ex.overwrite_grads = 1; ex.t_dev = t->t_dev; ex.weights = weights;
@@ -141,7 +144,7 @@ static int trainer_run(lnb_trainer *t, const lnb_step_args *batch, int nerf, boo
             ex.fuse_adam = 1; ex.param = t->params; ex.m = t->opt == LNB_OPT_ADAM ? t->m : nullptr; ex.v = t->v;
             ex.lr = t->lr; ex.b1 = t->b1; ex.b2 = t->b2; ex.eps = t->eps; ex.wimg_out = t->wimg;
         }
-        const int rc = lnb_step_ex(ctx, &t->mlp, &a, nerf != 0, &ex, comp);
+        const int rc = lnb_step_ex(ctx, &t->mlp, &a, nerf != 0, &ex, comp, views);
         if (rc == LNB_OK) { t->t_bumped = !fuse_update; return LNB_OK; }
         // the MLP fits the fused kernel but this batch does not (e.g. S > 128): the layerwise
         // tensor-core kernels below take it, exactly as lnb_nerf_step would
@@ -161,12 +164,12 @@ static int trainer_run(lnb_trainer *t, const lnb_step_args *batch, int nerf, boo
     int rc = LNB_ERR_UNSUPPORTED;
     if (a.path == LNB_PATH_F32 && !comp && !getenv("LNB_F32_NO_FUSED")) {
         // fused exact kernel writing the (zero-padded, never otherwise touched) gradient buffer: no memset
-        rc = lnb_step_f32_fused(ctx, &t->mlp, &a, nerf != 0, 1);
+        rc = lnb_step_f32_fused(ctx, &t->mlp, &a, nerf != 0, 1, views);
         if (rc != LNB_OK && rc != LNB_ERR_UNSUPPORTED) return rc;
     }
     if (rc == LNB_ERR_UNSUPPORTED) {
         LNB_CUDA(cudaMemsetAsync(t->grads, 0, (size_t)(t->n_w + t->n_b + 1) * 4, ctx->stream));
-        LNB_TRY(nerf ? lnb_step_ex(ctx, &t->mlp, &a, true, nullptr, comp) : lnb_fit_step(ctx, &t->mlp, &a));
+        LNB_TRY(nerf ? lnb_step_ex(ctx, &t->mlp, &a, true, nullptr, comp, views) : lnb_fit_step(ctx, &t->mlp, &a));
     }
     t->t_bumped = false;
     if (fuse_update) return lnb_trainer_apply(t);
@@ -188,6 +191,17 @@ extern "C" int lnb_trainer_set_background(lnb_trainer *t, const float *rgb)
     t->comp = lnb_composite{};
     t->comp.background = 1;
     for (int c = 0; c < 3; ++c) t->comp.bg[c] = rgb[c];
+    return LNB_OK;
+}
+
+extern "C" int lnb_trainer_set_views(lnb_trainer *t, const lnb_views *views)
+{
+    if (!t) return LNB_ERR_ARG;
+    lnb_ctx *ctx = t->ctx;
+    if (!views) { t->views = lnb_views{}; t->has_views = false; return LNB_OK; }
+    LNB_TRY(lnb_views_check(ctx, views, 0, 1));
+    t->views = *views;
+    t->has_views = true;
     return LNB_OK;
 }
 
@@ -248,6 +262,8 @@ static int host_inputs(lnb_trainer *t, lnb_step_args &a, lnb_camera &cam_dev, in
         ins[n_in++] = HostIn{&a.rays_d, R * 3 * rw};
         ins[n_in++] = HostIn{&a.t, R * S * rw};
     } else {
+        LNB_ARG(a.X || !nerf || !t->has_views, "trainer: a views batch (lnb_trainer_set_views) has its scene on the device; "
+                                                "the host-buffer steps do not take it");
         LNB_ARG(a.X, "trainer: X or rays required");
         ins[n_in++] = HostIn{(const void **)&a.X, N * c_in * 4};
         if (nerf) { LNB_ARG(a.dists, "trainer: dists required"); ins[n_in++] = HostIn{(const void **)&a.dists, R * S * 4}; }

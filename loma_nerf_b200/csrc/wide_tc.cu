@@ -876,7 +876,7 @@ int lnb_wide_tc_step(lnb_ctx *ctx, const lnb_mlp *mlp, const lnb_step_args *a, b
         float *de = (float *)take((size_t)R * S * 4);
         const int Ed = lnb_rays_dir_bands(c_in, a->pe_bands);
         if (N > 0 && cam)
-            LNB_TRY(lnb_launch_camera_encode(ctx, a->cam, R, S, a->pe_bands, Ed, nullptr, de, H[0], in_pad[0]));
+            LNB_TRY(lnb_launch_camera_encode(ctx, a->cam, lnb_cx_views(cx), R, S, a->pe_bands, Ed, nullptr, de, H[0], in_pad[0]));
         else if (N > 0)
             LNB_TRY(lnb_launch_sample_encode_bf16(ctx, a->rays_o, a->rays_d, a->t, a->ray_dtype == LNB_RAY_F64, R, S, a->pe_bands, Ed, nullptr, de, H[0],
                                                   in_pad[0]));
